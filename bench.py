@@ -2,6 +2,7 @@
 """bench.py -- MultiSURF fit throughput (sample-pair*features/s) on B200.
 
     python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload c3|c2|c4|c5|j1]
+                    [--dump-outputs DIR]
 
 A "step" is one pass of the scoring hot path (encode of the active columns, n x n
 distances, neighbour selection, weight accumulation, reduction) over one synthetic data
@@ -9,6 +10,9 @@ set.  `value` is measured with the raw matrix already resident in HBM; `e2e` is 
 metric through the estimator API (`MultiSURF(backend='gpu').fit`) from host buffers, with
 the host->device upload, the on-GPU column scan and the device->host read of the weights
 inside the timed region.
+
+The inputs are seeded: the same arguments give the same data on every run, so the outputs that
+--dump-outputs writes can be compared between two builds.
 
 Default workload (BASELINE.json configs[2], the config the metric's "1/2/4/8 B200" is
 quoted on): MultiSURF on synthetic 0/1/2 genotypes, 4000 samples x 100000 SNPs, epistatic
@@ -32,11 +36,13 @@ import numpy as np
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
+sys.dont_write_bytecode = True          # the benchmark leaves the tree as it found it (no __pycache__ of tests/ etc.)
 
 METRIC = "multisurf_fit_pair_features_per_s"
 UNIT = "sample-pair*features/s"
 WORKLOAD_SHAPES = {"c3": (4000, 100_000), "c2": (10_000, 10_000), "c4": (20_000, 50_000), "c4surf": (20_000, 50_000),
                    "c5": (20_000, 500_000)}
+DUMP_BYTES = 64 << 20
 
 
 # --------------------------------------------------------------------------- #
@@ -211,24 +217,24 @@ def cpu_sample(w, units=2.0e10):
 
 def run_cpu_port(w, xs, ys):
     """One timed pass of the oracle (C restatement of the reference CPU kernel, OpenMP over
-    target instances like the reference's prange)."""
+    target instances like the reference's prange); returns (seconds, feature scores)."""
     from oracle import ref_oracle as R
 
     if w["algo"] == "ReliefF":
         x32, y_enc, cp, recip, isd = R.relieff_prep(xs, ys, 10)
         t0 = time.perf_counter()
-        R.relieff_scores(x32, y_enc, recip, isd, 10, cp, 0)
+        scores = R.relieff_scores(x32, y_enc, recip, isd, 10, cp, 0)
     elif w["algo"] == "SURF":
         x64, recip, isd = R.surf_prep(xs, 10)
         y32 = np.asarray(ys).astype(np.int32)
         t0 = time.perf_counter()
-        R.surf_scores(x64, y32, recip, isd, w["star"], sum_mode=2)
+        scores = R.surf_scores(x64, y32, recip, isd, w["star"], sum_mode=2)
     else:
         x32, recip, isd = R.multisurf_prep(xs, 10)
         yc = np.unique(ys, return_inverse=True)[1].astype(np.int64)
         t0 = time.perf_counter()
-        R.multisurf_scores(x32, yc, recip, isd, w["star"])
-    return time.perf_counter() - t0
+        scores = R.multisurf_scores(x32, yc, recip, isd, w["star"])
+    return time.perf_counter() - t0, scores
 
 
 def cpu_baseline(w):
@@ -236,7 +242,7 @@ def cpu_baseline(w):
 
     R.set_threads(os.cpu_count() or 1)
     xs, ys, n_s, p_s = cpu_sample(w)
-    dt = run_cpu_port(w, xs, ys)
+    dt, _ = run_cpu_port(w, xs, ys)
     return {"value": n_s * n_s * p_s / dt, "unit": UNIT, "cores": R.max_threads(), "kind": "port",
             "sample": f"all {n_s} samples x first {p_s} features of the workload, one fit, {dt:.2f} s"}
 
@@ -259,7 +265,12 @@ def reference_arm(args):
     xs, ys, n_s, p_s = cpu_sample(w)
     for _ in range(args.warmup):
         run_cpu_port(w, xs[:200], ys[:200])
-    t = sum(run_cpu_port(w, xs, ys) for _ in range(args.steps))
+    t = 0.0
+    for _ in range(args.steps):
+        dt, scores = run_cpu_port(w, xs, ys)
+        t += dt
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"feature_importances": scores})
     value = args.steps * n_s * n_s * p_s / t
     desc = w["desc"].replace(f"x {p_gen}", f"x {p_full}")
     line = {"impl": "reference", "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": args.gpus,
@@ -285,6 +296,29 @@ def load_traffic(workload):
         return json.load(open(os.path.join(ROOT, "profiles", "traffic.json"))).get(workload, {})
     except Exception:
         return {}
+
+
+def dump_outputs(out_dir, outputs):
+    """--dump-outputs: each output of the timed path's last step (a numpy array, or a torch tensor left on
+    the device) as out_dir/<name>.npy in float32 or float64, DUMP_BYTES at most in all.  An output larger
+    than its share is replaced by the flat sample of the entries at np.unique(default_rng(0).integers(0,
+    size, share // 8)): fixed for a given shape, so two builds can be compared output for output."""
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_BYTES // len(outputs)
+    for name, a in outputs.items():
+        size = int(np.prod(a.shape))
+        if size * 8 > share:
+            pos = np.unique(np.random.default_rng(0).integers(0, size, share // 8))
+            if isinstance(a, np.ndarray):
+                a = a.reshape(-1)[pos]
+            else:
+                import torch
+
+                a = a.reshape(-1)[torch.from_numpy(pos).to(a.device)]
+        a = np.asarray(a) if isinstance(a, np.ndarray) else a.cpu().numpy()
+        if a.dtype not in (np.float32, np.float64):
+            a = a.astype(np.float64)
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 # --------------------------------------------------------------------------- #
@@ -453,6 +487,8 @@ def own_arm(args):
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     ms = float(t.item())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"weight_sums": buf})
     units = float(n) * n * p
     value = units * args.steps / (ms / 1e3)
     weights = (buf.cpu().numpy() / n).astype(np.float32)
@@ -652,6 +688,9 @@ def turf_arm(args):
         dist.all_reduce(tt, op=dist.ReduceOp.MAX)
     dt = float(tt.item())
     sess.close()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"feature_importances": resident.feature_importances_,
+                                         "top_features": resident.top_features_})
     value = units * args.steps / dt
 
     # ---- end to end: TuRF(...).fit from host buffers (upload, column scan, every pass)
@@ -734,15 +773,15 @@ def make_j1(n, p):
 
 def joint_cpu(x, y, threads):
     """One timed pass of the oracle's MI matrices (the C restatement of _batch_mi_cpu, OpenMP over
-    features like the reference's prange) on [x | y]."""
+    features like the reference's prange) on [x | y]; returns (seconds, (relevance, redundancy))."""
     from oracle import ref_oracle as R
 
     R.set_threads(threads)
     xi = np.ascontiguousarray(x, np.int32)
     yi = np.ascontiguousarray(y, np.int32)
     t0 = time.perf_counter()
-    R.mi_matrices(xi, yi)
-    return time.perf_counter() - t0
+    out = R.mi_matrices(xi, yi)
+    return time.perf_counter() - t0, out
 
 
 def joint_reference_arm(args):
@@ -758,7 +797,12 @@ def joint_reference_arm(args):
     w = make_j1(n_s, p_s)
     for _ in range(args.warmup):
         joint_cpu(w["x"][:200, :100], w["y"][:200], threads)
-    t = sum(joint_cpu(w["x"], w["y"], threads) for _ in range(args.steps))
+    t = 0.0
+    for _ in range(args.steps):
+        dt, (rel, red) = joint_cpu(w["x"], w["y"], threads)
+        t += dt
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"relevance": rel, "redundancy": red})
     units = float(n_s) * (p_s + 1) * p_s / 2
     value = args.steps * units / t
     line = {"impl": "reference", "metric": J_METRIC, "value": value, "unit": J_UNIT, "n_gpus": args.gpus,
@@ -829,6 +873,8 @@ def joint_arm(args):
         dist.all_reduce(tt, op=dist.ReduceOp.MAX)
     dt = float(tt.item())
     check = buf[p, :p].cpu().numpy()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"relevance": buf[p, :p], "mi_matrix": buf})
     ds.close()
 
     # ---- end to end through the public API, from host buffers
@@ -880,7 +926,7 @@ def joint_arm(args):
             "kernels": kernels, "phases_ms": phases, "bands": int(agg.get("n_chunks", 0) / steps),
             "cpu_baseline": None}
     n_s, p_s = min(n, 10_000), min(p, 6000)       # ~10 s of CPU work on 16 threads
-    tc = joint_cpu(w["x"][:n_s, :p_s], w["y"][:n_s], os.cpu_count() or 1)
+    tc, _ = joint_cpu(w["x"][:n_s, :p_s], w["y"][:n_s], os.cpu_count() or 1)
     from oracle import ref_oracle as R
     line["cpu_baseline"] = {"value": float(n_s) * (p_s + 1) * p_s / 2 / tc, "unit": J_UNIT, "cores": R.max_threads(),
                             "kind": "port", "sample": f"first {n_s} samples x {p_s} features, one pass, {tc:.2f} s"}
@@ -901,7 +947,12 @@ def main():
     # (--samples / --features: torchrun's own parser treats "--n" as an ambiguous abbreviation of its options)
     ap.add_argument("--n", "--samples", dest="n", type=int, default=None)
     ap.add_argument("--p", "--features", dest="p", type=int, default=None)
+    ap.add_argument("--dump-outputs", dest="dump_outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (float32 / float64, "
+                         "at most 64 MB in all: a fixed sample of the entries of a larger output)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     if args.impl == "reference" and args.workload == "j1":
         joint_reference_arm(args)
     elif args.workload == "j1":

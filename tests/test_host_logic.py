@@ -295,6 +295,26 @@ def test_bench_reference_arm_prints_the_contract_line():
     assert line["gpu_launches"] == 0 and line["vs_baseline"] is None
 
 
+def test_bench_dump_outputs_are_reproducible_and_bounded(tmp_path):
+    """bench.py --dump-outputs DIR: the last timed step's outputs as float32 / float64 .npy files, the same
+    for the same arguments whatever --steps is, and a fixed sample of an output above its share of 64 MB."""
+    def run(out, *args):
+        res = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--warmup", "0",
+                              "--dump-outputs", str(out), *args], capture_output=True, text=True, cwd=ROOT)
+        assert res.returncode == 0, res.stderr[-2000:]
+        return {f.stem: np.load(f) for f in out.iterdir()}
+
+    a = run(tmp_path / "a", "--n", "300", "--p", "400", "--steps", "1")
+    b = run(tmp_path / "b", "--n", "300", "--p", "400", "--steps", "2")
+    assert set(a) == set(b) == {"feature_importances"} and a["feature_importances"].shape == (400,)
+    assert np.array_equal(a["feature_importances"], b["feature_importances"])
+    j = run(tmp_path / "j", "--workload", "j1", "--n", "300", "--p", "2100", "--steps", "1")
+    assert j["relevance"].shape == (2100,)
+    assert j["redundancy"].ndim == 1 and 0 < j["redundancy"].size < 2100 * 2100       # 35 MB > 32 MB: sampled
+    assert sum(f.stat().st_size for f in (tmp_path / "j").iterdir()) <= 64 << 20
+    assert all(v.dtype in (np.float32, np.float64) for v in (*a.values(), *j.values()))
+
+
 def test_turf_resident_scoring_keeps_the_base_estimators_validation():
     """The reference re-fits the base estimator on X[:, active] every iteration (TuRF.py:110-111), so an
     integer n_features_to_select of the BASE estimator above the remaining column count raises there;
