@@ -7,7 +7,9 @@ parameters, validation and fitted attributes.  The pairwise statistics -- all of
 the p x p redundancy matrix the reference leaves to the CPU (mutual_information.py:191-193) --
 come from one tensor-core GEMM over the reduced one-hot rows of the columns plus a finishing
 kernel (fastselect_b200/csrc/joint.cu) through the C ABI; the greedy searches that follow are
-O(p k) host work, as in the reference.  There is no CPU fallback.
+O(p k) host work, as in the reference.  With ``pairs="selected"`` the estimators skip the p x p matrix
+and ask for the k + 1 columns their search reads (fs_joint_columns), which is what lets them run on
+genotype-scale p.  There is no CPU fallback.
 """
 from __future__ import annotations
 
@@ -69,23 +71,34 @@ def _stack_for_upload(x, y):
     return out
 
 
-def joint_matrix(codes, kind, log_base=1.0, stats_out=None):
-    """Pairwise statistic of every column pair of the integer matrix ``codes`` ([n, q]): float64
-    ``[q, q]`` with a zero diagonal.  One process per GPU: every rank uploads the matrix, computes a
-    band of rows balanced over the upper triangle, and ONE allreduce sums the bands.  ``stats_out``
-    (a dict) receives this rank's ``fs_stats``."""
-    codes = np.asarray(codes)
+def _open_discrete(codes):
+    """A data set over the integer matrix ``codes`` ([n, q]) with every column typed discrete."""
     n, q = codes.shape
     if n < 2:
         raise ValueError(f"need at least 2 samples, got {n}")
     arith = _native.FS_ARITH_F64 if codes.dtype == np.float64 else _native.FS_ARITH_F32
-    with _native.Dataset(codes, np.zeros(n, np.int32), 1) as ds:
+    ds = _native.Dataset(codes, np.zeros(n, np.int32), 1)
+    try:
         _, _, cnt = ds.column_stats()
         if int(cnt.max()) > MAX_STATES:
             bad = int(np.argmax(cnt > MAX_STATES))
             raise ValueError(f"GPU backend supports up to {MAX_STATES} unique states/bins "
                              f"(column {bad} has more).")
         ds.set_features(np.ones(q, np.uint8), np.ones(q, np.float32), arith)
+    except BaseException:
+        ds.close()
+        raise
+    return ds
+
+
+def joint_matrix(codes, kind, log_base=1.0, stats_out=None):
+    """Pairwise statistic of every column pair of the integer matrix ``codes`` ([n, q]): float64
+    ``[q, q]`` with a zero diagonal.  One process per GPU: every rank uploads the matrix, computes a
+    band of rows balanced over the upper triangle, and ONE allreduce sums the bands.  ``stats_out``
+    (a dict) receives this rank's ``fs_stats``."""
+    codes = np.asarray(codes)
+    q = codes.shape[1]
+    with _open_discrete(codes) as ds:
 
         def compute_band(lo, hi, out_ptr):
             res = ds.joint_matrix(kind, log_base, pos_begin=lo, pos_end=hi, out_device_ptr=out_ptr,
@@ -102,6 +115,43 @@ def joint_matrix(codes, kind, log_base=1.0, stats_out=None):
 
             nccl = dist.get_backend() == "nccl"
         return joint_sharded(q, compute_band, device_buffers=nccl)
+
+
+class JointColumns:
+    """One data set held open for a whole fit: ``columns(positions)`` returns the statistic of each
+    position of the integer matrix ``codes`` ([n, q]) against every position, float64
+    ``[len(positions), q]`` -- bitwise the rows of :func:`joint_matrix`, without the q x q matrix.  The
+    first call encodes the columns; later calls reuse the encoding.  Runs on this process's GPU with no
+    communication: under ``enable_distributed`` / ``set_gpus`` every rank computes the same columns."""
+
+    def __init__(self, codes, kind, log_base=1.0):
+        self.kind, self.log_base = kind, log_base
+        self._ds = _open_discrete(np.asarray(codes))
+
+    def columns(self, positions):
+        return self._ds.joint_columns(self.kind, self.log_base, positions)
+
+    def close(self):
+        self._ds.close()
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+
+def open_joint_columns(codes, kind, log_base=1.0):
+    """The GPU behind ``pairs="selected"``: a :class:`JointColumns` over ``codes``."""
+    return JointColumns(codes, kind, log_base)
+
+
+_PAIRS = ("all", "selected")
+
+
+def _check_pairs(pairs):
+    if pairs not in _PAIRS:
+        raise ValueError(f"pairs must be 'all' or 'selected' (got {pairs!r}).")
 
 
 def calculate_mi_matrices(X, y, *, backend="auto", unit="bit"):
@@ -142,14 +192,24 @@ class mRMR(BaseEstimator, TransformerMixin):
     """Minimum-redundancy maximum-relevance selection on discrete data (drop-in for
     ``fast_select.mRMR``, GPU backend; mRMR.py:30-152).
 
-    ``method``: 'MID' scores ``I(f; y) - mean I(f; S)``, 'MIQ' the quotient (:114-117)."""
+    ``method``: 'MID' scores ``I(f; y) - mean I(f; S)``, 'MIQ' the quotient (:114-117).
 
-    def __init__(self, n_features_to_select: int, method: str = "MID", backend: str = "gpu"):
+    ``pairs`` chooses what the fit returns.  ``"all"`` (the reference's behaviour) computes the whole
+    p x p redundancy matrix and keeps it as ``redundancy_matrix_``.  ``"selected"`` computes only the
+    columns the greedy search reads -- relevance, then one column per selected feature -- and keeps
+    those as ``redundancy_columns_`` (float64 ``[k, p]``, row i = ``I(top_features_[i]; .)``, equal to
+    ``redundancy_matrix_[top_features_]``); ``redundancy_matrix_`` is not set.  Everything else is
+    identical bit for bit.  Because the two differ in what they return, the choice is the caller's and
+    is never made automatically; use ``"selected"`` when p x p float64 does not fit (p = 100 000 is 80 GB)."""
+
+    def __init__(self, n_features_to_select: int, method: str = "MID", backend: str = "gpu", pairs: str = "all"):
         self.n_features_to_select = n_features_to_select
         self.method = method
         self.backend = backend
+        self.pairs = pairs
         if self.method not in ["MID", "MIQ"]:
             raise ValueError("Method must be either 'MID' or 'MIQ'.")
+        _check_pairs(self.pairs)
         if self.backend not in ["cpu", "gpu"]:
             raise ValueError("Backend must be either 'cpu' or 'gpu'.")
         if self.backend == "cpu":
@@ -170,25 +230,48 @@ class mRMR(BaseEstimator, TransformerMixin):
             if not np.issubdtype(arr.dtype, np.integer):
                 raise ValueError(f"{name} must be an integer-coded array (got {arr.dtype}). "
                                  "Discretise continuous data before calling this function.")
-        relevance, redundancy = _mi_matrices(X, y, math.log(2.0))
-        self.relevance_scores_ = relevance
-        self.redundancy_matrix_ = redundancy
-        self.top_features_ = self._select(relevance, redundancy, self.n_features_to_select, self.method)
+        _check_pairs(self.pairs)
+        for attr in ("redundancy_matrix_", "redundancy_columns_"):
+            self.__dict__.pop(attr, None)
+        if self.pairs == "all":
+            relevance, redundancy = _mi_matrices(X, y, math.log(2.0))
+            self.relevance_scores_ = relevance
+            self.redundancy_matrix_ = redundancy
+            self.top_features_ = self._select(relevance, redundancy, self.n_features_to_select, self.method)
+        else:
+            p = X.shape[1]
+            with open_joint_columns(_stack_for_upload(X, y), _native.FS_JOINT_MI, math.log(2.0)) as src:
+                relevance = src.columns([p])[0, :p].copy()
+                fetched = []
+
+                def column(f):
+                    fetched.append(src.columns([f])[0, :p])
+                    return fetched[-1]
+
+                self.relevance_scores_ = relevance
+                self.top_features_ = self._select_columns(relevance, column, self.n_features_to_select, self.method)
+            self.redundancy_columns_ = np.stack(fetched)
         self.feature_importances_ = self.relevance_scores_
         return self
 
     @staticmethod
     def _select(relevance, redundancy, n_select, method):
+        """Greedy forward selection of mRMR.py:102-131 on the full redundancy matrix."""
+        return mRMR._select_columns(relevance, lambda f: redundancy[:, f], n_select, method)
+
+    @staticmethod
+    def _select_columns(relevance, column, n_select, method):
         """Greedy forward selection of mRMR.py:102-131: start at the most relevant feature, then
         repeatedly take the best MID / MIQ score; candidates that ``np.isclose`` to the best score
-        are separated by the smaller mean redundancy."""
+        are separated by the smaller mean redundancy.  ``column(f)`` is ``redundancy[:, f]``; it is
+        asked once for every selected feature, in selection order."""
         p = relevance.size
         selected = np.zeros(n_select, dtype=np.int32)
         remaining = np.ones(p, dtype=bool)
         first = int(np.argmax(relevance))
         selected[0] = first
         remaining[first] = False
-        red_sum = redundancy[:, first].copy()
+        red_sum = column(first).copy()
         for i in range(1, n_select):
             idx = np.flatnonzero(remaining)
             mean_red = red_sum[idx] / i
@@ -200,7 +283,7 @@ class mRMR(BaseEstimator, TransformerMixin):
             best = cand[np.argmin(red_sum[cand] / i)] if cand.size > 1 else cand[0]
             selected[i] = best
             remaining[best] = False
-            red_sum += redundancy[:, best]
+            red_sum += column(best)
         return selected
 
     def transform(self, X):
@@ -226,9 +309,15 @@ def _cfs_merit(sum_r_cf, k, sum_r_ff):
 
 
 def _best_first_search(r_cf, r_ff, min_r_cf=0.1):
+    """Greedy forward search of CFS.py:114-162 on the full correlation matrix."""
+    return _best_first_search_columns(r_cf, lambda s: r_ff[:, s], min_r_cf)
+
+
+def _best_first_search_columns(r_cf, column, min_r_cf=0.1):
     """Greedy forward search of CFS.py:114-162: grow the subset by the candidate with the largest
     merit while the merit strictly improves.  The sums are formed in the reference's order (the
-    subset's own terms first, then the candidate's) so that ties fall the same way."""
+    subset's own terms first, then the candidate's) so that ties fall the same way.  ``column(s)`` is
+    ``r_ff[:, s]``; it is only asked for features already in the subset."""
     p = r_cf.size
     first = int(np.argmax(r_cf))
     if r_cf[first] < min_r_cf:
@@ -245,11 +334,11 @@ def _best_first_search(r_cf, r_ff, min_r_cf=0.1):
         for a in selected:
             for b in selected:
                 if a < b:
-                    base_ff += float(r_ff[a, b])
+                    base_ff += float(column(b)[a])
         sum_cf = base_cf + r_cf.astype(np.float64)
         sum_ff = np.full(p, base_ff)
         for s in selected:
-            sum_ff = sum_ff + r_ff[:, s].astype(np.float64)
+            sum_ff = sum_ff + column(s).astype(np.float64)
         merit = _cfs_merit(sum_cf, k, sum_ff)
         ok = eligible.copy()
         ok[selected] = False
@@ -266,17 +355,37 @@ def _best_first_search(r_cf, r_ff, min_r_cf=0.1):
 
 
 def _prune_redundant(selected, r_cf, r_ff):
+    """Redundancy filter of CFS.py:106-112 on the full correlation matrix."""
+    return _prune_redundant_columns(selected, r_cf, lambda s: r_ff[:, s])
+
+
+def _prune_redundant_columns(selected, r_cf, column):
     """Redundancy filter of CFS.py:106-112: visit the chosen features from the most to the least
     class-correlated (stable, so equal correlations keep their index order) and keep one only if no
-    feature kept so far is at least as correlated with it as the class is."""
+    feature kept so far is at least as correlated with it as the class is.  ``column(s)`` is
+    ``r_ff[:, s]`` and is only asked for features in ``selected``."""
     selected = np.asarray(selected, dtype=int)
     order = selected[np.argsort(-r_cf[selected], kind="stable")]
     kept = []
     for f in order.tolist():
-        if kept and bool((r_ff[f, kept] >= r_cf[f]).any()):
+        if kept and bool((np.array([column(k)[f] for k in kept]) >= r_cf[f]).any()):
             continue
         kept.append(f)
     return kept
+
+
+def _subset_merit(selected, r_cf, column):
+    """CFS.py:406-409 merit of the final subset: the float32 sums of the subset's ``r_cf`` and of the
+    upper triangle of its ``r_ff`` block, formed as ``np.sum`` forms them on the full matrix."""
+    k = len(selected)
+    if k == 0:
+        return 0.0
+    block = np.empty((k, k), np.float32)
+    for j, b in enumerate(selected):
+        block[:, j] = column(b)[selected]
+    sum_r_cf = np.sum(r_cf[selected])
+    sum_r_ff = np.sum(np.triu(block, k=1))
+    return float(_cfs_merit(np.float64(sum_r_cf), k, np.float64(sum_r_ff)))
 
 
 class CFS(BaseEstimator, SelectorMixin):
@@ -284,13 +393,21 @@ class CFS(BaseEstimator, SelectorMixin):
     ``fast_select.CFS``, GPU backend; CFS.py:246-429).  Continuous columns are binned with
     ``KBinsDiscretizer`` on the host exactly as the reference does; the correlations of all pairs
     come from the tensor-core joint-count kernels; ``n_bins`` and the number of distinct values of
-    a discrete column must not exceed 16 (the reference's own GPU kernel stops at 32, CFS.py:349-350)."""
+    a discrete column must not exceed 16 (the reference's own GPU kernel stops at 32, CFS.py:349-350).
 
-    def __init__(self, n_bins=10, strategy="uniform", backend="auto", n_jobs=-1):
+    ``pairs`` chooses what the fit returns.  ``"all"`` (the reference's behaviour) computes every
+    feature-feature correlation and keeps the p x p matrix as ``r_ff_``.  ``"selected"`` computes the
+    class column (``r_cf_``) and one column per feature the forward search accepts, and does not set
+    ``r_ff_``; ``selected_indices_``, ``support_mask_``, ``merit_`` and ``r_cf_`` are identical bit for
+    bit.  Because the two differ in what they return, the choice is the caller's and is never made
+    automatically; use ``"selected"`` when p x p does not fit."""
+
+    def __init__(self, n_bins=10, strategy="uniform", backend="auto", n_jobs=-1, pairs="all"):
         self.n_bins = n_bins
         self.strategy = strategy
         self.backend = backend
         self.n_jobs = n_jobs
+        self.pairs = pairs
 
     def fit(self, X, y):
         feature_names = np.asarray(X.columns) if hasattr(X, "columns") else None
@@ -304,30 +421,42 @@ class CFS(BaseEstimator, SelectorMixin):
             raise NotImplementedError(_NO_CPU)
         if self.backend not in ("auto", "gpu"):
             raise ValueError("backend must be one of 'auto', 'gpu', or 'cpu'")
+        _check_pairs(self.pairs)
         if _native.device_count() < 1:
             raise RuntimeError(_NO_GPU_CFS)
         if len(unique_y) > MAX_STATES or (n_states.size and int(n_states.max()) > MAX_STATES):
             raise ValueError(f"GPU backend supports up to {MAX_STATES} unique states/bins.")
         p = self.n_features_in_
-        su = joint_matrix(_stack_for_upload(codes, y_encoded), _native.FS_JOINT_SU)
-        r_cf = su[p, :p].astype(np.float32)                      # the reference's arrays are float32 (:88, :95)
-        r_ff = np.ascontiguousarray(su[:p, :p], dtype=np.float32)
-        self.r_cf_, self.r_ff_ = r_cf, r_ff
+        self.__dict__.pop("r_ff_", None)
+        if self.pairs == "all":
+            su = joint_matrix(_stack_for_upload(codes, y_encoded), _native.FS_JOINT_SU)
+            r_cf = su[p, :p].astype(np.float32)                      # the reference's arrays are float32 (:88, :95)
+            r_ff = np.ascontiguousarray(su[:p, :p], dtype=np.float32)
+            self.r_cf_, self.r_ff_ = r_cf, r_ff
+            self._search(r_cf, lambda s: r_ff[:, s])
+        else:
+            with open_joint_columns(_stack_for_upload(codes, y_encoded), _native.FS_JOINT_SU) as src:
+                self.r_cf_ = src.columns([p])[0, :p].astype(np.float32)
+                cache = {}
 
-        selected = _best_first_search(r_cf, r_ff)
+                def column(s):
+                    if s not in cache:
+                        cache[s] = src.columns([s])[0, :p].astype(np.float32)
+                    return cache[s]
+
+                self._search(self.r_cf_, column)
+        return self
+
+    def _search(self, r_cf, column):
+        """Best-first search, redundancy filter and merit (CFS.py:375-409); ``column(s)`` is ``r_ff[:, s]``."""
+        p = r_cf.size
+        selected = _best_first_search_columns(r_cf, column)
         selected = np.sort(np.array(selected, dtype=int))
-        self.selected_indices_ = np.sort(np.array(_prune_redundant(selected, r_cf, r_ff), dtype=int))
+        self.selected_indices_ = np.sort(np.array(_prune_redundant_columns(selected, r_cf, column), dtype=int))
         self.support_mask_ = np.zeros(p, dtype=bool)
         if len(self.selected_indices_) > 0:
             self.support_mask_[self.selected_indices_] = True
-        k = len(self.selected_indices_)
-        if k == 0:
-            self.merit_ = 0.0
-        else:
-            sum_r_cf = np.sum(r_cf[self.selected_indices_])
-            sum_r_ff = np.sum(np.triu(r_ff[np.ix_(self.selected_indices_, self.selected_indices_)], k=1))
-            self.merit_ = float(_cfs_merit(np.float64(sum_r_cf), k, np.float64(sum_r_ff)))
-        return self
+        self.merit_ = _subset_merit(self.selected_indices_, r_cf, column)
 
     def _encode(self, X):
         """CFS.py:319-334: floating columns -> ``n_bins`` ordinal bins, other columns -> the rank of

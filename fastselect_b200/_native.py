@@ -15,7 +15,7 @@ FS_U8, FS_I8, FS_F32, FS_F64 = 0, 1, 2, 3
 FS_ARITH_F32, FS_ARITH_F64 = 0, 1
 FS_JOINT_MI, FS_JOINT_SU = 0, 1
 FS_DISTINCT_CAP = 16
-FS_ABI_VERSION = 6
+FS_ABI_VERSION = 7
 
 _DTYPES = {np.dtype(np.uint8): FS_U8, np.dtype(np.int8): FS_I8,
            np.dtype(np.float32): FS_F32, np.dtype(np.float64): FS_F64}
@@ -81,6 +81,7 @@ def load():
     lib.fs_multi_destroy.argtypes = [vp]
     lib.fs_joint_matrix.argtypes = [vp, C.c_int, C.c_double, vp, i64, i64, i64, vp, C.c_int, C.POINTER(FsStats)]
     lib.fs_joint_tables.argtypes = [vp, vp, i64, vp, i64, vp]
+    lib.fs_joint_columns.argtypes = [vp, C.c_int, C.c_double, vp, i64, vp, i64, vp, C.c_int, C.POINTER(FsStats)]
     lib.fs_debug_slab.argtypes = [vp, i64, i64, vp, vp]
     if lib.fs_abi_version() != FS_ABI_VERSION:
         raise RuntimeError(f"fastselect_b200: {LIB_PATH} has ABI version {lib.fs_abi_version()}, "
@@ -266,6 +267,27 @@ class Dataset:
                                     int(pos_end), dst, on_dev, C.byref(stats) if stats is not None else None)
         if rc != 0:
             _raise(rc, "fs_joint_matrix")
+        return (out, stats.as_dict()) if want_stats else out
+
+    def joint_columns(self, kind, log_base, positions, feat_idx=None, want_stats=False):
+        """Rows ``positions`` of :meth:`joint_matrix` without the matrix: float64 ``[len(positions), n_kept]``,
+        row i = statistic of position ``positions[i]`` against every position (0 at itself), bitwise equal
+        to ``joint_matrix(kind, log_base, feat_idx)[positions]``.  The first call on a column list encodes
+        it; later calls on the same list reuse the encoding (see include/fastselect_b200.h)."""
+        positions = np.ascontiguousarray(np.atleast_1d(positions), np.int64)
+        if positions.ndim != 1 or positions.size < 1:
+            raise ValueError("positions must be a non-empty 1-D list of column positions")
+        if feat_idx is not None:
+            feat_idx = np.ascontiguousarray(feat_idx, np.int64)
+            n_kept = feat_idx.size
+        else:
+            n_kept = self.p
+        stats = FsStats() if want_stats else None
+        out = np.empty((positions.size, n_kept), np.float64)
+        rc = load().fs_joint_columns(self._h, int(kind), float(log_base), _ptr(feat_idx), n_kept, _ptr(positions),
+                                     positions.size, _ptr(out), 0, C.byref(stats) if stats is not None else None)
+        if rc != 0:
+            _raise(rc, "fs_joint_columns")
         return (out, stats.as_dict()) if want_stats else out
 
     def joint_tables(self, pairs, feat_idx=None):

@@ -240,6 +240,7 @@ struct WorkSet {
     // cache key
     std::vector<int64_t> key;
     bool valid = false;
+    uint64_t build_id = 0;          // bumped by every rebuild: state derived from At is stale when it changes
     // feature-sharded accumulation (multi-GPU group): At / codesT / krow hold only the tensor columns
     // [a0, a1) of the active list -- this rank's share -- with one-hot rows numbered from 0
     int64_t a0 = 0, a1 = 0;        // == [0, pt) on one GPU
@@ -361,6 +362,17 @@ struct fs_dataset {
     fs::DevBuf<int32_t> joint_slab;     // [band rows, ldd] negated reduced joint counts of one band
     fs::DevBuf<int32_t> joint_start;    // [n_kept + 1] first reduced row of every position
     fs::DevBuf<int64_t> joint_pairs, joint_tables;
+    // column path (fs_joint_columns): start offsets and marginals of the working set built for `jc_key`,
+    // valid while ws.build_id == jc_build
+    bool jc_valid = false;
+    uint64_t jc_build = 0;
+    std::vector<int64_t> jc_key;             // n_kept, then feat_idx (none for all columns)
+    std::vector<int32_t> jc_start_h;         // [n_kept + 1] host copy of jc_start
+    fs::DevBuf<int32_t> jc_start, jc_marg;
+    fs::DevBuf<int32_t> jc_counts;           // [selected rows of one launch, K] reduced joint counts
+    fs::DevBuf<int64_t> jc_pos;              // [n_pos] requested positions
+    fs::DevBuf<int32_t> jc_off;              // [n_pos] first count row of each position within its launch
+    fs::DevBuf<double> jc_out;               // [n_pos, n_kept] (host output)
 };
 
 namespace fs {

@@ -639,6 +639,7 @@ void build_workset(fs_dataset *ds, const int64_t *feat_idx, int64_t n_kept, bool
     }
     ws.key = std::move(key);
     ws.valid = true;
+    ++ws.build_id;
 }
 
 }  // namespace fs

@@ -19,6 +19,8 @@
 //            and the marginals (joint_math.cuh) and writes the statistic to both triangles of the
 //            p x p result.  Reads 4 * (V_a - 1)(V_b - 1) bytes per pair, writes 16.
 // Bands bound the slab (FS_B200_JOINT_SLAB_MB, default 1024 MB) whatever K is.
+// fs_joint_columns (bottom of the file) computes chosen rows of the same matrix from a CUDA-core count
+// kernel instead of the GEMM, with the same encode, marginals and finishing arithmetic.
 #include <algorithm>
 #include <cstring>
 
@@ -274,6 +276,245 @@ void run_joint(fs_dataset *ds, int kind, double log_base, const int64_t *feat_id
     }
 }
 
+// ---------------------------------------------------------------------------------------------------
+// Column path (fs_joint_columns): the statistic of a few positions against every position, for greedy
+// searches that read one column of the p x p matrix per step.  Counts come from the CUDA cores instead of
+// the GEMM: c(s, r) = #samples whose nibble is 0x2 in both selected reduced row s and At row r, one pass
+// over At per launch of up to kColsMaxSel selected rows -- K * ceil(n / 2) bytes, HBM-bound for 0/1/2
+// genotypes (two selected rows per position).  The finishing step is joint_statistic with the same
+// operand order (smaller position first) and the same marginals as joint_finish_kernel, so a row of the
+// result is bitwise the matching row of fs_joint_matrix.
+constexpr int kColsMaxSel = 16;                     // selected reduced rows per count launch (>= 15: one position)
+constexpr int kColsVecs = 4;                        // 16-byte At vectors per lane and sample chunk
+constexpr int kColsChunkVecs = 32 * kColsVecs;      // sample chunk of one block: 128 vectors = 4096 samples
+
+struct ColsSel {
+    int32_t row[kColsMaxSel];                       // At rows of the selected reduced rows
+};
+
+// The 0x2 bit of every nibble of a 16-byte At vector (32 samples) -> one bit per sample.  The bit order is
+// a fixed permutation of the samples, the same for every row, which is all the AND + POPC below needs.
+__device__ __forceinline__ uint32_t fold_ones(const uint4 q) {
+    return ((q.x >> 1) & 0x11111111u) | (q.y & 0x22222222u) | ((q.z << 1) & 0x44444444u) | ((q.w << 2) & 0x88888888u);
+}
+
+__device__ __forceinline__ uint32_t keep_bytes(uint32_t w, int64_t nb) {
+    return nb >= 4 ? w : nb <= 0 ? 0u : w & ((1u << (8 * nb)) - 1u);
+}
+
+// counts[s * K + r] += c(s, r) over the samples of chunk blockIdx.y (counts zeroed by the caller; integer
+// atomics, so the result does not depend on the order of the chunks).  The selected rows' masks of the chunk
+// sit in shared memory with the bytes past row_bytes cleared: the pitch padding of At is never trusted, the
+// AND removes it from the streamed rows.  One warp per At row: lane l reads vectors l, l + 32, ... of the
+// chunk (512 contiguous bytes per instruction), and one warp reduction per selected row ends the row.
+template <int S>
+__global__ void __launch_bounds__(256) joint_cols_count_kernel(const int8_t *__restrict__ At, int64_t pitch,
+                                                               int64_t row_bytes, int64_t K, ColsSel sel, int n_sel,
+                                                               int32_t *__restrict__ counts) {
+    __shared__ uint32_t sm[S][kColsChunkVecs];
+    const uint8_t *base = reinterpret_cast<const uint8_t *>(At);
+    const int64_t nvec = (row_bytes + 15) >> 4;
+    const int64_t v0 = (int64_t)blockIdx.y * kColsChunkVecs;
+    for (int t = threadIdx.x; t < S * kColsChunkVecs; t += blockDim.x) {
+        const int s = t / kColsChunkVecs, w = t % kColsChunkVecs;
+        const int64_t v = v0 + w;
+        uint32_t m = 0;
+        if (s < n_sel && v < nvec) {
+            uint4 q = reinterpret_cast<const uint4 *>(base + (int64_t)sel.row[s] * pitch)[v];
+            const int64_t nb = row_bytes - 16 * v;   // bytes of this vector inside the row (pitch: multiple of 64)
+            q.x = keep_bytes(q.x, nb);
+            q.y = keep_bytes(q.y, nb - 4);
+            q.z = keep_bytes(q.z, nb - 8);
+            q.w = keep_bytes(q.w, nb - 12);
+            m = fold_ones(q);
+        }
+        sm[s][w] = m;
+    }
+    __syncthreads();
+    const int lane = threadIdx.x & 31;
+    for (int64_t r = (int64_t)blockIdx.x * 8 + (threadIdx.x >> 5); r < K; r += (int64_t)gridDim.x * 8) {
+        const uint4 *row = reinterpret_cast<const uint4 *>(base + r * pitch);
+        uint4 q[kColsVecs];
+#pragma unroll
+        for (int j = 0; j < kColsVecs; ++j) {
+            const int64_t v = v0 + 32 * j + lane;
+            q[j] = v < nvec ? __ldg(row + v) : make_uint4(0u, 0u, 0u, 0u);
+        }
+        uint32_t c[S];
+#pragma unroll
+        for (int s = 0; s < S; ++s) c[s] = 0;
+#pragma unroll
+        for (int j = 0; j < kColsVecs; ++j) {
+            const uint32_t m = fold_ones(q[j]);
+#pragma unroll
+            for (int s = 0; s < S; ++s) c[s] += __popc(m & sm[s][32 * j + lane]);
+        }
+#pragma unroll
+        for (int s = 0; s < S; ++s) {
+            const uint32_t tot = __reduce_add_sync(0xffffffffu, c[s]);
+            if (lane == s && s < n_sel && tot) atomicAdd(counts + s * K + r, (int32_t)tot);
+        }
+    }
+}
+
+// out[i * n_kept + g] = statistic(positions[i], g) for the positions [i0, i0 + gridDim.y) of one count launch;
+// counts row off[i] + k holds reduced row k of positions[i] against every At row.
+__global__ void __launch_bounds__(256) joint_cols_finish_kernel(const int32_t *__restrict__ counts, int64_t K,
+                                                                const int32_t *__restrict__ start,
+                                                                const int32_t *__restrict__ marg, int64_t n_kept,
+                                                                const int64_t *__restrict__ positions,
+                                                                const int32_t *__restrict__ off, int64_t i0, int64_t n,
+                                                                int kind, double log_base, double *__restrict__ out) {
+    const int64_t g = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (g >= n_kept) return;
+    const int64_t i = i0 + blockIdx.y, c = positions[i];
+    double v = 0.0;
+    if (g != c) {
+        const int sc = start[c], lc = start[c + 1] - sc, sg = start[g], lg = start[g + 1] - sg;
+        const int32_t *C = counts + (int64_t)off[i] * K + sg;
+        // the smaller position is the first operand, as in joint_finish_kernel (joint_visit walks the cells
+        // in operand order, which fixes the float64 summation order)
+        if (c < g)
+            v = joint_statistic(kind, lc, lg, marg + sc, marg + sg, [=](int a, int b) { return C[a * K + b]; }, n, log_base);
+        else
+            v = joint_statistic(kind, lg, lc, marg + sg, marg + sc, [=](int a, int b) { return C[b * K + a]; }, n, log_base);
+    }
+    out[i * n_kept + g] = v;
+}
+
+template <int S>
+void launch_cols_count(const int8_t *At, int64_t pitch, int64_t row_bytes, int64_t K, const ColsSel &sel, int n_sel,
+                       int32_t *counts, int sms, cudaStream_t st) {
+    const int64_t chunks = ceil_div(ceil_div(row_bytes, 16), kColsChunkVecs);
+    // enough blocks for every SM several times over; each block walks many rows so that staging the
+    // selected rows' chunk (an L2 hit) stays small next to the At bytes it streams
+    const int64_t bx = std::max<int64_t>(1, std::min<int64_t>(ceil_div(K, 8), ceil_div((int64_t)sms * 16, chunks)));
+    joint_cols_count_kernel<S><<<dim3((unsigned)bx, (unsigned)chunks), 256, 0, st>>>(At, pitch, row_bytes, K, sel, n_sel, counts);
+}
+
+void run_joint_columns(fs_dataset *ds, int kind, double log_base, const int64_t *feat_idx, int64_t n_kept,
+                       const int64_t *positions, int64_t n_pos, double *d_out, fs_stats *stats) {
+    FS_REQUIRE(ds->have_features, FS_ERR_STATE, "joint counts: call fs_dataset_set_features first");
+    const int64_t n = ds->n;
+    const int64_t row_bytes = (n + 1) / 2;
+    FS_REQUIRE(ceil_div(ceil_div(row_bytes, 16), kColsChunkVecs) <= 65535, FS_ERR_INVALID,
+               "joint columns: n = %lld exceeds the sample range of the count kernel", (long long)n);
+    cudaStream_t st = ds->stream;
+    int launches = 0;
+    JointTimer tm(stats != nullptr, st);
+    enum { PH_ENCODE = 0, PH_COUNTS, PH_FINISH, PH_N };
+    tm.begin(PH_ENCODE);
+    // At, the start offsets and the marginals are built by the first call on a column list and reused by the
+    // following ones for as long as the working set is not rebuilt (new typing, another column list, fs_score)
+    std::vector<int64_t> key(1 + (feat_idx ? n_kept : 0));
+    key[0] = feat_idx ? n_kept : -1;
+    if (feat_idx) memcpy(key.data() + 1, feat_idx, n_kept * sizeof(int64_t));
+    WorkSet &ws = ds->ws;
+    if (!(ds->jc_valid && ws.valid && ws.build_id == ds->jc_build && ds->jc_key == key)) {
+        ds->jc_valid = false;
+        std::vector<int32_t> &start = ds->jc_start_h;
+        start.assign(n_kept + 1, 0);
+        for (int64_t c = 0; c < n_kept; ++c) {
+            const int64_t f = feat_idx ? feat_idx[c] : c;
+            FS_REQUIRE(f >= 0 && f < ds->p, FS_ERR_INVALID, "feat_idx[%lld]=%lld outside [0,%lld)", (long long)c,
+                       (long long)f, (long long)ds->p);
+            const unsigned ci = ds->col_info[f], path = ci & kColPathMask;
+            FS_REQUIRE(path == kColTensor || path == kColConst, FS_ERR_INVALID,
+                       "joint counts: column %lld is not a discrete column with at most %d distinct values", (long long)f,
+                       FS_DISTINCT_CAP);
+            start[c + 1] = start[c] + (path == kColTensor ? (int32_t)(ci >> 4) : 0);
+        }
+        ds->no_dist_ops = true;
+        try {
+            build_workset(ds, feat_idx, n_kept, true, false, 0, n, true, false, false, false, &launches);
+        } catch (...) {
+            ds->no_dist_ops = false;
+            throw;
+        }
+        ds->no_dist_ops = false;
+        const int64_t K = ws.K_used;
+        FS_REQUIRE(K == start[n_kept], FS_ERR_STATE, "joint counts: working set holds %lld reduced rows, expected %lld",
+                   (long long)K, (long long)start[n_kept]);
+        ds->jc_start.reserve(n_kept + 1);
+        FS_CUDA(cudaMemcpyAsync(ds->jc_start.ptr, start.data(), (n_kept + 1) * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+        ds->jc_marg.reserve(std::max<int64_t>(K, 1));
+        if (K > 0) {
+            joint_marginals_kernel<<<(unsigned)ceil_div(K, 8), 256, 0, st>>>(ws.At.ptr, ws.ldt / 2, row_bytes, K,
+                                                                              ds->jc_marg.ptr);
+            FS_CUDA(cudaGetLastError());
+            ++launches;
+        }
+        ds->jc_key = std::move(key);
+        ds->jc_build = ws.build_id;
+        ds->jc_valid = true;
+    }
+    tm.end();
+    const std::vector<int32_t> &start = ds->jc_start_h;
+    const int64_t K = ws.K_used, pitch = ws.ldt / 2;
+
+    // launches: consecutive runs of positions with at most kColsMaxSel reduced rows together
+    std::vector<int32_t> off(n_pos);
+    std::vector<int64_t> cuts{0};
+    for (int64_t i = 0, rows = 0; i < n_pos; ++i) {
+        const int l = start[positions[i] + 1] - start[positions[i]];
+        if (rows + l > kColsMaxSel) {
+            cuts.push_back(i);
+            rows = 0;
+        }
+        off[i] = (int32_t)rows;
+        rows += l;
+    }
+    cuts.push_back(n_pos);
+    ds->jc_pos.reserve(n_pos);
+    ds->jc_off.reserve(n_pos);
+    FS_CUDA(cudaMemcpyAsync(ds->jc_pos.ptr, positions, n_pos * sizeof(int64_t), cudaMemcpyHostToDevice, st));
+    FS_CUDA(cudaMemcpyAsync(ds->jc_off.ptr, off.data(), n_pos * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    ds->jc_counts.reserve((size_t)kColsMaxSel * std::max<int64_t>(K, 1));
+    int sms = 0;
+    FS_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, ds->device));
+    for (size_t q = 0; q + 1 < cuts.size(); ++q) {
+        const int64_t i0 = cuts[q], i1 = cuts[q + 1];
+        ColsSel sel{};
+        int n_sel = 0;
+        for (int64_t i = i0; i < i1; ++i)
+            for (int k = start[positions[i]]; k < start[positions[i] + 1]; ++k) sel.row[n_sel++] = k;
+        if (n_sel > 0) {
+            tm.begin(PH_COUNTS);
+            FS_CUDA(cudaMemsetAsync(ds->jc_counts.ptr, 0, (size_t)n_sel * K * sizeof(int32_t), st));
+            int32_t *cnt = ds->jc_counts.ptr;
+            if (n_sel <= 1) launch_cols_count<1>(ws.At.ptr, pitch, row_bytes, K, sel, n_sel, cnt, sms, st);
+            else if (n_sel <= 2) launch_cols_count<2>(ws.At.ptr, pitch, row_bytes, K, sel, n_sel, cnt, sms, st);
+            else if (n_sel <= 4) launch_cols_count<4>(ws.At.ptr, pitch, row_bytes, K, sel, n_sel, cnt, sms, st);
+            else if (n_sel <= 8) launch_cols_count<8>(ws.At.ptr, pitch, row_bytes, K, sel, n_sel, cnt, sms, st);
+            else launch_cols_count<16>(ws.At.ptr, pitch, row_bytes, K, sel, n_sel, cnt, sms, st);
+            FS_CUDA(cudaGetLastError());
+            ++launches;
+            tm.end();
+        }
+        tm.begin(PH_FINISH);
+        dim3 grid((unsigned)ceil_div(n_kept, 256), (unsigned)(i1 - i0));
+        joint_cols_finish_kernel<<<grid, 256, 0, st>>>(ds->jc_counts.ptr, K, ds->jc_start.ptr, ds->jc_marg.ptr, n_kept,
+                                                       ds->jc_pos.ptr, ds->jc_off.ptr, i0, n, kind, log_base, d_out);
+        FS_CUDA(cudaGetLastError());
+        ++launches;
+        tm.end();
+    }
+    // `positions`, `off` (pageable) were sources of asynchronous copies
+    FS_CUDA(cudaStreamSynchronize(st));
+    if (stats) {
+        memset(stats, 0, sizeof(*stats));
+        float ms[PH_N];
+        tm.finish(&stats->ms_total, ms, PH_N);
+        stats->ms_gather = ms[PH_ENCODE];
+        stats->ms_dist_general = ms[PH_COUNTS];
+        stats->ms_reduce = ms[PH_FINISH];
+        stats->launches = launches;
+        stats->n_chunks = (int32_t)(cuts.size() - 1);
+        stats->n_tensor_cols = ws.pt;
+        stats->onehot_k = K;
+    }
+}
+
 }  // namespace
 }  // namespace fs
 
@@ -336,6 +577,41 @@ int fs_joint_tables(fs_dataset *ds, const int64_t *feat_idx, int64_t n_kept, con
         return f.code;
     } catch (const std::exception &e) {
         set_error("fs_joint_tables: %s", e.what());
+        return FS_ERR_OOM;
+    }
+}
+
+int fs_joint_columns(fs_dataset *ds, int kind, double log_base, const int64_t *feat_idx, int64_t n_kept,
+                     const int64_t *positions, int64_t n_pos, double *out, int out_on_device, fs_stats *stats) {
+    try {
+        FS_REQUIRE(ds && out && positions, FS_ERR_INVALID, "fs_joint_columns: null pointer");
+        FS_REQUIRE(kind == FS_JOINT_MI || kind == FS_JOINT_SU, FS_ERR_INVALID, "fs_joint_columns: unknown kind %d", kind);
+        FS_REQUIRE(kind != FS_JOINT_MI || log_base > 0.0, FS_ERR_INVALID, "fs_joint_columns: log_base must be positive");
+        if (!feat_idx) n_kept = ds->p;
+        FS_REQUIRE(n_kept >= 1, FS_ERR_INVALID, "fs_joint_columns: no columns");
+        FS_REQUIRE(n_pos >= 1, FS_ERR_INVALID, "fs_joint_columns: no positions");
+        for (int64_t i = 0; i < n_pos; ++i)
+            FS_REQUIRE(positions[i] >= 0 && positions[i] < n_kept, FS_ERR_INVALID,
+                       "fs_joint_columns: position %lld = %lld outside [0, %lld)", (long long)i, (long long)positions[i],
+                       (long long)n_kept);
+        FS_CUDA(cudaSetDevice(ds->device));
+        alloc_stream() = ds->stream;
+        double *d_out = out;
+        const size_t cells = (size_t)n_pos * (size_t)n_kept;
+        if (!out_on_device) {
+            ds->jc_out.reserve(cells);
+            d_out = ds->jc_out.ptr;
+        }
+        run_joint_columns(ds, kind, log_base, feat_idx, n_kept, positions, n_pos, d_out, stats);
+        if (!out_on_device) {
+            FS_CUDA(cudaMemcpyAsync(out, d_out, cells * sizeof(double), cudaMemcpyDeviceToHost, ds->stream));
+            FS_CUDA(cudaStreamSynchronize(ds->stream));
+        }
+        return FS_OK;
+    } catch (const Fail &f) {
+        return f.code;
+    } catch (const std::exception &e) {
+        set_error("fs_joint_columns: %s", e.what());
         return FS_ERR_OOM;
     }
 }

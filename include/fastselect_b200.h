@@ -32,7 +32,7 @@ extern "C" {
 #define FS_API
 #endif
 
-#define FS_ABI_VERSION 6
+#define FS_ABI_VERSION 7
 /* distinct values tracked per column by fs_dataset_create; a column with more
  * distinct values reports FS_DISTINCT_CAP + 1 */
 #define FS_DISTINCT_CAP 16
@@ -236,12 +236,25 @@ FS_API int fs_multi_destroy(fs_multi *m);
  * fs_joint_tables: the contingency tables themselves for m pairs of positions (pairs[2 * q],
  *   pairs[2 * q + 1]), exact integers: tables_out[q * 256 + va * 16 + vb] = #samples with the va-th
  *   smallest value of the first column and the vb-th smallest value of the second (host pointer).
+ * fs_joint_columns: rows of the same matrix for n_pos chosen positions, without the p x p matrix:
+ *   out[i * n_kept + g] = statistic(feat_idx[positions[i]], feat_idx[g]) for every g in [0, n_kept),
+ *   0 at g == positions[i]; bitwise equal to row positions[i] of fs_joint_matrix.  Every position must
+ *   lie in [0, n_kept); the other checks and error codes are those of fs_joint_matrix.  The counts come
+ *   from one pass of the CUDA cores over the reduced one-hot rows per 16 selected reduced rows (one pass
+ *   for a call of up to 8 genotype or one 16-state position), so a greedy search that needs k columns
+ *   reads k passes, not p^2 statistics.  The one-hot rows, their marginals and the position offsets are
+ *   built by the first call on a (column list, typing) and reused by later calls until the data set's
+ *   working set is rebuilt (fs_dataset_set_features, another column list, fs_score).  In stats:
+ *   ms_gather = that build (about 0 on a reuse), ms_dist_general = count kernels, ms_reduce = finish
+ *   kernels, n_chunks = count launches.
  */
 typedef enum { FS_JOINT_MI = 0, FS_JOINT_SU = 1 } fs_joint_kind;
 FS_API int fs_joint_matrix(fs_dataset *ds, int kind, double log_base, const int64_t *feat_idx, int64_t n_kept,
                     int64_t pos_begin, int64_t pos_end, double *out, int out_on_device, fs_stats *stats);
 FS_API int fs_joint_tables(fs_dataset *ds, const int64_t *feat_idx, int64_t n_kept, const int64_t *pairs, int64_t m,
                     int64_t *tables_out);
+FS_API int fs_joint_columns(fs_dataset *ds, int kind, double log_base, const int64_t *feat_idx, int64_t n_kept,
+                            const int64_t *positions, int64_t n_pos, double *out, int out_on_device, fs_stats *stats);
 
 /*
  * Parity/debug view of the RESIDENT one-hot distance slab fs_score keeps between calls for TuRF's
