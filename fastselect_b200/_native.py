@@ -15,7 +15,8 @@ FS_U8, FS_I8, FS_F32, FS_F64 = 0, 1, 2, 3
 FS_ARITH_F32, FS_ARITH_F64 = 0, 1
 FS_JOINT_MI, FS_JOINT_SU = 0, 1
 FS_DISTINCT_CAP = 16
-FS_ABI_VERSION = 7
+FS_ABI_VERSION = 8
+FS_MDR_MAX_TOP = 2048
 
 _DTYPES = {np.dtype(np.uint8): FS_U8, np.dtype(np.int8): FS_I8,
            np.dtype(np.float32): FS_F32, np.dtype(np.float64): FS_F64}
@@ -83,6 +84,8 @@ def load():
     lib.fs_joint_tables.argtypes = [vp, vp, i64, vp, i64, vp]
     lib.fs_joint_columns.argtypes = [vp, C.c_int, C.c_double, vp, i64, vp, i64, vp, C.c_int, C.POINTER(FsStats)]
     lib.fs_debug_slab.argtypes = [vp, i64, i64, vp, vp]
+    lib.fs_mdr_scan.argtypes = [vp, vp, i64, i32, vp, i32, i64, vp, vp, vp, vp, vp, vp, C.POINTER(FsStats)]
+    lib.fs_mdr_tables.argtypes = [vp, vp, i64, i32, vp, i32, vp, i64, vp]
     if lib.fs_abi_version() != FS_ABI_VERSION:
         raise RuntimeError(f"fastselect_b200: {LIB_PATH} has ABI version {lib.fs_abi_version()}, "
                            f"this package needs {FS_ABI_VERSION}; rebuild it (make -C fastselect_b200/csrc)")
@@ -304,6 +307,57 @@ class Dataset:
         rc = load().fs_joint_tables(self._h, _ptr(feat_idx), n_kept, _ptr(pairs), pairs.shape[0], _ptr(out))
         if rc != 0:
             _raise(rc, "fs_joint_tables")
+        return out
+
+    def mdr_scan(self, fold, order, n_top, feat_idx=None, want_all=False, want_stats=False):
+        """MDR search over the combinations of order 1 or 2 of the positions of ``feat_idx`` (see
+        include/fastselect_b200.h): ``fold`` ([n], original sample order) assigns every sample to one of
+        ``max(fold) + 1`` cross-validation folds.  Returns a dict with ``top_idx`` (int64 ``[n_top]``),
+        ``top_train`` / ``top_test`` (mean balanced accuracies), ``fold_best`` (int64 ``[n_folds]``) and, with
+        ``want_all``, ``all_train`` / ``all_test`` (float64 ``[n_combos]``)."""
+        fold = np.ascontiguousarray(fold, np.int32)
+        if fold.shape != (self.n,):
+            raise ValueError(f"fold must have one entry per sample ({self.n})")
+        n_folds = int(fold.max()) + 1 if fold.size else 0
+        if feat_idx is not None:
+            feat_idx = np.ascontiguousarray(feat_idx, np.int64)
+            n_kept = feat_idx.size
+        else:
+            n_kept = self.p
+        n_combos = n_kept if order == 1 else n_kept * (n_kept - 1) // 2
+        out = dict(top_idx=np.empty(n_top, np.int64), top_train=np.empty(n_top, np.float64),
+                   top_test=np.empty(n_top, np.float64), fold_best=np.empty(max(n_folds, 1), np.int64))
+        if want_all:
+            out["all_train"] = np.empty(n_combos, np.float64)
+            out["all_test"] = np.empty(n_combos, np.float64)
+        stats = FsStats() if want_stats else None
+        rc = load().fs_mdr_scan(self._h, _ptr(feat_idx), n_kept, int(order), _ptr(fold), n_folds, int(n_top),
+                                _ptr(out["top_idx"]), _ptr(out["top_train"]), _ptr(out["top_test"]),
+                                _ptr(out["fold_best"]), _ptr(out.get("all_train")), _ptr(out.get("all_test")),
+                                C.byref(stats) if stats is not None else None)
+        if rc != 0:
+            _raise(rc, "fs_mdr_scan")
+        return (out, stats.as_dict()) if want_stats else out
+
+    def mdr_tables(self, fold, order, combos, feat_idx=None):
+        """Exact cell counts of the combinations ``combos`` (``[m, order]`` positions in ``feat_idx``): int64
+        ``[m, n_folds, 2, 9]``, entry ``[q, f, c, va * 3 + vb]`` counting the samples of fold f and class c whose
+        values have ranks va / vb among their columns' distinct values (order 1: vb = 0)."""
+        fold = np.ascontiguousarray(fold, np.int32)
+        if fold.shape != (self.n,):
+            raise ValueError(f"fold must have one entry per sample ({self.n})")
+        n_folds = int(fold.max()) + 1 if fold.size else 0
+        combos = np.ascontiguousarray(combos, np.int64).reshape(-1, int(order))
+        if feat_idx is not None:
+            feat_idx = np.ascontiguousarray(feat_idx, np.int64)
+            n_kept = feat_idx.size
+        else:
+            n_kept = self.p
+        out = np.empty((combos.shape[0], max(n_folds, 1), 2, 9), np.int64)
+        rc = load().fs_mdr_tables(self._h, _ptr(feat_idx), n_kept, int(order), _ptr(fold), n_folds, _ptr(combos),
+                                  combos.shape[0], _ptr(out))
+        if rc != 0:
+            _raise(rc, "fs_mdr_tables")
         return out
 
     def debug_slab(self, row_begin, nrows):

@@ -265,6 +265,15 @@ bool host_barrier_wait(HostBarrier *hb, double timeout_s);
 
 }  // namespace fs
 
+namespace fs {
+// Segments of the MDR bit-planes (mdr.cu): segment s = 2 * fold + class owns the words [w[s], w[s + 1]).
+constexpr int kMdrMaxSegments = 20;
+struct MdrSeg {
+    int32_t w[kMdrMaxSegments + 1];     // first word of every segment; w[nseg] = words in use
+    int32_t n[kMdrMaxSegments];         // samples of every segment
+};
+}  // namespace fs
+
 struct fs_comm {
     int rank = 0, world = 1, device = 0;
     std::shared_ptr<fs::HostBarrier> host_barrier;
@@ -373,6 +382,23 @@ struct fs_dataset {
     fs::DevBuf<int64_t> jc_pos;              // [n_pos] requested positions
     fs::DevBuf<int32_t> jc_off;              // [n_pos] first count row of each position within its launch
     fs::DevBuf<double> jc_out;               // [n_pos, n_kept] (host output)
+    // MDR (mdr.cu): bit-planes of the working set built for `mdr_key`, valid while ws.build_id == mdr_build
+    bool mdr_valid = false;
+    uint64_t mdr_build = 0;
+    std::vector<int64_t> mdr_key;            // n_kept (-1: all columns), n_folds, feat_idx, fold
+    std::vector<int32_t> mdr_start_h;        // [n_kept + 1] host copy of mdr_start
+    fs::MdrSeg mdr_seg{};
+    int64_t mdr_W = 0;                       // words of a plane row (multiple of 4)
+    int mdr_nseg = 0;
+    fs::DevBuf<int32_t> mdr_start;           // [n_kept + 1] first reduced row of every position
+    fs::DevBuf<int32_t> mdr_slot;            // [32 W] internal row of every bit slot, -1: padding
+    fs::DevBuf<uint8_t> mdr_wseg;            // [W] segment of every word
+    fs::DevBuf<uint32_t> mdr_planes;         // [K, W] bit-planes in segment order
+    fs::DevBuf<int32_t> mdr_marg;            // [K, nseg] popcount of every plane row in every segment
+    fs::DevBuf<double> mdr_all;              // [2, n_combos] mean training / test BA of every combination
+    fs::DevBuf<char> mdr_top, mdr_fold;      // block-local top lists (two merge buffers) and fold bests
+    fs::DevBuf<long long> mdr_best;          // [n_folds] merged fold bests
+    fs::DevBuf<int64_t> mdr_combos, mdr_tables;
 };
 
 namespace fs {

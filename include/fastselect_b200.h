@@ -32,7 +32,7 @@ extern "C" {
 #define FS_API
 #endif
 
-#define FS_ABI_VERSION 7
+#define FS_ABI_VERSION 8
 /* distinct values tracked per column by fs_dataset_create; a column with more
  * distinct values reports FS_DISTINCT_CAP + 1 */
 #define FS_DISTINCT_CAP 16
@@ -255,6 +255,41 @@ FS_API int fs_joint_tables(fs_dataset *ds, const int64_t *feat_idx, int64_t n_ke
                     int64_t *tables_out);
 FS_API int fs_joint_columns(fs_dataset *ds, int kind, double log_base, const int64_t *feat_idx, int64_t n_kept,
                             const int64_t *positions, int64_t n_pos, double *out, int out_on_device, fs_stats *stats);
+
+/*
+ * MDR (multifactor dimensionality reduction; the semantics are this project's own, see DESIGN.md "MDR"):
+ * exhaustive search over the combinations of order 1 or 2 of the positions of feat_idx (NULL = all p) for
+ * the one whose high-risk cells best separate the two classes, scored by cross-validated balanced accuracy.
+ * The data set's y_enc is the class (n_classes must be 2; class 1 is the case class).  fold[n] gives every
+ * sample's cross-validation fold in [0, n_folds), in ORIGINAL sample order; 2 <= n_folds <= 10, and every
+ * fold must hold samples of both classes.  Every scanned column must be discrete in fs_dataset_set_features
+ * and hold at most 3 distinct values (FS_ERR_INVALID otherwise); a column's cell index is the rank of its
+ * value among its sorted distinct values.  n < 2^26.
+ *
+ * Combination index: order 1, the position a; order 2, the lexicographic rank of (a, b), a < b:
+ *   idx = a * n_kept - a * (a + 1) / 2 + (b - a - 1),   n_combos = n_kept * (n_kept - 1) / 2.
+ * Per combination and fold f: training counts over the samples with fold != f, test counts over fold f;
+ * a cell is high-risk iff T1 * N0 > T0 * N1 (int64; ties and empty cells are low-risk); balanced accuracy
+ * = (TP * N0 + TN * N1) / (2 N1 N0) with one float64 division, the test one with the training labels; the
+ * means over the folds are summed in fold order, then divided by n_folds.
+ *
+ * fs_mdr_scan: top_idx / top_train / top_test [n_top]: the n_top combinations with the highest mean test
+ *   balanced accuracy (lower index first on ties), with their mean training / test values;
+ *   1 <= n_top <= min(FS_MDR_MAX_TOP, n_combos).  fold_best[n_folds]: per fold, the combination with the
+ *   highest training balanced accuracy (lower index first on ties).  all_train / all_test (nullable, both
+ *   or neither, [n_combos] host arrays): the means of every combination.  The bit-planes of a (column
+ *   list, fold vector) are built by the first call and reused by later calls until the working set is
+ *   rebuilt.  In stats: ms_gather = encode + pack (about 0 on a reuse), ms_dist_general = scan kernel,
+ *   ms_reduce = merges, n_chunks = scan blocks, pairs_selected = n_combos.
+ * fs_mdr_tables: tables_out[((q * n_folds + f) * 2 + c) * 9 + va * 3 + vb], int64: samples of fold f and
+ *   class c in cell (va, vb) of combination q = combos[q * order ..] (positions, any order; order 1: vb = 0).
+ */
+#define FS_MDR_MAX_TOP 2048
+FS_API int fs_mdr_scan(fs_dataset *ds, const int64_t *feat_idx, int64_t n_kept, int32_t order, const int32_t *fold,
+                       int32_t n_folds, int64_t n_top, int64_t *top_idx, double *top_train, double *top_test,
+                       int64_t *fold_best, double *all_train, double *all_test, fs_stats *stats);
+FS_API int fs_mdr_tables(fs_dataset *ds, const int64_t *feat_idx, int64_t n_kept, int32_t order, const int32_t *fold,
+                         int32_t n_folds, const int64_t *combos, int64_t m, int64_t *tables_out);
 
 /*
  * Parity/debug view of the RESIDENT one-hot distance slab fs_score keeps between calls for TuRF's
