@@ -198,7 +198,7 @@ using namespace fs;
 extern "C" {
 
 int fs_comm_create(fs_comm **out, int32_t rank, int32_t world, int32_t device) {
-    try {
+    return api_call("fs_comm_create", [&] {
         FS_REQUIRE(out, FS_ERR_INVALID, "fs_comm_create: null pointer");
         FS_REQUIRE(world >= 1 && world <= kMaxRanks && rank >= 0 && rank < world, FS_ERR_INVALID,
                    "fs_comm_create: bad rank/world %d/%d (at most %d ranks)", rank, world, kMaxRanks);
@@ -215,13 +215,11 @@ int fs_comm_create(fs_comm **out, int32_t rank, int32_t world, int32_t device) {
         c->peers.world = world;
         *out = c;
         return FS_OK;
-    } catch (const Fail &f) {
-        return f.code;
-    }
+    });
 }
 
 int fs_comm_reserve(fs_comm *c, uint64_t bytes, void *ipc_handle_out, int32_t *changed_out) {
-    try {
+    return api_call("fs_comm_reserve", [&] {
         FS_REQUIRE(c, FS_ERR_INVALID, "fs_comm_reserve: null communicator");
         FS_CUDA(cudaSetDevice(c->device));
         bool changed = false;
@@ -246,9 +244,7 @@ int fs_comm_reserve(fs_comm *c, uint64_t bytes, void *ipc_handle_out, int32_t *c
         }
         if (changed_out) *changed_out = changed ? 1 : 0;
         return FS_OK;
-    } catch (const Fail &f) {
-        return f.code;
-    }
+    });
 }
 
 void *fs_comm_arena(fs_comm *c) { return c ? c->arena : nullptr; }
@@ -256,7 +252,7 @@ uint64_t fs_comm_arena_bytes(fs_comm *c) { return c ? c->arena_bytes : 0; }
 int fs_comm_connected(fs_comm *c) { return c && c->connected ? 1 : 0; }
 
 int fs_comm_connect(fs_comm *c, const void *ipc_handles, void *const *raw_ptrs) {
-    try {
+    return api_call("fs_comm_connect", [&] {
         FS_REQUIRE(c && c->arena, FS_ERR_STATE, "fs_comm_connect: reserve the arena first");
         FS_REQUIRE(ipc_handles || raw_ptrs || c->world == 1, FS_ERR_INVALID, "fs_comm_connect: no handles");
         FS_CUDA(cudaSetDevice(c->device));
@@ -301,9 +297,7 @@ int fs_comm_connect(fs_comm *c, const void *ipc_handles, void *const *raw_ptrs) 
         c->epoch = 0;
         c->connected = true;
         return FS_OK;
-    } catch (const Fail &f) {
-        return f.code;
-    }
+    });
 }
 
 int fs_comm_destroy(fs_comm *c) {

@@ -7,6 +7,7 @@
 #include <cstdarg>
 #include <cstdio>
 #include <cstdlib>
+#include <exception>
 #include <memory>
 #include <string>
 #include <vector>
@@ -42,6 +43,20 @@ struct Fail {
             throw fs::Fail{code};            \
         }                                    \
     } while (0)
+
+// Body of a C-ABI entry point: a Fail returns its code, any other exception (std::bad_alloc from a host
+// container, ...) sets "<name>: <what>" and returns FS_ERR_OOM.  Nothing crosses the C ABI.
+template <class F>
+int api_call(const char *name, F &&body) noexcept {
+    try {
+        return body();
+    } catch (const Fail &f) {
+        return f.code;
+    } catch (const std::exception &e) {
+        set_error("%s: %s", name, e.what());
+        return FS_ERR_OOM;
+    }
+}
 
 // Stream used by DevBuf allocations of the current API call (set at every C-ABI entry).
 cudaStream_t &alloc_stream();
@@ -101,6 +116,60 @@ struct PinnedBuf {
         count = 0;
         ptr = static_cast<T *>(pinned_take(n * sizeof(T), &bytes));
         count = bytes / sizeof(T);
+    }
+};
+
+// Device-time phases of one call (stats != nullptr only): begin(&fs_stats::ms_x) / end() record a span on the
+// stream, and finish() adds every span into its field and sets ms_total from construction to stop() (or to
+// finish() itself).  finish() adds: the caller zeroes *out first.
+struct PhaseTimer {
+    using Field = float fs_stats::*;
+    struct Span { Field field; cudaEvent_t a, b; };
+    bool on;
+    cudaStream_t st;
+    std::vector<Span> spans;
+    cudaEvent_t t0 = nullptr, t1 = nullptr;
+    bool stopped = false;
+    PhaseTimer(bool enable, cudaStream_t s) : on(enable), st(s) {
+        if (on) {
+            cudaEventCreate(&t0);
+            cudaEventCreate(&t1);
+            cudaEventRecord(t0, st);
+        }
+    }
+    void begin(Field f) {
+        if (!on) return;
+        Span s{f, nullptr, nullptr};
+        cudaEventCreate(&s.a);
+        cudaEventCreate(&s.b);
+        cudaEventRecord(s.a, st);
+        spans.push_back(s);
+    }
+    void end() {
+        if (on) cudaEventRecord(spans.back().b, st);
+    }
+    void stop() {
+        if (on && !stopped) cudaEventRecord(t1, st);
+        stopped = true;
+    }
+    void finish(fs_stats *out) {
+        if (!on) return;
+        stop();
+        cudaEventSynchronize(t1);
+        for (auto &s : spans) {
+            float t = 0.f;
+            cudaEventElapsedTime(&t, s.a, s.b);
+            out->*s.field += t;
+        }
+        cudaEventElapsedTime(&out->ms_total, t0, t1);
+    }
+    ~PhaseTimer() {
+        for (auto &s : spans) {
+            cudaEventDestroy(s.a);
+            cudaEventDestroy(s.b);
+        }
+        if (t0) cudaEventDestroy(t0);
+        if (t1) cudaEventDestroy(t1);
     }
 };
 
@@ -266,6 +335,21 @@ bool host_barrier_wait(HostBarrier *hb, double timeout_s);
 }  // namespace fs
 
 namespace fs {
+// The reduced one-hot operand At of a list of discrete columns (ws.At, built without the distance operands)
+// with its per-position offsets: what the joint-count and MDR paths read.  Built by discrete_operand for the
+// first call on a column list and kept while the working set is not rebuilt.
+struct DiscreteOperand {
+    bool valid = false;
+    std::vector<int64_t> key;       // n_kept (-1: all columns), then feat_idx
+    uint64_t build_id = 0;          // ws.build_id it was built for
+    uint64_t generation = 0;        // bumped by every rebuild: state derived from the operand is stale when it changes
+    int max_rows = 0;               // largest reduced-row count (V - 1) of a column of the list
+    std::vector<int32_t> start_h;   // [n_kept + 1] first reduced row of every position (none for a constant column)
+    DevBuf<int32_t> start;          // device copy of start_h
+    bool have_marg = false;
+    DevBuf<int32_t> marg;           // [K] marginal counts of the reduced rows, computed when first asked for
+};
+
 // Segments of the MDR bit-planes (mdr.cu): segment s = 2 * fold + class owns the words [w[s], w[s + 1]).
 constexpr int kMdrMaxSegments = 20;
 struct MdrSeg {
@@ -362,35 +446,24 @@ struct fs_dataset {
     fs::DevBuf<int32_t> tie_flag, tie_order, tie_list;   // ReliefF reference tie order (select.cu)
     fs::DevBuf<float> tie_keys;
     fs::DevBuf<unsigned long long> counters;
-    // joint-count path (joint.cu)
-    bool no_dist_ops = false;     // build_workset: skip the distance operands (U / Wd / srow)
+    // joint-count and MDR paths: the shared operand (joint.cu)
+    fs::DiscreteOperand disc;
     fs::DevBuf<double> joint_out;       // [n_kept, n_kept]
-    fs::DevBuf<int32_t> joint_marg;     // [K] marginal counts of the reduced one-hot rows
     fs::DevBuf<int32_t> joint_zero;     // zeros: the s_i / s_j vector of the reused distance kernel
     fs::DevBuf<int64_t> joint_ids;      // zeros: its row-id vector
     fs::DevBuf<int32_t> joint_slab;     // [band rows, ldd] negated reduced joint counts of one band
-    fs::DevBuf<int32_t> joint_start;    // [n_kept + 1] first reduced row of every position
     fs::DevBuf<int64_t> joint_pairs, joint_tables;
-    // column path (fs_joint_columns): start offsets and marginals of the working set built for `jc_key`,
-    // valid while ws.build_id == jc_build
-    bool jc_valid = false;
-    uint64_t jc_build = 0;
-    std::vector<int64_t> jc_key;             // n_kept, then feat_idx (none for all columns)
-    std::vector<int32_t> jc_start_h;         // [n_kept + 1] host copy of jc_start
-    fs::DevBuf<int32_t> jc_start, jc_marg;
+    // column path (fs_joint_columns)
     fs::DevBuf<int32_t> jc_counts;           // [selected rows of one launch, K] reduced joint counts
     fs::DevBuf<int64_t> jc_pos;              // [n_pos] requested positions
     fs::DevBuf<int32_t> jc_off;              // [n_pos] first count row of each position within its launch
     fs::DevBuf<double> jc_out;               // [n_pos, n_kept] (host output)
-    // MDR (mdr.cu): bit-planes of the working set built for `mdr_key`, valid while ws.build_id == mdr_build
-    bool mdr_valid = false;
-    uint64_t mdr_build = 0;
-    std::vector<int64_t> mdr_key;            // n_kept (-1: all columns), n_folds, feat_idx, fold
-    std::vector<int32_t> mdr_start_h;        // [n_kept + 1] host copy of mdr_start
+    // MDR (mdr.cu): bit-planes of the operand of generation mdr_gen (0: none) and the folds `mdr_key`
+    uint64_t mdr_gen = 0;
+    std::vector<int64_t> mdr_key;            // n_folds, fold
     fs::MdrSeg mdr_seg{};
     int64_t mdr_W = 0;                       // words of a plane row (multiple of 4)
     int mdr_nseg = 0;
-    fs::DevBuf<int32_t> mdr_start;           // [n_kept + 1] first reduced row of every position
     fs::DevBuf<int32_t> mdr_slot;            // [32 W] internal row of every bit slot, -1: padding
     fs::DevBuf<uint8_t> mdr_wseg;            // [W] segment of every word
     fs::DevBuf<uint32_t> mdr_planes;         // [K, W] bit-planes in segment order
@@ -407,9 +480,17 @@ namespace fs {
 // r0 / R / slab_cacheable: the (contiguous) target rows of this call and whether their distance
 // slab fits one chunk -- decides between a full, an incremental and no distance computation
 // want_split: a multi-GPU group call that may shard the accumulation by one-hot columns (WorkSet::acc_split)
+// dist_ops: build the distance operands U / Wd / srow too (the joint-count and MDR paths read only At)
 void build_workset(fs_dataset *ds, const int64_t *feat_idx, int64_t n_kept, bool allow_tensor, bool need_codes,
                    int64_t r0, int64_t R, bool contiguous, bool slab_cacheable, bool want_split, bool group_call,
-                   int *launches);
+                   bool dist_ops, int *launches);
+
+// joint.cu: the operand of the discrete columns feat_idx (all p columns when null) of a data set whose features
+// are set.  Every column must be constant or a tensor-path column with at most max_values distinct values
+// (FS_ERR_INVALID "<what>: column ... is not a discrete column with at most <max_values> distinct values"); with
+// need_marg the marginals are there too.
+const DiscreteOperand &discrete_operand(fs_dataset *ds, const int64_t *feat_idx, int64_t n_kept, int max_values,
+                                        const char *what, bool need_marg, int *launches);
 
 // comm.cu
 void comm_barrier(fs_comm *c, cudaStream_t st, int *launches);

@@ -447,7 +447,7 @@ static int plan_dist(fs_dataset *ds, const int64_t *tcol, int64_t pt, int64_t r0
 
 void build_workset(fs_dataset *ds, const int64_t *feat_idx, int64_t n_kept, bool allow_tensor, bool need_codes,
                    int64_t r0, int64_t R, bool contiguous, bool slab_cacheable, bool want_split, bool group_call,
-                   int *launches) {
+                   bool dist_ops, int *launches) {
     WorkSet &ws = ds->ws;
     // sample rows the target-side distance operand U has to hold
     const int64_t want_lo = contiguous ? r0 : 0, want_hi = contiguous ? r0 + R : ds->n;
@@ -464,7 +464,7 @@ void build_workset(fs_dataset *ds, const int64_t *feat_idx, int64_t n_kept, bool
         // same columns as the last call: the slab is either still there or recomputed in full
         const int mode = plan_dist(ds, ws.p_tcol.ptr, ws.pt, r0, R, slab_cacheable, ws.removed);
         if (mode == kDistReuse || (ws.have_dist_ops && ws.u_lo <= want_lo && want_hi <= ws.u_hi) || ws.pt == 0 ||
-            ds->no_dist_ops) {               // joint-count path: only At is needed, and it is always built
+            !dist_ops) {                     // only At is needed, and it is always built
             ws.dist_mode = mode == kDistReuse ? kDistReuse : kDistFull;
             return;
         }
@@ -630,7 +630,7 @@ void build_workset(fs_dataset *ds, const int64_t *feat_idx, int64_t n_kept, bool
         Trace tr("  plan_dist");
         ws.dist_mode = plan_dist(ds, ws.p_tcol.ptr, ws.pt, r0, R, slab_cacheable, ws.removed);
     }
-    ws.have_dist_ops = ws.dist_mode == kDistFull && !ds->no_dist_ops;
+    ws.have_dist_ops = ws.dist_mode == kDistFull && dist_ops;
     ws.u_lo = want_lo;
     ws.u_hi = want_hi;
     if (ws.pt > 0) {
@@ -657,10 +657,10 @@ int fs_abi_version(void) { return FS_ABI_VERSION; }
 
 int fs_dataset_create(fs_dataset **out, const void *x, int dtype, int64_t n, int64_t p, int64_t row_stride_elems,
                       const int32_t *y_enc, int32_t n_classes, int32_t device, void *stream) {
-    fs_dataset *ds = nullptr;
-    try {
+    return api_call("fs_dataset_create", [&] {
         FS_REQUIRE(out && x, FS_ERR_INVALID, "fs_dataset_create: null pointer");
-        ds = create_common(dtype, n, p, row_stride_elems, y_enc, n_classes, device, stream);
+        std::unique_ptr<fs_dataset> owner(create_common(dtype, n, p, row_stride_elems, y_enc, n_classes, device, stream));
+        fs_dataset *ds = owner.get();
         size_t es = dtype_size(dtype);
         ds->ldx = round_up(p, 16 / (int64_t)es > 0 ? 16 / (int64_t)es : 1);
         ds->x_owned.alloc((size_t)n * ds->ldx * es);
@@ -764,40 +764,26 @@ int fs_dataset_create(fs_dataset **out, const void *x, int dtype, int64_t n, int
         for (auto e : done)
             if (e) cudaEventDestroy(e);
         cudaStreamDestroy(copy_stream);
-        *out = ds;
+        *out = owner.release();
         return FS_OK;
-    } catch (const Fail &f) {
-        delete ds;
-        return f.code;
-    } catch (const std::exception &e) {
-        set_error("fs_dataset_create: %s", e.what());
-        delete ds;
-        return FS_ERR_OOM;
-    }
+    });
 }
 
 int fs_dataset_create_device(fs_dataset **out, const void *x_dev, int dtype, int64_t n, int64_t p,
                              int64_t row_stride_elems, const int32_t *y_enc, int32_t n_classes, int32_t device,
                              void *stream) {
-    fs_dataset *ds = nullptr;
-    try {
+    return api_call("fs_dataset_create_device", [&] {
         FS_REQUIRE(out && x_dev, FS_ERR_INVALID, "fs_dataset_create_device: null pointer");
-        ds = create_common(dtype, n, p, row_stride_elems, y_enc, n_classes, device, stream);
+        std::unique_ptr<fs_dataset> owner(create_common(dtype, n, p, row_stride_elems, y_enc, n_classes, device, stream));
+        fs_dataset *ds = owner.get();
         ds->x = x_dev;
         ds->ldx = row_stride_elems;
         prepare_create(ds, y_enc);
         scan_rows(ds, 0, n, true, true);
         finish_create(ds);
-        *out = ds;
+        *out = owner.release();
         return FS_OK;
-    } catch (const Fail &f) {
-        delete ds;
-        return f.code;
-    } catch (const std::exception &e) {
-        set_error("fs_dataset_create_device: %s", e.what());
-        delete ds;
-        return FS_ERR_OOM;
-    }
+    });
 }
 
 int fs_dataset_column_stats(const fs_dataset *ds, double *col_min, double *col_max, int32_t *n_distinct) {
@@ -868,7 +854,7 @@ int fs_dataset_row_order(const fs_dataset *ds, int64_t *perm_out) {
 }
 
 int fs_dataset_attach_comm(fs_dataset *ds, fs_comm *comm, const int64_t *row_starts) {
-    try {
+    return api_call("fs_dataset_attach_comm", [&] {
         FS_REQUIRE(ds, FS_ERR_INVALID, "fs_dataset_attach_comm: null data set");
         if (comm == nullptr || comm->world <= 1) {         // detach: plain single-rank behaviour
             ds->comm = nullptr;
@@ -926,9 +912,7 @@ int fs_dataset_attach_comm(fs_dataset *ds, fs_comm *comm, const int64_t *row_sta
         ++ds->typing_epoch;          // the accumulation shares changed: cached column lists are stale
         compute_owner_bounds(ds);
         return FS_OK;
-    } catch (const Fail &f) {
-        return f.code;
-    }
+    });
 }
 
 // Sharded upload: this rank copies rows [n * rank / world, n * (rank + 1) / world) of the host matrix into
@@ -936,11 +920,11 @@ int fs_dataset_attach_comm(fs_dataset *ds, fs_comm *comm, const int64_t *row_sta
 // barrier every rank holds all of X having moved 1/world of it over PCIe.
 int fs_dataset_create_group(fs_dataset **out, fs_comm *comm, const void *x, int dtype, int64_t n, int64_t p,
                             int64_t row_stride_elems, const int32_t *y_enc, int32_t n_classes, void *stream) {
-    fs_dataset *ds = nullptr;
-    try {
+    return api_call("fs_dataset_create_group", [&] {
         FS_REQUIRE(out && x && comm, FS_ERR_INVALID, "fs_dataset_create_group: null pointer");
         FS_REQUIRE(comm->connected, FS_ERR_STATE, "fs_dataset_create_group: the communicator is not connected");
-        ds = create_common(dtype, n, p, row_stride_elems, y_enc, n_classes, comm->device, stream);
+        std::unique_ptr<fs_dataset> owner(create_common(dtype, n, p, row_stride_elems, y_enc, n_classes, comm->device, stream));
+        fs_dataset *ds = owner.get();
         const size_t es = dtype_size(dtype);
         ds->ldx = round_up(p, 16 / (int64_t)es > 0 ? 16 / (int64_t)es : 1);
         const int world = comm->world, rank = comm->rank;
@@ -964,16 +948,9 @@ int fs_dataset_create_group(fs_dataset **out, fs_comm *comm, const void *x, int 
         scan_rows(ds, 0, n, true, true);
         finish_create(ds);
         comm_check(comm);
-        *out = ds;
+        *out = owner.release();
         return FS_OK;
-    } catch (const Fail &f) {
-        delete ds;
-        return f.code;
-    } catch (const std::exception &e) {
-        set_error("fs_dataset_create_group: %s", e.what());
-        delete ds;
-        return FS_ERR_OOM;
-    }
+    });
 }
 
 int fs_dataset_destroy(fs_dataset *ds) {

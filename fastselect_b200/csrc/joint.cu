@@ -59,6 +59,64 @@ __global__ void __launch_bounds__(256) joint_marginals_kernel(const int8_t *__re
     if (lane == 0) marg[row] = cnt;
 }
 
+}  // namespace
+
+const DiscreteOperand &discrete_operand(fs_dataset *ds, const int64_t *feat_idx, int64_t n_kept, int max_values,
+                                        const char *what, bool need_marg, int *launches) {
+    FS_REQUIRE(ds->have_features, FS_ERR_STATE, "%s: call fs_dataset_set_features first", what);
+    DiscreteOperand &op = ds->disc;
+    const WorkSet &ws = ds->ws;
+    std::vector<int64_t> key(1 + (feat_idx ? n_kept : 0));
+    key[0] = feat_idx ? n_kept : -1;
+    if (feat_idx) std::copy(feat_idx, feat_idx + n_kept, key.begin() + 1);
+    // a list encoded for a laxer caller is checked again (and fails) below
+    if (!(op.valid && ws.valid && ws.build_id == op.build_id && op.max_rows < max_values && op.key == key)) {
+        // reduced rows of every position: V - 1 for a tensor-path column, none for a constant one
+        std::vector<int32_t> start(n_kept + 1, 0);
+        int max_rows = 0;
+        for (int64_t c = 0; c < n_kept; ++c) {
+            const int64_t f = feat_idx ? feat_idx[c] : c;
+            FS_REQUIRE(f >= 0 && f < ds->p, FS_ERR_INVALID, "feat_idx[%lld]=%lld outside [0,%lld)", (long long)c,
+                       (long long)f, (long long)ds->p);
+            const unsigned ci = ds->col_info[f], path = ci & kColPathMask;
+            const int rows = path == kColTensor ? (int)(ci >> 4) : 0;
+            FS_REQUIRE((path == kColTensor && rows < max_values) || path == kColConst, FS_ERR_INVALID,
+                       "%s: column %lld is not a discrete column with at most %d distinct values", what, (long long)f,
+                       max_values);
+            start[c + 1] = start[c] + rows;
+            max_rows = std::max(max_rows, rows);
+        }
+        op.valid = false;
+        build_workset(ds, feat_idx, n_kept, true, false, 0, ds->n, true, false, false, false, false, launches);
+        FS_REQUIRE(ws.K_used == start[n_kept], FS_ERR_STATE, "%s: working set holds %lld reduced rows, expected %lld",
+                   what, (long long)ws.K_used, (long long)start[n_kept]);
+        op.start_h = std::move(start);
+        op.start.reserve(n_kept + 1);
+        FS_CUDA(cudaMemcpyAsync(op.start.ptr, op.start_h.data(), (n_kept + 1) * sizeof(int32_t), cudaMemcpyHostToDevice,
+                                ds->stream));
+        op.key = std::move(key);
+        op.build_id = ws.build_id;
+        op.max_rows = max_rows;
+        op.have_marg = false;
+        ++op.generation;
+        op.valid = true;
+    }
+    if (need_marg && !op.have_marg) {
+        const int64_t K = ws.K_used;
+        op.marg.reserve(std::max<int64_t>(K, 1));
+        if (K > 0) {
+            joint_marginals_kernel<<<(unsigned)ceil_div(K, 8), 256, 0, ds->stream>>>(ws.At.ptr, ws.ldt / 2, (ds->n + 1) / 2,
+                                                                                      K, op.marg.ptr);
+            FS_CUDA(cudaGetLastError());
+            ++*launches;
+        }
+        op.have_marg = true;
+    }
+    return op;
+}
+
+namespace {
+
 // out[c, g] = out[g, c] = statistic of the columns at positions c in [c_lo, c_hi) and g in (c, n_kept).
 // start[c] .. start[c + 1]: reduced rows of position c (an empty range for a constant column);
 // D: the band's negated counts, its row 0 / column 0 being reduced row b0.
@@ -101,56 +159,9 @@ __global__ void __launch_bounds__(128) joint_tables_kernel(const int32_t *__rest
     });
 }
 
-struct JointTimer {
-    bool on;
-    cudaStream_t st;
-    struct Span { int ph; cudaEvent_t a, b; };
-    std::vector<Span> spans;
-    cudaEvent_t t0 = nullptr, t1 = nullptr;
-    JointTimer(bool enable, cudaStream_t s) : on(enable), st(s) {
-        if (on) {
-            cudaEventCreate(&t0);
-            cudaEventCreate(&t1);
-            cudaEventRecord(t0, st);
-        }
-    }
-    void begin(int ph) {
-        if (!on) return;
-        Span s{ph, nullptr, nullptr};
-        cudaEventCreate(&s.a);
-        cudaEventCreate(&s.b);
-        cudaEventRecord(s.a, st);
-        spans.push_back(s);
-    }
-    void end() {
-        if (on) cudaEventRecord(spans.back().b, st);
-    }
-    void finish(float *ms_total, float *ms_phase, int n_phase) {
-        if (!on) return;
-        cudaEventRecord(t1, st);
-        cudaEventSynchronize(t1);
-        for (int i = 0; i < n_phase; ++i) ms_phase[i] = 0.f;
-        for (auto &s : spans) {
-            float t = 0.f;
-            cudaEventElapsedTime(&t, s.a, s.b);
-            ms_phase[s.ph] += t;
-        }
-        cudaEventElapsedTime(ms_total, t0, t1);
-    }
-    ~JointTimer() {
-        for (auto &s : spans) {
-            cudaEventDestroy(s.a);
-            cudaEventDestroy(s.b);
-        }
-        if (t0) cudaEventDestroy(t0);
-        if (t1) cudaEventDestroy(t1);
-    }
-};
-
 // The GEMM bands shared by fs_joint_matrix (kind >= 0, d_out) and fs_joint_tables (d_pairs / d_tables).
 void run_joint(fs_dataset *ds, int kind, double log_base, const int64_t *feat_idx, int64_t n_kept, int64_t pos_begin,
                int64_t pos_end, double *d_out, const int64_t *d_pairs, int64_t m, int64_t *d_tables, fs_stats *stats) {
-    FS_REQUIRE(ds->have_features, FS_ERR_STATE, "joint counts: call fs_dataset_set_features first");
     FS_REQUIRE(n_kept >= 1 && pos_begin >= 0 && pos_begin <= pos_end && pos_end <= n_kept, FS_ERR_INVALID,
                "joint counts: bad position range [%lld, %lld) of %lld columns", (long long)pos_begin, (long long)pos_end,
                (long long)n_kept);
@@ -158,45 +169,15 @@ void run_joint(fs_dataset *ds, int kind, double log_base, const int64_t *feat_id
     FS_REQUIRE(ds->n < (1LL << 24), FS_ERR_INVALID, "joint counts: n = %lld exceeds the exact range (2^24)", (long long)ds->n);
     const int64_t n = ds->n;
     cudaStream_t st = ds->stream;
-    // reduced rows of every position: V - 1 for a tensor-path column, none for a constant one
-    std::vector<int32_t> start(n_kept + 1, 0);
-    for (int64_t c = 0; c < n_kept; ++c) {
-        const int64_t f = feat_idx ? feat_idx[c] : c;
-        FS_REQUIRE(f >= 0 && f < ds->p, FS_ERR_INVALID, "feat_idx[%lld]=%lld outside [0,%lld)", (long long)c, (long long)f,
-                   (long long)ds->p);
-        const unsigned ci = ds->col_info[f], path = ci & kColPathMask;
-        FS_REQUIRE(path == kColTensor || path == kColConst, FS_ERR_INVALID,
-                   "joint counts: column %lld is not a discrete column with at most %d distinct values", (long long)f,
-                   FS_DISTINCT_CAP);
-        start[c + 1] = start[c] + (path == kColTensor ? (int32_t)(ci >> 4) : 0);
-    }
     int launches = 0;
     double ops = 0.0;
-    JointTimer tm(stats != nullptr, st);
-    enum { PH_ENCODE = 0, PH_COUNTS, PH_FINISH, PH_N };
-    tm.begin(PH_ENCODE);
-    ds->no_dist_ops = true;
-    try {
-        build_workset(ds, feat_idx, n_kept, true, false, 0, n, true, false, false, false, &launches);
-    } catch (...) {
-        ds->no_dist_ops = false;
-        throw;
-    }
-    ds->no_dist_ops = false;
+    PhaseTimer tm(stats != nullptr, st);
+    tm.begin(&fs_stats::ms_gather);
+    const DiscreteOperand &op = discrete_operand(ds, feat_idx, n_kept, FS_DISTINCT_CAP, "joint counts", true, &launches);
+    const std::vector<int32_t> &start = op.start_h;
     const WorkSet &ws = ds->ws;
     const int64_t K = ws.K_used;
-    FS_REQUIRE(K == start[n_kept], FS_ERR_STATE, "joint counts: working set holds %lld reduced rows, expected %lld",
-               (long long)K, (long long)start[n_kept]);
-    ds->joint_start.reserve(n_kept + 1);
-    // pageable source: the copy is staged before the call returns
-    FS_CUDA(cudaMemcpyAsync(ds->joint_start.ptr, start.data(), (n_kept + 1) * sizeof(int32_t), cudaMemcpyHostToDevice, st));
     const int64_t row_bytes = (n + 1) / 2, pitch = ws.ldt / 2;     // At: two samples per byte
-    ds->joint_marg.reserve(std::max<int64_t>(K, 1));
-    if (K > 0) {
-        joint_marginals_kernel<<<(unsigned)ceil_div(K, 8), 256, 0, st>>>(ws.At.ptr, pitch, row_bytes, K, ds->joint_marg.ptr);
-        FS_CUDA(cudaGetLastError());
-        ++launches;
-    }
     tm.end();
 
     // the reused distance kernel adds s_i + s_j (zeros here) and looks its rows up through an id vector
@@ -220,7 +201,7 @@ void run_joint(fs_dataset *ds, int kind, double log_base, const int64_t *feat_id
             R = start[c_hi] - b0;
         }
         if (R > 0) {
-            tm.begin(PH_COUNTS);
+            tm.begin(&fs_stats::ms_dist_tensor);
             ds->joint_slab.reserve((size_t)round_up(R, 128) * ldd);
             ds->joint_ids.reserve(round_up(R, 128));
             FS_CUDA(cudaMemsetAsync(ds->joint_ids.ptr, 0, round_up(R, 128) * sizeof(int64_t), st));
@@ -241,17 +222,17 @@ void run_joint(fs_dataset *ds, int kind, double log_base, const int64_t *feat_id
                            &launches, &ops);
             tm.end();
         }
-        tm.begin(PH_FINISH);
+        tm.begin(&fs_stats::ms_reduce);
         if (d_out && c_lo + 1 < n_kept) {
             dim3 grid((unsigned)ceil_div(n_kept - c_lo - 1, 256), (unsigned)std::min<int64_t>(c_hi - c_lo, 4096));
-            joint_finish_kernel<<<grid, 256, 0, st>>>(ds->joint_slab.ptr, ldd, b0, ds->joint_start.ptr, c_lo, c_hi, n_kept,
-                                                      ds->joint_marg.ptr, n, kind, log_base, d_out);
+            joint_finish_kernel<<<grid, 256, 0, st>>>(ds->joint_slab.ptr, ldd, b0, op.start.ptr, c_lo, c_hi, n_kept,
+                                                      op.marg.ptr, n, kind, log_base, d_out);
             FS_CUDA(cudaGetLastError());
             ++launches;
         }
         if (d_tables && m > 0) {
-            joint_tables_kernel<<<(unsigned)ceil_div(m, 128), 128, 0, st>>>(ds->joint_slab.ptr, ldd, b0, ds->joint_start.ptr,
-                                                                            c_lo, c_hi, ds->joint_marg.ptr, n, d_pairs, m,
+            joint_tables_kernel<<<(unsigned)ceil_div(m, 128), 128, 0, st>>>(ds->joint_slab.ptr, ldd, b0, op.start.ptr,
+                                                                            c_lo, c_hi, op.marg.ptr, n, d_pairs, m,
                                                                             d_tables);
             FS_CUDA(cudaGetLastError());
             ++launches;
@@ -259,15 +240,10 @@ void run_joint(fs_dataset *ds, int kind, double log_base, const int64_t *feat_id
         tm.end();
         c_lo = c_hi;
     }
-    // `start` (pageable) was the source of an asynchronous copy
     FS_CUDA(cudaStreamSynchronize(st));
     if (stats) {
         memset(stats, 0, sizeof(*stats));
-        float ms[PH_N];
-        tm.finish(&stats->ms_total, ms, PH_N);
-        stats->ms_gather = ms[PH_ENCODE];
-        stats->ms_dist_tensor = ms[PH_COUNTS];
-        stats->ms_reduce = ms[PH_FINISH];
+        tm.finish(stats);
         stats->launches = launches;
         stats->n_chunks = bands;
         stats->n_tensor_cols = ws.pt;
@@ -394,62 +370,18 @@ void launch_cols_count(const int8_t *At, int64_t pitch, int64_t row_bytes, int64
 
 void run_joint_columns(fs_dataset *ds, int kind, double log_base, const int64_t *feat_idx, int64_t n_kept,
                        const int64_t *positions, int64_t n_pos, double *d_out, fs_stats *stats) {
-    FS_REQUIRE(ds->have_features, FS_ERR_STATE, "joint counts: call fs_dataset_set_features first");
     const int64_t n = ds->n;
     const int64_t row_bytes = (n + 1) / 2;
     FS_REQUIRE(ceil_div(ceil_div(row_bytes, 16), kColsChunkVecs) <= 65535, FS_ERR_INVALID,
                "joint columns: n = %lld exceeds the sample range of the count kernel", (long long)n);
     cudaStream_t st = ds->stream;
     int launches = 0;
-    JointTimer tm(stats != nullptr, st);
-    enum { PH_ENCODE = 0, PH_COUNTS, PH_FINISH, PH_N };
-    tm.begin(PH_ENCODE);
-    // At, the start offsets and the marginals are built by the first call on a column list and reused by the
-    // following ones for as long as the working set is not rebuilt (new typing, another column list, fs_score)
-    std::vector<int64_t> key(1 + (feat_idx ? n_kept : 0));
-    key[0] = feat_idx ? n_kept : -1;
-    if (feat_idx) memcpy(key.data() + 1, feat_idx, n_kept * sizeof(int64_t));
-    WorkSet &ws = ds->ws;
-    if (!(ds->jc_valid && ws.valid && ws.build_id == ds->jc_build && ds->jc_key == key)) {
-        ds->jc_valid = false;
-        std::vector<int32_t> &start = ds->jc_start_h;
-        start.assign(n_kept + 1, 0);
-        for (int64_t c = 0; c < n_kept; ++c) {
-            const int64_t f = feat_idx ? feat_idx[c] : c;
-            FS_REQUIRE(f >= 0 && f < ds->p, FS_ERR_INVALID, "feat_idx[%lld]=%lld outside [0,%lld)", (long long)c,
-                       (long long)f, (long long)ds->p);
-            const unsigned ci = ds->col_info[f], path = ci & kColPathMask;
-            FS_REQUIRE(path == kColTensor || path == kColConst, FS_ERR_INVALID,
-                       "joint counts: column %lld is not a discrete column with at most %d distinct values", (long long)f,
-                       FS_DISTINCT_CAP);
-            start[c + 1] = start[c] + (path == kColTensor ? (int32_t)(ci >> 4) : 0);
-        }
-        ds->no_dist_ops = true;
-        try {
-            build_workset(ds, feat_idx, n_kept, true, false, 0, n, true, false, false, false, &launches);
-        } catch (...) {
-            ds->no_dist_ops = false;
-            throw;
-        }
-        ds->no_dist_ops = false;
-        const int64_t K = ws.K_used;
-        FS_REQUIRE(K == start[n_kept], FS_ERR_STATE, "joint counts: working set holds %lld reduced rows, expected %lld",
-                   (long long)K, (long long)start[n_kept]);
-        ds->jc_start.reserve(n_kept + 1);
-        FS_CUDA(cudaMemcpyAsync(ds->jc_start.ptr, start.data(), (n_kept + 1) * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-        ds->jc_marg.reserve(std::max<int64_t>(K, 1));
-        if (K > 0) {
-            joint_marginals_kernel<<<(unsigned)ceil_div(K, 8), 256, 0, st>>>(ws.At.ptr, ws.ldt / 2, row_bytes, K,
-                                                                              ds->jc_marg.ptr);
-            FS_CUDA(cudaGetLastError());
-            ++launches;
-        }
-        ds->jc_key = std::move(key);
-        ds->jc_build = ws.build_id;
-        ds->jc_valid = true;
-    }
+    PhaseTimer tm(stats != nullptr, st);
+    tm.begin(&fs_stats::ms_gather);
+    const DiscreteOperand &op = discrete_operand(ds, feat_idx, n_kept, FS_DISTINCT_CAP, "joint counts", true, &launches);
     tm.end();
-    const std::vector<int32_t> &start = ds->jc_start_h;
+    const std::vector<int32_t> &start = op.start_h;
+    const WorkSet &ws = ds->ws;
     const int64_t K = ws.K_used, pitch = ws.ldt / 2;
 
     // launches: consecutive runs of positions with at most kColsMaxSel reduced rows together
@@ -479,7 +411,7 @@ void run_joint_columns(fs_dataset *ds, int kind, double log_base, const int64_t 
         for (int64_t i = i0; i < i1; ++i)
             for (int k = start[positions[i]]; k < start[positions[i] + 1]; ++k) sel.row[n_sel++] = k;
         if (n_sel > 0) {
-            tm.begin(PH_COUNTS);
+            tm.begin(&fs_stats::ms_dist_general);
             FS_CUDA(cudaMemsetAsync(ds->jc_counts.ptr, 0, (size_t)n_sel * K * sizeof(int32_t), st));
             int32_t *cnt = ds->jc_counts.ptr;
             if (n_sel <= 1) launch_cols_count<1>(ws.At.ptr, pitch, row_bytes, K, sel, n_sel, cnt, sms, st);
@@ -491,9 +423,9 @@ void run_joint_columns(fs_dataset *ds, int kind, double log_base, const int64_t 
             ++launches;
             tm.end();
         }
-        tm.begin(PH_FINISH);
+        tm.begin(&fs_stats::ms_reduce);
         dim3 grid((unsigned)ceil_div(n_kept, 256), (unsigned)(i1 - i0));
-        joint_cols_finish_kernel<<<grid, 256, 0, st>>>(ds->jc_counts.ptr, K, ds->jc_start.ptr, ds->jc_marg.ptr, n_kept,
+        joint_cols_finish_kernel<<<grid, 256, 0, st>>>(ds->jc_counts.ptr, K, op.start.ptr, op.marg.ptr, n_kept,
                                                        ds->jc_pos.ptr, ds->jc_off.ptr, i0, n, kind, log_base, d_out);
         FS_CUDA(cudaGetLastError());
         ++launches;
@@ -503,11 +435,7 @@ void run_joint_columns(fs_dataset *ds, int kind, double log_base, const int64_t 
     FS_CUDA(cudaStreamSynchronize(st));
     if (stats) {
         memset(stats, 0, sizeof(*stats));
-        float ms[PH_N];
-        tm.finish(&stats->ms_total, ms, PH_N);
-        stats->ms_gather = ms[PH_ENCODE];
-        stats->ms_dist_general = ms[PH_COUNTS];
-        stats->ms_reduce = ms[PH_FINISH];
+        tm.finish(stats);
         stats->launches = launches;
         stats->n_chunks = (int32_t)(cuts.size() - 1);
         stats->n_tensor_cols = ws.pt;
@@ -524,7 +452,7 @@ extern "C" {
 
 int fs_joint_matrix(fs_dataset *ds, int kind, double log_base, const int64_t *feat_idx, int64_t n_kept,
                     int64_t pos_begin, int64_t pos_end, double *out, int out_on_device, fs_stats *stats) {
-    try {
+    return api_call("fs_joint_matrix", [&] {
         FS_REQUIRE(ds && out, FS_ERR_INVALID, "fs_joint_matrix: null pointer");
         FS_REQUIRE(kind == FS_JOINT_MI || kind == FS_JOINT_SU, FS_ERR_INVALID, "fs_joint_matrix: unknown kind %d", kind);
         FS_REQUIRE(kind != FS_JOINT_MI || log_base > 0.0, FS_ERR_INVALID, "fs_joint_matrix: log_base must be positive");
@@ -545,17 +473,12 @@ int fs_joint_matrix(fs_dataset *ds, int kind, double log_base, const int64_t *fe
             FS_CUDA(cudaStreamSynchronize(ds->stream));
         }
         return FS_OK;
-    } catch (const Fail &f) {
-        return f.code;
-    } catch (const std::exception &e) {
-        set_error("fs_joint_matrix: %s", e.what());
-        return FS_ERR_OOM;
-    }
+    });
 }
 
 int fs_joint_tables(fs_dataset *ds, const int64_t *feat_idx, int64_t n_kept, const int64_t *pairs, int64_t m,
                     int64_t *tables_out) {
-    try {
+    return api_call("fs_joint_tables", [&] {
         FS_REQUIRE(ds && pairs && tables_out && m >= 1, FS_ERR_INVALID, "fs_joint_tables: invalid argument");
         if (!feat_idx) n_kept = ds->p;
         for (int64_t q = 0; q < m; ++q)
@@ -573,17 +496,12 @@ int fs_joint_tables(fs_dataset *ds, const int64_t *feat_idx, int64_t n_kept, con
         FS_CUDA(cudaMemcpyAsync(tables_out, ds->joint_tables.ptr, 256 * m * sizeof(int64_t), cudaMemcpyDeviceToHost, ds->stream));
         FS_CUDA(cudaStreamSynchronize(ds->stream));
         return FS_OK;
-    } catch (const Fail &f) {
-        return f.code;
-    } catch (const std::exception &e) {
-        set_error("fs_joint_tables: %s", e.what());
-        return FS_ERR_OOM;
-    }
+    });
 }
 
 int fs_joint_columns(fs_dataset *ds, int kind, double log_base, const int64_t *feat_idx, int64_t n_kept,
                      const int64_t *positions, int64_t n_pos, double *out, int out_on_device, fs_stats *stats) {
-    try {
+    return api_call("fs_joint_columns", [&] {
         FS_REQUIRE(ds && out && positions, FS_ERR_INVALID, "fs_joint_columns: null pointer");
         FS_REQUIRE(kind == FS_JOINT_MI || kind == FS_JOINT_SU, FS_ERR_INVALID, "fs_joint_columns: unknown kind %d", kind);
         FS_REQUIRE(kind != FS_JOINT_MI || log_base > 0.0, FS_ERR_INVALID, "fs_joint_columns: log_base must be positive");
@@ -608,12 +526,7 @@ int fs_joint_columns(fs_dataset *ds, int kind, double log_base, const int64_t *f
             FS_CUDA(cudaStreamSynchronize(ds->stream));
         }
         return FS_OK;
-    } catch (const Fail &f) {
-        return f.code;
-    } catch (const std::exception &e) {
-        set_error("fs_joint_columns: %s", e.what());
-        return FS_ERR_OOM;
-    }
+    });
 }
 
 }  // extern "C"

@@ -4,8 +4,8 @@
 // project's own (DESIGN.md, "MDR"); oracle/mdr_oracle.py restates them in numpy.
 //
 // Data flow (all on the data set's stream):
-//   encode   the reduced one-hot rows At [K, n] of the columns, as fs_joint_columns builds them
-//            (build_workset; a column with V <= 3 values owns V - 1 rows, a constant column none).
+//   encode   the reduced one-hot rows At [K, n] of the columns, shared with the joint-count path
+//            (discrete_operand; a column with V <= 3 values owns V - 1 rows, a constant column none).
 //   pack     At -> uint32 bit-planes [K, W] in SEGMENT order: segment s = 2 * fold + class holds the words
 //            [seg.w[s], seg.w[s + 1]), padded with zero bits to whole words, so every word belongs to one
 //            segment; plus the popcount of every row in every segment (marg [K, 2 cv]).  Reads K * n / 2
@@ -446,52 +446,22 @@ __global__ void __launch_bounds__(128) mdr_tables_kernel(const uint32_t *__restr
                 [&](int i, int j, int64_t nij, int64_t, int64_t) { t[i * 3 + j] = nij; });
 }
 
-struct MdrTimer {
-    bool on;
-    cudaStream_t st;
-    cudaEvent_t ev[4] = {};
-    MdrTimer(bool enable, cudaStream_t s) : on(enable), st(s) {
-        if (on)
-            for (auto &e : ev) cudaEventCreate(&e);
-    }
-    void mark(int i) {
-        if (on) cudaEventRecord(ev[i], st);
-    }
-    ~MdrTimer() {
-        if (on)
-            for (auto &e : ev) cudaEventDestroy(e);
-    }
-};
-
-// Encode + pack of (feat_idx, fold), cached in ds->mdr_* while the working set is not rebuilt.
+// Encode (the shared discrete operand) + pack of (feat_idx, fold); the planes are kept for the operand's
+// generation and the folds.
 void mdr_prepare(fs_dataset *ds, const int64_t *feat_idx, int64_t n_kept, const int32_t *fold, int n_folds, int *launches) {
-    FS_REQUIRE(ds->have_features, FS_ERR_STATE, "mdr: call fs_dataset_set_features first");
     FS_REQUIRE(ds->n_classes == 2, FS_ERR_INVALID, "mdr: the data set must have 2 classes (has %d)", ds->n_classes);
     const int64_t n = ds->n;
     // balanced accuracies are ratios of integers below 2^53 (2 N1 N0 < 2^53)
     FS_REQUIRE(n < (1LL << 26), FS_ERR_INVALID, "mdr: n = %lld exceeds 2^26 samples", (long long)n);
+    const DiscreteOperand &op = discrete_operand(ds, feat_idx, n_kept, 3, "mdr", false, launches);
     const int nseg = 2 * n_folds;
-    std::vector<int64_t> key(2 + (feat_idx ? n_kept : 0) + n);
-    key[0] = feat_idx ? n_kept : -1;
-    key[1] = n_folds;
-    if (feat_idx) std::copy(feat_idx, feat_idx + n_kept, key.begin() + 2);
-    std::copy(fold, fold + n, key.begin() + 2 + (feat_idx ? n_kept : 0));
-    WorkSet &ws = ds->ws;
-    if (ds->mdr_valid && ws.valid && ws.build_id == ds->mdr_build && ds->mdr_key == key) return;
-    ds->mdr_valid = false;
+    std::vector<int64_t> key(1 + n);
+    key[0] = n_folds;
+    std::copy(fold, fold + n, key.begin() + 1);
+    if (ds->mdr_gen == op.generation && ds->mdr_key == key) return;
+    ds->mdr_gen = 0;
     cudaStream_t st = ds->stream;
 
-    std::vector<int32_t> &start = ds->mdr_start_h;
-    start.assign(n_kept + 1, 0);
-    for (int64_t c = 0; c < n_kept; ++c) {
-        const int64_t f = feat_idx ? feat_idx[c] : c;
-        FS_REQUIRE(f >= 0 && f < ds->p, FS_ERR_INVALID, "feat_idx[%lld]=%lld outside [0,%lld)", (long long)c, (long long)f,
-                   (long long)ds->p);
-        const unsigned ci = ds->col_info[f], path = ci & kColPathMask;
-        FS_REQUIRE((path == kColTensor && (ci >> 4) <= 2) || path == kColConst, FS_ERR_INVALID,
-                   "mdr: column %lld is not a discrete column with at most 3 distinct values", (long long)f);
-        start[c + 1] = start[c] + (path == kColTensor ? (int32_t)(ci >> 4) : 0);
-    }
     // segments: s = 2 * fold + class, each padded to whole words; slots filled in internal row order
     std::vector<int64_t> seg_n(nseg, 0);
     for (int64_t r = 0; r < n; ++r) {
@@ -519,24 +489,13 @@ void mdr_prepare(fs_dataset *ds, const int64_t *feat_idx, int64_t n_kept, const 
         slot[32 * (int64_t)seg.w[s] + fill[s]++] = (int32_t)r;
     }
 
-    ds->no_dist_ops = true;
-    try {
-        build_workset(ds, feat_idx, n_kept, true, false, 0, n, true, false, false, false, launches);
-    } catch (...) {
-        ds->no_dist_ops = false;
-        throw;
-    }
-    ds->no_dist_ops = false;
+    const WorkSet &ws = ds->ws;
     const int64_t K = ws.K_used;
-    FS_REQUIRE(K == start[n_kept], FS_ERR_STATE, "mdr: working set holds %lld reduced rows, expected %lld", (long long)K,
-               (long long)start[n_kept]);
-    ds->mdr_start.reserve(n_kept + 1);
     ds->mdr_slot.reserve(32 * W);
     ds->mdr_wseg.reserve(W);
     ds->mdr_planes.reserve((size_t)std::max<int64_t>(K, 1) * W);
     ds->mdr_marg.reserve((size_t)std::max<int64_t>(K, 1) * nseg);
     // pageable sources: each copy is staged before the call returns
-    FS_CUDA(cudaMemcpyAsync(ds->mdr_start.ptr, start.data(), (n_kept + 1) * sizeof(int32_t), cudaMemcpyHostToDevice, st));
     FS_CUDA(cudaMemcpyAsync(ds->mdr_slot.ptr, slot.data(), slot.size() * sizeof(int32_t), cudaMemcpyHostToDevice, st));
     FS_CUDA(cudaMemcpyAsync(ds->mdr_wseg.ptr, wseg.data(), W, cudaMemcpyHostToDevice, st));
     FS_CUDA(cudaMemsetAsync(ds->mdr_marg.ptr, 0, (size_t)std::max<int64_t>(K, 1) * nseg * sizeof(int32_t), st));
@@ -552,8 +511,7 @@ void mdr_prepare(fs_dataset *ds, const int64_t *feat_idx, int64_t n_kept, const 
     ds->mdr_W = W;
     ds->mdr_nseg = nseg;
     ds->mdr_key = std::move(key);
-    ds->mdr_build = ws.build_id;
-    ds->mdr_valid = true;
+    ds->mdr_gen = op.generation;
 }
 
 template <int NSEG, bool PAIR>
@@ -612,7 +570,7 @@ extern "C" {
 int fs_mdr_scan(fs_dataset *ds, const int64_t *feat_idx, int64_t n_kept, int32_t order, const int32_t *fold, int32_t n_folds,
                 int64_t n_top, int64_t *top_idx, double *top_train, double *top_test, int64_t *fold_best,
                 double *all_train, double *all_test, fs_stats *stats) {
-    try {
+    return api_call("fs_mdr_scan", [&] {
         if (ds && !feat_idx) n_kept = ds->p;
         check_common(ds, n_kept, order, fold, n_folds);
         FS_REQUIRE(top_idx && top_train && top_test && fold_best, FS_ERR_INVALID, "fs_mdr_scan: null output");
@@ -626,17 +584,18 @@ int fs_mdr_scan(fs_dataset *ds, const int64_t *feat_idx, int64_t n_kept, int32_t
         alloc_stream() = ds->stream;
         cudaStream_t st = ds->stream;
         int launches = 0;
-        MdrTimer tm(stats != nullptr, st);
-        tm.mark(0);
+        PhaseTimer tm(stats != nullptr, st);
+        tm.begin(&fs_stats::ms_gather);
         mdr_prepare(ds, feat_idx, n_kept, fold, n_folds, &launches);
-        tm.mark(1);
+        tm.end();
+        tm.begin(&fs_stats::ms_dist_general);
         const int nseg = ds->mdr_nseg;
         int sms = 0;
         FS_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, ds->device));
         MdrScanArgs args{};
         args.planes = ds->mdr_planes.ptr;
         args.marg = ds->mdr_marg.ptr;
-        args.start = ds->mdr_start.ptr;
+        args.start = ds->disc.start.ptr;
         args.W = ds->mdr_W;
         args.n_kept = n_kept;
         args.n_top = (int)n_top;
@@ -662,7 +621,8 @@ int fs_mdr_scan(fs_dataset *ds, const int64_t *feat_idx, int64_t n_kept, int32_t
         static_assert(sizeof(MdrCand) == 24, "MdrCand layout");
         const int64_t G = launch_scan(nseg, order == 2, args, ds->mdr_seg, sms, max_blocks, st);
         ++launches;
-        tm.mark(2);
+        tm.end();
+        tm.begin(&fs_stats::ms_reduce);
         MdrCand *cur = args.top_out, *nxt = cur + max_blocks * n_top;
         for (int64_t L = G; L > 1; L = ceil_div(L, 2)) {
             mdr_merge_kernel<<<(unsigned)ceil_div(L, 2), 256, 0, st>>>(cur, L, (int)n_top, nxt);
@@ -673,7 +633,8 @@ int fs_mdr_scan(fs_dataset *ds, const int64_t *feat_idx, int64_t n_kept, int32_t
         mdr_fold_best_kernel<<<1, 32, 0, st>>>(args.fold_out, G, n_folds, ds->mdr_best.ptr);
         FS_CUDA(cudaGetLastError());
         ++launches;
-        tm.mark(3);
+        tm.end();
+        tm.stop();          // ms_total ends before the results are copied back
         std::vector<MdrCand> top(n_top);
         FS_CUDA(cudaMemcpyAsync(top.data(), cur, n_top * sizeof(MdrCand), cudaMemcpyDeviceToHost, st));
         FS_CUDA(cudaMemcpyAsync(fold_best, ds->mdr_best.ptr, n_folds * sizeof(long long), cudaMemcpyDeviceToHost, st));
@@ -689,14 +650,7 @@ int fs_mdr_scan(fs_dataset *ds, const int64_t *feat_idx, int64_t n_kept, int32_t
         }
         if (stats) {
             memset(stats, 0, sizeof(*stats));
-            float ms = 0.f;
-            cudaEventElapsedTime(&stats->ms_total, tm.ev[0], tm.ev[3]);
-            cudaEventElapsedTime(&ms, tm.ev[0], tm.ev[1]);
-            stats->ms_gather = ms;
-            cudaEventElapsedTime(&ms, tm.ev[1], tm.ev[2]);
-            stats->ms_dist_general = ms;
-            cudaEventElapsedTime(&ms, tm.ev[2], tm.ev[3]);
-            stats->ms_reduce = ms;
+            tm.finish(stats);
             stats->launches = launches;
             stats->n_chunks = (int32_t)G;
             stats->n_tensor_cols = ds->ws.pt;
@@ -704,17 +658,12 @@ int fs_mdr_scan(fs_dataset *ds, const int64_t *feat_idx, int64_t n_kept, int32_t
             stats->pairs_selected = n_combos;
         }
         return FS_OK;
-    } catch (const Fail &f) {
-        return f.code;
-    } catch (const std::exception &e) {
-        set_error("fs_mdr_scan: %s", e.what());
-        return FS_ERR_OOM;
-    }
+    });
 }
 
 int fs_mdr_tables(fs_dataset *ds, const int64_t *feat_idx, int64_t n_kept, int32_t order, const int32_t *fold,
                   int32_t n_folds, const int64_t *combos, int64_t m, int64_t *tables_out) {
-    try {
+    return api_call("fs_mdr_tables", [&] {
         if (ds && !feat_idx) n_kept = ds->p;
         check_common(ds, n_kept, order, fold, n_folds);
         FS_REQUIRE(combos && tables_out && m >= 1, FS_ERR_INVALID, "fs_mdr_tables: invalid argument");
@@ -735,18 +684,13 @@ int fs_mdr_tables(fs_dataset *ds, const int64_t *feat_idx, int64_t n_kept, int32
         ds->mdr_tables.reserve(cells);
         FS_CUDA(cudaMemcpyAsync(ds->mdr_combos.ptr, combos, (size_t)m * order * sizeof(int64_t), cudaMemcpyHostToDevice, st));
         mdr_tables_kernel<<<(unsigned)ceil_div(m * nseg, 128), 128, 0, st>>>(ds->mdr_planes.ptr, ds->mdr_W, ds->mdr_marg.ptr,
-                                                                             ds->mdr_start.ptr, ds->mdr_seg, nseg,
+                                                                             ds->disc.start.ptr, ds->mdr_seg, nseg,
                                                                              ds->mdr_combos.ptr, order, m, ds->mdr_tables.ptr);
         FS_CUDA(cudaGetLastError());
         FS_CUDA(cudaMemcpyAsync(tables_out, ds->mdr_tables.ptr, cells * sizeof(int64_t), cudaMemcpyDeviceToHost, st));
         FS_CUDA(cudaStreamSynchronize(st));
         return FS_OK;
-    } catch (const Fail &f) {
-        return f.code;
-    } catch (const std::exception &e) {
-        set_error("fs_mdr_tables: %s", e.what());
-        return FS_ERR_OOM;
-    }
+    });
 }
 
 }  // extern "C"

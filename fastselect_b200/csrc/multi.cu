@@ -53,15 +53,8 @@ void run_ranks(int world, const std::function<int(int)> &fn) {
     th.reserve(world);
     for (int r = 0; r < world; ++r)
         th.emplace_back([&, r]() {
-            int rc = FS_ERR_CUDA;
-            try {
-                rc = fn(r);
-            } catch (const Fail &f) {
-                rc = f.code;
-            } catch (const std::exception &e) {
-                set_error("rank %d: %s", r, e.what());
-                rc = FS_ERR_OOM;
-            }
+            const std::string name = "rank " + std::to_string(r);
+            const int rc = api_call(name.c_str(), [&] { return fn(r); });
             errs[r].code = rc;
             if (rc != FS_OK) errs[r].msg = get_error();
         });
@@ -97,7 +90,7 @@ extern "C" {
 int fs_multi_create(fs_multi **out, const void *x, int dtype, int64_t n, int64_t p, int64_t row_stride_elems,
                     const int32_t *y_enc, int32_t n_classes, const int32_t *devices, int32_t n_devices) {
     fs_multi *m = nullptr;
-    try {
+    const int rc = api_call("fs_multi_create", [&] {
         FS_REQUIRE(out && x && devices, FS_ERR_INVALID, "fs_multi_create: null pointer");
         FS_REQUIRE(n_devices >= 1 && n_devices <= kMaxRanks, FS_ERR_INVALID, "fs_multi_create: 1..%d devices", kMaxRanks);
         FS_REQUIRE(fs_device_count() > 0, FS_ERR_NO_DEVICE, "no usable NVIDIA sm_100 (B200) GPU: this library has no CPU fallback");
@@ -170,20 +163,12 @@ int fs_multi_create(fs_multi **out, const void *x, int dtype, int64_t n, int64_t
         if (world > 1) run_ranks(world, [&](int r) { return fs_dataset_attach_comm(m->sets[r], m->comms[r], m->starts.data()); });
         *out = m;
         return FS_OK;
-    } catch (const Fail &f) {
-        if (m) {
-            for (auto *ds : m->sets) fs_dataset_destroy(ds);
-            delete m;
-        }
-        return f.code;
-    } catch (const std::exception &e) {
-        set_error("fs_multi_create: %s", e.what());
-        if (m) {
-            for (auto *ds : m->sets) fs_dataset_destroy(ds);
-            delete m;
-        }
-        return FS_ERR_OOM;
+    });
+    if (rc != FS_OK && m) {
+        for (auto *ds : m->sets) fs_dataset_destroy(ds);
+        delete m;
     }
+    return rc;
 }
 
 int fs_multi_world(const fs_multi *m) { return m ? m->world : 0; }
@@ -210,7 +195,7 @@ int fs_multi_set_features(fs_multi *m, const uint8_t *is_discrete, const float *
 
 int fs_multi_score(fs_multi *m, int algo, int use_star, int32_t k, const float *class_probs, const int64_t *feat_idx,
                    int64_t n_kept, double *wsum_out, fs_stats *stats) {
-    try {
+    return api_call("fs_multi_score", [&] {
         FS_REQUIRE(m && wsum_out, FS_ERR_INVALID, "fs_multi_score: null pointer");
         if (!feat_idx) n_kept = m->p;
         const int world = m->world;
@@ -227,12 +212,7 @@ int fs_multi_score(fs_multi *m, int algo, int use_star, int32_t k, const float *
                             m->outs[r]->ptr, 1, nullptr);
         });
         return FS_OK;
-    } catch (const Fail &f) {
-        return f.code;
-    } catch (const std::exception &e) {
-        set_error("fs_multi_score: %s", e.what());
-        return FS_ERR_OOM;
-    }
+    });
 }
 
 int fs_multi_destroy(fs_multi *m) {

@@ -23,61 +23,6 @@ void launch_accum_tensor(fs_dataset *ds, const WorkSet &ws, int algo, const int6
                          const int32_t *nbr_cnt, int32_t nbr_cap, double *wsum, cudaStream_t st, int *launches,
                          double *ops);
 
-enum Phase { PH_GATHER = 0, PH_DIST_T, PH_DIST_G, PH_SELECT, PH_ACC_T, PH_ACC_G, PH_REDUCE, PH_COUNT };
-
-struct Timer {
-    bool on;
-    cudaStream_t st;
-    struct Span { int ph; cudaEvent_t a, b; };
-    std::vector<Span> spans;
-    cudaEvent_t t0 = nullptr, t1 = nullptr;
-    Timer(bool enable, cudaStream_t s) : on(enable), st(s) {
-        if (on) {
-            cudaEventCreate(&t0);
-            cudaEventCreate(&t1);
-            cudaEventRecord(t0, st);
-        }
-    }
-    void begin(int ph) {
-        if (!on) return;
-        Span s{ph, nullptr, nullptr};
-        cudaEventCreate(&s.a);
-        cudaEventCreate(&s.b);
-        cudaEventRecord(s.a, st);
-        spans.push_back(s);
-    }
-    void end() {
-        if (on) cudaEventRecord(spans.back().b, st);
-    }
-    void finish(fs_stats *out) {
-        if (!on) return;
-        cudaEventRecord(t1, st);
-        cudaEventSynchronize(t1);
-        float ms[PH_COUNT] = {0};
-        for (auto &s : spans) {
-            float t = 0.f;
-            cudaEventElapsedTime(&t, s.a, s.b);
-            ms[s.ph] += t;
-        }
-        cudaEventElapsedTime(&out->ms_total, t0, t1);
-        out->ms_gather = ms[PH_GATHER];
-        out->ms_dist_tensor = ms[PH_DIST_T];
-        out->ms_dist_general = ms[PH_DIST_G];
-        out->ms_select = ms[PH_SELECT];
-        out->ms_accum_tensor = ms[PH_ACC_T];
-        out->ms_accum_general = ms[PH_ACC_G];
-        out->ms_reduce = ms[PH_REDUCE];
-    }
-    ~Timer() {
-        for (auto &s : spans) {
-            cudaEventDestroy(s.a);
-            cudaEventDestroy(s.b);
-        }
-        if (t0) cudaEventDestroy(t0);
-        if (t1) cudaEventDestroy(t1);
-    }
-};
-
 struct DebugOut {
     double *dist = nullptr;    // [nt, n] original sample order
     double *thresh = nullptr;  // [nt]
@@ -127,7 +72,7 @@ static void run_pipeline(fs_dataset *ds, int algo, int use_star, int32_t k, cons
     const int64_t n = ds->n;
     int launches = 0;
     double ops_dist = 0.0, ops_accum = 0.0;
-    Timer timer(stats != nullptr, st);
+    PhaseTimer timer(stats != nullptr, st);
 
     const char *env_t = getenv("FS_B200_TENSOR");
     const bool allow_tensor = tensor_path_available() && !(env_t && env_t[0] == '0');
@@ -154,10 +99,10 @@ static void run_pipeline(fs_dataset *ds, int algo, int use_star, int32_t k, cons
     const int64_t cache_rows = std::max<int64_t>((int64_t)targets.size(), max_shard);
     const bool slab_cacheable = contiguous && dbg == nullptr && round_up(cache_rows, 128) <= chunk_rows(true, true, ldn, algo);
     if (!slab_cacheable) ds->dd_valid = false;
-    timer.begin(PH_GATHER);
+    timer.begin(&fs_stats::ms_gather);
     const auto prep0 = std::chrono::steady_clock::now();
     build_workset(ds, feat_idx, n_kept, allow_tensor, algo == FS_RELIEFF, targets[0], (int64_t)targets.size(),
-                  contiguous, slab_cacheable, want_split, group_call, &launches);
+                  contiguous, slab_cacheable, want_split, group_call, true, &launches);
     const double ms_prep = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - prep0).count();
     timer.end();
     const WorkSet &ws = ds->ws;
@@ -182,7 +127,7 @@ static void run_pipeline(fs_dataset *ds, int algo, int use_star, int32_t k, cons
                 ds->dd_valid = false;
                 ds->ws.valid = false;
                 build_workset(ds, feat_idx, n_kept, allow_tensor, algo == FS_RELIEFF, targets[0], (int64_t)targets.size(),
-                              contiguous, slab_cacheable, want_split, group_call, &launches);
+                              contiguous, slab_cacheable, want_split, group_call, true, &launches);
             }
             ds->dd_valid = false;
         }
@@ -256,7 +201,7 @@ static void run_pipeline(fs_dataset *ds, int algo, int use_star, int32_t k, cons
         // ---- distances
         if (ws.pt > 0 && ws.dist_mode != kDistReuse) {
             ds->dd_valid = false;
-            timer.begin(PH_DIST_T);
+            timer.begin(&fs_stats::ms_dist_tensor);
             launch_dist_tensor(ds, ws, h_ids[0], h_ids, ds->row_ids.ptr, contiguous, R, Dd, ldn, st, &launches, &ops_dist);
             timer.end();
             if (ds->last_dist_exchanged) {
@@ -278,12 +223,12 @@ static void run_pipeline(fs_dataset *ds, int algo, int use_star, int32_t k, cons
             ds->dd_valid = true;
         }
         if (ws.pg > 0) {
-            timer.begin(PH_DIST_G);
+            timer.begin(&fs_stats::ms_dist_general);
             launch_dist_general(ws, xa, R, ws.xg.ptr, n, ds->Dc.ptr, ldn, st, &launches);
             timer.end();
         }
         // ---- neighbour selection
-        timer.begin(PH_SELECT);
+        timer.begin(&fs_stats::ms_select);
         launch_select(ds, algo, use_star, k, ds->row_ids.ptr, R, ws.pg > 0 ? ds->Dc.ptr : nullptr,
                       ws.pt > 0 ? Dd : nullptr, ldn, ds->sel.ptr, use_masks ? mask_h : nullptr,
                       use_masks ? mask_m : nullptr, rinfo_buf, ds->nbr_idx.ptr,
@@ -298,7 +243,7 @@ static void run_pipeline(fs_dataset *ds, int algo, int use_star, int32_t k, cons
             // sharded by one-hot columns: every rank sends the masks / constants of its target rows to all
             // peers, then contracts ITS columns against the masks of ALL n targets (the complete weight of
             // those columns, with the tiling of a single-GPU pass: bitwise the single-GPU result)
-            timer.begin(PH_ACC_T);
+            timer.begin(&fs_stats::ms_accum_tensor);
             const size_t mrow = (size_t)(ldn / 2);
             comm_push(comm, ds->glayout.off_mask_h + (size_t)shard0 * mrow, (size_t)R * mrow, st, &launches);
             comm_push(comm, ds->glayout.off_mask_m + (size_t)shard0 * mrow, (size_t)R * mrow, st, &launches);
@@ -317,7 +262,7 @@ static void run_pipeline(fs_dataset *ds, int algo, int use_star, int32_t k, cons
                                 acc_out, st, &launches, &ops_accum);
             timer.end();
         } else if (ws.pt > 0) {
-            timer.begin(PH_ACC_T);
+            timer.begin(&fs_stats::ms_accum_tensor);
             launch_accum_tensor(ds, ws, algo, ds->row_ids.ptr, h_ids, contiguous, R, mask_h, mask_m, ldn,
                                 rinfo_buf, ds->nbr_idx.ptr, ds->nbr_w.ptr, ds->nbr_cnt.ptr, nbr_cap, acc_out,
                                 st, &launches, &ops_accum);
@@ -326,7 +271,7 @@ static void run_pipeline(fs_dataset *ds, int algo, int use_star, int32_t k, cons
         if (ws.pg > 0) {
             const int64_t n_part = accum_general_partials(ws, R);
             ds->partial.reserve((size_t)n_part * ws.ldg);
-            timer.begin(PH_ACC_G);
+            timer.begin(&fs_stats::ms_accum_general);
             if (algo == FS_RELIEFF)
                 launch_relieff_gather(ws, n, xa, ds->nbr_idx.ptr, ds->nbr_w.ptr, ds->nbr_cnt.ptr, nbr_cap, R,
                                       ds->partial.ptr, n_part, st, &launches);
@@ -334,7 +279,7 @@ static void run_pipeline(fs_dataset *ds, int algo, int use_star, int32_t k, cons
                 launch_accum_general(ws, n, xa, ds->sel.ptr, ldn, rinfo_buf, R, ds->partial.ptr, n_part, st,
                                      &launches);
             timer.end();
-            timer.begin(PH_REDUCE);
+            timer.begin(&fs_stats::ms_reduce);
             launch_reduce_partials(ws, ds->partial.ptr, n_part, acc_out, st, &launches);
             timer.end();
         }
@@ -375,7 +320,7 @@ static void run_pipeline(fs_dataset *ds, int algo, int use_star, int32_t k, cons
     if (group_call) {
         // every rank's contribution (its share of the one-hot columns in full, or partial sums over its
         // target rows) goes into its slot of every arena; the slots are added in rank order
-        timer.begin(PH_REDUCE);
+        timer.begin(&fs_stats::ms_reduce);
         const size_t slot_bytes = (size_t)round_up(n_kept * (int64_t)sizeof(double), 16);
         comm_push(comm, ds->glayout.off_w + (size_t)comm->rank * ds->p * sizeof(double), slot_bytes, st, &launches);
         comm_barrier(comm, st, &launches);
@@ -415,7 +360,7 @@ extern "C" {
 int fs_score(fs_dataset *ds, int algo, int use_star, int32_t k, const float *class_probs,
              const int64_t *feat_idx, int64_t n_kept, int64_t row_begin, int64_t row_end, double *wsum_out,
              int out_on_device, fs_stats *stats) {
-    try {
+    return api_call("fs_score", [&] {
         FS_REQUIRE(ds && wsum_out, FS_ERR_INVALID, "fs_score: null pointer");
         if (!feat_idx) n_kept = ds->p;
         FS_REQUIRE(row_begin >= 0 && row_begin <= row_end && row_end <= ds->n, FS_ERR_INVALID,
@@ -441,18 +386,13 @@ int fs_score(fs_dataset *ds, int algo, int use_star, int32_t k, const float *cla
             FS_CUDA(cudaStreamSynchronize(ds->stream));
         }
         return FS_OK;
-    } catch (const Fail &f) {
-        return f.code;
-    } catch (const std::exception &e) {
-        set_error("fs_score: %s", e.what());
-        return FS_ERR_OOM;
-    }
+    });
 }
 
 int fs_debug_rows(fs_dataset *ds, int algo, int use_star, int32_t k, const float *class_probs,
                   const int64_t *feat_idx, int64_t n_kept, const int64_t *targets, int64_t nt, double *dist_out,
                   double *thresh_out, int8_t *mask_out, double *wsum_out) {
-    try {
+    return api_call("fs_debug_rows", [&] {
         FS_REQUIRE(ds && targets && nt >= 1, FS_ERR_INVALID, "fs_debug_rows: invalid argument");
         if (!feat_idx) n_kept = ds->p;
         FS_CUDA(cudaSetDevice(ds->device));
@@ -468,16 +408,11 @@ int fs_debug_rows(fs_dataset *ds, int algo, int use_star, int32_t k, const float
         run_pipeline(ds, algo, use_star, k, class_probs, feat_idx, n_kept, ids, false, ds->wsum.ptr, &dbg, nullptr);
         if (wsum_out) FS_CUDA(cudaMemcpy(wsum_out, ds->wsum.ptr, n_kept * sizeof(double), cudaMemcpyDeviceToHost));
         return FS_OK;
-    } catch (const Fail &f) {
-        return f.code;
-    } catch (const std::exception &e) {
-        set_error("fs_debug_rows: %s", e.what());
-        return FS_ERR_OOM;
-    }
+    });
 }
 
 int fs_debug_slab(fs_dataset *ds, int64_t row_begin, int64_t nrows, int32_t *out, int64_t *info_out) {
-    try {
+    return api_call("fs_debug_slab", [&] {
         FS_REQUIRE(ds && out && nrows >= 1, FS_ERR_INVALID, "fs_debug_slab: invalid argument");
         FS_REQUIRE(ds->dd_valid && ds->dd_buf != nullptr, FS_ERR_STATE, "fs_debug_slab: no distance slab is cached");
         FS_REQUIRE(row_begin >= ds->dd_r0 && row_begin + nrows <= ds->dd_r0 + ds->dd_R, FS_ERR_STATE,
@@ -494,9 +429,7 @@ int fs_debug_slab(fs_dataset *ds, int64_t row_begin, int64_t nrows, int32_t *out
             info_out[2] = (int64_t)ds->dd_cols.size();
         }
         return FS_OK;
-    } catch (const Fail &f) {
-        return f.code;
-    }
+    });
 }
 
 }  // extern "C"

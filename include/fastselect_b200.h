@@ -233,6 +233,10 @@ FS_API int fs_multi_destroy(fs_multi *m);
  *   kind FS_JOINT_SU: 2 I(x; y) / (H(x) + H(y)) in bits                  (CFS.py:26-77; the reference
  *        keeps float32 intermediates there, this is the float64 value: |difference| < 1e-6)
  *   out_on_device != 0: out is a device pointer on the data set's device.
+ *   The one-hot rows, their marginals and the position offsets of a column list are shared by
+ *   fs_joint_matrix, fs_joint_tables, fs_joint_columns and fs_mdr_*: built by the first of these calls
+ *   on a (column list, typing) and reused by the following ones until the data set's working set is
+ *   rebuilt (fs_dataset_set_features, another column list, fs_score).
  * fs_joint_tables: the contingency tables themselves for m pairs of positions (pairs[2 * q],
  *   pairs[2 * q + 1]), exact integers: tables_out[q * 256 + va * 16 + vb] = #samples with the va-th
  *   smallest value of the first column and the vb-th smallest value of the second (host pointer).
@@ -242,10 +246,8 @@ FS_API int fs_multi_destroy(fs_multi *m);
  *   lie in [0, n_kept); the other checks and error codes are those of fs_joint_matrix.  The counts come
  *   from one pass of the CUDA cores over the reduced one-hot rows per 16 selected reduced rows (one pass
  *   for a call of up to 8 genotype or one 16-state position), so a greedy search that needs k columns
- *   reads k passes, not p^2 statistics.  The one-hot rows, their marginals and the position offsets are
- *   built by the first call on a (column list, typing) and reused by later calls until the data set's
- *   working set is rebuilt (fs_dataset_set_features, another column list, fs_score).  In stats:
- *   ms_gather = that build (about 0 on a reuse), ms_dist_general = count kernels, ms_reduce = finish
+ *   reads k passes, not p^2 statistics.  The one-hot rows, offsets and marginals are shared with
+ *   fs_joint_matrix (see there).  In stats: ms_gather = their build (about 0 on a reuse), ms_dist_general = count kernels, ms_reduce = finish
  *   kernels, n_chunks = count launches.
  */
 typedef enum { FS_JOINT_MI = 0, FS_JOINT_SU = 1 } fs_joint_kind;
@@ -277,9 +279,9 @@ FS_API int fs_joint_columns(fs_dataset *ds, int kind, double log_base, const int
  *   balanced accuracy (lower index first on ties), with their mean training / test values;
  *   1 <= n_top <= min(FS_MDR_MAX_TOP, n_combos).  fold_best[n_folds]: per fold, the combination with the
  *   highest training balanced accuracy (lower index first on ties).  all_train / all_test (nullable, both
- *   or neither, [n_combos] host arrays): the means of every combination.  The bit-planes of a (column
- *   list, fold vector) are built by the first call and reused by later calls until the working set is
- *   rebuilt.  In stats: ms_gather = encode + pack (about 0 on a reuse), ms_dist_general = scan kernel,
+ *   or neither, [n_combos] host arrays): the means of every combination.  The one-hot rows and offsets
+ *   are shared with fs_joint_matrix (see there); the bit-planes of a (column list, fold vector) are built
+ *   from them by the first call and reused by later calls until they are rebuilt.  In stats: ms_gather = encode + pack (about 0 on a reuse), ms_dist_general = scan kernel,
  *   ms_reduce = merges, n_chunks = scan blocks, pairs_selected = n_combos.
  * fs_mdr_tables: tables_out[((q * n_folds + f) * 2 + c) * 9 + va * 3 + vb], int64: samples of fold f and
  *   class c in cell (va, vb) of combination q = combos[q * order ..] (positions, any order; order 1: vb = 0).

@@ -155,3 +155,50 @@ def test_planted_interaction_at_c3_shape(native):
     fold = _mdr.make_folds(y, 5, None)
     with _mdr.MDRData(X, y) as src:
         check_scan(src, X, y, fold, 5, 2, feat_idx=idx, n_top=100)
+
+
+def test_encoding_is_shared_with_the_joint_path(native):
+    """joint_columns, mdr_scan, joint_matrix and mdr_scan again on one column list of one data set: each result
+    is bitwise the same call's on a freshly opened data set, and the second scan packs nothing."""
+    X, y = make_data(7, 3001, 30, np.uint8, 5)
+    fold = _mdr.make_folds(y, 5, None)
+    idx = np.random.RandomState(7).permutation(30)[:24]
+    calls = [lambda ds: ds.joint_columns(0, 1.0, [0, 5, 23], feat_idx=idx),
+             lambda ds: ds.mdr_scan(fold, 2, 50, feat_idx=idx, want_all=True, want_stats=True),
+             lambda ds: ds.joint_matrix(1, 1.0, feat_idx=idx),
+             lambda ds: ds.mdr_scan(fold, 2, 50, feat_idx=idx, want_all=True, want_stats=True)]
+    fresh = []
+    for call in calls:
+        with _mdr.MDRData(X, y) as src:
+            fresh.append(call(src._ds))
+    with _mdr.MDRData(X, y) as src:
+        got = [call(src._ds) for call in calls]
+    for i in (0, 2):
+        assert np.array_equal(bits(got[i]), bits(fresh[i])), i
+    for i in (1, 3):
+        for k in fresh[i][0]:
+            assert np.array_equal(np.asarray(got[i][0][k]).view(np.int64), np.asarray(fresh[i][0][k]).view(np.int64)), k
+    # the first scan packs the planes (encode done by joint_columns); the second only scans and merges
+    assert got[1][1]["launches"] == got[3][1]["launches"] + 1
+    assert got[3][1]["ms_gather"] < 0.05, got[3][1]
+
+
+def test_encoding_of_the_joint_path_keeps_the_mdr_limit(native):
+    X, y = make_data(8, 400, 12, np.uint8, 5)
+    X[0, 4] = 9                                                 # 4 states: a joint column, not an MDR one
+    fold = _mdr.make_folds(y, 5, None)
+    with _mdr.MDRData(X, y) as src:
+        src._ds.joint_columns(0, 1.0, [4])
+        with pytest.raises(ValueError, match="at most 3"):
+            src._ds.mdr_scan(fold, 2, 1)
+
+
+def test_scan_after_a_rebuild_of_the_working_set(native):
+    X, y = make_data(9, 1500, 20, np.int8, 3)
+    fold = _mdr.make_folds(y, 3, None)
+    with _mdr.MDRData(X, y) as src:
+        first = src._ds.mdr_scan(fold, 2, 40, want_all=True)
+        src._ds.joint_columns(0, 1.0, [1], feat_idx=np.arange(0, 20, 3))
+        again = src._ds.mdr_scan(fold, 2, 40, want_all=True)
+    for k in first:
+        assert np.array_equal(np.asarray(first[k]).view(np.int64), np.asarray(again[k]).view(np.int64)), k

@@ -85,6 +85,39 @@ def test_c_abi_exports_every_declared_symbol():
     assert not [s for s in exported if "fso_" in s], "the oracle must not be linked into the product"
 
 
+# Every C entry point that can fail inside turns that failure into a return code and a message; a null
+# handle is rejected before any device work, so this runs without a GPU.
+_NULL_HANDLE_CALLS = [
+    ("fs_score", (None, 0, 0, 0, None, None, 0, 0, 0, None, 0, None), -1, "fs_score: null pointer"),
+    ("fs_debug_rows", (None, 0, 0, 0, None, None, 0, None, 0, None, None, None, None), -1,
+     "fs_debug_rows: invalid argument"),
+    ("fs_debug_slab", (None, 0, 1, None, None), -1, "fs_debug_slab: invalid argument"),
+    ("fs_joint_matrix", (None, 0, 1.0, None, 0, 0, 0, None, 0, None), -1, "fs_joint_matrix: null pointer"),
+    ("fs_joint_tables", (None, None, 0, None, 0, None), -1, "fs_joint_tables: invalid argument"),
+    ("fs_joint_columns", (None, 0, 1.0, None, 0, None, 0, None, 0, None), -1, "fs_joint_columns: null pointer"),
+    ("fs_mdr_scan", (None, None, 0, 2, None, 2, 1, None, None, None, None, None, None, None), -1, "mdr: null pointer"),
+    ("fs_mdr_tables", (None, None, 0, 2, None, 2, None, 0, None), -1, "mdr: null pointer"),
+    ("fs_dataset_create", (None, None, 0, 1, 1, 1, None, 2, 0, None), -1, "fs_dataset_create: null pointer"),
+    ("fs_dataset_create_device", (None, None, 0, 1, 1, 1, None, 2, 0, None), -1,
+     "fs_dataset_create_device: null pointer"),
+    ("fs_dataset_create_group", (None, None, None, 0, 1, 1, 1, None, 2, None), -1,
+     "fs_dataset_create_group: null pointer"),
+    ("fs_dataset_attach_comm", (None, None, None), -1, "fs_dataset_attach_comm: null data set"),
+    ("fs_comm_create", (None, 0, 1, 0), -1, "fs_comm_create: null pointer"),
+    ("fs_comm_reserve", (None, 0, None, None), -1, "fs_comm_reserve: null communicator"),
+    ("fs_comm_connect", (None, None, None), -5, "fs_comm_connect: reserve the arena first"),
+    ("fs_multi_create", (None, None, 0, 1, 1, 1, None, 2, None, 1), -1, "fs_multi_create: null pointer"),
+    ("fs_multi_score", (None, 0, 0, 0, None, None, 0, None, None), -1, "fs_multi_score: null pointer"),
+]
+
+
+@pytest.mark.parametrize("name,args,code,message", _NULL_HANDLE_CALLS, ids=[c[0] for c in _NULL_HANDLE_CALLS])
+def test_c_entry_points_reject_a_null_handle(name, args, code, message):
+    lib = _native.load()
+    assert getattr(lib, name)(*args) == code
+    assert lib.fs_last_error().decode().startswith(message)
+
+
 def test_product_never_imports_the_oracle():
     pkg = os.path.join(ROOT, "fastselect_b200")
     for dirpath, _, files in os.walk(pkg):
