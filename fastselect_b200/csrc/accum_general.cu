@@ -234,9 +234,8 @@ void launch_accum_general(const WorkSet &ws, int64_t n, const void *xa, const in
     // Target rows given as a view into xg (the production path); a gathered copy (fs_debug_rows) stays on
     // the float64 kernel.
     const char *xg_lo = ws.xg.ptr, *xg_hi = ws.xg.ptr + (size_t)n * ws.ldg * ws.elem;
-    const char *env32 = getenv("FS_B200_SURF_ACCUM_F32");
     const bool view = static_cast<const char *>(xa) >= xg_lo && static_cast<const char *>(xa) < xg_hi;
-    if (ws.elem == 8 && ws.have_xg32 && view && !(env32 && env32[0] == '0')) {
+    if (ws.elem == 8 && ws.have_xg32 && view) {
         const int64_t row0 = (static_cast<const char *>(xa) - xg_lo) / ((int64_t)ws.ldg * ws.elem);
         accum_general_kernel<float><<<grid, kAccThreads, 0, st>>>(
             ws.xg32.ptr, n, ws.ldg, ws.rg.ptr, ws.ctype.ptr, ws.xg32.ptr + (size_t)row0 * ws.ldg, sel, ldn, rinfo, R, rows,

@@ -481,7 +481,7 @@ namespace fs {
 // slab fits one chunk -- decides between a full, an incremental and no distance computation
 // want_split: a multi-GPU group call that may shard the accumulation by one-hot columns (WorkSet::acc_split)
 // dist_ops: build the distance operands U / Wd / srow too (the joint-count and MDR paths read only At)
-void build_workset(fs_dataset *ds, const int64_t *feat_idx, int64_t n_kept, bool allow_tensor, bool need_codes,
+void build_workset(fs_dataset *ds, const int64_t *feat_idx, int64_t n_kept, bool need_codes,
                    int64_t r0, int64_t R, bool contiguous, bool slab_cacheable, bool want_split, bool group_call,
                    bool dist_ops, int *launches);
 

@@ -445,7 +445,7 @@ static int plan_dist(fs_dataset *ds, const int64_t *tcol, int64_t pt, int64_t r0
     return kDistIncremental;
 }
 
-void build_workset(fs_dataset *ds, const int64_t *feat_idx, int64_t n_kept, bool allow_tensor, bool need_codes,
+void build_workset(fs_dataset *ds, const int64_t *feat_idx, int64_t n_kept, bool need_codes,
                    int64_t r0, int64_t R, bool contiguous, bool slab_cacheable, bool want_split, bool group_call,
                    bool dist_ops, int *launches) {
     WorkSet &ws = ds->ws;
@@ -455,7 +455,7 @@ void build_workset(fs_dataset *ds, const int64_t *feat_idx, int64_t n_kept, bool
     // cache key: flags + the explicit column list (none when every column is active)
     const bool all = feat_idx == nullptr;
     std::vector<int64_t> key(3 + (all ? 0 : n_kept));
-    key[0] = (allow_tensor ? 1 : 0) | (want_split ? 2 : 0) | (group_call ? 4 : 0);
+    key[0] = (want_split ? 1 : 0) | (group_call ? 2 : 0);
     ws.group_call = group_call;
     key[1] = ds->arith;
     key[2] = all ? -1 : n_kept;
@@ -501,18 +501,13 @@ void build_workset(fs_dataset *ds, const int64_t *feat_idx, int64_t n_kept, bool
         const unsigned ci = info[f];
         switch (ci & kColPathMask) {
             case kColTensor:
-                if (allow_tensor) {
-                    tcol[pt] = f;
-                    tout[pt] = c;
-                    toff[pt] = (int32_t)K;
-                    K += ci >> 4;                  // V - 1 reduced one-hot rows
-                    ident &= ci;
-                    v3 = v3 && (ci >> 4) == 2;
-                    ++pt;
-                } else {
-                    cmp_col.push_back(f);
-                    cmp_out.push_back(c);
-                }
+                tcol[pt] = f;
+                tout[pt] = c;
+                toff[pt] = (int32_t)K;
+                K += ci >> 4;                      // V - 1 reduced one-hot rows
+                ident &= ci;
+                v3 = v3 && (ci >> 4) == 2;
+                ++pt;
                 break;
             case kColConst:
                 // a constant column: every per-feature term is 0 (MultiSURF.py:184-185), so it

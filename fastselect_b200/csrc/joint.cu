@@ -34,8 +34,8 @@ namespace fs {
 // onehot.cu / tc_dist.cu
 CUtensorMap make_tmap_u8_sw128(const void *base, uint64_t row_bytes, uint64_t rows, uint64_t pitch_bytes,
                                uint32_t box_rows);
-void launch_tc_dist(const CUtensorMap &tmap_a, const CUtensorMap &tmap_b, const CUtensorMap *tmap_b_half, int64_t K,
-                    const int32_t *srow, const int64_t *d_ids, int64_t R, int64_t n, int64_t ldd, bool symmetric, bool subtract,
+void launch_tc_dist(const CUtensorMap &tmap_a, const CUtensorMap &tmap_b, int64_t K, const int32_t *srow,
+                    const int64_t *d_ids, int64_t R, int64_t n, int64_t ldd, bool symmetric, bool subtract,
                     const DistPeers &peers, cudaStream_t st, int *launches, double *ops);
 
 namespace {
@@ -87,7 +87,7 @@ const DiscreteOperand &discrete_operand(fs_dataset *ds, const int64_t *feat_idx,
             max_rows = std::max(max_rows, rows);
         }
         op.valid = false;
-        build_workset(ds, feat_idx, n_kept, true, false, 0, ds->n, true, false, false, false, false, launches);
+        build_workset(ds, feat_idx, n_kept, false, 0, ds->n, true, false, false, false, false, launches);
         FS_REQUIRE(ws.K_used == start[n_kept], FS_ERR_STATE, "%s: working set holds %lld reduced rows, expected %lld",
                    what, (long long)ws.K_used, (long long)start[n_kept]);
         op.start_h = std::move(start);
@@ -207,7 +207,7 @@ void run_joint(fs_dataset *ds, int kind, double log_base, const int64_t *feat_id
             FS_CUDA(cudaMemsetAsync(ds->joint_ids.ptr, 0, round_up(R, 128) * sizeof(int64_t), st));
             const int8_t *base = ws.At.ptr + (size_t)b0 * pitch;
             const CUtensorMap ta = make_tmap_u8_sw128(base, row_bytes, R, pitch, 128);
-            const CUtensorMap tb = make_tmap_u8_sw128(base, row_bytes, ncols, pitch, 256);
+            const CUtensorMap tb = make_tmap_u8_sw128(base, row_bytes, ncols, pitch, 128);      // half a super-block per CTA
             DistPeers peers{};
             peers.world = 1;
             peers.rank = 0;
@@ -217,8 +217,7 @@ void run_joint(fs_dataset *ds, int kind, double log_base, const int64_t *feat_id
             peers.sb_base[0] = 0;
             peers.sb_base[1] = (int32_t)ceil_div(ncols, 256);
             peers.coarse_shift = 3;
-            const CUtensorMap tbh = make_tmap_u8_sw128(base, row_bytes, ncols, pitch, 128);      // CTA pairs
-            launch_tc_dist(ta, tb, &tbh, k_bytes, ds->joint_zero.ptr, ds->joint_ids.ptr, R, ncols, ldd, false, false, peers, st,
+            launch_tc_dist(ta, tb, k_bytes, ds->joint_zero.ptr, ds->joint_ids.ptr, R, ncols, ldd, false, false, peers, st,
                            &launches, &ops);
             tm.end();
         }

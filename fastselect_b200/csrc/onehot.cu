@@ -20,8 +20,8 @@
 
 namespace fs {
 
-void launch_tc_dist(const CUtensorMap &tmap_a, const CUtensorMap &tmap_b, const CUtensorMap *tmap_b_half, int64_t K,
-                    const int32_t *srow, const int64_t *d_ids, int64_t R, int64_t n, int64_t ldd, bool symmetric, bool subtract,
+void launch_tc_dist(const CUtensorMap &tmap_a, const CUtensorMap &tmap_b, int64_t K, const int32_t *srow,
+                    const int64_t *d_ids, int64_t R, int64_t n, int64_t ldd, bool symmetric, bool subtract,
                     const DistPeers &peers, cudaStream_t st, int *launches, double *ops);
 int tc_accum_tile_desc_ints();
 int launch_tc_accum(const CUtensorMap &tmap_at, const CUtensorMap &tmap_mh, const CUtensorMap &tmap_mm, int64_t n,
@@ -29,8 +29,6 @@ int launch_tc_accum(const CUtensorMap &tmap_at, const CUtensorMap &tmap_mh, cons
                     int64_t ldt, const uint32_t *krow, int64_t K_rows, DevBuf<double> &tpartial, int32_t *d_tiles,
                     DevBuf<int32_t> &consts, cudaStream_t st, int *launches, const int64_t *h_ids, const int32_t *h_y,
                     const int64_t *h_cls_start, double *ops);
-
-bool tensor_path_available() { return true; }
 
 // ---------------------------------------------------------------------------
 // TMA descriptor (driver entry point fetched through the runtime: no -lcuda)
@@ -738,16 +736,13 @@ void build_onehot(fs_dataset *ds, WorkSet &ws, int *launches) {
     // samples), then the accumulation operands of this rank's slice only.
     // Wd rows this rank's distance kernel reads (see WdRows)
     WdRows wr{0, n, 0, 0};
-    {
-        const char *env_sym = getenv("FS_B200_SYMMETRIC");
-        if (ws.group_call && ds->peers_on && ds->peers.world > 1 && !(env_sym && env_sym[0] == '0')) {
-            const DistPeers &pr = ds->peers;
-            const int G = pr.world, r = pr.rank, last = r + G / 2;          // ranks r .. r + floor(G / 2) on the ring
-            if (last < G) {
-                wr = WdRows{pr.starts[r], pr.starts[last + 1], 0, 0};
-            } else {
-                wr = WdRows{pr.starts[r], n, 0, pr.starts[last - G + 1]};
-            }
+    if (ws.group_call && ds->peers_on && ds->peers.world > 1) {
+        const DistPeers &pr = ds->peers;
+        const int G = pr.world, r = pr.rank, last = r + G / 2;          // ranks r .. r + floor(G / 2) on the ring
+        if (last < G) {
+            wr = WdRows{pr.starts[r], pr.starts[last + 1], 0, 0};
+        } else {
+            wr = WdRows{pr.starts[r], n, 0, pr.starts[last - G + 1]};
         }
     }
     auto launch = [&](int64_t c_lo, int64_t c_hi, bool want_dist, bool want_acc, bool want_codes) {
@@ -836,11 +831,9 @@ void launch_dist_tensor(fs_dataset *ds, const WorkSet &ws, int64_t r0_internal, 
     // is the trivial case; with peers configured (fs_dataset_set_peers) this rank's rows must be
     // exactly its shard and Dd its exported slab.  An incremental update across ranks stays
     // non-symmetric (it would need remote read-modify-writes).
-    const char *env = getenv("FS_B200_SYMMETRIC");
-    const bool allow = contiguous && !(env && env[0] == '0');
     DistPeers peers{};
     bool symmetric = false;
-    if (allow && ds->peers_on && Dd == ds->peer_slab && r0_internal == ds->peers.starts[ds->peers.rank] &&
+    if (contiguous && ds->peers_on && Dd == ds->peer_slab && r0_internal == ds->peers.starts[ds->peers.rank] &&
         R == ds->peers.starts[ds->peers.rank + 1] - ds->peers.starts[ds->peers.rank] && !incr) {
         peers = ds->peers;
         symmetric = true;
@@ -853,12 +846,11 @@ void launch_dist_tensor(fs_dataset *ds, const WorkSet &ws, int64_t r0_internal, 
         peers.sb_base[0] = 0;
         peers.sb_base[1] = (int32_t)ceil_div(ds->n, 256);
         peers.coarse_shift = 3;                 // groups of 8 super-blocks = one rasterisation band of 16 tiles
-        symmetric = allow && r0_internal == 0 && R == ds->n;
+        symmetric = contiguous && r0_internal == 0 && R == ds->n;
     }
     const CUtensorMap ta = make_tmap_u8_sw128(a_rows, K, R, K, 128);
-    const CUtensorMap tb = make_tmap_u8_sw128(Wop, K, ds->n, K, 256);
-    const CUtensorMap tbh = make_tmap_u8_sw128(Wop, K, ds->n, K, 128);      // CTA pairs: each CTA stages half of the sample rows
-    launch_tc_dist(ta, tb, &tbh, K, sop, d_row_ids, R, ds->n, ldn, symmetric, incr, peers, st, launches, ops);
+    const CUtensorMap tb = make_tmap_u8_sw128(Wop, K, ds->n, K, 128);       // each CTA of a pair stages half of the sample rows
+    launch_tc_dist(ta, tb, K, sop, d_row_ids, R, ds->n, ldn, symmetric, incr, peers, st, launches, ops);
     ds->last_dist_exchanged = symmetric && peers.world > 1;
 }
 
@@ -956,23 +948,22 @@ void launch_accum_tensor(fs_dataset *ds, const WorkSet &ws, int algo, const int6
     CUtensorMap tat = make_tmap_u8_sw128(ws.At.ptr, row_bytes, (uint64_t)ws.Ka, (uint64_t)(ws.ldt / 2), 128);
     CUtensorMap tmh = make_tmap_u8_sw128(mask_h, row_bytes, (uint64_t)R, (uint64_t)(ldn / 2), 240);
     CUtensorMap tmm = make_tmap_u8_sw128(mask_m, row_bytes, (uint64_t)R, (uint64_t)(ldn / 2), 240);
-    // every column with exactly three values: one-hot rows 2c, 2c + 1 are column c's two planes.  Default: the
-    // merged-plane epilogue, whose operands are staged in a permuted row order (tc_accum.cu): At rows as
-    // (column mod 8, plane, column / 8), mask rows as (e, j, g, chunk) with row strides 1, 4, 2, 16 -- the box of a
-    // tile may run up to 239 rows past the tile's first row, hence the padding behind both masks.
+    // every column with exactly three values: one-hot rows 2c, 2c + 1 are column c's two planes.  Default (3): the
+    // merged-plane kernel as clusters of two CTAs (cta_group::2), whose operands are staged in a permuted row order
+    // (tc_accum.cu): At rows as (column mod 8, plane, column / 8), mask rows as (e, j, g, chunk) with row strides
+    // 1, 4, 2, 16 -- tiles of <= 224 rows, every CTA stages half of a tile's chunks (box of 7); the box of a tile
+    // may run up to 223 rows past the tile's first row, hence the padding behind both masks.
     // FS_B200_ACCUM_PAIR = 1: paired epilogue (planes meet by shuffle), 0: one thread per one-hot row.
-    // 3 (default): the merged-plane kernel as clusters of two CTAs (cta_group::2): tiles of <= 224 rows, every CTA
-    // stages half of a tile's chunks (box of 7)
     // (the merged kernel's per-column 64-bit sums need n^2 * 2^27 < 2^63)
     int pair_mode = ws.all_v3 ? (n < (1 << 17) ? 3 : 1) : 0;
     if (const char *e = getenv("FS_B200_ACCUM_PAIR"))
-        if (ws.all_v3 && e[0] >= '0' && e[0] <= (n < (1 << 17) ? '3' : '1')) pair_mode = e[0] - '0';
-    if (pair_mode >= 2) {
+        if (ws.all_v3 && (e[0] == '0' || e[0] == '1' || (e[0] == '3' && n < (1 << 17)))) pair_mode = e[0] - '0';
+    if (pair_mode == 3) {
         const uint64_t pa_b = (uint64_t)(ws.ldt / 2), pm_b = (uint64_t)(ldn / 2);
         const uint64_t da[4] = {row_bytes, 8, 2, (uint64_t)(ws.Ka / 16)}, sa[3] = {2 * pa_b, pa_b, 16 * pa_b};
         const uint32_t ba[4] = {128, 8, 2, 8};
-        const uint64_t dm[5] = {row_bytes, (uint64_t)R, 4, 2, pair_mode == 3 ? 14u : 15u}, sm[4] = {pm_b, 4 * pm_b, 2 * pm_b, 16 * pm_b};
-        const uint32_t bm[5] = {128, 2, 4, 2, pair_mode == 3 ? 7u : 15u};
+        const uint64_t dm[5] = {row_bytes, (uint64_t)R, 4, 2, 14}, sm[4] = {pm_b, 4 * pm_b, 2 * pm_b, 16 * pm_b};
+        const uint32_t bm[5] = {128, 2, 4, 2, 7};
         const bool ok = make_tmap_u8_sw128_nd(&tat, ws.At.ptr, 4, da, sa, ba) && make_tmap_u8_sw128_nd(&tmh, mask_h, 5, dm, sm, bm) &&
                         make_tmap_u8_sw128_nd(&tmm, mask_m, 5, dm, sm, bm);
         if (!ok) {   // the driver refused a permuted map: the 2-D maps above and the paired epilogue still apply

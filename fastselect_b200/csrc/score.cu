@@ -13,7 +13,6 @@
 namespace fs {
 
 // tensor path (onehot.cu / tc_dist.cu / tc_accum.cu)
-bool tensor_path_available();
 void launch_dist_tensor(fs_dataset *ds, const WorkSet &ws, int64_t r0_internal, const int64_t *h_row_ids,
                         const int64_t *d_row_ids, bool contiguous, int64_t R, int32_t *Dd, int64_t ldn,
                         cudaStream_t st, int *launches, double *ops);
@@ -74,8 +73,6 @@ static void run_pipeline(fs_dataset *ds, int algo, int use_star, int32_t k, cons
     double ops_dist = 0.0, ops_accum = 0.0;
     PhaseTimer timer(stats != nullptr, st);
 
-    const char *env_t = getenv("FS_B200_TENSOR");
-    const bool allow_tensor = tensor_path_available() && !(env_t && env_t[0] == '0');
     const int64_t ldn = round_up(n, 128);
     // Multi-GPU group call: this rank scores exactly its shard of the target rows, every rank does the
     // same with the same arguments, and the shard fits one chunk on every rank (the decision must be
@@ -101,7 +98,7 @@ static void run_pipeline(fs_dataset *ds, int algo, int use_star, int32_t k, cons
     if (!slab_cacheable) ds->dd_valid = false;
     timer.begin(&fs_stats::ms_gather);
     const auto prep0 = std::chrono::steady_clock::now();
-    build_workset(ds, feat_idx, n_kept, allow_tensor, algo == FS_RELIEFF, targets[0], (int64_t)targets.size(),
+    build_workset(ds, feat_idx, n_kept, algo == FS_RELIEFF, targets[0], (int64_t)targets.size(),
                   contiguous, slab_cacheable, want_split, group_call, true, &launches);
     const double ms_prep = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - prep0).count();
     timer.end();
@@ -126,7 +123,7 @@ static void run_pipeline(fs_dataset *ds, int algo, int use_star, int32_t k, cons
             if (ds->dd_valid && ws.dist_mode != kDistFull) {
                 ds->dd_valid = false;
                 ds->ws.valid = false;
-                build_workset(ds, feat_idx, n_kept, allow_tensor, algo == FS_RELIEFF, targets[0], (int64_t)targets.size(),
+                build_workset(ds, feat_idx, n_kept, algo == FS_RELIEFF, targets[0], (int64_t)targets.size(),
                               contiguous, slab_cacheable, want_split, group_call, true, &launches);
             }
             ds->dd_valid = false;

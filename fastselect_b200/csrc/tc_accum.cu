@@ -77,12 +77,8 @@ constexpr int SF_COL = 2 * BN;            // 8 columns of UE8M0 1.0 (0x7f) for b
 // CTA pairs (merged-plane kernel): tiles of <= 224 target rows, each CTA stages half of them (7 chunks of 16)
 constexpr int CG2_BN = 224;
 constexpr int CG2_B_BYTES = (CG2_BN / 2) * BK;   // 14 KB
-#ifndef FS_CG2_STAGES
-#define FS_CG2_STAGES 6
-#endif
-constexpr int CG2_STAGES = FS_CG2_STAGES;
+constexpr int CG2_STAGES = 6;
 constexpr int CG2_SMEM_BYTES = CG2_STAGES * (A_BYTES + CG2_B_BYTES) + 1024 + BAR_BYTES;
-constexpr int MERGED_SMEM_BYTES = STAGES * STAGE_BYTES + 1024 + BAR_BYTES;
 static_assert(CG2_B_BYTES % 1024 == 0 && CG2_SMEM_BYTES <= 232448, "pair stage shape");
 
 // A tile of target rows and the K blocks (of 128 samples) its two masks can be non-zero in:
@@ -141,7 +137,7 @@ __global__ void __launch_bounds__(256) accum_consts_kernel(const TileDesc *__res
     }
     limbs[(size_t)blockIdx.x * 256 + e] = coef_limbs(c);
     // the paired epilogue works on the FP32 accumulators directly: |rs| <= n < 2^22 is exact in float;
-    // the merged-plane epilogue (mode 2) wants it with the float -> int bias already added
+    // the merged-plane epilogue (rsum_as_float = 2) wants it with the float -> int bias already added
     rsum[(size_t)blockIdx.x * 256 + e] =
         rsum_as_float == 2 ? __float_as_int((float)rs + 12582912.0f) : (rsum_as_float ? __float_as_int((float)rs) : rs);
 }
@@ -508,19 +504,12 @@ struct ChunkConsts {
 };
 
 //
-// kCg2: the kernel runs as CLUSTERS OF TWO CTAs (tcgen05.mma.cta_group::2, M = 256): the pair takes two adjacent
+// The kernel runs as CLUSTERS OF TWO CTAs (tcgen05.mma.cta_group::2, M = 256): the pair takes two adjacent
 // blocks of 128 one-hot rows through the same tiles; each CTA stages its own At block and HALF of the mask
 // tile (chunks [0, nch / 2) or [nch / 2, nch), N rounded up to 32), the leader issues the MMAs for both and waits
-// for both epilogues.  The single-CTA kernel moves 46 KB from L2 into shared memory per four MMAs -- with
+// for both epilogues.  One CTA staging a whole tile moved 46 KB from L2 into shared memory per four MMAs -- with
 // the epilogue switched off it still ran C3 in 1.12 ms against 0.78 ms of MMA time (18.5 TB/s out of L2 over the
 // GPU: the same ceiling the distance GEMM hit before it became CTA pairs) -- the pair moves 30 KB.
-#ifdef FS_ACCUM_EXPERIMENTS
-#define FS_EXP(bit) ((kExp & (bit)) != 0)
-template <bool kCg2, int kExp>
-#else
-#define FS_EXP(bit) false
-template <bool kCg2>
-#endif
 __global__ void __launch_bounds__(M_THREADS, 1)
 tc_accum_merged_kernel(const __grid_constant__ CUtensorMap tmap_at, const __grid_constant__ CUtensorMap tmap_mh,
                        const __grid_constant__ CUtensorMap tmap_mm, int num_k_blocks, int64_t R,
@@ -530,9 +519,8 @@ tc_accum_merged_kernel(const __grid_constant__ CUtensorMap tmap_at, const __grid
                        const uint32_t *__restrict__ krow, int64_t K_rows, double *__restrict__ tpartial) {
     extern __shared__ __align__(1024) unsigned char smem_raw[];
     unsigned char *smem = smem_raw + ((1024u - (tc::smem_u32(smem_raw) & 1023u)) & 1023u);
-    constexpr int kStages = kCg2 ? CG2_STAGES : STAGES;
-    constexpr int kBBytes = kCg2 ? CG2_B_BYTES : B_BYTES;            // mask rows this CTA stages per K block
-    constexpr int kStageBytes = A_BYTES + kBBytes;
+    constexpr int kStages = CG2_STAGES;
+    constexpr int kStageBytes = A_BYTES + CG2_B_BYTES;               // At block + the mask rows this CTA stages per K block
     uint64_t *full_bar = reinterpret_cast<uint64_t *>(smem + kStages * kStageBytes);
     uint64_t *empty_bar = full_bar + kStages;
     uint64_t *tfull_bar = empty_bar + kStages;    // [2] accumulator buffer ready
@@ -540,15 +528,15 @@ tc_accum_merged_kernel(const __grid_constant__ CUtensorMap tmap_at, const __grid
     uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(tempty_bar + 2);
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    // pairs: both CTAs of a cluster walk the same units; the CTA's block of one-hot rows is 2 * (u / groups) + rank
-    const uint32_t crank = kCg2 ? tc::cluster_ctarank() : 0u;
-    const int worker = kCg2 ? (int)(blockIdx.x >> 1) : (int)blockIdx.x;
-    const int workers = kCg2 ? (int)(gridDim.x >> 1) : (int)gridDim.x;
+    // both CTAs of a cluster walk the same units; the CTA's block of one-hot rows is 2 * (u / groups) + rank
+    const uint32_t crank = tc::cluster_ctarank();
+    const int worker = (int)(blockIdx.x >> 1);
+    const int workers = (int)(gridDim.x >> 1);
     // work units: (block of one-hot rows, group of tiles), walked in bands of `group_span` groups: inside a band the
     // blocks advance slowest-varying-last (unit = band, block, group within band), so that the workers running at one
     // time cover group_span groups x (workers / group_span) blocks -- their mask tiles AND their At rows stay in L2
     // (group_span = groups: all groups of a block together; 1: one group for all workers)
-    const int m_units = kCg2 ? (m_blocks + 1) / 2 : m_blocks;
+    const int m_units = (m_blocks + 1) / 2;
     const int units = m_units * groups;
     const int band_units = m_units * group_span;
     auto unit_block = [&](int u, int &g) {
@@ -568,18 +556,15 @@ tc_accum_merged_kernel(const __grid_constant__ CUtensorMap tmap_at, const __grid
         }
         for (int b = 0; b < 2; ++b) {
             tc::mbar_init(&tfull_bar[b], 1);
-            // single CTA: every epilogue thread arrives; pairs: one lane per epilogue warp of BOTH CTAs
-            tc::mbar_init(&tempty_bar[b], kCg2 ? 2 * M_EPI_WARPS : 32 * M_EPI_WARPS);
+            // one lane per epilogue warp of BOTH CTAs arrives
+            tc::mbar_init(&tempty_bar[b], 2 * M_EPI_WARPS);
         }
         tc::fence_barrier_init();
     }
-    if (warp == MMA_WARP) {
-        if constexpr (kCg2) tc::tmem_alloc_pair<TMEM_COLS>(tmem_slot);
-        else tc::tmem_alloc<TMEM_COLS>(tmem_slot);
-    }
+    if (warp == MMA_WARP) tc::tmem_alloc_pair<TMEM_COLS>(tmem_slot);
     tc::tc_fence_before();
     __syncthreads();
-    if constexpr (kCg2) tc::cluster_sync_all();       // the peer's barriers exist before anything signals them
+    tc::cluster_sync_all();                           // the peer's barriers exist before anything signals them
     tc::tc_fence_after();
     // the kernel owns ALL 512 TMEM columns, so the allocation starts at column 0, lane 0: a constant the compiler
     // can keep in uniform registers (checked here, trapped otherwise)
@@ -591,7 +576,7 @@ tc_accum_merged_kernel(const __grid_constant__ CUtensorMap tmap_at, const __grid
     }
     tc::tc_fence_before();
     __syncthreads();
-    if constexpr (kCg2) tc::cluster_sync_all();       // both CTAs' scale factors are in place before the leader issues
+    tc::cluster_sync_all();                           // both CTAs' scale factors are in place before the leader issues
     tc::tc_fence_after();
 
     if (warp == PRODUCER_WARP) {
@@ -603,12 +588,12 @@ tc_accum_merged_kernel(const __grid_constant__ CUtensorMap tmap_at, const __grid
             for (int u = worker; u < units; u += workers) {
                 int g;
                 const int ub = unit_block(u, g);
-                const int m0 = (ub * (kCg2 ? 2 : 1) + (int)crank) * BM;
+                const int m0 = (ub * 2 + (int)crank) * BM;
                 const int tile_end = (g + 1) * group_tiles < num_tiles ? (g + 1) * group_tiles : num_tiles;
                 for (int t = g * group_tiles; t < tile_end; ++t) {
                     const TileDesc d = tt.t[t];
-                    // pairs: this CTA's half of the tile's chunks of 16 target rows (N is a multiple of 32)
-                    const int c_half = kCg2 ? (int)crank * ((d.rows + 31) >> 5) : 0;
+                    // this CTA's half of the tile's chunks of 16 target rows (N is a multiple of 32)
+                    const int c_half = (int)crank * ((d.rows + 31) >> 5);
                     for (int phase = 0; phase < 2; ++phase) {
                         const CUtensorMap *tm = phase == 0 ? &tmap_mh : &tmap_mm;
                         int kb = phase == 0 ? d.hb0 : (d.ib0 > 0 ? 0 : d.ib1);
@@ -619,18 +604,10 @@ tc_accum_merged_kernel(const __grid_constant__ CUtensorMap tmap_at, const __grid
                             ++it;
                             tc::mbar_wait(&empty_bar[s], ph ^ 1);
                             unsigned char *st = smem + s * kStageBytes;
-                            if (FS_EXP(16)) {      // experiment: no operand traffic at all
-                                if (crank == 0) tc::mbar_arrive(&full_bar[s]);
-                            } else if constexpr (kCg2) {
-                                // both CTAs' bytes are credited to the LEADER's barrier
-                                if (crank == 0) tc::mbar_arrive_expect_tx(&full_bar[s], 2 * kStageBytes);
-                                tc::tma_load_4d_pair(st, &tmap_at, &full_bar[s], kb * BK, 0, 0, m0 >> 4);
-                                tc::tma_load_5d_pair(st + A_BYTES, tm, &full_bar[s], kb * BK, d.row0, 0, 0, c_half);
-                            } else {
-                                tc::mbar_arrive_expect_tx(&full_bar[s], kStageBytes);
-                                tc::tma_load_4d(st, &tmap_at, &full_bar[s], kb * BK, 0, 0, m0 >> 4);
-                                tc::tma_load_5d(st + A_BYTES, tm, &full_bar[s], kb * BK, d.row0, 0, 0, 0);
-                            }
+                            // both CTAs' bytes are credited to the LEADER's barrier
+                            if (crank == 0) tc::mbar_arrive_expect_tx(&full_bar[s], 2 * kStageBytes);
+                            tc::tma_load_4d_pair(st, &tmap_at, &full_bar[s], kb * BK, 0, 0, m0 >> 4);
+                            tc::tma_load_5d_pair(st + A_BYTES, tm, &full_bar[s], kb * BK, d.row0, 0, 0, c_half);
                             ++kb;
                             if (phase == 1 && kb == d.ib0) kb = d.ib1;
                         }
@@ -639,7 +616,7 @@ tc_accum_merged_kernel(const __grid_constant__ CUtensorMap tmap_at, const __grid
             }
         }
     } else if (warp == MMA_WARP) {
-        // ===== MMA issuer: one thread (pairs: of the leader CTA, for both).  Everything the tcgen05 instructions
+        // ===== MMA issuer: one thread of the leader CTA, for both.  Everything the tcgen05 instructions
         // take is derived from kernel parameters (the tile table is one) and loop counters, so that it stays in
         // uniform registers: with the table in shared memory every tcgen05.mma was wrapped in an elect / broadcast
         // sequence of ~20 instructions and the issuing thread, not the tensor pipe, set the pace. =====
@@ -651,8 +628,7 @@ tc_accum_merged_kernel(const __grid_constant__ CUtensorMap tmap_at, const __grid
                 const int tile_end = (g + 1) * group_tiles < num_tiles ? (g + 1) * group_tiles : num_tiles;
                 for (int t = g * group_tiles; t < tile_end; ++t) {
                     const TileDesc d = tt.t[t];
-                    const uint32_t idesc = kCg2 ? tc::make_idesc_mxf4(2 * BM, ((d.rows + 31) >> 5) << 5)
-                                                : tc::make_idesc_mxf4(BM, ((d.rows + 15) >> 4) << 4);
+                    const uint32_t idesc = tc::make_idesc_mxf4(2 * BM, ((d.rows + 31) >> 5) << 5);
                     for (int phase = 0; phase < 2; ++phase) {
                         const int nblk = phase == 0 ? d.hb1 - d.hb0 : d.ib0 + (num_k_blocks - d.ib1);
                         if (nblk == 0) continue;
@@ -674,20 +650,13 @@ tc_accum_merged_kernel(const __grid_constant__ CUtensorMap tmap_at, const __grid
                             const uint64_t db = tc::make_smem_desc_sw128(sa + A_BYTES);
 #pragma unroll
                             for (int k = 0; k < BK / 32; ++k) {
-                                if (FS_EXP(16)) break;
-                                if constexpr (kCg2)
-                                    tc::mma_mxf4_pair(acc, da + (uint64_t)(2 * k), db + (uint64_t)(2 * k), idesc, tmem_base + SF_COL,
-                                                      tmem_base + SF_COL, have);
-                                else
-                                    tc::mma_mxf4(acc, da + (uint64_t)(2 * k), db + (uint64_t)(2 * k), idesc, tmem_base + SF_COL,
-                                                 tmem_base + SF_COL, have);
+                                tc::mma_mxf4_pair(acc, da + (uint64_t)(2 * k), db + (uint64_t)(2 * k), idesc, tmem_base + SF_COL,
+                                                  tmem_base + SF_COL, have);
                                 have = 1;
                             }
-                            if constexpr (kCg2) tc::tc_commit_pair(&empty_bar[s]);
-                            else tc::tc_commit(&empty_bar[s]);
+                            tc::tc_commit_pair(&empty_bar[s]);
                         }
-                        if constexpr (kCg2) tc::tc_commit_pair(&tfull_bar[buf]);
-                        else tc::tc_commit(&tfull_bar[buf]);
+                        tc::tc_commit_pair(&tfull_bar[buf]);
                     }
                 }
             }
@@ -704,12 +673,8 @@ tc_accum_merged_kernel(const __grid_constant__ CUtensorMap tmap_at, const __grid
         // hand an accumulator buffer back to the MMA issuer (this thread's TMEM loads have completed)
         auto release_acc = [&](uint64_t *bar) {
             tc::tc_fence_before();
-            if constexpr (kCg2) {
-                __syncwarp();
-                if (lane == 0) tc::mbar_arrive_cluster_relaxed(bar, 0);   // no memory fence: TMEM reads are ordered by tcgen05.fence
-            } else {
-                tc::mbar_arrive(bar);
-            }
+            __syncwarp();
+            if (lane == 0) tc::mbar_arrive_cluster_relaxed(bar, 0);   // no memory fence: TMEM reads are ordered by tcgen05.fence
         };
         int item = 0;
         for (int u = worker; u < units; u += workers) {
@@ -717,23 +682,20 @@ tc_accum_merged_kernel(const __grid_constant__ CUtensorMap tmap_at, const __grid
             const int ub = unit_block(u, g);
             const int tile_end = (g + 1) * group_tiles < num_tiles ? (g + 1) * group_tiles : num_tiles;
             // this thread's two columns: the tile's columns (2q + h) * 8 + r8, h = 0, 1 (lane offsets 0, 16)
-            const int64_t mrow0 = (int64_t)(ub * (kCg2 ? 2 : 1) + (int)crank) * BM + 2 * ((2 * q) * 8 + r8);
+            const int64_t mrow0 = (int64_t)(ub * 2 + (int)crank) * BM + 2 * ((2 * q) * 8 + r8);
             const int64_t mrow1 = mrow0 + 16;
             const uint8_t *at0 = codesT + (int64_t)((mrow0 < K_rows ? krow[mrow0] : 0u) & 0xffffffu) * ldt;
             const uint8_t *at1 = codesT + (int64_t)((mrow1 < K_rows ? krow[mrow1] : 0u) & 0xffffffu) * ldt;
             unsigned long long ah0 = 0, al0 = 0, ah1 = 0, al1 = 0;   // exact fixed-point sums, one pair per column
             for (int t = g * group_tiles; t < tile_end; ++t) {
                 const TileDesc d = tt.t[t];
-                const int nch = kCg2 ? ((d.rows + 31) >> 5) << 1 : (d.rows + 15) >> 4;   // chunks of 16 targets in this tile
+                const int nch = ((d.rows + 31) >> 5) << 1;   // chunks of 16 targets in this tile (N rounded up to 32)
                 const int n_my = nch > part ? (nch - part + M_PARTS - 1) / M_PARTS : 0;   // this part's chunks: part, part + M_PARTS, ...
                 // value codes of the thread's targets in its two columns: one word per chunk and column
                 // (issued before the accumulator wait; shared by both phases).  Targets beyond the tile's
                 // rows get whatever follows: their coefficient is 0.
                 uint32_t oh0[M_CHUNKS], oh1[M_CHUNKS];
-                if (FS_EXP(1)) {
-#pragma unroll
-                    for (int i = 0; i < M_CHUNKS; ++i) { oh0[i] = 0x00010200u; oh1[i] = 0x02000100u; }
-                } else if (contiguous) {
+                if (contiguous) {
                     const int64_t a0 = ids0 + d.row0 + 16 * part + 4 * j;   // chunk i: + 16 M_PARTS i
                     if ((a0 & 3) == 0) {
 #pragma unroll
@@ -781,9 +743,7 @@ tc_accum_merged_kernel(const __grid_constant__ CUtensorMap tmap_at, const __grid
                     const int2 *s_c = limbs + ((size_t)t * 2 + phase) * 256 + 16 * part + 4 * j;
                     const float *s_rs = reinterpret_cast<const float *>(rsum) + ((size_t)t * 2 + phase) * 256 + 16 * part + 4 * j;
                     ChunkConsts kc{}, kn{};
-                    if (FS_EXP(2)) {
-                        kc.ca = make_int4(3, 5, 7, 9); kc.cb = make_int4(11, 13, 15, 17); kc.rs = make_float4(kMagic, kMagic, kMagic, kMagic);
-                    } else if (n_my > 0) {
+                    if (n_my > 0) {
                         kc.ca = __ldg(reinterpret_cast<const int4 *>(s_c));
                         kc.cb = __ldg(reinterpret_cast<const int4 *>(s_c + 2));
                         kc.rs = __ldg(reinterpret_cast<const float4 *>(s_rs));
@@ -794,10 +754,6 @@ tc_accum_merged_kernel(const __grid_constant__ CUtensorMap tmap_at, const __grid
                     const uint32_t tacc = tquarter + (uint32_t)(buf * BN + 16 * part);   // chunk i: + 16 M_PARTS i
                     // v[buffer][column h][group g of 8 TMEM columns][r0..r3]
                     uint32_t v[2][2][2][4];
-                    if (FS_EXP(8)) {
-                        release_acc(&tempty_bar[buf]);
-                        continue;
-                    }
                     if (n_my > 0) {
                         tc::tmem_ld_16x256b(tacc, v[0][0][0]);
                         tc::tmem_ld_16x256b(tacc + 8, v[0][0][1]);
@@ -818,11 +774,9 @@ tc_accum_merged_kernel(const __grid_constant__ CUtensorMap tmap_at, const __grid
                                 tc::tmem_ld_16x256b(ta + 8, vn[0][1]);
                                 tc::tmem_ld_16x256b(ta + (16u << 16), vn[1][0]);
                                 tc::tmem_ld_16x256b(ta + (16u << 16) + 8, vn[1][1]);
-                                if (!FS_EXP(2)) {
                                 kn.ca = __ldg(reinterpret_cast<const int4 *>(s_c + 16 * M_PARTS * (i + 1)));
                                 kn.cb = __ldg(reinterpret_cast<const int4 *>(s_c + 16 * M_PARTS * (i + 1) + 2));
                                 kn.rs = __ldg(reinterpret_cast<const float4 *>(s_rs + 16 * M_PARTS * (i + 1)));
-                                }
                             } else {
                                 // the last chunk is in registers: the MMA issuer may reuse the buffer
                                 release_acc(&tempty_bar[buf]);
@@ -830,13 +784,6 @@ tc_accum_merged_kernel(const __grid_constant__ CUtensorMap tmap_at, const __grid
                             const int chi[4] = {kc.ca.x, kc.ca.z, kc.cb.x, kc.cb.z};
                             const int clo[4] = {kc.ca.y, kc.ca.w, kc.cb.y, kc.cb.w};
                             const float rsb[4] = {kc.rs.x, kc.rs.y, kc.rs.z, kc.rs.w};
-                            if (FS_EXP(4)) {
-#pragma unroll
-                                for (int b = 0; b < 4; ++b) {
-                                    ah0 += vc[0][b >> 1][b & 1] ^ vc[0][b >> 1][2 + (b & 1)] ^ (uint32_t)chi[b] ^ oh0[i];
-                                    ah1 += vc[1][b >> 1][b & 1] ^ vc[1][b >> 1][2 + (b & 1)] ^ (uint32_t)clo[b] ^ oh1[i] ^ __float_as_uint(rsb[b]);
-                                }
-                            } else
 #pragma unroll
                             for (int h = 0; h < 2; ++h) {
                                 const uint32_t w = h == 0 ? oh0[i] : oh1[i];
@@ -891,11 +838,10 @@ tc_accum_merged_kernel(const __grid_constant__ CUtensorMap tmap_at, const __grid
         }
     }
     __syncthreads();
-    if constexpr (kCg2) tc::cluster_sync_all();       // neither CTA leaves (or frees TMEM) while the pair is in flight
+    tc::cluster_sync_all();                           // neither CTA leaves (or frees TMEM) while the pair is in flight
     if (warp == MMA_WARP) {
         tc::tc_fence_after();
-        if constexpr (kCg2) tc::tmem_dealloc_pair<TMEM_COLS>(tmem_base);
-        else tc::tmem_dealloc<TMEM_COLS>(tmem_base);
+        tc::tmem_dealloc_pair<TMEM_COLS>(tmem_base);
     }
 }
 
@@ -959,68 +905,44 @@ int launch_tc_accum(const CUtensorMap &tmap_at, const CUtensorMap &tmap_mh, cons
                     int64_t ldt, const uint32_t *krow, int64_t K_rows, DevBuf<double> &tpartial, int32_t *d_tiles,
                     DevBuf<int32_t> &consts, cudaStream_t st, int *launches, const int64_t *h_ids, const int32_t *h_y,
                     const int64_t *h_cls_start, double *ops) {
-    // pair_mode 1 / 2 / 3: every column owns exactly two one-hot rows (2c, 2c + 1): paired epilogue (planes meet by
-    // shuffle), merged-plane epilogue (planes meet in one thread; the caller built the permuted tensor maps), and
-    // the merged-plane kernel as clusters of two CTAs (cta_group::2; tiles of <= 224 rows)
-    const bool cg2 = pair_mode == 3;
-#ifdef FS_ACCUM_EXPERIMENTS
-    // diagnostic build (-DFS_ACCUM_EXPERIMENTS): FS_B200_ACCUM_EXP compiles parts of the merged kernel out --
-    // 1 no value-code loads, 2 no constants loads, 4 no arithmetic, 8 epilogue only waits and arrives, 16 no operand
-    // traffic and no MMAs (sums of these as listed); the results are then wrong on purpose
-    // (profiles/r02_accum_kernel_experiments.txt)
-    int exp_mode = 0;
-    if (const char *e = getenv("FS_B200_ACCUM_EXP")) exp_mode = atoi(e);
-#define FS_PICK(c) (exp_mode == 8 ? tc_accum_merged_kernel<c, 8> : exp_mode == 16 ? tc_accum_merged_kernel<c, 16> : \
-                    exp_mode == 17 ? tc_accum_merged_kernel<c, 17> : exp_mode == 18 ? tc_accum_merged_kernel<c, 18> : \
-                    exp_mode == 20 ? tc_accum_merged_kernel<c, 20> : exp_mode == 23 ? tc_accum_merged_kernel<c, 23> : \
-                    exp_mode == 24 ? tc_accum_merged_kernel<c, 24> : tc_accum_merged_kernel<c, 0>)
-    auto merged = cg2 ? FS_PICK(true) : FS_PICK(false);
-#undef FS_PICK
-#else
-    auto merged = cg2 ? tc_accum_merged_kernel<true> : tc_accum_merged_kernel<false>;
-#endif
+    // pair_mode 1 / 3: every column owns exactly two one-hot rows (2c, 2c + 1): paired epilogue (planes meet by
+    // shuffle), or the merged-plane kernel as clusters of two CTAs (planes meet in one thread; cta_group::2; tiles of
+    // <= 224 rows; the caller built the permuted tensor maps).  0: one thread per one-hot row.
+    const bool merged = pair_mode == 3;
     auto kernel = pair_mode == 1 ? tc_accum_kernel<true> : tc_accum_kernel<false>;
-    const int smem_bytes = pair_mode >= 2 ? (cg2 ? CG2_SMEM_BYTES : MERGED_SMEM_BYTES) : SMEM_BYTES;
-    if (pair_mode >= 2) FS_CUDA(cudaFuncSetAttribute(merged, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes));
+    const int smem_bytes = merged ? CG2_SMEM_BYTES : SMEM_BYTES;
+    if (merged) FS_CUDA(cudaFuncSetAttribute(tc_accum_merged_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes));
     else FS_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes));
     int dev = 0, sms = 0;
     FS_CUDA(cudaGetDevice(&dev));
     FS_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
     FS_REQUIRE(n < (1LL << 22), FS_ERR_INVALID, "one-hot accumulation supports up to 2^22 samples (got %lld)", (long long)n);
-    const AccumPlan plan = make_plan(n, R, contiguous, h_ids, h_y, h_cls_start, cg2 ? CG2_BN : BN, cg2 ? 32 : 16);
+    const AccumPlan plan = make_plan(n, R, contiguous, h_ids, h_y, h_cls_start, merged ? CG2_BN : BN, merged ? 32 : 16);
     const int m_blocks = (int)ceil_div(K_rows, BM);
     // Tile groups.  Work units (128 one-hot rows x one group) are dealt round-robin, so the ~sms
     // units resident at one time span sms / groups one-hot row blocks, each streaming its own
     // 128 x n bytes of At again for every tile of the group: keep that footprint within about half
     // of L2 (else every re-read goes to HBM and the kernel turns DRAM-bound for large n) by
     // cutting the tiles into more, smaller groups of equal size.
-    // merged kernel: band of groups walked together (see the kernel); 0 = all groups of a block together
-    // Large n (the two masks, n^2 bytes, no longer fit L2): groups of two tiles walked in bands of twelve keep the
-    // mask tiles and the At rows of the ~74 running clusters inside L2 -- measured on a C5 cut (20 000 x 100 000):
-    // 226 -> 204 ms of accumulation per TuRF run (profiles/r02_accum_l2_blocking_c5cut.txt)
-    int group_span = 0, group_tiles_env = 0;
-    if (pair_mode >= 2 && n > 8192) {
-        group_span = 12;
-        group_tiles_env = 2;
-    }
-    if (const char *e = getenv("FS_B200_ACCUM_SPAN")) group_span = atoi(e);
-    if (const char *e = getenv("FS_B200_ACCUM_GROUP_TILES")) group_tiles_env = atoi(e);
+    // Merged kernel at large n (the two masks, n^2 bytes, no longer fit L2): groups of two tiles walked in bands of
+    // twelve (see the kernel) keep the mask tiles and the At rows of the ~74 running clusters inside L2 -- measured
+    // on a C5 cut (20 000 x 100 000): 226 -> 204 ms of accumulation per TuRF run
+    // (profiles/r02_accum_l2_blocking_c5cut.txt).  Otherwise all groups of a block are walked together.
+    const bool l2_bands = merged && n > 8192;
     auto groups_for = [&](int nt) {
+        if (l2_bands) return (int)ceil_div(nt, 2);
         const int64_t want = ceil_div((int64_t)sms * BM * (n / 2), (int64_t)60 << 20);   // At rows are n / 2 bytes
-        const int64_t g = std::max<int64_t>(ceil_div(nt, GROUP), std::min<int64_t>(nt, want));
-        if (pair_mode >= 2 && group_tiles_env > 0) return (int)ceil_div(nt, group_tiles_env);
-        return (int)g;
+        return (int)std::max<int64_t>(ceil_div(nt, GROUP), std::min<int64_t>(nt, want));
     };
-    const size_t max_tiles = pair_mode >= 2 ? MERGED_MAX_TILES : MAX_TILES;
+    const size_t max_tiles = merged ? MERGED_MAX_TILES : MAX_TILES;
     int total_groups = 0;
     for (size_t t0 = 0; t0 < plan.tiles.size(); t0 += max_tiles)
         total_groups += groups_for((int)std::min<size_t>(max_tiles, plan.tiles.size() - t0));
     // merged kernel: one pair of exact 64-bit sums per column for the whole call (zeroed here, finished below)
-    const int parts = pair_mode >= 2 ? 0 : PARTS;
-    tpartial.reserve(pair_mode >= 2 ? (size_t)K_rows + 2 : (size_t)total_groups * parts * K_rows);
-    if (pair_mode >= 2) FS_CUDA(cudaMemsetAsync(tpartial.ptr, 0, (size_t)K_rows * sizeof(double), st));
+    tpartial.reserve(merged ? (size_t)K_rows + 2 : (size_t)total_groups * PARTS * K_rows);
+    if (merged) FS_CUDA(cudaMemsetAsync(tpartial.ptr, 0, (size_t)K_rows * sizeof(double), st));
     int groups_done = 0;
-    // at most MAX_TILES tile descriptors per launch
+    // at most max_tiles tile descriptors per launch
     for (size_t t0 = 0; t0 < plan.tiles.size(); t0 += max_tiles) {
         const int nt = (int)std::min<size_t>(max_tiles, plan.tiles.size() - t0);
         // equal-sized groups (work units are dealt round-robin: unequal units would unbalance the SMs)
@@ -1032,31 +954,31 @@ int launch_tc_accum(const CUtensorMap &tmap_at, const CUtensorMap &tmap_mh, cons
         consts.reserve((size_t)nt * 2 * 256 * 3 + 512);   // slack: the epilogue prefetches one item ahead
         int2 *limbs = reinterpret_cast<int2 *>(consts.ptr);
         int32_t *rsum = consts.ptr + (size_t)nt * 2 * 256 * 2;
-        accum_consts_kernel<<<2 * nt, 256, 0, st>>>(reinterpret_cast<const TileDesc *>(d_tiles), nt, rinfo, limbs, rsum, pair_mode >= 2 ? 2 : pair_mode);
+        accum_consts_kernel<<<2 * nt, 256, 0, st>>>(reinterpret_cast<const TileDesc *>(d_tiles), nt, rinfo, limbs, rsum, merged ? 2 : pair_mode);
         ++*launches;
-        if (pair_mode >= 2) {
-            // single CTAs, or clusters of two CTAs: a cluster takes two adjacent blocks of one-hot rows through a
-            // group of tiles.  The tile table is a kernel parameter.
+        if (merged) {
+            // clusters of two CTAs: a cluster takes two adjacent blocks of one-hot rows through a group of tiles.
+            // The tile table is a kernel parameter.
             TileTable table;
             memcpy(table.t, plan.tiles.data() + t0, (size_t)nt * sizeof(TileDesc));
-            const int units = (cg2 ? (m_blocks + 1) / 2 : m_blocks) * groups;
-            const int workers = cg2 ? sms / 2 : sms;
+            const int units = (m_blocks + 1) / 2 * groups;
+            const int workers = sms / 2;
+            const int group_span = l2_bands && 12 < groups ? 12 : groups;
             cudaLaunchConfig_t cfg{};
-            cfg.gridDim = dim3((unsigned)((cg2 ? 2 : 1) * (units < workers ? units : workers)));
+            cfg.gridDim = dim3((unsigned)(2 * (units < workers ? units : workers)));
             cfg.blockDim = dim3(M_THREADS);
             cfg.dynamicSmemBytes = (size_t)smem_bytes;
             cfg.stream = st;
             cudaLaunchAttribute attr{};
             attr.id = cudaLaunchAttributeClusterDimension;
-            attr.val.clusterDim.x = cg2 ? 2 : 1;
+            attr.val.clusterDim.x = 2;
             attr.val.clusterDim.y = 1;
             attr.val.clusterDim.z = 1;
             cfg.attrs = &attr;
             cfg.numAttrs = 1;
-            FS_CUDA(cudaLaunchKernelEx(&cfg, merged, tmap_at, tmap_mh, tmap_mm, (int)ceil_div(n, KS), R, table, nt, groups,
-                                       group_tiles, m_blocks, group_span > 0 && group_span < groups ? group_span : groups, d_ids, contiguous ? 1 : 0, (const int2 *)limbs,
-                                       (const int32_t *)rsum, codesT, ldt, krow, K_rows,
-                                       tpartial.ptr + (size_t)groups_done * parts * K_rows));
+            FS_CUDA(cudaLaunchKernelEx(&cfg, tc_accum_merged_kernel, tmap_at, tmap_mh, tmap_mm, (int)ceil_div(n, KS), R, table,
+                                       nt, groups, group_tiles, m_blocks, group_span, d_ids, contiguous ? 1 : 0,
+                                       (const int2 *)limbs, (const int32_t *)rsum, codesT, ldt, krow, K_rows, tpartial.ptr));
         } else {
             const int units = m_blocks * groups;
             const int grid = units < sms ? units : sms;
@@ -1069,14 +991,14 @@ int launch_tc_accum(const CUtensorMap &tmap_at, const CUtensorMap &tmap_mh, cons
         ++*launches;
         groups_done += groups;
     }
-    if (ops) *ops += 2.0 * BM * BN * KS * plan.blocks * (double)(cg2 ? (m_blocks + 1) / 2 * 2 : m_blocks);
-    if (pair_mode >= 2) {
+    if (ops) *ops += 2.0 * BM * BN * KS * plan.blocks * (double)(merged ? (m_blocks + 1) / 2 * 2 : m_blocks);
+    if (merged) {
         merged_finish_kernel<<<(unsigned)ceil_div(K_rows / 2 + 1, 256), 256, 0, st>>>(tpartial.ptr, K_rows);
         FS_CUDA(cudaGetLastError());
         ++*launches;
         return 1;
     }
-    return parts * groups_done;
+    return PARTS * groups_done;
 }
 
 int tc_accum_tile_desc_ints() { return MAX_TILES * (int)(sizeof(TileDesc) / sizeof(int32_t)); }

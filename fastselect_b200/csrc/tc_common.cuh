@@ -50,24 +50,6 @@ __device__ __forceinline__ void tma_load_2d(void *smem_dst, const CUtensorMap *m
         : "memory");
 }
 
-// 4-D / 5-D tile loads: the outer box dimensions enumerate ROWS of the operand in a permuted order (the
-// accumulation kernel's merged-plane epilogue); c0 = coordinate along the contiguous (byte) dimension
-__device__ __forceinline__ void tma_load_4d(void *smem_dst, const CUtensorMap *m, uint64_t *bar, int32_t c0, int32_t c1,
-                                            int32_t c2, int32_t c3) {
-    asm volatile(
-        "cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];" ::"r"(
-            smem_u32(smem_dst)),
-        "l"(reinterpret_cast<uint64_t>(m)), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
-        : "memory");
-}
-__device__ __forceinline__ void tma_load_5d(void *smem_dst, const CUtensorMap *m, uint64_t *bar, int32_t c0, int32_t c1,
-                                            int32_t c2, int32_t c3, int32_t c4) {
-    asm volatile(
-        "cp.async.bulk.tensor.5d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6, %7}], [%2];" ::"r"(
-            smem_u32(smem_dst)),
-        "l"(reinterpret_cast<uint64_t>(m)), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "r"(c4)
-        : "memory");
-}
 // L2 prefetches: a 4-D tile of a tensor map, and a run of bytes (16-byte aligned, size a multiple of 16)
 __device__ __forceinline__ void tma_prefetch_4d(const CUtensorMap *m, int32_t c0, int32_t c1, int32_t c2, int32_t c3) {
     asm volatile("cp.async.bulk.prefetch.tensor.4d.L2.global [%0, {%1, %2, %3, %4}];" ::"l"(reinterpret_cast<uint64_t>(m)), "r"(c0),
@@ -237,7 +219,8 @@ __device__ __forceinline__ void tma_load_2d_pair(void *smem_dst, const CUtensorM
         "l"(reinterpret_cast<uint64_t>(m)), "r"(smem_u32(bar) & kLeaderMask), "r"(c0), "r"(c1)
         : "memory");
 }
-// the permuted 4-D / 5-D tile loads of the accumulation kernel, by either CTA of the pair
+// 4-D / 5-D tile loads, by either CTA of the pair: the outer box dimensions enumerate ROWS of the operand in a
+// permuted order (the accumulation kernel's merged-plane epilogue); c0 = coordinate along the contiguous (byte) dimension
 __device__ __forceinline__ void tma_load_4d_pair(void *smem_dst, const CUtensorMap *m, uint64_t *bar, int32_t c0, int32_t c1,
                                                  int32_t c2, int32_t c3) {
     asm volatile(

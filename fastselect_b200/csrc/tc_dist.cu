@@ -10,12 +10,18 @@
 // accumulation (tcgen05 kind::mxf4, twice the int8 rate): every product and every partial sum is a
 // small integer, so the FP32 accumulators are exact up to 2^24 and the distances are exact.
 //
-// Kernel: one CTA per 128 x 256 tile of D.  Warp 0 streams 128-byte-wide K slabs of
-// both operands with TMA (128B swizzle) through a 4-stage mbarrier ring; one elected
-// thread of warp 1 issues tcgen05.mma.cta_group::1.kind::mxf4 (M=128, N=256, K=64) into
-// a 256-column TMEM accumulator; warps 2-5 read the accumulator back with
-// tcgen05.ld (32 lanes x 32 columns per instruction), form s_i + s_j - acc and store
-// int32 rows (each thread writes whole 128-byte lines).
+// Kernel: one cluster of two CTAs (tcgen05 cta_group::2) per 256 x 256 super-block of D.  Warp 0
+// of each CTA streams 128-byte-wide K slabs of its own 128 target rows and of HALF of the 256
+// sample rows with TMA (128B swizzle) through a 6-stage mbarrier ring; one elected thread of the
+// leader CTA's warp 1 issues tcgen05.mma.cta_group::2.kind::mxf4 (M=256, N=256, K=64) for the
+// pair, which reads the B operand from both CTAs' shared memory, into a 256-column TMEM
+// accumulator; commits are multicast to both CTAs' barriers.  Warps 2-5 of each CTA read its 128
+// TMEM lanes back with tcgen05.ld (32 lanes x 32 columns per instruction), form s_i + s_j - acc
+// and store int32 rows (each thread writes whole 128-byte lines).
+// Pairs, because one CTA staging a whole 128 x 256 tile was bound by the operand feed from L2:
+// about 190 cycles per M128 N256 K64 MMA against the 128 that tools/fp4_peak.cu reaches from
+// resident operands.  Probed stand-alone first (tools/tc_dist_cg2_probe.cu,
+// profiles/r02_tc_dist_cg2_probe_run1.txt: exact).
 //
 // Symmetric mode.  D is symmetric, so when the target rows of all ranks together cover every
 // sample (one GPU scoring all rows, or one process per GPU each scoring its row shard) only
@@ -35,17 +41,17 @@
 namespace fs {
 
 namespace {
-constexpr int BM = 128;        // target rows per tile   (UMMA M)
-constexpr int BN = 256;        // sample columns per tile (UMMA N)
+constexpr int BM = 128;        // target rows per CTA (half of UMMA M)
+constexpr int BN = 256;        // sample columns per super-block (UMMA N)
 constexpr int BK = 128;        // bytes of K per stage (one swizzle atom)
-constexpr int STAGES = 4;
-constexpr int A_BYTES = BM * BK;   // 16 KB
-constexpr int B_BYTES = BN * BK;   // 32 KB
+constexpr int STAGES = 6;
+constexpr int A_BYTES = BM * BK;         // 16 KB
+constexpr int B_BYTES = (BN / 2) * BK;   // 16 KB: this CTA's half of the sample rows
 constexpr int SMEM_BYTES = STAGES * (A_BYTES + B_BYTES) + 1024 /*align*/ + 256 /*barriers*/;
 constexpr int THREADS = 192;
 constexpr int TMEM_COLS = 512;  // 256 accumulator columns + 8 scale-factor columns, rounded up to a power of two
 constexpr int SF_COL = BN;      // 8 columns of UE8M0 1.0 (0x7f): block scales of both operands
-constexpr int BAND = 16;        // row blocks per rasterisation band
+constexpr int BAND = 8;         // super-block rows per rasterisation band
 }  // namespace
 
 // Symmetric mode: is super-block (sb_i, sb_j) computed on the side that owns rows sb_i?  Exactly
@@ -140,152 +146,25 @@ __device__ __forceinline__ void dist_store_tile(uint32_t tmem_base, int q, int64
         }
 }
 
-__global__ void __launch_bounds__(THREADS, 1)
-tc_dist_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b,
-               int num_k_blocks, const int32_t *__restrict__ srow, const int64_t *__restrict__ ids, int64_t R,
-               int64_t n, int64_t ldd, int symmetric, int subtract, int tiles_y, int tiles_x,
-               const __grid_constant__ DistPeers peers) {
-    // L2-friendly rasterisation: bands of BAND row blocks, walked column by column, so that the
-    // ~148 concurrently resident tiles form a roughly square region and share their operand
-    // K-slabs through L2 (16 x 128 target rows and ~9 x 256 sample rows per wave) instead of
-    // streaming a different 256-row slab of the sample operand per tile.
-    int tile_y, tile_x;
-    {
-        const int lin = (int)blockIdx.x;
-        const int band = lin / (BAND * tiles_x);
-        const int band_rows = tiles_y - band * BAND < BAND ? tiles_y - band * BAND : BAND;
-        const int in_band = lin - band * BAND * tiles_x;
-        tile_y = band * BAND + in_band % band_rows;
-        tile_x = in_band / band_rows;
-    }
-    // column tile -> the rank that owns those samples as target rows, and the sample range.
-    // Column tiles are the 256-row super-blocks of every rank's shard, numbered globally.
-    int owner = 0;
-    while (owner + 1 < peers.world && tile_x >= peers.sb_base[owner + 1]) ++owner;
-    const int64_t n0 = peers.starts[owner] + (int64_t)(tile_x - peers.sb_base[owner]) * BN;
-    const int64_t cend = n0 + BN < peers.starts[owner + 1] ? n0 + BN : peers.starts[owner + 1];
-    // symmetric mode: checkerboard over super-blocks (see the header); sb_i = this tile's super-row
-    const int sb_i = peers.sb_base[peers.rank] + (tile_y >> 1), sb_j = tile_x;
-    const bool diagonal = sb_i == sb_j;
-    if (symmetric && !dist_row_side(sb_i, sb_j, peers.coarse_shift, peers.rank, owner, peers.world)) return;
-    const bool mirror = symmetric && !diagonal;
-    int32_t *Dd = peers.slab[peers.rank];                         // may alias Dm: no __restrict__
-    int32_t *Dm = peers.slab[owner];                  // slab that receives the transposed tile
-    const int64_t row_global0 = peers.starts[peers.rank];          // global sample index of slab row 0
-    extern __shared__ __align__(1024) unsigned char smem_raw[];
-    unsigned char *smem = reinterpret_cast<unsigned char *>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
-    unsigned char *smem_a = smem;
-    unsigned char *smem_b = smem + STAGES * A_BYTES;
-    uint64_t *full_bar = reinterpret_cast<uint64_t *>(smem + STAGES * (A_BYTES + B_BYTES));
-    uint64_t *empty_bar = full_bar + STAGES;
-    uint64_t *accum_bar = empty_bar + STAGES;
-    uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(accum_bar + 1);
-
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int m0 = tile_y * BM;
-
-    if (warp == 0 && lane == 0) {
-        tc::prefetch_tmap(&tmap_a);
-        tc::prefetch_tmap(&tmap_b);
-        for (int s = 0; s < STAGES; ++s) {
-            tc::mbar_init(&full_bar[s], 1);
-            tc::mbar_init(&empty_bar[s], 1);
-        }
-        tc::mbar_init(accum_bar, 1);
-        tc::fence_barrier_init();
-    }
-    if (warp == 1) tc::tmem_alloc<TMEM_COLS>(tmem_slot);
-    tc::tc_fence_before();
-    __syncthreads();
-    tc::tc_fence_after();
-    const uint32_t tmem_base = *tmem_slot;
-    if (warp >= 2) {
-        // block scale factors: 1.0 everywhere (warps 2..5 cover the four TMEM lane quarters)
-        for (int c = 0; c < 8; ++c) tc::tmem_st_32x1(tmem_base + ((uint32_t)((warp & 3) * 32) << 16) + SF_COL + c, 0x7f7f7f7fu);
-        tc::tmem_st_wait();
-    }
-    tc::tc_fence_before();
-    __syncthreads();
-    tc::tc_fence_after();
-
-    if (warp == 0) {
-        // ===== TMA producer =====
-        if (tc::elect_one()) {   // one thread, and the compiler knows it: uniform-register issue code
-            for (int kb = 0; kb < num_k_blocks; ++kb) {
-                const int s = kb % STAGES;
-                const uint32_t ph = (kb / STAGES) & 1;
-                tc::mbar_wait(&empty_bar[s], ph ^ 1);
-                tc::mbar_arrive_expect_tx(&full_bar[s], A_BYTES + B_BYTES);
-                tc::tma_load_2d(smem_a + s * A_BYTES, &tmap_a, &full_bar[s], kb * BK, m0);
-                tc::tma_load_2d(smem_b + s * B_BYTES, &tmap_b, &full_bar[s], kb * BK, (int32_t)n0);
-            }
-        }
-    } else if (warp == 1) {
-        // ===== MMA issuer (one thread) =====
-        if (tc::elect_one()) {   // one thread, and the compiler knows it: uniform-register issue code
-            constexpr uint32_t idesc = tc::make_idesc_mxf4(BM, BN);
-            for (int kb = 0; kb < num_k_blocks; ++kb) {
-                const int s = kb % STAGES;
-                const uint32_t ph = (kb / STAGES) & 1;
-                tc::mbar_wait(&full_bar[s], ph);
-                tc::tc_fence_after();
-                const uint64_t da = tc::make_smem_desc_sw128(tc::smem_u32(smem_a + s * A_BYTES));
-                const uint64_t db = tc::make_smem_desc_sw128(tc::smem_u32(smem_b + s * B_BYTES));
-#pragma unroll
-                for (int k = 0; k < BK / 32; ++k)   // +32 bytes of K = +2 in the (addr >> 4) field
-                    tc::mma_mxf4(tmem_base, da + (uint64_t)(2 * k), db + (uint64_t)(2 * k), idesc, tmem_base + SF_COL,
-                                 tmem_base + SF_COL, (kb | k) != 0);
-                tc::tc_commit(&empty_bar[s]);       // frees the smem stage when these MMAs retire
-            }
-            tc::tc_commit(accum_bar);               // accumulator complete
-        }
-    } else {
-        // ===== epilogue: warps 2..5 own TMEM lanes 32*(warp%4) .. +32 =====
-        const int q = warp & 3;
-        const int64_t row = (int64_t)m0 + q * 32 + lane;
-        const int32_t s_i = row < R ? srow[ids[row]] : 0;      // issued before the accumulator wait
-        tc::mbar_wait(accum_bar, 0);
-        tc::tc_fence_after();
-        dist_store_tile(tmem_base, q, row, s_i, R, n0, cend, srow, ldd, subtract, mirror, Dd, Dm, peers.starts[owner], row_global0);
-        tc::tc_fence_before();
-    }
-    __syncthreads();
-    if (warp == 1) {
-        tc::tc_fence_after();
-        tc::tmem_dealloc<TMEM_COLS>(tmem_base);
-    }
-}
-
-// ---------------------------------------------------------------------------------------------
-// CTA-pair version (tcgen05 cta_group::2): one cluster of two CTAs per 256 x 256 super-block of D.
-// Each CTA stages its own 128 target rows and HALF of the 256 sample rows (32 KB per K slab instead
-// of 48 KB -- the single-CTA kernel is bound by the operand feed from L2, not by the tensor pipe:
-// tools/fp4_peak.cu reaches 128 cycles per M128 N256 K64 MMA from resident operands, the kernel
-// above ~190), six stages deep; the leader CTA issues one M256 N256 MMA for the pair, which reads the
-// B operand from both CTAs' shared memory; commits are multicast to both CTAs' barriers; each CTA
-// drains its own 128 TMEM lanes.  A pair is exactly one super-block of the symmetric scheme.
-// Probed stand-alone first (tools/tc_dist_cg2_probe.cu, profiles/r02_tc_dist_cg2_probe_run1.txt: exact).
-namespace {
-constexpr int P_STAGES = 6;
-constexpr int P_B_BYTES = (BN / 2) * BK;                       // 16 KB: this CTA's half of the sample rows
-constexpr int P_SMEM_BYTES = P_STAGES * (A_BYTES + P_B_BYTES) + 1024 + 256;
-constexpr int P_BAND = BAND / 2;                               // rasterisation band in super-block rows
-}  // namespace
-
+// One cluster of two CTAs per super-block (see the header); a pair is exactly one super-block of the
+// symmetric scheme.
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(THREADS, 1)
 tc_dist_pair_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b,
                     int num_k_blocks, const int32_t *__restrict__ srow, const int64_t *__restrict__ ids, int64_t R,
                     int64_t n, int64_t ldd, int symmetric, int subtract, int pair_rows, int tiles_x,
                     const __grid_constant__ DistPeers peers) {
     const uint32_t crank = tc::cluster_ctarank();
-    // the same L2-friendly raster as above, in super-block rows
+    // L2-friendly rasterisation: bands of BAND super-block rows, walked column by column, so that the
+    // ~74 concurrently resident pairs form a roughly square region and share their operand K-slabs
+    // through L2 (8 x 256 target rows and ~9 x 256 sample rows per wave) instead of streaming a
+    // different 256-row slab of the sample operand per pair.
     int pair_y, tile_x;
     {
         const int lin = (int)(blockIdx.x >> 1);
-        const int band = lin / (P_BAND * tiles_x);
-        const int band_rows = pair_rows - band * P_BAND < P_BAND ? pair_rows - band * P_BAND : P_BAND;
-        const int in_band = lin - band * P_BAND * tiles_x;
-        pair_y = band * P_BAND + in_band % band_rows;
+        const int band = lin / (BAND * tiles_x);
+        const int band_rows = pair_rows - band * BAND < BAND ? pair_rows - band * BAND : BAND;
+        const int in_band = lin - band * BAND * tiles_x;
+        pair_y = band * BAND + in_band % band_rows;
         tile_x = in_band / band_rows;
     }
     int owner = 0;
@@ -302,10 +181,10 @@ tc_dist_pair_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
     extern __shared__ __align__(1024) unsigned char smem_raw[];
     unsigned char *smem = reinterpret_cast<unsigned char *>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
     unsigned char *smem_a = smem;
-    unsigned char *smem_b = smem + P_STAGES * A_BYTES;
-    uint64_t *full_bar = reinterpret_cast<uint64_t *>(smem + P_STAGES * (A_BYTES + P_B_BYTES));
-    uint64_t *empty_bar = full_bar + P_STAGES;
-    uint64_t *accum_bar = empty_bar + P_STAGES;
+    unsigned char *smem_b = smem + STAGES * A_BYTES;
+    uint64_t *full_bar = reinterpret_cast<uint64_t *>(smem + STAGES * (A_BYTES + B_BYTES));
+    uint64_t *empty_bar = full_bar + STAGES;
+    uint64_t *accum_bar = empty_bar + STAGES;
     uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(accum_bar + 1);
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -314,7 +193,7 @@ tc_dist_pair_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
     if (warp == 0 && lane == 0) {
         tc::prefetch_tmap(&tmap_a);
         tc::prefetch_tmap(&tmap_b);
-        for (int s = 0; s < P_STAGES; ++s) {
+        for (int s = 0; s < STAGES; ++s) {
             tc::mbar_init(&full_bar[s], 1);       // the leader's producer arrives with the pair's byte count
             tc::mbar_init(&empty_bar[s], 1);      // the pair's MMA commit arrives (multicast)
         }
@@ -340,12 +219,12 @@ tc_dist_pair_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
         // ===== TMA producer (one per CTA: own A rows, own half of the B rows) =====
         if (tc::elect_one()) {   // one thread, and the compiler knows it: uniform-register issue code
             for (int kb = 0; kb < num_k_blocks; ++kb) {
-                const int s = kb % P_STAGES;
-                const uint32_t ph = (kb / P_STAGES) & 1;
+                const int s = kb % STAGES;
+                const uint32_t ph = (kb / STAGES) & 1;
                 tc::mbar_wait(&empty_bar[s], ph ^ 1);
-                if (crank == 0) tc::mbar_arrive_expect_tx(&full_bar[s], 2 * (A_BYTES + P_B_BYTES));
+                if (crank == 0) tc::mbar_arrive_expect_tx(&full_bar[s], 2 * (A_BYTES + B_BYTES));
                 tc::tma_load_2d_pair(smem_a + s * A_BYTES, &tmap_a, &full_bar[s], kb * BK, m0);
-                tc::tma_load_2d_pair(smem_b + s * P_B_BYTES, &tmap_b, &full_bar[s], kb * BK, (int32_t)(n0 + crank * (BN / 2)));
+                tc::tma_load_2d_pair(smem_b + s * B_BYTES, &tmap_b, &full_bar[s], kb * BK, (int32_t)(n0 + crank * (BN / 2)));
             }
         }
     } else if (warp == 1) {
@@ -353,12 +232,12 @@ tc_dist_pair_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
         if (crank == 0 && tc::elect_one()) {
             constexpr uint32_t idesc = tc::make_idesc_mxf4(2 * BM, BN);
             for (int kb = 0; kb < num_k_blocks; ++kb) {
-                const int s = kb % P_STAGES;
-                const uint32_t ph = (kb / P_STAGES) & 1;
+                const int s = kb % STAGES;
+                const uint32_t ph = (kb / STAGES) & 1;
                 tc::mbar_wait(&full_bar[s], ph);
                 tc::tc_fence_after();
                 const uint64_t da = tc::make_smem_desc_sw128(tc::smem_u32(smem_a + s * A_BYTES));
-                const uint64_t db = tc::make_smem_desc_sw128(tc::smem_u32(smem_b + s * P_B_BYTES));
+                const uint64_t db = tc::make_smem_desc_sw128(tc::smem_u32(smem_b + s * B_BYTES));
 #pragma unroll
                 for (int k = 0; k < BK / 32; ++k)
                     tc::mma_mxf4_pair(tmem_base, da + (uint64_t)(2 * k), db + (uint64_t)(2 * k), idesc, tmem_base + SF_COL,
@@ -385,37 +264,26 @@ tc_dist_pair_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
     }
 }
 
-void launch_tc_dist(const CUtensorMap &tmap_a, const CUtensorMap &tmap_b, const CUtensorMap *tmap_b_half, int64_t K,
-                    const int32_t *srow, const int64_t *d_ids, int64_t R, int64_t n, int64_t ldd, bool symmetric, bool subtract,
+// tmap_b: the sample operand with a box of BN / 2 rows (each CTA of a pair stages half of a super-block)
+void launch_tc_dist(const CUtensorMap &tmap_a, const CUtensorMap &tmap_b, int64_t K, const int32_t *srow,
+                    const int64_t *d_ids, int64_t R, int64_t n, int64_t ldd, bool symmetric, bool subtract,
                     const DistPeers &peers, cudaStream_t st, int *launches, double *ops) {
-    const int tiles_x = peers.sb_base[peers.world], tiles_y = (int)ceil_div(R, BM);
-    // CTA pairs (cta_group::2) unless switched off: FS_B200_DIST_PAIR=0 keeps the single-CTA kernel
-    const char *env = getenv("FS_B200_DIST_PAIR");
-    const bool pair = tmap_b_half != nullptr && !(env && env[0] == '0');
-    if (pair) {
-        // per launch: the attribute belongs to the CURRENT device (several devices per process: fs_multi_*)
-        FS_CUDA(cudaFuncSetAttribute(tc_dist_pair_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, P_SMEM_BYTES));
-        const int pair_rows = (int)ceil_div(R, 2 * BM);
-        tc_dist_pair_kernel<<<(unsigned)(2 * tiles_x * pair_rows), THREADS, P_SMEM_BYTES, st>>>(
-            tmap_a, *tmap_b_half, (int)(K / BK), srow, d_ids, R, n, ldd, symmetric ? 1 : 0, subtract ? 1 : 0, pair_rows, tiles_x,
-            peers);
-    } else {
-        FS_CUDA(cudaFuncSetAttribute(tc_dist_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
-        tc_dist_kernel<<<(unsigned)(tiles_x * tiles_y), THREADS, SMEM_BYTES, st>>>(
-            tmap_a, tmap_b, (int)(K / BK), srow, d_ids, R, n, ldd, symmetric ? 1 : 0, subtract ? 1 : 0, tiles_y, tiles_x,
-            peers);
-    }
+    const int tiles_x = peers.sb_base[peers.world], pair_rows = (int)ceil_div(R, 2 * BM);
+    // per launch: the attribute belongs to the CURRENT device (several devices per process: fs_multi_*)
+    FS_CUDA(cudaFuncSetAttribute(tc_dist_pair_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
+    tc_dist_pair_kernel<<<(unsigned)(2 * tiles_x * pair_rows), THREADS, SMEM_BYTES, st>>>(
+        tmap_a, tmap_b, (int)(K / BK), srow, d_ids, R, n, ldd, symmetric ? 1 : 0, subtract ? 1 : 0, pair_rows, tiles_x, peers);
     FS_CUDA(cudaGetLastError());
     ++*launches;
     if (ops) {
         int64_t tiles = 0;
-        const int rows_y = pair ? 2 * (int)ceil_div(R, 2 * BM) : tiles_y;       // a pair always runs both of its row tiles
-        for (int by = 0; by < rows_y; ++by)
+        for (int py = 0; py < pair_rows; ++py)
             for (int bx = 0; bx < tiles_x; ++bx) {
-                const int sb_i = peers.sb_base[peers.rank] + (by >> 1);
                 int owner = 0;
                 while (owner + 1 < peers.world && bx >= peers.sb_base[owner + 1]) ++owner;
-                tiles += (!symmetric || dist_row_side(sb_i, bx, peers.coarse_shift, peers.rank, owner, peers.world)) ? 1 : 0;
+                const int sb_i = peers.sb_base[peers.rank] + py;
+                // a pair always runs both of its 128-row tiles
+                tiles += (!symmetric || dist_row_side(sb_i, bx, peers.coarse_shift, peers.rank, owner, peers.world)) ? 2 : 0;
             }
         *ops += 2.0 * BM * BN * (2.0 * (double)K) * (double)tiles;      // K is the operand row length in bytes
     }

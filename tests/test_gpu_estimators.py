@@ -238,10 +238,9 @@ def test_accumulation_kernels_agree_many_tiles(native, monkeypatch):
     x = rs.randint(0, 3, (n, p)).astype(np.int8)
     x[:, 5] = (y + rs.randint(0, 2, n)) % 3
     w = {}
-    for mode in ("3", "2", "1"):
+    for mode in ("3", "1"):
         monkeypatch.setenv("FS_B200_ACCUM_PAIR", mode)
         w[mode] = fsb.MultiSURF(n_features_to_select=3, backend="gpu").fit(x, y).feature_importances_
     scale = float(np.abs(w["1"]).max())
     np.testing.assert_allclose(w["3"], w["1"], rtol=0, atol=1e-6 * scale)
-    np.testing.assert_allclose(w["2"], w["1"], rtol=0, atol=1e-6 * scale)
     assert np.argmax(w["3"]) == 5
