@@ -1,6 +1,7 @@
 // accum_general.cu -- CUDA-core per-feature weight accumulation for continuous
-// (and wide discrete) columns, the ReliefF neighbour gather, and the final
-// reduction of the partial weight vectors.
+// (and wide discrete) columns, the ReliefF neighbour gathers (general columns, and
+// the value codes of the one-hot columns), and the final reduction of the partial
+// weight vectors.
 //
 // Replaces the hit/miss accumulation loops and normalisation of the reference
 // kernels (MultiSURF.py:198-251, SURF.py:165-195, ReliefF.py:181-216) in the
@@ -269,6 +270,70 @@ void launch_relieff_gather(const WorkSet &ws, int64_t n, const void *xa, const i
             static_cast<const double *>(xa), nbr_idx, nbr_w, nbr_cnt, nbr_cap, R, rows, partial);
     FS_CUDA(cudaGetLastError());
     ++*launches;
+}
+
+// ReliefF on the one-hot columns: sparse neighbour lists, value codes compared directly
+// (ReliefF.py:181-216; at most C*k neighbours per target) -- HBM/L2-bound gather.
+__global__ void __launch_bounds__(128) relieff_codes_gather_kernel(
+    const uint8_t *__restrict__ codes, int64_t ldc, int64_t pt, const int64_t *__restrict__ ids,
+    const int32_t *__restrict__ nbr_idx, const double *__restrict__ nbr_w, const int32_t *__restrict__ nbr_cnt,
+    int nbr_cap, int64_t R, int64_t rows_per_cta, double *__restrict__ partial) {
+    __shared__ int32_t sidx[256];
+    __shared__ double sw[256];
+    const int tid = threadIdx.x;
+    const int64_t c = (int64_t)blockIdx.y * 128 + tid;
+    const bool live = c < pt;
+    const int64_t cc = live ? c : pt - 1;
+    const int64_t r_begin = (int64_t)blockIdx.x * rows_per_cta;
+    const int64_t r_end = r_begin + rows_per_cta < R ? r_begin + rows_per_cta : R;
+    double total = 0.0;
+    for (int64_t row = r_begin; row < r_end; ++row) {
+        const uint8_t ci = codes[ids[row] * ldc + cc];
+        const int cnt = nbr_cnt[row];
+        for (int s0 = 0; s0 < cnt; s0 += 256) {
+            const int m = cnt - s0 < 256 ? cnt - s0 : 256;
+            __syncthreads();
+            for (int e = tid; e < m; e += 128) {
+                sidx[e] = nbr_idx[row * nbr_cap + s0 + e];
+                sw[e] = nbr_w[row * nbr_cap + s0 + e];
+            }
+            __syncthreads();
+#pragma unroll 4
+            for (int e = 0; e < m; ++e) {
+                const uint8_t cj = codes[(int64_t)sidx[e] * ldc + cc];
+                total += (ci != cj) ? sw[e] : 0.0;
+            }
+        }
+    }
+    if (live) partial[(int64_t)blockIdx.x * pt + c] = total;
+}
+
+__global__ void __launch_bounds__(256) reduce_code_partials_kernel(const double *__restrict__ partial, int64_t n_part,
+                                                                   int64_t pt, const int64_t *__restrict__ tout,
+                                                                   double *__restrict__ wsum) {
+    const int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (c >= pt) return;
+    double s = 0.0;
+    for (int64_t q = 0; q < n_part; ++q) s += partial[q * pt + c];
+    wsum[tout[c]] += s;
+}
+
+// Grid: 128-column strips x chunks of target rows, about 8 CTAs per SM of a B200 (148 SMs) in all.
+void launch_relieff_codes(const WorkSet &ws, const int64_t *ids, const int32_t *nbr_idx, const double *nbr_w,
+                          const int32_t *nbr_cnt, int32_t nbr_cap, int64_t R, DevBuf<double> &partial, double *wsum,
+                          cudaStream_t st, int *launches) {
+    const int64_t ctiles = ceil_div(ws.pt, 128);
+    const int64_t want = std::max<int64_t>(1, ceil_div(148 * 8, ctiles));
+    const int64_t rows = std::max<int64_t>(1, ceil_div(R, want));
+    const int64_t n_part = ceil_div(R, rows);
+    partial.reserve((size_t)n_part * ws.pt);
+    dim3 grid((unsigned)n_part, (unsigned)ctiles);
+    relieff_codes_gather_kernel<<<grid, 128, 0, st>>>(ws.codes.ptr, ws.ldc, ws.pt, ids, nbr_idx, nbr_w, nbr_cnt, nbr_cap, R,
+                                                      rows, partial.ptr);
+    FS_CUDA(cudaGetLastError());
+    reduce_code_partials_kernel<<<(unsigned)ceil_div(ws.pt, 256), 256, 0, st>>>(partial.ptr, n_part, ws.pt, ws.tout.ptr, wsum);
+    FS_CUDA(cudaGetLastError());
+    *launches += 2;
 }
 
 __global__ void __launch_bounds__(256) reduce_partials_kernel(const double *__restrict__ partial, int64_t n_part,

@@ -90,12 +90,11 @@ GroupLayout group_layout(int64_t n, int64_t p, int64_t max_shard_rows, int world
     size_t o = align_up(sizeof(CommHeader));
     L.off_slab = o;
     o += align_up((size_t)round_up(std::max<int64_t>(max_shard_rows, 1), 128) * ldn * sizeof(int32_t));
-    // 256 rows of padding behind each mask: the accumulation kernel's permuted tile box may run up to 239
-    // rows past a tile's first row (onehot.cu::launch_accum_tensor)
+    // padding behind each mask: the accumulation kernels' mask box may reach into it
     L.off_mask_h = o;
-    o += align_up((size_t)(ldn + 256) * (ldn / 2));
+    o += align_up((size_t)(ldn + kAccumMaskPadRows) * (ldn / 2));
     L.off_mask_m = o;
-    o += align_up((size_t)(ldn + 256) * (ldn / 2));
+    o += align_up((size_t)(ldn + kAccumMaskPadRows) * (ldn / 2));
     L.off_rinfo = o;
     o += align_up((size_t)ldn * sizeof(RowInfo));
     L.off_w = o;

@@ -224,6 +224,17 @@ struct DistPeers {
     int32_t world, rank;
     int32_t coarse_shift;           // symmetric mode: log2 of the super-block group size (see tc_dist.cu)
 };
+// One rank whose slab holds all `cols` sample columns (the trivial case above), in symmetric mode with groups of 8
+// super-blocks: one rasterisation band of 16 tiles
+inline DistPeers single_rank_peers(int32_t *slab, int64_t cols) {
+    DistPeers p{};
+    p.world = 1;
+    p.slab[0] = slab;
+    p.starts[1] = cols;
+    p.sb_base[1] = (int32_t)ceil_div(cols, 256);
+    p.coarse_shift = 3;
+    return p;
+}
 
 // ---------------------------------------------------------------------------
 // multi-GPU group (comm.cu): every rank owns one exchange arena with the same layout
@@ -249,6 +260,9 @@ struct GroupLayout {
 };
 // a rank's shard may exceed n / world by this many rows (shard boundaries on super-blocks of 256 target rows)
 constexpr int64_t kShardSlack = 256;
+// Rows of padding behind each neighbour mask (score.cu, group_layout): the accumulation kernels' tensor-map box of a
+// target tile may reach that many rows past the tile's first row (tc_accum.cu checks the bound)
+constexpr int64_t kAccumMaskPadRows = 256;
 GroupLayout group_layout(int64_t n, int64_t p, int64_t max_shard_rows, int world, size_t x_bytes);
 
 // Working set of one fs_score call: the active columns split by path.
@@ -497,6 +511,31 @@ void comm_barrier(fs_comm *c, cudaStream_t st, int *launches);
 void comm_check(fs_comm *c);
 void comm_push(fs_comm *c, size_t off, size_t bytes, cudaStream_t st, int *launches);
 
+// onehot.cu: the reduced one-hot operands of the working set's tensor-path columns (U, Wd, srow when
+// ws.have_dist_ops; At, krow, codesT or tpos; codes when ws.have_codes) and, for an incremental distance
+// update, those of the removed columns
+void build_onehot(fs_dataset *ds, WorkSet &ws, int *launches);
+
+// tc_dist.cu: the one-hot mismatch counts of R target rows (internal order; h_row_ids / d_row_ids, or the
+// contiguous range from r0_internal) against all samples, into the slab Dd [R, ldn] (or subtracted from it for
+// an incremental update); symmetric and mirrored into the peers' slabs when this rank scores its shard
+void launch_dist_tensor(fs_dataset *ds, const WorkSet &ws, int64_t r0_internal, const int64_t *h_row_ids,
+                        const int64_t *d_row_ids, bool contiguous, int64_t R, int32_t *Dd, int64_t ldn,
+                        cudaStream_t st, int *launches, double *ops);
+// The distance GEMM itself: D[r, j] = srow[ids[r]] + srow[j] - sum_k a[r, k] b[j, k] (subtract: D[r, j] -= that)
+// over the FP4 operands a (R rows) and b (n rows), row_bytes wide at a pitch of `pitch` bytes, contracted over K
+// bytes (a multiple of 128; bytes past row_bytes are the tensor maps' zero fill)
+void launch_tc_dist(const int8_t *a, const int8_t *b, int64_t row_bytes, int64_t pitch, int64_t K, const int32_t *srow,
+                    const int64_t *d_ids, int64_t R, int64_t n, int64_t ldd, bool symmetric, bool subtract,
+                    const DistPeers &peers, cudaStream_t st, int *launches, double *ops);
+
+// tc_accum.cu: wsum[tout[c]] += the MultiSURF / SURF weight of every one-hot column c of the working set's
+// accumulation slice over R target rows, from the FP4 neighbour masks (rows of ldn / 2 bytes, kAccumMaskPadRows
+// rows of padding behind them) and the row constants rinfo
+void launch_accum_tensor(fs_dataset *ds, const WorkSet &ws, const int64_t *d_row_ids, const int64_t *h_row_ids,
+                         bool contiguous, int64_t R, const int8_t *mask_h, const int8_t *mask_m, int64_t ldn,
+                         const RowInfo *rinfo, double *wsum, cudaStream_t st, int *launches, double *ops);
+
 // dist_general.cu: D[r, j] = sum over general columns of the per-feature term
 // between target row r (rows of xa) and sample j (rows of xb).
 void launch_dist_general(const WorkSet &ws, const void *xa, int64_t na, const void *xb, int64_t nb,
@@ -517,6 +556,11 @@ void launch_accum_general(const WorkSet &ws, int64_t n, const void *xa, const in
 void launch_relieff_gather(const WorkSet &ws, int64_t n, const void *xa, const int32_t *nbr_idx,
                            const double *nbr_w, const int32_t *nbr_cnt, int32_t nbr_cap, int64_t R,
                            double *partial, int64_t n_part, cudaStream_t st, int *launches);
+// ReliefF on the one-hot columns: wsum[tout[c]] += the weight of every tensor-path column c from the value codes
+// (ws.codes) of the R target rows ids and of their neighbours; partial is scratch
+void launch_relieff_codes(const WorkSet &ws, const int64_t *ids, const int32_t *nbr_idx, const double *nbr_w,
+                          const int32_t *nbr_cnt, int32_t nbr_cap, int64_t R, DevBuf<double> &partial, double *wsum,
+                          cudaStream_t st, int *launches);
 // wsum[gout[c]] += sum_q partial[q, c]  (fixed order => bitwise reproducible)
 void launch_reduce_partials(const WorkSet &ws, const double *partial, int64_t n_part, double *wsum,
                             cudaStream_t st, int *launches);

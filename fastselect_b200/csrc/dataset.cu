@@ -415,8 +415,6 @@ static void run_gather(fs_dataset *ds, WorkSet &ws, int *launches) {
     ++*launches;
 }
 
-void build_onehot(fs_dataset *ds, WorkSet &ws, int *launches);  // onehot.cu
-
 // Can the cached distance slab serve this call?  tcol[0..pt) are the tensor-path columns now active.
 static int plan_dist(fs_dataset *ds, const int64_t *tcol, int64_t pt, int64_t r0, int64_t R, bool cacheable,
                      std::vector<int64_t> &removed) {

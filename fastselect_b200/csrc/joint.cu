@@ -24,19 +24,10 @@
 #include <algorithm>
 #include <cstring>
 
-#include <cuda.h>
-
 #include "common.cuh"
 #include "joint_math.cuh"
 
 namespace fs {
-
-// onehot.cu / tc_dist.cu
-CUtensorMap make_tmap_u8_sw128(const void *base, uint64_t row_bytes, uint64_t rows, uint64_t pitch_bytes,
-                               uint32_t box_rows);
-void launch_tc_dist(const CUtensorMap &tmap_a, const CUtensorMap &tmap_b, int64_t K, const int32_t *srow,
-                    const int64_t *d_ids, int64_t R, int64_t n, int64_t ldd, bool symmetric, bool subtract,
-                    const DistPeers &peers, cudaStream_t st, int *launches, double *ops);
 
 namespace {
 
@@ -206,19 +197,8 @@ void run_joint(fs_dataset *ds, int kind, double log_base, const int64_t *feat_id
             ds->joint_ids.reserve(round_up(R, 128));
             FS_CUDA(cudaMemsetAsync(ds->joint_ids.ptr, 0, round_up(R, 128) * sizeof(int64_t), st));
             const int8_t *base = ws.At.ptr + (size_t)b0 * pitch;
-            const CUtensorMap ta = make_tmap_u8_sw128(base, row_bytes, R, pitch, 128);
-            const CUtensorMap tb = make_tmap_u8_sw128(base, row_bytes, ncols, pitch, 128);      // half a super-block per CTA
-            DistPeers peers{};
-            peers.world = 1;
-            peers.rank = 0;
-            peers.slab[0] = ds->joint_slab.ptr;
-            peers.starts[0] = 0;
-            peers.starts[1] = ncols;
-            peers.sb_base[0] = 0;
-            peers.sb_base[1] = (int32_t)ceil_div(ncols, 256);
-            peers.coarse_shift = 3;
-            launch_tc_dist(ta, tb, k_bytes, ds->joint_zero.ptr, ds->joint_ids.ptr, R, ncols, ldd, false, false, peers, st,
-                           &launches, &ops);
+            launch_tc_dist(base, base, row_bytes, pitch, k_bytes, ds->joint_zero.ptr, ds->joint_ids.ptr, R, ncols, ldd, false,
+                           false, single_rank_peers(ds->joint_slab.ptr, ncols), st, &launches, &ops);
             tm.end();
         }
         tm.begin(&fs_stats::ms_reduce);

@@ -12,15 +12,6 @@
 
 #include "common.cuh"
 
-extern "C" {
-int fs_comm_create(fs_comm **out, int32_t rank, int32_t world, int32_t device);
-uint64_t fs_comm_required_bytes(int64_t n, int64_t p, int32_t dtype, int32_t world, int32_t with_x);
-int fs_comm_reserve(fs_comm *comm, uint64_t bytes, void *ipc_handle_out, int32_t *changed_out);
-int fs_comm_connect(fs_comm *comm, const void *ipc_handles, void *const *raw_ptrs);
-void *fs_comm_arena(fs_comm *comm);
-int fs_comm_connected(fs_comm *comm);
-}
-
 struct fs_multi {
     int world = 0;
     std::vector<int> devices;

@@ -1,5 +1,5 @@
-// onehot.cu -- one-hot tensor-core path: encoding of the active discrete columns, TMA
-// tensor maps, and the host side of the tcgen05 distance / accumulation kernels.
+// onehot.cu -- encoding of the active discrete columns into the operands of the one-hot
+// tensor-core path (tc_dist.cu, tc_accum.cu) and of ReliefF's one-hot gather (accum_general.cu).
 //
 // K0 "encode" of the design: every active discrete column f with 2 <= V_f <= FS_DISTINCT_CAP
 // distinct values becomes V_f - 1 reduced one-hot rows/columns (only equality matters,
@@ -13,75 +13,9 @@
 // reads n*pt elements once, writes 1.5*n*K + n*pt bytes.
 #include <algorithm>
 
-#include <cuda.h>
-
 #include "common.cuh"
-#include "tc_common.cuh"
 
 namespace fs {
-
-void launch_tc_dist(const CUtensorMap &tmap_a, const CUtensorMap &tmap_b, int64_t K, const int32_t *srow,
-                    const int64_t *d_ids, int64_t R, int64_t n, int64_t ldd, bool symmetric, bool subtract,
-                    const DistPeers &peers, cudaStream_t st, int *launches, double *ops);
-int tc_accum_tile_desc_ints();
-int launch_tc_accum(const CUtensorMap &tmap_at, const CUtensorMap &tmap_mh, const CUtensorMap &tmap_mm, int64_t n,
-                    int64_t R, const int64_t *d_ids, bool contiguous, int pair_mode, const RowInfo *rinfo, const uint8_t *codesT,
-                    int64_t ldt, const uint32_t *krow, int64_t K_rows, DevBuf<double> &tpartial, int32_t *d_tiles,
-                    DevBuf<int32_t> &consts, cudaStream_t st, int *launches, const int64_t *h_ids, const int32_t *h_y,
-                    const int64_t *h_cls_start, double *ops);
-
-// ---------------------------------------------------------------------------
-// TMA descriptor (driver entry point fetched through the runtime: no -lcuda)
-// ---------------------------------------------------------------------------
-typedef CUresult (*EncodeTiledFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *,
-                                  const cuuint64_t *, const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-static EncodeTiledFn encode_fn() {
-    static EncodeTiledFn fn = nullptr;
-    if (!fn) {
-        void *p = nullptr;
-        cudaDriverEntryPointQueryResult q;
-        FS_CUDA(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q));
-        FS_REQUIRE(p != nullptr && q == cudaDriverEntryPointSuccess, FS_ERR_CUDA, "cuTensorMapEncodeTiled not available");
-        fn = reinterpret_cast<EncodeTiledFn>(p);
-    }
-    return fn;
-}
-
-CUtensorMap make_tmap_u8_sw128(const void *base, uint64_t row_bytes, uint64_t rows, uint64_t pitch_bytes,
-                               uint32_t box_rows) {
-    CUtensorMap m;
-    cuuint64_t dims[2] = {row_bytes, rows};
-    cuuint64_t strides[1] = {pitch_bytes};
-    cuuint32_t box[2] = {128, box_rows};
-    cuuint32_t estr[2] = {1, 1};
-    CUresult rc = encode_fn()(&m, CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, const_cast<void *>(base), dims, strides, box, estr,
-                              CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
-                              CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    FS_REQUIRE(rc == CUDA_SUCCESS, FS_ERR_CUDA, "cuTensorMapEncodeTiled failed (%d): base=%p row_bytes=%llu rows=%llu pitch=%llu",
-               (int)rc, base, (unsigned long long)row_bytes, (unsigned long long)rows, (unsigned long long)pitch_bytes);
-    return m;
-}
-
-bool make_tmap_u8_sw128_nd(CUtensorMap *out, const void *base, int rank, const uint64_t *dims, const uint64_t *strides,
-                           const uint32_t *box) {
-    CUtensorMap m;
-    cuuint64_t gd[5], gs[4];
-    cuuint32_t bx[5], estr[5];
-    for (int i = 0; i < rank; ++i) {
-        gd[i] = dims[i];
-        bx[i] = box[i];
-        estr[i] = 1;
-        if (i + 1 < rank) gs[i] = strides[i];
-    }
-    const CUresult rc = encode_fn()(&m, CU_TENSOR_MAP_DATA_TYPE_UINT8, (cuuint32_t)rank, const_cast<void *>(base), gd, gs, bx, estr,
-                                    CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
-                                    CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (rc != CUDA_SUCCESS) return false;
-    *out = m;
-    return true;
-}
 
 // ---------------------------------------------------------------------------
 // encode
@@ -585,6 +519,38 @@ __global__ void __launch_bounds__(256, 6) onehot_encode_v3_kernel(
     }
 }
 
+// One launch of the encode over the columns tcol[0, pc): the lean kernel (every column holds exactly the values 0/1/2
+// of a one-byte input), else the general kernel in the input's type.  off: the columns' first reduced rows; uk0 /
+// ucol0: the reduced row / column of U and Wd that the launch's first one stands for.  Null outputs are not written.
+static void launch_encode(const fs_dataset *ds, bool lean, int all_ident, const int64_t *tcol, const int32_t *off, int64_t pc,
+                          int64_t K, int64_t ldt, int64_t ldc, int8_t *U, int8_t *Wd, int8_t *At, uint8_t *codesT,
+                          uint8_t *codes, int32_t *srow, uint32_t *krow, int64_t u_lo, int64_t u_hi, const int32_t *tpos,
+                          int uk0, int64_t ucol0, WdRows wr, cudaStream_t st, int *launches) {
+    const int64_t n = ds->n;
+    const unsigned grid = (unsigned)(ceil_div(pc, ENC_COLS) * ceil_div(n, ENC_ROWS));
+    const int as_f32 = (ds->arith == FS_ARITH_F32 && ds->dtype == FS_F64) ? 1 : 0;
+    auto general = [&](auto type_tag) {
+        using T = decltype(type_tag);
+        onehot_encode_kernel<T><<<grid, 256, 0, st>>>(static_cast<const T *>(ds->x), ds->ldx, ds->d_perm.ptr, tcol, off,
+                                                      ds->d_vals.ptr, as_f32, n, pc, K, ldt, ldc, U, Wd, At, codesT, codes,
+                                                      srow, krow, all_ident, u_lo, u_hi, tpos, uk0, wr);
+    };
+    if (lean) {
+        onehot_encode_v3_kernel<<<grid, 256, 0, st>>>(static_cast<const uint8_t *>(ds->x), ds->ldx, ds->d_perm.ptr, tcol, n, pc,
+                                                      K, ldt, ldc, U, Wd, At, codesT, codes, srow, krow, u_lo, u_hi, tpos,
+                                                      ucol0, wr);
+    } else {
+        switch (ds->dtype) {
+            case FS_U8: general(uint8_t{}); break;
+            case FS_I8: general(int8_t{}); break;
+            case FS_F32: general(float{}); break;
+            case FS_F64: general(double{}); break;
+        }
+    }
+    FS_CUDA(cudaGetLastError());
+    ++*launches;
+}
+
 // Distance operands (Ur, Wdr, srow_r) of the columns removed since the cached slab was built.
 static void build_removed(fs_dataset *ds, WorkSet &ws, int *launches) {
     Trace tr("    build_removed");
@@ -627,30 +593,8 @@ static void build_removed(fs_dataset *ds, WorkSet &ws, int *launches) {
         FS_CUDA(cudaMemset2DAsync(ws.Ur.ptr + ws.Kr_used / 2, Kb, 0, (size_t)(ws.Kr - ws.Kr_used) / 2, (size_t)n, st));
         FS_CUDA(cudaMemset2DAsync(ws.Wdr.ptr + ws.Kr_used / 2, Kb, 0, (size_t)(ws.Kr - ws.Kr_used) / 2, (size_t)n, st));
     }
-    const unsigned grid = (unsigned)(ceil_div(pr, ENC_COLS) * ceil_div(n, ENC_ROWS));
-    const int as_f32 = (ds->arith == FS_ARITH_F32 && ds->dtype == FS_F64) ? 1 : 0;
-    if (lean) {
-        onehot_encode_v3_kernel<<<grid, 256, 0, st>>>(static_cast<const uint8_t *>(ds->x), ds->ldx, ds->d_perm.ptr,
-                                                      ws.rcol.ptr, n, pr, (int64_t)Kb, ws.ldt, 0, ws.Ur.ptr, ws.Wdr.ptr, nullptr,
-                                                      nullptr, nullptr, ws.srow_r.ptr, nullptr, 0, n, nullptr, 0, WdRows{0, n, 0, 0});
-        FS_CUDA(cudaGetLastError());
-        ++*launches;
-        return;
-    }
-#define FS_ENCODE_R(T)                                                                                            \
-    onehot_encode_kernel<T><<<grid, 256, 0, st>>>(static_cast<const T *>(ds->x), ds->ldx, ds->d_perm.ptr,        \
-                                                  ws.rcol.ptr, ws.roff.ptr, ds->d_vals.ptr, as_f32, n, pr, (int64_t)Kb, \
-                                                  ws.ldt, 0, ws.Ur.ptr, ws.Wdr.ptr, nullptr, nullptr, nullptr,    \
-                                                  ws.srow_r.ptr, nullptr, all_ident, 0, n, nullptr, 0, WdRows{0, n, 0, 0})
-    switch (ds->dtype) {
-        case FS_U8: FS_ENCODE_R(uint8_t); break;
-        case FS_I8: FS_ENCODE_R(int8_t); break;
-        case FS_F32: FS_ENCODE_R(float); break;
-        case FS_F64: FS_ENCODE_R(double); break;
-    }
-#undef FS_ENCODE_R
-    FS_CUDA(cudaGetLastError());
-    ++*launches;
+    launch_encode(ds, lean, all_ident, ws.rcol.ptr, ws.roff.ptr, pr, (int64_t)Kb, ws.ldt, 0, ws.Ur.ptr, ws.Wdr.ptr, nullptr,
+                  nullptr, nullptr, ws.srow_r.ptr, nullptr, 0, n, nullptr, 0, 0, WdRows{0, n, 0, 0}, st, launches);
 }
 
 void build_onehot(fs_dataset *ds, WorkSet &ws, int *launches) {
@@ -728,9 +672,7 @@ void build_onehot(fs_dataset *ds, WorkSet &ws, int *launches) {
     }
     if (ws.Ka > ws.Ka_used)
         FS_CUDA(cudaMemsetAsync(ws.At.ptr + (size_t)ws.Ka_used * (ws.ldt / 2), 0, (size_t)(ws.Ka - ws.Ka_used) * (ws.ldt / 2), st));
-    const int as_f32 = (ds->arith == FS_ARITH_F32 && ds->dtype == FS_F64) ? 1 : 0;
     const int all_ident = ws.all_ident ? 1 : 0;
-    const unsigned row_tiles = (unsigned)ceil_div(n, ENC_ROWS);
     // One fused launch when the accumulation operands cover the same columns as the distance operands;
     // in a multi-GPU group two: the distance operands of ALL active columns (every rank needs Wd of all
     // samples), then the accumulation operands of this rank's slice only.
@@ -748,7 +690,6 @@ void build_onehot(fs_dataset *ds, WorkSet &ws, int *launches) {
     auto launch = [&](int64_t c_lo, int64_t c_hi, bool want_dist, bool want_acc, bool want_codes) {
         const int64_t pc = c_hi - c_lo;
         if (pc <= 0 || (!want_dist && !want_acc && !want_codes)) return;
-        const unsigned grid = (unsigned)ceil_div(pc, ENC_COLS) * row_tiles;
         // slice-local offsets: one-hot rows from 0, codesT rows from 0
         const bool local_rows = want_acc && c_lo == a0;        // At / krow rows numbered from the slice's first column
         const int32_t *off = local_rows ? ws.atoff.ptr : ws.toff.ptr + c_lo;
@@ -760,26 +701,8 @@ void build_onehot(fs_dataset *ds, WorkSet &ws, int *launches) {
         const int32_t *To = want_acc && reuse_ct ? ws.tpos.ptr : nullptr;
         int32_t *So = want_dist ? ws.srow.ptr : nullptr;
         uint8_t *codes = want_codes ? ws.codes.ptr : nullptr;       // sample-major value codes (ReliefF)
-        if (lean) {
-            onehot_encode_v3_kernel<<<grid, 256, 0, st>>>(static_cast<const uint8_t *>(ds->x), ds->ldx, ds->d_perm.ptr,
-                                                          ws.tcol.ptr + c_lo, n, pc, (int64_t)Kb, ws.ldt, ws.ldc, Uo, Wo, Ao, Co,
-                                                          codes, So, Ko, ws.u_lo, ws.u_hi, To, c_lo, wr);
-        } else {
-#define FS_ENCODE(T)                                                                                              \
-    onehot_encode_kernel<T><<<grid, 256, 0, st>>>(static_cast<const T *>(ds->x), ds->ldx, ds->d_perm.ptr,        \
-                                                  ws.tcol.ptr + c_lo, off, ds->d_vals.ptr, as_f32, n, pc, (int64_t)Kb, \
-                                                  ws.ldt, ws.ldc, Uo, Wo, Ao, Co, codes, So, Ko, all_ident, ws.u_lo,    \
-                                                  ws.u_hi, To, uk0, wr)
-            switch (ds->dtype) {
-                case FS_U8: FS_ENCODE(uint8_t); break;
-                case FS_I8: FS_ENCODE(int8_t); break;
-                case FS_F32: FS_ENCODE(float); break;
-                case FS_F64: FS_ENCODE(double); break;
-            }
-#undef FS_ENCODE
-        }
-        FS_CUDA(cudaGetLastError());
-        ++*launches;
+        launch_encode(ds, lean, all_ident, ws.tcol.ptr + c_lo, off, pc, (int64_t)Kb, ws.ldt, ws.ldc, Uo, Wo, Ao, Co, codes, So,
+                      Ko, ws.u_lo, ws.u_hi, To, uk0, c_lo, wr, st, launches);
     };
     if (!split) {
         launch(0, pt, ops, true, ws.have_codes);
@@ -799,187 +722,6 @@ void build_onehot(fs_dataset *ds, WorkSet &ws, int *launches) {
     // no synchronisation here: the pinned staging buffers live in the working set and are only
     // rewritten by the next build, which starts after fs_score's final stream synchronisation
     if (ws.dist_mode == kDistIncremental) build_removed(ds, ws, launches);
-}
-
-// ---------------------------------------------------------------------------
-// distance
-// ---------------------------------------------------------------------------
-void launch_dist_tensor(fs_dataset *ds, const WorkSet &ws, int64_t r0_internal, const int64_t *h_row_ids,
-                        const int64_t *d_row_ids, bool contiguous, int64_t R, int32_t *Dd, int64_t ldn,
-                        cudaStream_t st, int *launches, double *ops) {
-    // incremental update: the operands are those of the removed columns and the result is subtracted
-    const bool incr = ws.dist_mode == kDistIncremental;
-    const int8_t *Uop = incr ? ws.Ur.ptr : ws.U.ptr, *Wop = incr ? ws.Wdr.ptr : ws.Wd.ptr;
-    const int32_t *sop = incr ? ws.srow_r.ptr : ws.srow.ptr;
-    const int64_t K = (incr ? ws.Kr : ws.K) / 2;        // operand row bytes (FP4 nibbles)
-    // every column adds at most 2 to an FP32 accumulator: exact while the sums stay below 2^24
-    FS_REQUIRE(2 * ws.pt < (1LL << 24), FS_ERR_INVALID, "too many one-hot columns for exact FP32 accumulation (%lld)", (long long)ws.pt);
-    const int8_t *a_rows;
-    const int64_t u_lo = incr ? 0 : ws.u_lo;           // first sample row held by the target-side operand
-    if (contiguous) {
-        a_rows = Uop + (size_t)(r0_internal - u_lo) * K;
-    } else {
-        DevBuf<int8_t> &g = ds->a_gather;
-        g.reserve((size_t)R * K);
-        for (int64_t r = 0; r < R; ++r)
-            FS_CUDA(cudaMemcpyAsync(g.ptr + (size_t)r * K, Uop + (size_t)(h_row_ids[r] - u_lo) * K, K,
-                                    cudaMemcpyDeviceToDevice, st));
-        a_rows = g.ptr;
-    }
-    // Symmetric mode: the target rows of all ranks together cover every sample, so half of the
-    // off-diagonal super-blocks are computed and mirrored (tc_dist.cu).  One rank scoring all rows
-    // is the trivial case; with peers configured (fs_dataset_set_peers) this rank's rows must be
-    // exactly its shard and Dd its exported slab.  An incremental update across ranks stays
-    // non-symmetric (it would need remote read-modify-writes).
-    DistPeers peers{};
-    bool symmetric = false;
-    if (contiguous && ds->peers_on && Dd == ds->peer_slab && r0_internal == ds->peers.starts[ds->peers.rank] &&
-        R == ds->peers.starts[ds->peers.rank + 1] - ds->peers.starts[ds->peers.rank] && !incr) {
-        peers = ds->peers;
-        symmetric = true;
-    } else {
-        peers.world = 1;
-        peers.rank = 0;
-        peers.slab[0] = Dd;
-        peers.starts[0] = 0;
-        peers.starts[1] = ds->n;
-        peers.sb_base[0] = 0;
-        peers.sb_base[1] = (int32_t)ceil_div(ds->n, 256);
-        peers.coarse_shift = 3;                 // groups of 8 super-blocks = one rasterisation band of 16 tiles
-        symmetric = contiguous && r0_internal == 0 && R == ds->n;
-    }
-    const CUtensorMap ta = make_tmap_u8_sw128(a_rows, K, R, K, 128);
-    const CUtensorMap tb = make_tmap_u8_sw128(Wop, K, ds->n, K, 128);       // each CTA of a pair stages half of the sample rows
-    launch_tc_dist(ta, tb, K, sop, d_row_ids, R, ds->n, ldn, symmetric, incr, peers, st, launches, ops);
-    ds->last_dist_exchanged = symmetric && peers.world > 1;
-}
-
-// ---------------------------------------------------------------------------
-// accumulation
-// ---------------------------------------------------------------------------
-// wsum[tout[c]] += sum over groups g and one-hot rows of column c of tpartial[g, row]
-__global__ void __launch_bounds__(256) reduce_tensor_partials_kernel(const double *__restrict__ tpartial, int groups,
-                                                                     int64_t K_rows, const int32_t *__restrict__ toff,
-                                                                     const int64_t *__restrict__ tout, int64_t pt,
-                                                                     double *__restrict__ wsum) {
-    const int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (c >= pt) return;
-    double s = 0.0;
-    for (int g = 0; g < groups; ++g)
-        for (int r = toff[c]; r < toff[c + 1]; ++r) s += tpartial[(int64_t)g * K_rows + r];
-    wsum[tout[c]] += s;
-}
-
-// ReliefF on the one-hot columns: sparse neighbour lists, value codes compared directly
-// (ReliefF.py:181-216; at most C*k neighbours per target) -- HBM/L2-bound gather.
-__global__ void __launch_bounds__(128) relieff_codes_gather_kernel(
-    const uint8_t *__restrict__ codes, int64_t ldc, int64_t pt, const int64_t *__restrict__ ids,
-    const int32_t *__restrict__ nbr_idx, const double *__restrict__ nbr_w, const int32_t *__restrict__ nbr_cnt,
-    int nbr_cap, int64_t R, int64_t rows_per_cta, double *__restrict__ partial) {
-    __shared__ int32_t sidx[256];
-    __shared__ double sw[256];
-    const int tid = threadIdx.x;
-    const int64_t c = (int64_t)blockIdx.y * 128 + tid;
-    const bool live = c < pt;
-    const int64_t cc = live ? c : pt - 1;
-    const int64_t r_begin = (int64_t)blockIdx.x * rows_per_cta;
-    const int64_t r_end = r_begin + rows_per_cta < R ? r_begin + rows_per_cta : R;
-    double total = 0.0;
-    for (int64_t row = r_begin; row < r_end; ++row) {
-        const uint8_t ci = codes[ids[row] * ldc + cc];
-        const int cnt = nbr_cnt[row];
-        for (int s0 = 0; s0 < cnt; s0 += 256) {
-            const int m = cnt - s0 < 256 ? cnt - s0 : 256;
-            __syncthreads();
-            for (int e = tid; e < m; e += 128) {
-                sidx[e] = nbr_idx[row * nbr_cap + s0 + e];
-                sw[e] = nbr_w[row * nbr_cap + s0 + e];
-            }
-            __syncthreads();
-#pragma unroll 4
-            for (int e = 0; e < m; ++e) {
-                const uint8_t cj = codes[(int64_t)sidx[e] * ldc + cc];
-                total += (ci != cj) ? sw[e] : 0.0;
-            }
-        }
-    }
-    if (live) partial[(int64_t)blockIdx.x * pt + c] = total;
-}
-
-__global__ void __launch_bounds__(256) reduce_code_partials_kernel(const double *__restrict__ partial, int64_t n_part,
-                                                                   int64_t pt, const int64_t *__restrict__ tout,
-                                                                   double *__restrict__ wsum) {
-    const int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (c >= pt) return;
-    double s = 0.0;
-    for (int64_t q = 0; q < n_part; ++q) s += partial[q * pt + c];
-    wsum[tout[c]] += s;
-}
-
-void launch_accum_tensor(fs_dataset *ds, const WorkSet &ws, int algo, const int64_t *d_row_ids,
-                         const int64_t *h_row_ids, bool contiguous, int64_t R, const int8_t *mask_h, const int8_t *mask_m,
-                         int64_t ldn, const RowInfo *rinfo, const int32_t *nbr_idx, const double *nbr_w,
-                         const int32_t *nbr_cnt, int32_t nbr_cap, double *wsum, cudaStream_t st, int *launches,
-                         double *ops) {
-    const int64_t n = ds->n;
-    if (algo == FS_RELIEFF) {
-        const int64_t ctiles = ceil_div(ws.pt, 128);
-        const int64_t want = std::max<int64_t>(1, ceil_div(148 * 8, ctiles));
-        const int64_t rows = std::max<int64_t>(1, ceil_div(R, want));
-        const int64_t n_part = ceil_div(R, rows);
-        ds->tpartial.reserve((size_t)n_part * ws.pt);
-        dim3 grid((unsigned)n_part, (unsigned)ctiles);
-        relieff_codes_gather_kernel<<<grid, 128, 0, st>>>(ws.codes.ptr, ws.ldc, ws.pt, d_row_ids, nbr_idx, nbr_w,
-                                                          nbr_cnt, nbr_cap, R, rows, ds->tpartial.ptr);
-        FS_CUDA(cudaGetLastError());
-        reduce_code_partials_kernel<<<(unsigned)ceil_div(ws.pt, 256), 256, 0, st>>>(ds->tpartial.ptr, n_part, ws.pt,
-                                                                                   ws.tout.ptr, wsum);
-        FS_CUDA(cudaGetLastError());
-        *launches += 2;
-        return;
-    }
-    // the accumulation operands hold the columns [a0, a1) of the active list (everything outside a
-    // multi-GPU group; this rank's share inside one), one-hot rows numbered from 0
-    const int64_t pa = ws.a1 - ws.a0;
-    if (pa <= 0 || ws.Ka_used <= 0) return;
-    ds->tile_desc.reserve(tc_accum_tile_desc_ints());
-    // K of this GEMM is the sample index; At and the masks hold FP4 nibbles: rows of (n + 1) / 2 bytes
-    const uint64_t row_bytes = (uint64_t)((n + 1) / 2);
-    CUtensorMap tat = make_tmap_u8_sw128(ws.At.ptr, row_bytes, (uint64_t)ws.Ka, (uint64_t)(ws.ldt / 2), 128);
-    CUtensorMap tmh = make_tmap_u8_sw128(mask_h, row_bytes, (uint64_t)R, (uint64_t)(ldn / 2), 240);
-    CUtensorMap tmm = make_tmap_u8_sw128(mask_m, row_bytes, (uint64_t)R, (uint64_t)(ldn / 2), 240);
-    // every column with exactly three values: one-hot rows 2c, 2c + 1 are column c's two planes.  Default (3): the
-    // merged-plane kernel as clusters of two CTAs (cta_group::2), whose operands are staged in a permuted row order
-    // (tc_accum.cu): At rows as (column mod 8, plane, column / 8), mask rows as (e, j, g, chunk) with row strides
-    // 1, 4, 2, 16 -- tiles of <= 224 rows, every CTA stages half of a tile's chunks (box of 7); the box of a tile
-    // may run up to 223 rows past the tile's first row, hence the padding behind both masks.
-    // FS_B200_ACCUM_PAIR = 1: paired epilogue (planes meet by shuffle), 0: one thread per one-hot row.
-    // (the merged kernel's per-column 64-bit sums need n^2 * 2^27 < 2^63)
-    int pair_mode = ws.all_v3 ? (n < (1 << 17) ? 3 : 1) : 0;
-    if (const char *e = getenv("FS_B200_ACCUM_PAIR"))
-        if (ws.all_v3 && (e[0] == '0' || e[0] == '1' || (e[0] == '3' && n < (1 << 17)))) pair_mode = e[0] - '0';
-    if (pair_mode == 3) {
-        const uint64_t pa_b = (uint64_t)(ws.ldt / 2), pm_b = (uint64_t)(ldn / 2);
-        const uint64_t da[4] = {row_bytes, 8, 2, (uint64_t)(ws.Ka / 16)}, sa[3] = {2 * pa_b, pa_b, 16 * pa_b};
-        const uint32_t ba[4] = {128, 8, 2, 8};
-        const uint64_t dm[5] = {row_bytes, (uint64_t)R, 4, 2, 14}, sm[4] = {pm_b, 4 * pm_b, 2 * pm_b, 16 * pm_b};
-        const uint32_t bm[5] = {128, 2, 4, 2, 7};
-        const bool ok = make_tmap_u8_sw128_nd(&tat, ws.At.ptr, 4, da, sa, ba) && make_tmap_u8_sw128_nd(&tmh, mask_h, 5, dm, sm, bm) &&
-                        make_tmap_u8_sw128_nd(&tmm, mask_m, 5, dm, sm, bm);
-        if (!ok) {   // the driver refused a permuted map: the 2-D maps above and the paired epilogue still apply
-            tat = make_tmap_u8_sw128(ws.At.ptr, row_bytes, (uint64_t)ws.Ka, (uint64_t)(ws.ldt / 2), 128);
-            tmh = make_tmap_u8_sw128(mask_h, row_bytes, (uint64_t)R, (uint64_t)(ldn / 2), 240);
-            tmm = make_tmap_u8_sw128(mask_m, row_bytes, (uint64_t)R, (uint64_t)(ldn / 2), 240);
-            pair_mode = 1;
-        }
-    }
-    const int parts = launch_tc_accum(tat, tmh, tmm, n, R, d_row_ids, contiguous, pair_mode, rinfo, ws.codesT.ptr, ws.ldt,
-                                      ws.krow.ptr, ws.Ka_used, ds->tpartial, ds->tile_desc.ptr, ds->tile_consts, st, launches,
-                                      h_row_ids, ds->y_sorted.data(), ds->cls_start.data(), ops);
-    reduce_tensor_partials_kernel<<<(unsigned)ceil_div(pa, 256), 256, 0, st>>>(ds->tpartial.ptr, parts, ws.Ka_used,
-                                                                              ws.atoff.ptr, ws.tout.ptr + ws.a0, pa, wsum);
-    FS_CUDA(cudaGetLastError());
-    ++*launches;
 }
 
 }  // namespace fs

@@ -12,16 +12,6 @@
 
 namespace fs {
 
-// tensor path (onehot.cu / tc_dist.cu / tc_accum.cu)
-void launch_dist_tensor(fs_dataset *ds, const WorkSet &ws, int64_t r0_internal, const int64_t *h_row_ids,
-                        const int64_t *d_row_ids, bool contiguous, int64_t R, int32_t *Dd, int64_t ldn,
-                        cudaStream_t st, int *launches, double *ops);
-void launch_accum_tensor(fs_dataset *ds, const WorkSet &ws, int algo, const int64_t *d_row_ids,
-                         const int64_t *h_row_ids, bool contiguous, int64_t R, const int8_t *mask_h, const int8_t *mask_m,
-                         int64_t ldn, const RowInfo *rinfo, const int32_t *nbr_idx, const double *nbr_w,
-                         const int32_t *nbr_cnt, int32_t nbr_cap, double *wsum, cudaStream_t st, int *launches,
-                         double *ops);
-
 struct DebugOut {
     double *dist = nullptr;    // [nt, n] original sample order
     double *thresh = nullptr;  // [nt]
@@ -143,10 +133,9 @@ static void run_pipeline(fs_dataset *ds, int algo, int use_star, int32_t k, cons
         rinfo_buf = reinterpret_cast<RowInfo *>(arena + ds->glayout.off_rinfo) + shard0;
     } else {
         if (use_masks) {
-            // rows of ldn / 2 bytes; 256 rows of padding: the accumulation kernel's permuted tile box may
-            // run up to 239 rows past a tile's first row (onehot.cu::launch_accum_tensor)
-            ds->maskH.reserve((size_t)(Rmax + 256) * (ldn / 2));
-            ds->maskM.reserve((size_t)(Rmax + 256) * (ldn / 2));
+            // rows of ldn / 2 bytes, and the padding the accumulation kernels' mask box may reach into
+            ds->maskH.reserve((size_t)(Rmax + kAccumMaskPadRows) * (ldn / 2));
+            ds->maskM.reserve((size_t)(Rmax + kAccumMaskPadRows) * (ldn / 2));
             mask_h = ds->maskH.ptr;
             mask_m = ds->maskM.ptr;
         }
@@ -252,17 +241,20 @@ static void run_pipeline(fs_dataset *ds, int algo, int use_star, int32_t k, cons
                 ds->all_ids.alloc(n);
                 FS_CUDA(cudaMemcpyAsync(ds->all_ids.ptr, ds->all_ids_h.data(), n * sizeof(int64_t), cudaMemcpyHostToDevice, st));
             }
-            launch_accum_tensor(ds, ws, algo, ds->all_ids.ptr, ds->all_ids_h.data(), true, n,
+            launch_accum_tensor(ds, ws, ds->all_ids.ptr, ds->all_ids_h.data(), true, n,
                                 reinterpret_cast<const int8_t *>(arena + ds->glayout.off_mask_h),
                                 reinterpret_cast<const int8_t *>(arena + ds->glayout.off_mask_m), ldn,
-                                reinterpret_cast<const RowInfo *>(arena + ds->glayout.off_rinfo), nullptr, nullptr, nullptr, 0,
-                                acc_out, st, &launches, &ops_accum);
+                                reinterpret_cast<const RowInfo *>(arena + ds->glayout.off_rinfo), acc_out, st, &launches,
+                                &ops_accum);
             timer.end();
         } else if (ws.pt > 0) {
             timer.begin(&fs_stats::ms_accum_tensor);
-            launch_accum_tensor(ds, ws, algo, ds->row_ids.ptr, h_ids, contiguous, R, mask_h, mask_m, ldn,
-                                rinfo_buf, ds->nbr_idx.ptr, ds->nbr_w.ptr, ds->nbr_cnt.ptr, nbr_cap, acc_out,
-                                st, &launches, &ops_accum);
+            if (algo == FS_RELIEFF)
+                launch_relieff_codes(ws, ds->row_ids.ptr, ds->nbr_idx.ptr, ds->nbr_w.ptr, ds->nbr_cnt.ptr, nbr_cap, R,
+                                     ds->tpartial, acc_out, st, &launches);
+            else
+                launch_accum_tensor(ds, ws, ds->row_ids.ptr, h_ids, contiguous, R, mask_h, mask_m, ldn, rinfo_buf,
+                                    acc_out, st, &launches, &ops_accum);
             timer.end();
         }
         if (ws.pg > 0) {

@@ -80,6 +80,16 @@ constexpr int CG2_B_BYTES = (CG2_BN / 2) * BK;   // 14 KB
 constexpr int CG2_STAGES = 6;
 constexpr int CG2_SMEM_BYTES = CG2_STAGES * (A_BYTES + CG2_B_BYTES) + 1024 + BAR_BYTES;
 static_assert(CG2_B_BYTES % 1024 == 0 && CG2_SMEM_BYTES <= 232448, "pair stage shape");
+// Permuted mask box of the merged kernel (see above the kernel): target rows (e, j, g, chunk) with row strides 1, 4, 2,
+// 16; each CTA's box covers its half of a tile's chunks, the second CTA's from chunk CG2_BN / 32 on.
+constexpr uint32_t kMaskStride[4] = {1, 4, 2, 16};
+constexpr uint32_t kMaskBox[4] = {2, 4, 2, CG2_BN / 32};
+// How far past a tile's first row a mask box reaches: BN - 1 rows for the 2-D box (which TMA also clips at the map's R
+// rows), kMaskReach = 223 for the permuted box (not clipped: its row index is split over four dimensions).  The masks
+// carry kAccumMaskPadRows rows of padding behind them for this.
+constexpr uint32_t kMaskReach = (kMaskBox[0] - 1) * kMaskStride[0] + (kMaskBox[1] - 1) * kMaskStride[1] +
+                                (kMaskBox[2] - 1) * kMaskStride[2] + (CG2_BN / 32 + kMaskBox[3] - 1) * kMaskStride[3];
+static_assert(BN - 1 < kAccumMaskPadRows && kMaskReach < kAccumMaskPadRows, "mask box reaches past the mask padding");
 
 // A tile of target rows and the K blocks (of 128 samples) its two masks can be non-zero in:
 // hit mask: blocks [hb0, hb1); miss mask: blocks [0, ib0) and [ib1, num_k_blocks).
@@ -899,15 +909,58 @@ static AccumPlan make_plan(int64_t n, int64_t R, bool contiguous, const int64_t 
     return plan;
 }
 
-// Returns the number of partial vectors written ([groups x PARTS][K_rows] doubles).
-int launch_tc_accum(const CUtensorMap &tmap_at, const CUtensorMap &tmap_mh, const CUtensorMap &tmap_mm, int64_t n,
-                    int64_t R, const int64_t *d_ids, bool contiguous, int pair_mode, const RowInfo *rinfo, const uint8_t *codesT,
-                    int64_t ldt, const uint32_t *krow, int64_t K_rows, DevBuf<double> &tpartial, int32_t *d_tiles,
-                    DevBuf<int32_t> &consts, cudaStream_t st, int *launches, const int64_t *h_ids, const int32_t *h_y,
-                    const int64_t *h_cls_start, double *ops) {
-    // pair_mode 1 / 3: every column owns exactly two one-hot rows (2c, 2c + 1): paired epilogue (planes meet by
-    // shuffle), or the merged-plane kernel as clusters of two CTAs (planes meet in one thread; cta_group::2; tiles of
-    // <= 224 rows; the caller built the permuted tensor maps).  0: one thread per one-hot row.
+// wsum[tout[c]] += sum over groups g and one-hot rows of column c of tpartial[g, row]
+__global__ void __launch_bounds__(256) reduce_tensor_partials_kernel(const double *__restrict__ tpartial, int groups,
+                                                                     int64_t K_rows, const int32_t *__restrict__ toff,
+                                                                     const int64_t *__restrict__ tout, int64_t pt,
+                                                                     double *__restrict__ wsum) {
+    const int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (c >= pt) return;
+    double s = 0.0;
+    for (int g = 0; g < groups; ++g)
+        for (int r = toff[c]; r < toff[c + 1]; ++r) s += tpartial[(int64_t)g * K_rows + r];
+    wsum[tout[c]] += s;
+}
+
+void launch_accum_tensor(fs_dataset *ds, const WorkSet &ws, const int64_t *d_row_ids, const int64_t *h_row_ids,
+                         bool contiguous, int64_t R, const int8_t *mask_h, const int8_t *mask_m, int64_t ldn,
+                         const RowInfo *rinfo, double *wsum, cudaStream_t st, int *launches, double *ops) {
+    const int64_t n = ds->n;
+    // the accumulation operands hold the columns [a0, a1) of the active list (everything outside a
+    // multi-GPU group; this rank's share inside one), one-hot rows numbered from 0
+    const int64_t pa = ws.a1 - ws.a0, K_rows = ws.Ka_used;
+    if (pa <= 0 || K_rows <= 0) return;
+    ds->tile_desc.reserve(MAX_TILES * sizeof(TileDesc) / sizeof(int32_t));
+    TileDesc *d_tiles = reinterpret_cast<TileDesc *>(ds->tile_desc.ptr);
+    // K of this GEMM is the sample index; At and the masks hold FP4 nibbles: rows of (n + 1) / 2 bytes
+    const uint64_t row_bytes = (uint64_t)((n + 1) / 2), pa_b = (uint64_t)(ws.ldt / 2), pm_b = (uint64_t)(ldn / 2);
+    CUtensorMap tmap_at = make_tmap_u8_sw128(ws.At.ptr, row_bytes, (uint64_t)ws.Ka, pa_b, BM);
+    CUtensorMap tmap_mh = make_tmap_u8_sw128(mask_h, row_bytes, (uint64_t)R, pm_b, BN);
+    CUtensorMap tmap_mm = make_tmap_u8_sw128(mask_m, row_bytes, (uint64_t)R, pm_b, BN);
+    // Kernel choice.  Every column with exactly three values (one-hot rows 2c, 2c + 1 are column c's two planes):
+    // 3, the merged-plane kernel, whose operands are staged in a permuted row order (see above the kernel; the
+    // default below n = 2^17, where its per-column 64-bit sums stay exact: n^2 * 2^27 < 2^63), or 1, the paired
+    // epilogue (planes meet by shuffle).  Otherwise 0: one thread per one-hot row.  FS_B200_ACCUM_PAIR = 0 / 1 / 3
+    // forces a mode for three-valued columns.
+    int pair_mode = ws.all_v3 ? (n < (1 << 17) ? 3 : 1) : 0;
+    if (const char *e = getenv("FS_B200_ACCUM_PAIR"))
+        if (ws.all_v3 && (e[0] == '0' || e[0] == '1' || (e[0] == '3' && n < (1 << 17)))) pair_mode = e[0] - '0';
+    if (pair_mode == 3) {
+        const uint64_t da[4] = {row_bytes, 8, 2, (uint64_t)(ws.Ka / 16)}, sa[3] = {2 * pa_b, pa_b, 16 * pa_b};
+        const uint32_t ba[4] = {BK, 8, 2, 8};
+        const uint64_t dm[5] = {row_bytes, (uint64_t)R, 4, 2, CG2_BN / 16};
+        const uint64_t sm[4] = {kMaskStride[0] * pm_b, kMaskStride[1] * pm_b, kMaskStride[2] * pm_b, kMaskStride[3] * pm_b};
+        const uint32_t bm[5] = {BK, kMaskBox[0], kMaskBox[1], kMaskBox[2], kMaskBox[3]};
+        CUtensorMap at4, mh5, mm5;
+        if (make_tmap_u8_sw128_nd(&at4, ws.At.ptr, 4, da, sa, ba) && make_tmap_u8_sw128_nd(&mh5, mask_h, 5, dm, sm, bm) &&
+            make_tmap_u8_sw128_nd(&mm5, mask_m, 5, dm, sm, bm)) {
+            tmap_at = at4;
+            tmap_mh = mh5;
+            tmap_mm = mm5;
+        } else {
+            pair_mode = 1;   // the driver refused a permuted map: the 2-D maps and the paired epilogue still apply
+        }
+    }
     const bool merged = pair_mode == 3;
     auto kernel = pair_mode == 1 ? tc_accum_kernel<true> : tc_accum_kernel<false>;
     const int smem_bytes = merged ? CG2_SMEM_BYTES : SMEM_BYTES;
@@ -917,7 +970,8 @@ int launch_tc_accum(const CUtensorMap &tmap_at, const CUtensorMap &tmap_mh, cons
     FS_CUDA(cudaGetDevice(&dev));
     FS_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
     FS_REQUIRE(n < (1LL << 22), FS_ERR_INVALID, "one-hot accumulation supports up to 2^22 samples (got %lld)", (long long)n);
-    const AccumPlan plan = make_plan(n, R, contiguous, h_ids, h_y, h_cls_start, merged ? CG2_BN : BN, merged ? 32 : 16);
+    const AccumPlan plan = make_plan(n, R, contiguous, h_row_ids, ds->y_sorted.data(), ds->cls_start.data(),
+                                     merged ? CG2_BN : BN, merged ? 32 : 16);
     const int m_blocks = (int)ceil_div(K_rows, BM);
     // Tile groups.  Work units (128 one-hot rows x one group) are dealt round-robin, so the ~sms
     // units resident at one time span sms / groups one-hot row blocks, each streaming its own
@@ -939,6 +993,7 @@ int launch_tc_accum(const CUtensorMap &tmap_at, const CUtensorMap &tmap_mh, cons
     for (size_t t0 = 0; t0 < plan.tiles.size(); t0 += max_tiles)
         total_groups += groups_for((int)std::min<size_t>(max_tiles, plan.tiles.size() - t0));
     // merged kernel: one pair of exact 64-bit sums per column for the whole call (zeroed here, finished below)
+    DevBuf<double> &tpartial = ds->tpartial;
     tpartial.reserve(merged ? (size_t)K_rows + 2 : (size_t)total_groups * PARTS * K_rows);
     if (merged) FS_CUDA(cudaMemsetAsync(tpartial.ptr, 0, (size_t)K_rows * sizeof(double), st));
     int groups_done = 0;
@@ -951,10 +1006,10 @@ int launch_tc_accum(const CUtensorMap &tmap_at, const CUtensorMap &tmap_mh, cons
         // pageable source: the copy is staged before cudaMemcpyAsync returns
         FS_CUDA(cudaMemcpyAsync(d_tiles, plan.tiles.data() + t0, nt * sizeof(TileDesc), cudaMemcpyHostToDevice, st));
         // per-item constants: [nt x 2 phases x 256] (Chi, Clo) pairs, then as many row sums
-        consts.reserve((size_t)nt * 2 * 256 * 3 + 512);   // slack: the epilogue prefetches one item ahead
-        int2 *limbs = reinterpret_cast<int2 *>(consts.ptr);
-        int32_t *rsum = consts.ptr + (size_t)nt * 2 * 256 * 2;
-        accum_consts_kernel<<<2 * nt, 256, 0, st>>>(reinterpret_cast<const TileDesc *>(d_tiles), nt, rinfo, limbs, rsum, merged ? 2 : pair_mode);
+        ds->tile_consts.reserve((size_t)nt * 2 * 256 * 3 + 512);   // slack: the epilogue prefetches one item ahead
+        int2 *limbs = reinterpret_cast<int2 *>(ds->tile_consts.ptr);
+        int32_t *rsum = ds->tile_consts.ptr + (size_t)nt * 2 * 256 * 2;
+        accum_consts_kernel<<<2 * nt, 256, 0, st>>>(d_tiles, nt, rinfo, limbs, rsum, merged ? 2 : pair_mode);
         ++*launches;
         if (merged) {
             // clusters of two CTAs: a cluster takes two adjacent blocks of one-hot rows through a group of tiles.
@@ -977,14 +1032,14 @@ int launch_tc_accum(const CUtensorMap &tmap_at, const CUtensorMap &tmap_mh, cons
             cfg.attrs = &attr;
             cfg.numAttrs = 1;
             FS_CUDA(cudaLaunchKernelEx(&cfg, tc_accum_merged_kernel, tmap_at, tmap_mh, tmap_mm, (int)ceil_div(n, KS), R, table,
-                                       nt, groups, group_tiles, m_blocks, group_span, d_ids, contiguous ? 1 : 0,
-                                       (const int2 *)limbs, (const int32_t *)rsum, codesT, ldt, krow, K_rows, tpartial.ptr));
+                                       nt, groups, group_tiles, m_blocks, group_span, d_row_ids, contiguous ? 1 : 0,
+                                       (const int2 *)limbs, (const int32_t *)rsum, ws.codesT.ptr, ws.ldt, ws.krow.ptr, K_rows, tpartial.ptr));
         } else {
             const int units = m_blocks * groups;
             const int grid = units < sms ? units : sms;
             kernel<<<grid, THREADS, smem_bytes, st>>>(
-                tmap_at, tmap_mh, tmap_mm, (int)ceil_div(n, KS), R, reinterpret_cast<const TileDesc *>(d_tiles), nt,
-                groups, group_tiles, m_blocks, d_ids, contiguous ? 1 : 0, limbs, rsum, codesT, ldt, krow, K_rows,
+                tmap_at, tmap_mh, tmap_mm, (int)ceil_div(n, KS), R, d_tiles, nt,
+                groups, group_tiles, m_blocks, d_row_ids, contiguous ? 1 : 0, limbs, rsum, ws.codesT.ptr, ws.ldt, ws.krow.ptr, K_rows,
                 tpartial.ptr + (size_t)groups_done * PARTS * K_rows);
         }
         FS_CUDA(cudaGetLastError());
@@ -996,11 +1051,12 @@ int launch_tc_accum(const CUtensorMap &tmap_at, const CUtensorMap &tmap_mh, cons
         merged_finish_kernel<<<(unsigned)ceil_div(K_rows / 2 + 1, 256), 256, 0, st>>>(tpartial.ptr, K_rows);
         FS_CUDA(cudaGetLastError());
         ++*launches;
-        return 1;
     }
-    return PARTS * groups_done;
+    const int parts = merged ? 1 : PARTS * groups_done;
+    reduce_tensor_partials_kernel<<<(unsigned)ceil_div(pa, 256), 256, 0, st>>>(tpartial.ptr, parts, K_rows, ws.atoff.ptr,
+                                                                              ws.tout.ptr + ws.a0, pa, wsum);
+    FS_CUDA(cudaGetLastError());
+    ++*launches;
 }
-
-int tc_accum_tile_desc_ints() { return MAX_TILES * (int)(sizeof(TileDesc) / sizeof(int32_t)); }
 
 }  // namespace fs

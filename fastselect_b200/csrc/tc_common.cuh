@@ -365,7 +365,7 @@ __device__ __forceinline__ bool elect_one() {
 
 }  // namespace tc
 
-// Host: 2-D uint8 tensor map, box = 128 bytes x box_rows, 128-byte swizzle.
+// Host (tc_dist.cu): 2-D uint8 tensor map, box = 128 bytes x box_rows, 128-byte swizzle.
 CUtensorMap make_tmap_u8_sw128(const void *base, uint64_t row_bytes, uint64_t rows, uint64_t pitch_bytes,
                                uint32_t box_rows);
 // Host: rank-`rank` (3..5) uint8 tensor map, 128-byte swizzle; dims[0] / box[0] along the contiguous bytes,

@@ -40,6 +40,59 @@
 
 namespace fs {
 
+// ---------------------------------------------------------------------------
+// TMA descriptors (driver entry point fetched through the runtime: no -lcuda)
+// ---------------------------------------------------------------------------
+typedef CUresult (*EncodeTiledFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *,
+                                  const cuuint64_t *, const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave,
+                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+
+static EncodeTiledFn encode_fn() {
+    static EncodeTiledFn fn = nullptr;
+    if (!fn) {
+        void *p = nullptr;
+        cudaDriverEntryPointQueryResult q;
+        FS_CUDA(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q));
+        FS_REQUIRE(p != nullptr && q == cudaDriverEntryPointSuccess, FS_ERR_CUDA, "cuTensorMapEncodeTiled not available");
+        fn = reinterpret_cast<EncodeTiledFn>(p);
+    }
+    return fn;
+}
+
+CUtensorMap make_tmap_u8_sw128(const void *base, uint64_t row_bytes, uint64_t rows, uint64_t pitch_bytes,
+                               uint32_t box_rows) {
+    CUtensorMap m;
+    cuuint64_t dims[2] = {row_bytes, rows};
+    cuuint64_t strides[1] = {pitch_bytes};
+    cuuint32_t box[2] = {128, box_rows};
+    cuuint32_t estr[2] = {1, 1};
+    CUresult rc = encode_fn()(&m, CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, const_cast<void *>(base), dims, strides, box, estr,
+                              CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
+                              CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    FS_REQUIRE(rc == CUDA_SUCCESS, FS_ERR_CUDA, "cuTensorMapEncodeTiled failed (%d): base=%p row_bytes=%llu rows=%llu pitch=%llu",
+               (int)rc, base, (unsigned long long)row_bytes, (unsigned long long)rows, (unsigned long long)pitch_bytes);
+    return m;
+}
+
+bool make_tmap_u8_sw128_nd(CUtensorMap *out, const void *base, int rank, const uint64_t *dims, const uint64_t *strides,
+                           const uint32_t *box) {
+    CUtensorMap m;
+    cuuint64_t gd[5], gs[4];
+    cuuint32_t bx[5], estr[5];
+    for (int i = 0; i < rank; ++i) {
+        gd[i] = dims[i];
+        bx[i] = box[i];
+        estr[i] = 1;
+        if (i + 1 < rank) gs[i] = strides[i];
+    }
+    const CUresult rc = encode_fn()(&m, CU_TENSOR_MAP_DATA_TYPE_UINT8, (cuuint32_t)rank, const_cast<void *>(base), gd, gs, bx, estr,
+                                    CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
+                                    CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    if (rc != CUDA_SUCCESS) return false;
+    *out = m;
+    return true;
+}
+
 namespace {
 constexpr int BM = 128;        // target rows per CTA (half of UMMA M)
 constexpr int BN = 256;        // sample columns per super-block (UMMA N)
@@ -264,10 +317,11 @@ tc_dist_pair_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
     }
 }
 
-// tmap_b: the sample operand with a box of BN / 2 rows (each CTA of a pair stages half of a super-block)
-void launch_tc_dist(const CUtensorMap &tmap_a, const CUtensorMap &tmap_b, int64_t K, const int32_t *srow,
+void launch_tc_dist(const int8_t *a, const int8_t *b, int64_t row_bytes, int64_t pitch, int64_t K, const int32_t *srow,
                     const int64_t *d_ids, int64_t R, int64_t n, int64_t ldd, bool symmetric, bool subtract,
                     const DistPeers &peers, cudaStream_t st, int *launches, double *ops) {
+    const CUtensorMap tmap_a = make_tmap_u8_sw128(a, row_bytes, R, pitch, BM);
+    const CUtensorMap tmap_b = make_tmap_u8_sw128(b, row_bytes, n, pitch, BN / 2);   // each CTA of a pair stages half of the sample rows
     const int tiles_x = peers.sb_base[peers.world], pair_rows = (int)ceil_div(R, 2 * BM);
     // per launch: the attribute belongs to the CURRENT device (several devices per process: fs_multi_*)
     FS_CUDA(cudaFuncSetAttribute(tc_dist_pair_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
@@ -287,6 +341,41 @@ void launch_tc_dist(const CUtensorMap &tmap_a, const CUtensorMap &tmap_b, int64_
             }
         *ops += 2.0 * BM * BN * (2.0 * (double)K) * (double)tiles;      // K is the operand row length in bytes
     }
+}
+
+void launch_dist_tensor(fs_dataset *ds, const WorkSet &ws, int64_t r0_internal, const int64_t *h_row_ids,
+                        const int64_t *d_row_ids, bool contiguous, int64_t R, int32_t *Dd, int64_t ldn,
+                        cudaStream_t st, int *launches, double *ops) {
+    // incremental update: the operands are those of the removed columns and the result is subtracted
+    const bool incr = ws.dist_mode == kDistIncremental;
+    const int8_t *Uop = incr ? ws.Ur.ptr : ws.U.ptr, *Wop = incr ? ws.Wdr.ptr : ws.Wd.ptr;
+    const int32_t *sop = incr ? ws.srow_r.ptr : ws.srow.ptr;
+    const int64_t K = (incr ? ws.Kr : ws.K) / 2;        // operand row bytes (FP4 nibbles)
+    // every column adds at most 2 to an FP32 accumulator: exact while the sums stay below 2^24
+    FS_REQUIRE(2 * ws.pt < (1LL << 24), FS_ERR_INVALID, "too many one-hot columns for exact FP32 accumulation (%lld)", (long long)ws.pt);
+    const int8_t *a_rows;
+    const int64_t u_lo = incr ? 0 : ws.u_lo;           // first sample row held by the target-side operand
+    if (contiguous) {
+        a_rows = Uop + (size_t)(r0_internal - u_lo) * K;
+    } else {
+        DevBuf<int8_t> &g = ds->a_gather;
+        g.reserve((size_t)R * K);
+        for (int64_t r = 0; r < R; ++r)
+            FS_CUDA(cudaMemcpyAsync(g.ptr + (size_t)r * K, Uop + (size_t)(h_row_ids[r] - u_lo) * K, K,
+                                    cudaMemcpyDeviceToDevice, st));
+        a_rows = g.ptr;
+    }
+    // Symmetric mode: the target rows of all ranks together cover every sample, so half of the
+    // off-diagonal super-blocks are computed and mirrored (see the file head).  One rank scoring all rows
+    // is the trivial case; with peers configured (fs_dataset_set_peers) this rank's rows must be
+    // exactly its shard and Dd its exported slab.  An incremental update across ranks stays
+    // non-symmetric (it would need remote read-modify-writes).
+    const bool own_shard = contiguous && ds->peers_on && Dd == ds->peer_slab && r0_internal == ds->peers.starts[ds->peers.rank] &&
+                           R == ds->peers.starts[ds->peers.rank + 1] - ds->peers.starts[ds->peers.rank] && !incr;
+    const DistPeers peers = own_shard ? ds->peers : single_rank_peers(Dd, ds->n);
+    const bool symmetric = own_shard || (contiguous && r0_internal == 0 && R == ds->n);
+    launch_tc_dist(a_rows, Wop, K, K, K, sop, d_row_ids, R, ds->n, ldn, symmetric, incr, peers, st, launches, ops);
+    ds->last_dist_exchanged = symmetric && peers.world > 1;
 }
 
 }  // namespace fs
