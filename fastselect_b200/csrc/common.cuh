@@ -457,8 +457,9 @@ struct fs_dataset {
     std::vector<int64_t> tcol_all_sorted;    // tensor-path columns of the whole data set (ascending): static ownership
     std::vector<int64_t> owner_bound;        // [world + 1] original-column boundaries of the ranks' accumulation shares
     fs::DevBuf<int8_t> a_gather;  // gathered one-hot target rows (fs_debug_rows)
-    fs::DevBuf<int32_t> tie_flag, tie_order, tie_list;   // ReliefF reference tie order (select.cu)
-    fs::DevBuf<float> tie_keys;
+    // ReliefF reference tie order (select.cu): compacted list of tied rows, [R, n] (key, index) pairs
+    fs::DevBuf<int32_t> tie_list;
+    fs::DevBuf<uint2> tie_pairs;
     fs::DevBuf<unsigned long long> counters;
     // joint-count and MDR paths: the shared operand (joint.cu)
     fs::DiscreteOperand disc;

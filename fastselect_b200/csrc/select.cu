@@ -210,7 +210,7 @@ __global__ void __launch_bounds__(256) relieff_select_kernel(
     const int64_t *__restrict__ row_ids, const int32_t *__restrict__ y, const int64_t *__restrict__ cls_start,
     int n_classes, int k, const float *__restrict__ class_probs, int8_t *__restrict__ sel,
     RowInfo *__restrict__ rinfo, int32_t *__restrict__ nbr_idx, double *__restrict__ nbr_w,
-    int32_t *__restrict__ nbr_cnt, int nbr_cap, int32_t *__restrict__ tie_flag, int32_t *__restrict__ tie_list) {
+    int32_t *__restrict__ nbr_cnt, int nbr_cap, int32_t *__restrict__ tie_list) {
     __shared__ int hist[256];
     __shared__ int warp_tot[8];
     __shared__ unsigned s_prefix;
@@ -308,11 +308,8 @@ __global__ void __launch_bounds__(256) relieff_select_kernel(
         slot_base = slot;
     }
     if (tid == 0) {
-        if (tie_flag) {
-            tie_flag[r] = ambiguous ? 1 : 0;
-            // compacted list of the rows that need the reference's tie order: [0] = count
-            if (ambiguous) tie_list[1 + atomicAdd(&tie_list[0], 1)] = (int32_t)r;
-        }
+        // compacted list of the rows that need the reference's tie order: [0] = count
+        if (tie_list && ambiguous) tie_list[1 + atomicAdd(&tie_list[0], 1)] = (int32_t)r;
         nbr_cnt[r] = slot_base < nbr_cap ? slot_base : nbr_cap;
         RowInfo ri;
         ri.thresh = 0.0;
@@ -330,19 +327,30 @@ __global__ void __launch_bounds__(256) relieff_select_kernel(
 // ReliefF tie order of the reference.  When several candidates are tied at the k-th
 // distance (discrete data), which of them the reference takes is decided by the order
 // numba's np.argsort leaves them in (ReliefF.py:157; numba/misc/quicksort.py: median-of-
-// three partition with an explicit stack, insertion sort below 15 elements).  For the
-// target rows flagged by relieff_select_kernel this kernel replays that quicksort on the
-// float32 distance row in ORIGINAL sample order -- one thread per row, the algorithm is
+// three partition with an explicit stack, insertion sort below 15 elements).  For each row
+// of relieff_select_kernel's compacted tie list, one CTA stages the float32 distance row in
+// ORIGINAL sample order, one thread replays that quicksort on it -- the algorithm is
 // sequential -- then scans the order exactly as ReliefF.py:164-175 does and rewrites the
-// row's neighbour codes and list.  Untied rows (all rows of continuous data) exit at once.
+// row's neighbour codes and list.  Untied rows (all rows of continuous data) are not listed.
 // ---------------------------------------------------------------------------
 constexpr int kMaxTieClasses = 64;
+// A row's (key, index) pairs are staged in shared memory up to this size (n <= 25 600), in a
+// global scratch of one row per CTA beyond it.
+constexpr size_t kTieSmemBytes = 200 * 1024;
+// The CTA's threads only stage the row.  With global scratch a one-warp CTA lets an SM run 32
+// sorts at once instead of 8 (B200, n = 30 000, 2 048 tied rows: 55 ms against 92 ms).
+constexpr int kTieThreadsSmem = 256, kTieThreadsGlobal = 32;
 
-__device__ __forceinline__ void nbq_swap(int32_t *R, int64_t a, int64_t b) {
-    const int32_t t = R[a]; R[a] = R[b]; R[b] = t;
+// numba's quicksort on (key, index) pairs: the reference permutes an index array R and
+// compares A[R[i]]; moving the pairs themselves performs exactly the same swaps.  Keys are
+// non-negative float32 distances (and +inf), whose order is that of their bit patterns; only
+// the key half is compared, so equal distances stay ties.  Inlined, so that pairs in shared
+// memory are accessed as such.
+__device__ __forceinline__ uint32_t pkey(const uint2 *P, int64_t i) { return P[i].x; }
+__device__ __forceinline__ void pswap(uint2 *P, int64_t a, int64_t b) {
+    const uint2 t = P[a]; P[a] = P[b]; P[b] = t;
 }
-
-__device__ void numba_argsort_f32(const float *A, int32_t *R, int64_t n) {
+__device__ __forceinline__ void numba_argsort_pairs(uint2 *P, int64_t n) {
     if (n < 2) return;
     int32_t stack_lo[100], stack_hi[100];
     int sp = 1;
@@ -352,57 +360,6 @@ __device__ void numba_argsort_f32(const float *A, int32_t *R, int64_t n) {
         int64_t low = stack_lo[sp], high = stack_hi[sp];
         while (high - low >= 15) {
             // partition around the median of {low, mid, high}
-            const int64_t mid = (low + high) >> 1;
-            if (A[R[mid]] < A[R[low]]) nbq_swap(R, low, mid);
-            if (A[R[high]] < A[R[mid]]) nbq_swap(R, high, mid);
-            if (A[R[mid]] < A[R[low]]) nbq_swap(R, low, mid);
-            const float pivot = A[R[mid]];
-            nbq_swap(R, high, mid);
-            int64_t i = low, j = high - 1;
-            for (;;) {
-                while (i < high && A[R[i]] < pivot) ++i;
-                while (j >= low && pivot < A[R[j]]) --j;
-                if (i >= j) break;
-                nbq_swap(R, i, j);
-                ++i; --j;
-            }
-            nbq_swap(R, i, high);
-            if (high - i > i - low) {
-                if (high > i) { stack_lo[sp] = (int32_t)(i + 1); stack_hi[sp] = (int32_t)high; ++sp; }
-                high = i - 1;
-            } else {
-                if (i > low) { stack_lo[sp] = (int32_t)low; stack_hi[sp] = (int32_t)(i - 1); ++sp; }
-                low = i + 1;
-            }
-        }
-        // insertion sort of [low, high]
-        for (int64_t i = low + 1; i <= high; ++i) {
-            const int32_t kk = R[i];
-            const float v = A[kk];
-            int64_t j = i;
-            while (j > low && v < A[R[j - 1]]) { R[j] = R[j - 1]; --j; }
-            R[j] = kk;
-        }
-    }
-}
-
-// The same quicksort on (key, index) pairs held in shared memory: the reference permutes an
-// index array R and compares A[R[i]]; moving the pairs themselves performs exactly the same
-// swaps.  Keys are non-negative float32 distances (and +inf), whose order is that of their bit
-// patterns; only the key half is compared, so equal distances stay ties.
-__device__ __forceinline__ uint32_t pkey(const uint2 *P, int64_t i) { return P[i].x; }
-__device__ __forceinline__ void pswap(uint2 *P, int64_t a, int64_t b) {
-    const uint2 t = P[a]; P[a] = P[b]; P[b] = t;
-}
-__device__ void numba_argsort_pairs(uint2 *P, int64_t n) {
-    if (n < 2) return;
-    int32_t stack_lo[100], stack_hi[100];
-    int sp = 1;
-    stack_lo[0] = 0; stack_hi[0] = (int32_t)(n - 1);
-    while (sp > 0) {
-        --sp;
-        int64_t low = stack_lo[sp], high = stack_hi[sp];
-        while (high - low >= 15) {
             const int64_t mid = (low + high) >> 1;
             if (pkey(P, mid) < pkey(P, low)) pswap(P, low, mid);
             if (pkey(P, high) < pkey(P, mid)) pswap(P, high, mid);
@@ -426,6 +383,7 @@ __device__ void numba_argsort_pairs(uint2 *P, int64_t n) {
                 low = i + 1;
             }
         }
+        // insertion sort of [low, high]
         for (int64_t i = low + 1; i <= high; ++i) {
             const uint2 kv = P[i];
             int64_t j = i;
@@ -435,18 +393,19 @@ __device__ void numba_argsort_pairs(uint2 *P, int64_t n) {
     }
 }
 
-// One CTA per ambiguous row (compacted list): the row's float32 distances are staged in shared
-// memory by all threads, one thread replays the quicksort there (shared-memory latency instead of
-// a dependent global access per comparison) and re-selects exactly as ReliefF.py:164-175.
-__global__ void __launch_bounds__(256) relieff_ties_smem_kernel(
+// kShared: the pairs live in dynamic shared memory (shared-memory latency instead of a global
+// access per comparison); otherwise in `scratch`, n pairs per CTA.  A template parameter rather
+// than a pointer chosen at run time, so that the shared instantiation keeps shared loads/stores.
+template <bool kShared>
+__global__ void __launch_bounds__(kShared ? kTieThreadsSmem : kTieThreadsGlobal) relieff_ties_kernel(
     const double *__restrict__ Dc, const int32_t *__restrict__ Dd, int64_t ldn, int64_t n,
     const int64_t *__restrict__ row_ids, const int32_t *__restrict__ y, const int64_t *__restrict__ inv_perm,
     int n_classes, int k, const float *__restrict__ class_probs, const int32_t *__restrict__ tie_list,
-    int8_t *__restrict__ sel, int32_t *__restrict__ nbr_idx, double *__restrict__ nbr_w,
+    uint2 *scratch, int8_t *__restrict__ sel, int32_t *__restrict__ nbr_idx, double *__restrict__ nbr_w,
     int32_t *__restrict__ nbr_cnt, int nbr_cap) {
     extern __shared__ __align__(16) unsigned char ties_smem[];
-    uint2 *P = reinterpret_cast<uint2 *>(ties_smem);
     if ((int)blockIdx.x >= tie_list[0]) return;
+    uint2 *P = kShared ? reinterpret_cast<uint2 *>(ties_smem) : scratch + (int64_t)blockIdx.x * n;
     const int64_t r = tie_list[1 + blockIdx.x];
     const int64_t self = row_ids[r];
     const int64_t base = r * ldn;
@@ -464,58 +423,11 @@ __global__ void __launch_bounds__(256) relieff_ties_smem_kernel(
     if (denom == 0.0) denom = 1.0;
     int found[kMaxTieClasses];
     for (int c = 0; c < n_classes; ++c) found[c] = 0;
-    int slot = 0, filled = 0;
-    for (int64_t q = 0; q < n && filled < n_classes; ++q) {
-        const int64_t j = inv_perm[P[q].y];
-        const int c = y[j];
-        if (found[c] >= k) continue;
-        if (++found[c] == k) ++filled;
-        sel[base + j] = c == ci ? FS_MASK_NEAR_HIT : FS_MASK_NEAR_MISS;
-        if (slot < nbr_cap) {
-            nbr_idx[r * nbr_cap + slot] = (int32_t)j;
-            nbr_w[r * nbr_cap + slot] = c == ci ? -1.0 : ((double)class_probs[c] / denom) / (double)k;
-        }
-        ++slot;
-    }
-    const double wh = found[ci] > 0 ? -1.0 / (double)found[ci] : 0.0;   // ReliefF.py:211-212
-    const int m = slot < nbr_cap ? slot : nbr_cap;
-    for (int e = 0; e < m; ++e)
-        if (nbr_w[r * nbr_cap + e] == -1.0) nbr_w[r * nbr_cap + e] = wh;
-    nbr_cnt[r] = m;
-}
-
-__global__ void __launch_bounds__(32) relieff_ties_kernel(
-    const double *__restrict__ Dc, const int32_t *__restrict__ Dd, int64_t ldn, int64_t n,
-    const int64_t *__restrict__ row_ids, const int32_t *__restrict__ y, const int64_t *__restrict__ inv_perm,
-    int n_classes, int k, const float *__restrict__ class_probs, const int32_t *__restrict__ tie_flag,
-    float *__restrict__ keys, int32_t *__restrict__ order, int8_t *__restrict__ sel,
-    int32_t *__restrict__ nbr_idx, double *__restrict__ nbr_w, int32_t *__restrict__ nbr_cnt, int nbr_cap,
-    int64_t R) {
-    const int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (r >= R || !tie_flag[r]) return;
-    const int64_t self = row_ids[r];
-    const int64_t base = r * ldn;
-    float *A = keys + r * n;
-    int32_t *ord = order + r * n;
-    for (int64_t o = 0; o < n; ++o) {
-        const int64_t j = inv_perm[o];
-        A[o] = j == self ? __int_as_float(0x7f800000) : (float)load_d(Dc, Dd, base + j);   // ReliefF.py:146-155
-        ord[o] = (int32_t)o;
-    }
-    numba_argsort_f32(A, ord, n);
-    const int ci = y[self];
-    double denom = 1.0 - (double)class_probs[ci];
-    if (denom == 0.0) denom = 1.0;
-    int found[kMaxTieClasses];
-    for (int c = 0; c < n_classes; ++c) found[c] = 0;
-    for (int64_t j = 0; j < n; ++j) sel[base + j] = FS_MASK_NONE;
     // ReliefF.py:164-175 (the scan never ends early in the reference: the target's own class
     // cannot reach k misses; stopping once every class is served selects the same samples)
     int slot = 0, filled = 0;
-    const int64_t own_len = 0;
-    (void)own_len;
     for (int64_t q = 0; q < n && filled < n_classes; ++q) {
-        const int64_t j = inv_perm[ord[q]];
+        const int64_t j = inv_perm[P[q].y];
         const int c = y[j];
         if (found[c] >= k) continue;
         if (++found[c] == k) ++filled;
@@ -552,33 +464,27 @@ void launch_select(fs_dataset *ds, int algo, int use_star, int32_t k, const int6
         const char *env = getenv("FS_B200_RELIEFF_TIES");
         const bool emulate = !(env && env[0] == 'i') && ds->n_classes <= kMaxTieClasses;
         if (emulate) {
-            ds->tie_flag.reserve(R);
             ds->tie_list.reserve(R + 1);
             FS_CUDA(cudaMemsetAsync(ds->tie_list.ptr, 0, sizeof(int32_t), st));
         }
         relieff_select_kernel<<<grid, 256, 0, st>>>(Dc, Dd, ldn, ds->n, row_ids, ds->d_y.ptr, ds->d_cls_start.ptr,
                                                     ds->n_classes, k, class_probs, sel, rinfo, nbr_idx, nbr_w,
-                                                    nbr_cnt, nbr_cap, emulate ? ds->tie_flag.ptr : nullptr,
-                                                    emulate ? ds->tie_list.ptr : nullptr);
+                                                    nbr_cnt, nbr_cap, emulate ? ds->tie_list.ptr : nullptr);
         if (emulate) {
             FS_CUDA(cudaGetLastError());
             ++*launches;
+            // one CTA per row of the compacted list (CTAs beyond the list's length exit at once; no
+            // host round trip for the count)
             const size_t pair_bytes = (size_t)ds->n * sizeof(uint2);
-            if (pair_bytes <= 200 * 1024) {
-                // the row fits in shared memory: one CTA per ambiguous row of the compacted list
-                // (CTAs beyond the list's length exit at once; no host round trip for the count)
-                FS_CUDA(cudaFuncSetAttribute(relieff_ties_smem_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                             (int)pair_bytes));
-                relieff_ties_smem_kernel<<<grid, 256, pair_bytes, st>>>(
-                    Dc, Dd, ldn, ds->n, row_ids, ds->d_y.ptr, ds->d_inv_perm.ptr, ds->n_classes, k, class_probs,
-                    ds->tie_list.ptr, sel, nbr_idx, nbr_w, nbr_cnt, nbr_cap);
-            } else {
-                ds->tie_keys.reserve((size_t)R * ds->n);
-                ds->tie_order.reserve((size_t)R * ds->n);
-                relieff_ties_kernel<<<(unsigned)ceil_div(R, 32), 32, 0, st>>>(
-                    Dc, Dd, ldn, ds->n, row_ids, ds->d_y.ptr, ds->d_inv_perm.ptr, ds->n_classes, k, class_probs,
-                    ds->tie_flag.ptr, ds->tie_keys.ptr, ds->tie_order.ptr, sel, nbr_idx, nbr_w, nbr_cnt, nbr_cap, R);
-            }
+            const bool smem = pair_bytes <= kTieSmemBytes;
+            auto kernel = smem ? relieff_ties_kernel<true> : relieff_ties_kernel<false>;
+            if (smem)
+                FS_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pair_bytes));
+            else
+                ds->tie_pairs.reserve((size_t)R * ds->n);
+            kernel<<<grid, smem ? kTieThreadsSmem : kTieThreadsGlobal, smem ? pair_bytes : 0, st>>>(
+                Dc, Dd, ldn, ds->n, row_ids, ds->d_y.ptr, ds->d_inv_perm.ptr, ds->n_classes, k, class_probs,
+                ds->tie_list.ptr, smem ? nullptr : ds->tie_pairs.ptr, sel, nbr_idx, nbr_w, nbr_cnt, nbr_cap);
         }
     }
     FS_CUDA(cudaGetLastError());

@@ -123,6 +123,29 @@ def test_relieff_rows_match_oracle(native, monkeypatch, name, k, ties):
         np.testing.assert_allclose(full, want["wsum"], rtol=RTOL, atol=atol_for(want["wsum"]) * n)
 
 
+@pytest.mark.parametrize("k", [1, 10])
+def test_relieff_reference_ties_beyond_shared_memory(native, monkeypatch, k):
+    """n = 26 000 genotypes: a row's (distance, index) pairs take 208 000 bytes, more than the
+    tie replay stages in shared memory, so the quicksort runs on global scratch.  18 targets
+    spread over the classes (all of them would need a 5 GB distance output)."""
+    monkeypatch.delenv("FS_B200_RELIEFF_TIES", raising=False)
+    x, y = genotype(41, 26_000, 24, 3)
+    ds, (x32, y_enc, recip, isd, cp) = open_relieff(native, x, y)
+    tg = []
+    for c in range(len(cp)):
+        idx = np.flatnonzero(y_enc == c)
+        tg.append(idx[np.linspace(0, idx.size - 1, 6).astype(np.int64)])
+    tg = np.concatenate(tg)
+    with ds:
+        got = ds.debug_rows(native.FS_RELIEFF, tg, k=k, class_probs=cp)
+    want = R.relieff_targets(x32, y_enc, recip, isd, k, cp, tg, tie_mode=0)
+    other = R.relieff_targets(x32, y_enc, recip, isd, k, cp, tg, tie_mode=1, want_dist=False)
+    assert np.array_equal(got["dist"], want["dist"])
+    assert np.array_equal(got["mask"], want["mask"])
+    np.testing.assert_allclose(got["wsum"], want["wsum"], rtol=RTOL, atol=atol_for(want["wsum"]) * tg.size)
+    assert not np.array_equal(want["mask"], other["mask"])      # the tie order decides neighbours
+
+
 def test_surf_mean_uses_the_reference_summation_order(native, golden):
     """gauss2_long: the float32 row sum decides two neighbour pairs; only the order the
     reference's compiled code uses (oracle sum_mode 2) reproduces the reference scores."""
