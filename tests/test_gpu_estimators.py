@@ -230,17 +230,24 @@ def test_staged_upload_of_pageable_views(native, monkeypatch):
 
 
 def test_accumulation_kernels_agree_many_tiles(native, monkeypatch):
-    """More target tiles than one launch of the merged-plane accumulation kernel takes (112 tiles of 224 rows):
-    the launches add into the same exact column sums; the older paired kernel (one launch) must agree."""
+    """More target tiles than one launch of the merged-plane accumulation kernel takes (117 tiles of <= 224 rows
+    > 112): the launches add into the same exact column sums.  Both it and the paired kernel (one launch) must
+    match the oracle to the exactness of the one-hot path (see test_gpu_onehot_exact.py)."""
+    from test_gpu_onehot_exact import oracle_multisurf
+
     rs = np.random.RandomState(12)
     n, p = 26000, 48
     y = rs.randint(0, 3, n)
     x = rs.randint(0, 3, (n, p)).astype(np.int8)
     x[:, 5] = (y + rs.randint(0, 2, n)) % 3
-    w = {}
+    assert sum(-(-int(c) // 224) for c in np.bincount(y)) > 112
+    want, _, atol = oracle_multisurf(x, y, False, np.arange(n))
     for mode in ("3", "1"):
         monkeypatch.setenv("FS_B200_ACCUM_PAIR", mode)
-        w[mode] = fsb.MultiSURF(n_features_to_select=3, backend="gpu").fit(x, y).feature_importances_
-    scale = float(np.abs(w["1"]).max())
-    np.testing.assert_allclose(w["3"], w["1"], rtol=0, atol=1e-6 * scale)
-    assert np.argmax(w["3"]) == 5
+        # the float64 sums fit() divides by n and rounds to float32
+        with native.Dataset(x, y.astype(np.int32), 3) as ds:
+            ds.set_features(np.ones(p, bool), np.ones(p, np.float32), native.FS_ARITH_F32)
+            w, st = ds.score(native.FS_MULTISURF, want_stats=True)
+        assert st["n_tensor_cols"] == p and st["ops_accum_tensor"] > 0
+        assert np.abs(w - want).max() <= atol, (mode, np.abs(w - want).max(), atol)
+        assert np.argmax(fsb.MultiSURF(n_features_to_select=3, backend="gpu").fit(x, y).feature_importances_) == 5

@@ -300,15 +300,31 @@ def test_general_encode_path_matches_oracle(native, make):
 
 
 def test_chunked_target_rows_give_the_same_result(native, monkeypatch):
-    x, y = mixed(36, 300, 40, 2)
+    """A 16 MB slab budget at n = 3000 (rows of round_up(n, 128) = 3072 samples) splits the target rows into chunks:
+    3072 x 15 bytes per row (float64 and int32 distances, selection, masks) gives 256-row chunks on mixed data,
+    3072 x 7 bytes (no float64 slab) 768-row chunks on genotypes.  Mixed data must match the single-chunk run;
+    genotypes must match the oracle to the exactness of the one-hot path (see test_gpu_onehot_exact.py)."""
+    from test_gpu_onehot_exact import oracle_multisurf
+
+    n = 3000
+    x, y = mixed(36, n, 40, 2)
+    g, gy = epistatic_genotypes(36, n, 40)
     ds, _ = open_multisurf(native, x, y)
     with ds:
         a = ds.score(native.FS_MULTISURF, use_star=True)
-    monkeypatch.setenv("FS_B200_CHUNK_MB", "16")    # forces 128-row chunks at this size? (small budget)
+    monkeypatch.setenv("FS_B200_CHUNK_MB", "16")
     ds, _ = open_multisurf(native, x, y)
     with ds:
         b, st = ds.score(native.FS_MULTISURF, use_star=True, want_stats=True)
+    assert st["n_chunks"] == 12, st["n_chunks"]
     np.testing.assert_allclose(a, b, rtol=1e-12, atol=1e-12)
+    with native.Dataset(g, gy.astype(np.int32), 2) as ds:
+        ds.set_features(np.ones(40, bool), np.ones(40, np.float32), native.FS_ARITH_F32)
+        for star in (False, True):
+            w, st = ds.score(native.FS_MULTISURF, use_star=star, want_stats=True)
+            assert st["n_chunks"] == 4 and st["n_general_cols"] == 0, st
+            want, _, atol = oracle_multisurf(g, gy, star, ds.row_order())
+            assert np.abs(w - want).max() <= atol, (star, np.abs(w - want).max(), atol)
 
 
 def test_c3_shape_subset_of_targets(native):
