@@ -333,10 +333,12 @@ __global__ void __launch_bounds__(256) relieff_select_kernel(
 // sequential -- then scans the order exactly as ReliefF.py:164-175 does and rewrites the
 // row's neighbour codes and list.  Untied rows (all rows of continuous data) are not listed.
 // ---------------------------------------------------------------------------
-constexpr int kMaxTieClasses = 64;
-// A row's (key, index) pairs are staged in shared memory up to this size (n <= 25 600), in a
-// global scratch of one row per CTA beyond it.
+// A row's (key, index) pairs and its per-class neighbour counters (n * 8 + n_classes * 4 bytes) are
+// staged in shared memory up to this size (n <= 25 599 with 2 classes), in a global scratch of one row
+// per CTA beyond it.
 constexpr size_t kTieSmemBytes = 200 * 1024;
+// uint2 slots of one row of the global scratch: n pairs, then the counters (padded to a whole pair)
+__host__ __device__ __forceinline__ int64_t tie_row_pairs(int64_t n, int n_classes) { return n + (n_classes + 1) / 2; }
 // The CTA's threads only stage the row.  With global scratch a one-warp CTA lets an SM run 32
 // sorts at once instead of 8 (B200, n = 30 000, 2 048 tied rows: 55 ms against 92 ms).
 constexpr int kTieThreadsSmem = 256, kTieThreadsGlobal = 32;
@@ -393,9 +395,10 @@ __device__ __forceinline__ void numba_argsort_pairs(uint2 *P, int64_t n) {
     }
 }
 
-// kShared: the pairs live in dynamic shared memory (shared-memory latency instead of a global
-// access per comparison); otherwise in `scratch`, n pairs per CTA.  A template parameter rather
-// than a pointer chosen at run time, so that the shared instantiation keeps shared loads/stores.
+// kShared: the pairs and counters live in dynamic shared memory (shared-memory latency instead of a
+// global access per comparison); otherwise in `scratch`, tie_row_pairs(n, n_classes) pairs per CTA.
+// A template parameter rather than a pointer chosen at run time, so that the shared instantiation
+// keeps shared loads/stores.
 template <bool kShared>
 __global__ void __launch_bounds__(kShared ? kTieThreadsSmem : kTieThreadsGlobal) relieff_ties_kernel(
     const double *__restrict__ Dc, const int32_t *__restrict__ Dd, int64_t ldn, int64_t n,
@@ -405,7 +408,8 @@ __global__ void __launch_bounds__(kShared ? kTieThreadsSmem : kTieThreadsGlobal)
     int32_t *__restrict__ nbr_cnt, int nbr_cap) {
     extern __shared__ __align__(16) unsigned char ties_smem[];
     if ((int)blockIdx.x >= tie_list[0]) return;
-    uint2 *P = kShared ? reinterpret_cast<uint2 *>(ties_smem) : scratch + (int64_t)blockIdx.x * n;
+    uint2 *P = kShared ? reinterpret_cast<uint2 *>(ties_smem) : scratch + (int64_t)blockIdx.x * tie_row_pairs(n, n_classes);
+    int32_t *found = reinterpret_cast<int32_t *>(P + n);      // neighbours taken per class
     const int64_t r = tie_list[1 + blockIdx.x];
     const int64_t self = row_ids[r];
     const int64_t base = r * ldn;
@@ -415,14 +419,13 @@ __global__ void __launch_bounds__(kShared ? kTieThreadsSmem : kTieThreadsGlobal)
         P[o] = make_uint2(__float_as_uint(d), (uint32_t)o);
     }
     for (int64_t j = threadIdx.x; j < n; j += blockDim.x) sel[base + j] = FS_MASK_NONE;
+    for (int c = threadIdx.x; c < n_classes; c += blockDim.x) found[c] = 0;
     __syncthreads();
     if (threadIdx.x != 0) return;
     numba_argsort_pairs(P, n);
     const int ci = y[self];
     double denom = 1.0 - (double)class_probs[ci];
     if (denom == 0.0) denom = 1.0;
-    int found[kMaxTieClasses];
-    for (int c = 0; c < n_classes; ++c) found[c] = 0;
     // ReliefF.py:164-175 (the scan never ends early in the reference: the target's own class
     // cannot reach k misses; stopping once every class is served selects the same samples)
     int slot = 0, filled = 0;
@@ -462,7 +465,7 @@ void launch_select(fs_dataset *ds, int algo, int use_star, int32_t k, const int6
     else {
         // reference tie order unless FS_B200_RELIEFF_TIES=index (ties then go by sample index)
         const char *env = getenv("FS_B200_RELIEFF_TIES");
-        const bool emulate = !(env && env[0] == 'i') && ds->n_classes <= kMaxTieClasses;
+        const bool emulate = !(env && env[0] == 'i');
         if (emulate) {
             ds->tie_list.reserve(R + 1);
             FS_CUDA(cudaMemsetAsync(ds->tie_list.ptr, 0, sizeof(int32_t), st));
@@ -475,14 +478,14 @@ void launch_select(fs_dataset *ds, int algo, int use_star, int32_t k, const int6
             ++*launches;
             // one CTA per row of the compacted list (CTAs beyond the list's length exit at once; no
             // host round trip for the count)
-            const size_t pair_bytes = (size_t)ds->n * sizeof(uint2);
-            const bool smem = pair_bytes <= kTieSmemBytes;
+            const size_t row_bytes = (size_t)ds->n * sizeof(uint2) + (size_t)ds->n_classes * sizeof(int32_t);
+            const bool smem = row_bytes <= kTieSmemBytes;
             auto kernel = smem ? relieff_ties_kernel<true> : relieff_ties_kernel<false>;
             if (smem)
-                FS_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pair_bytes));
+                FS_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)row_bytes));
             else
-                ds->tie_pairs.reserve((size_t)R * ds->n);
-            kernel<<<grid, smem ? kTieThreadsSmem : kTieThreadsGlobal, smem ? pair_bytes : 0, st>>>(
+                ds->tie_pairs.reserve((size_t)R * tie_row_pairs(ds->n, ds->n_classes));
+            kernel<<<grid, smem ? kTieThreadsSmem : kTieThreadsGlobal, smem ? row_bytes : 0, st>>>(
                 Dc, Dd, ldn, ds->n, row_ids, ds->d_y.ptr, ds->d_inv_perm.ptr, ds->n_classes, k, class_probs,
                 ds->tie_list.ptr, smem ? nullptr : ds->tie_pairs.ptr, sel, nbr_idx, nbr_w, nbr_cnt, nbr_cap);
         }
