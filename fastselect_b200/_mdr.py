@@ -134,6 +134,9 @@ class MDRData:
     def tables(self, fold, order, combos):
         return self._ds.mdr_tables(fold, order, combos)
 
+    def interaction_scan(self, n_top, want_all=False):
+        return self._ds.interaction_scan(n_top, want_all=want_all)
+
     def close(self):
         self._ds.close()
 

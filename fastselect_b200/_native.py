@@ -15,7 +15,7 @@ FS_U8, FS_I8, FS_F32, FS_F64 = 0, 1, 2, 3
 FS_ARITH_F32, FS_ARITH_F64 = 0, 1
 FS_JOINT_MI, FS_JOINT_SU = 0, 1
 FS_DISTINCT_CAP = 16
-FS_ABI_VERSION = 8
+FS_ABI_VERSION = 9
 FS_MDR_MAX_TOP = 2048
 
 _DTYPES = {np.dtype(np.uint8): FS_U8, np.dtype(np.int8): FS_I8,
@@ -86,6 +86,7 @@ def load():
     lib.fs_debug_slab.argtypes = [vp, i64, i64, vp, vp]
     lib.fs_mdr_scan.argtypes = [vp, vp, i64, i32, vp, i32, i64, vp, vp, vp, vp, vp, vp, C.POINTER(FsStats)]
     lib.fs_mdr_tables.argtypes = [vp, vp, i64, i32, vp, i32, vp, i64, vp]
+    lib.fs_interaction_scan.argtypes = [vp, vp, i64, i64, vp, vp, vp, vp, C.POINTER(FsStats)]
     if lib.fs_abi_version() != FS_ABI_VERSION:
         raise RuntimeError(f"fastselect_b200: {LIB_PATH} has ABI version {lib.fs_abi_version()}, "
                            f"this package needs {FS_ABI_VERSION}; rebuild it (make -C fastselect_b200/csrc)")
@@ -351,6 +352,22 @@ class Dataset(_DeviceData):
         _call("fs_mdr_tables", self._h, _ptr(feat_idx), n_kept, int(order), _ptr(fold), n_folds, _ptr(combos),
               combos.shape[0], _ptr(out))
         return out
+
+    def interaction_scan(self, n_top, feat_idx=None, want_all=False, want_stats=False):
+        """KSA screen of every pair of the positions of ``feat_idx`` (see include/fastselect_b200.h): returns a
+        dict with ``top_idx`` (int64 ``[n_top]``, pair indices of :meth:`mdr_scan` order 2), ``top_ksa``
+        (float64 ``[n_top]``, highest first), ``top_tables`` (int64 ``[n_top, 2, 9]``, entry ``[q, k, i * 3 + j]``
+        counting the samples of class k with state i in the first and j in the second column) and, with
+        ``want_all``, ``all_ksa`` (float64 ``[n_pairs]``)."""
+        feat_idx, n_kept = _columns(feat_idx, self.p)
+        out = dict(top_idx=np.empty(n_top, np.int64), top_ksa=np.empty(n_top, np.float64),
+                   top_tables=np.empty((n_top, 2, 9), np.int64))
+        if want_all:
+            out["all_ksa"] = np.empty(n_kept * (n_kept - 1) // 2, np.float64)
+        stats, stats_arg = _stats(want_stats)
+        _call("fs_interaction_scan", self._h, _ptr(feat_idx), n_kept, int(n_top), _ptr(out["top_idx"]),
+              _ptr(out["top_ksa"]), _ptr(out["top_tables"]), _ptr(out.get("all_ksa")), stats_arg)
+        return (out, stats.as_dict()) if want_stats else out
 
     def debug_slab(self, row_begin, nrows):
         """Rows of the resident one-hot distance slab (internal row and sample order) as the last

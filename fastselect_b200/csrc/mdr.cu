@@ -20,6 +20,11 @@
 //            fold bests.  Every comparison is on (score, index), a total order, so the result does not
 //            depend on which block saw which pair.
 // fs_mdr_tables counts the per-segment tables of chosen combinations from the same planes.
+//
+// fs_interaction_scan (DESIGN.md section 11) is the same pack, scan and merge with a single fold, so the two
+// segments are the two classes, and another evaluation policy: the KSA statistic of BOOST from the two
+// class tables instead of balanced accuracies, and no fold bests.  The tables of the listed pairs follow
+// from mdr_tables_kernel on the same planes.
 #include <algorithm>
 #include <climits>
 #include <cmath>
@@ -106,9 +111,9 @@ struct MdrScanArgs {
     const int32_t *start;                           // [n_kept + 1] first reduced row of every position
     int64_t W, n_kept, n_tiles, tiles_side;
     int n_top;
-    double *all_train, *all_test;                   // [n_combos] or null
+    double *all_train, *all_test;                   // [n_combos] or null: cand.train (MDR only), cand.score
     MdrCand *top_out;                               // [gridDim.x, n_top]
-    MdrCand *fold_out;                              // [gridDim.x, n_folds]
+    MdrCand *fold_out;                              // [gridDim.x, n_folds] (MDR only)
 };
 
 // Full 3 x 3 table of one segment, cell va * 3 + vb, from the pair's reduced counts c[i][j] and the
@@ -193,6 +198,83 @@ __device__ __forceinline__ void mdr_evaluate(int la, int lb, int ka, int kb, con
     mean_test = acc_test / (double)NF;
 }
 
+// KSA statistic of one pair from its class tables t[k][i * 3 + j] and class sizes nk[k], in the operation
+// order of DESIGN.md section 11 (cells in (i, j, k) order, products left to right).  The explicit
+// round-to-nearest intrinsics keep the compiler from contracting the sum into FMAs, so the order holds.
+__device__ __forceinline__ double ksa_statistic(const int32_t (&t)[2][9], const int32_t (&nk)[2]) {
+    int32_t ni[3], nj[3], nik[3][2], njk[3][2];
+#pragma unroll
+    for (int i = 0; i < 3; ++i) {
+        ni[i] = nj[i] = 0;
+        nik[i][0] = nik[i][1] = njk[i][0] = njk[i][1] = 0;
+    }
+#pragma unroll
+    for (int i = 0; i < 3; ++i)
+#pragma unroll
+        for (int j = 0; j < 3; ++j)
+#pragma unroll
+            for (int k = 0; k < 2; ++k) {
+                const int32_t v = t[k][i * 3 + j];
+                ni[i] += v;
+                nj[j] += v;
+                nik[i][k] += v;
+                njk[j][k] += v;
+            }
+    double q[18];
+    double eta = 0.0;
+#pragma unroll
+    for (int i = 0; i < 3; ++i)
+#pragma unroll
+        for (int j = 0; j < 3; ++j)
+#pragma unroll
+            for (int k = 0; k < 2; ++k) {
+                const int32_t nij = t[0][i * 3 + j] + t[1][i * 3 + j];
+                double v = 0.0;
+                if (nij > 0 && nik[i][k] > 0 && njk[j][k] > 0)
+                    v = __dmul_rn(__dmul_rn((double)nij, (double)nik[i][k]), (double)njk[j][k]) /
+                        __dmul_rn(__dmul_rn((double)ni[i], (double)nj[j]), (double)nk[k]);
+                q[(i * 3 + j) * 2 + k] = v;
+                eta = __dadd_rn(eta, v);
+            }
+    const double N = (double)(nk[0] + nk[1]);
+    double L = 0.0;
+#pragma unroll
+    for (int g = 0; g < 18; ++g) {
+        const int32_t n = t[g & 1][g >> 1];
+        if (n > 0) L = __dadd_rn(L, __dmul_rn((double)n, log(__dmul_rn((double)n, eta) / __dmul_rn(N, q[g]))));
+    }
+    return 2.0 * L;
+}
+
+// Evaluation policies of mdr_scan_kernel: eval turns a pair's (or column's) per-segment counts into the
+// candidate's score (the top-list key) and train value, and the fold bests of the NF folds it reports in train.
+template <int NSEG>
+struct MdrEval {                                    // MDR: mean test / training balanced accuracy, fold bests
+    static constexpr int NF = NSEG / 2;
+    static __device__ __forceinline__ void eval(int la, int lb, int ka, int kb, const int32_t *__restrict__ marg,
+                                                const MdrSeg &seg, const uint32_t (&c)[NSEG][4], double (&train)[NF],
+                                                MdrCand &cand) {
+        mdr_evaluate<NSEG>(la, lb, ka, kb, marg, seg, c, train, cand.train, cand.score);
+    }
+};
+
+struct KsaEval {                                    // one fold, segments = classes: L_KSA, no fold bests
+    static constexpr int NF = 0;
+    static __device__ __forceinline__ void eval(int la, int lb, int ka, int kb, const int32_t *__restrict__ marg,
+                                                const MdrSeg &seg, const uint32_t (&c)[2][4], double (&)[1],
+                                                MdrCand &cand) {
+        auto m = [&](int k, int have, int s) -> int32_t { return have ? __ldg(marg + (int64_t)k * 2 + s) : 0; };
+        int32_t t[2][9];
+#pragma unroll
+        for (int s = 0; s < 2; ++s)
+            seg_table(la, lb, m(ka, la > 0, s), m(ka + 1, la > 1, s), m(kb, lb > 0, s), m(kb + 1, lb > 1, s), c[s][0],
+                      c[s][1], c[s][2], c[s][3], seg.n[s], t[s]);
+        const int32_t nk[2] = {seg.n[0], seg.n[1]};
+        cand.score = ksa_statistic(t, nk);
+        cand.train = 0.0;
+    }
+};
+
 // first linear tile of tile row i of the upper triangle (T tile rows): i * T - i (i - 1) / 2
 __device__ __forceinline__ int64_t tri_off(int64_t i, int64_t T) { return i * T - i * (i - 1) / 2; }
 
@@ -202,9 +284,10 @@ __host__ __device__ inline size_t mdr_smem_bytes(bool pair, int n_top) {
            (2 * (size_t)n_top + 2 * kMdrThreads) * sizeof(MdrCand);
 }
 
-template <int NSEG, bool PAIR>
+template <int NSEG, bool PAIR, class Eval>
 __global__ void __launch_bounds__(kMdrThreads) mdr_scan_kernel(const MdrScanArgs args, const MdrSeg seg) {
-    constexpr int NF = NSEG / 2;
+    constexpr int NF = Eval::NF;
+    constexpr int NFA = NF > 0 ? NF : 1;              // array extent: KsaEval keeps no fold bests
     extern __shared__ __align__(16) unsigned char smem[];
     uint32_t *stile = reinterpret_cast<uint32_t *>(smem);                 // [4 * kMdrTile rows][kMdrLd]: A rows, then B rows
     MdrCand *list = reinterpret_cast<MdrCand *>(smem + (PAIR ? (size_t)4 * kMdrTile * kMdrLd * sizeof(uint32_t) : 0));
@@ -213,8 +296,8 @@ __global__ void __launch_bounds__(kMdrThreads) mdr_scan_kernel(const MdrScanArgs
     MdrCand *sbuf = buf + kMdrThreads;
     __shared__ int s_rows[4 * kMdrTile];              // plane row of every staged row, -1: none
     __shared__ int s_cnt, s_nbuf;
-    __shared__ double s_fb[kMdrThreads / 32][NF];     // per warp: best training BA of every fold
-    __shared__ long long s_fi[kMdrThreads / 32][NF];
+    __shared__ double s_fb[kMdrThreads / 32][NFA];    // per warp: best training BA of every fold
+    __shared__ long long s_fi[kMdrThreads / 32][NFA];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int tx = tid % kMdrTile, ty = tid / kMdrTile;
     if (tid == 0) {
@@ -294,16 +377,16 @@ __global__ void __launch_bounds__(kMdrThreads) mdr_scan_kernel(const MdrScanArgs
             }
         }
         MdrCand cand{-INFINITY, 0.0, LLONG_MAX};
-        double train[NF];
+        double train[NFA];
 #pragma unroll
         for (int f = 0; f < NF; ++f) train[f] = -INFINITY;
         if (valid) {
             const int ka = args.start[a], la = args.start[a + 1] - ka;
             const int kb = PAIR ? args.start[b] : 0, lb = PAIR ? args.start[b + 1] - kb : 0;
-            mdr_evaluate<NSEG>(la, lb, ka, kb, args.marg, seg, c, train, cand.train, cand.score);
+            Eval::eval(la, lb, ka, kb, args.marg, seg, c, train, cand);
             cand.idx = PAIR ? (long long)(a * nk - a * (a + 1) / 2 + (b - a - 1)) : (long long)a;
-            if (args.all_train) {
-                args.all_train[cand.idx] = cand.train;
+            if (args.all_test) {
+                if (NF > 0) args.all_train[cand.idx] = cand.train;
                 args.all_test[cand.idx] = cand.score;
             }
         }
@@ -448,12 +531,14 @@ __global__ void __launch_bounds__(128) mdr_tables_kernel(const uint32_t *__restr
 
 // Encode (the shared discrete operand) + pack of (feat_idx, fold); the planes are kept for the operand's
 // generation and the folds.
-void mdr_prepare(fs_dataset *ds, const int64_t *feat_idx, int64_t n_kept, const int32_t *fold, int n_folds, int *launches) {
-    FS_REQUIRE(ds->n_classes == 2, FS_ERR_INVALID, "mdr: the data set must have 2 classes (has %d)", ds->n_classes);
+// `what` names the caller in error messages.
+void mdr_prepare(fs_dataset *ds, const int64_t *feat_idx, int64_t n_kept, const int32_t *fold, int n_folds, int *launches,
+                 const char *what = "mdr") {
+    FS_REQUIRE(ds->n_classes == 2, FS_ERR_INVALID, "%s: the data set must have 2 classes (has %d)", what, ds->n_classes);
     const int64_t n = ds->n;
-    // balanced accuracies are ratios of integers below 2^53 (2 N1 N0 < 2^53)
-    FS_REQUIRE(n < (1LL << 26), FS_ERR_INVALID, "mdr: n = %lld exceeds 2^26 samples", (long long)n);
-    const DiscreteOperand &op = discrete_operand(ds, feat_idx, n_kept, 3, "mdr", false, launches);
+    // balanced accuracies are ratios of integers below 2^53 (2 N1 N0 < 2^53); KSA products of two counts too
+    FS_REQUIRE(n < (1LL << 26), FS_ERR_INVALID, "%s: n = %lld exceeds 2^26 samples", what, (long long)n);
+    const DiscreteOperand &op = discrete_operand(ds, feat_idx, n_kept, 3, what, false, launches);
     const int nseg = 2 * n_folds;
     std::vector<int64_t> key(1 + n);
     key[0] = n_folds;
@@ -466,14 +551,14 @@ void mdr_prepare(fs_dataset *ds, const int64_t *feat_idx, int64_t n_kept, const 
     std::vector<int64_t> seg_n(nseg, 0);
     for (int64_t r = 0; r < n; ++r) {
         const int32_t f = fold[ds->perm[r]];
-        FS_REQUIRE(f >= 0 && f < n_folds, FS_ERR_INVALID, "mdr: fold[%lld] = %d outside [0, %d)", (long long)ds->perm[r], f,
-                   n_folds);
+        FS_REQUIRE(f >= 0 && f < n_folds, FS_ERR_INVALID, "%s: fold[%lld] = %d outside [0, %d)", what,
+                   (long long)ds->perm[r], f, n_folds);
         ++seg_n[2 * f + ds->y_sorted[r]];
     }
     MdrSeg &seg = ds->mdr_seg;
     seg.w[0] = 0;
     for (int s = 0; s < nseg; ++s) {
-        FS_REQUIRE(seg_n[s] > 0, FS_ERR_INVALID, "mdr: fold %d has no sample of class %d", s / 2, s & 1);
+        FS_REQUIRE(seg_n[s] > 0, FS_ERR_INVALID, "%s: fold %d has no sample of class %d", what, s / 2, s & 1);
         seg.n[s] = (int32_t)seg_n[s];
         seg.w[s + 1] = seg.w[s] + (int32_t)ceil_div(seg_n[s], 32);
     }
@@ -514,9 +599,9 @@ void mdr_prepare(fs_dataset *ds, const int64_t *feat_idx, int64_t n_kept, const 
     ds->mdr_gen = op.generation;
 }
 
-template <int NSEG, bool PAIR>
+template <int NSEG, bool PAIR, class Eval>
 int64_t launch_scan_t(const MdrScanArgs &args, const MdrSeg &seg, int sms, int64_t max_blocks, cudaStream_t st) {
-    auto kern = mdr_scan_kernel<NSEG, PAIR>;
+    auto kern = mdr_scan_kernel<NSEG, PAIR, Eval>;
     const size_t smem = mdr_smem_bytes(PAIR, args.n_top);
     FS_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int per_sm = 0;
@@ -530,10 +615,11 @@ int64_t launch_scan_t(const MdrScanArgs &args, const MdrSeg &seg, int sms, int64
 
 template <int NSEG>
 int64_t launch_scan_n(bool pair, const MdrScanArgs &args, const MdrSeg &seg, int sms, int64_t max_blocks, cudaStream_t st) {
-    return pair ? launch_scan_t<NSEG, true>(args, seg, sms, max_blocks, st)
-                : launch_scan_t<NSEG, false>(args, seg, sms, max_blocks, st);
+    return pair ? launch_scan_t<NSEG, true, MdrEval<NSEG>>(args, seg, sms, max_blocks, st)
+                : launch_scan_t<NSEG, false, MdrEval<NSEG>>(args, seg, sms, max_blocks, st);
 }
 
+// MDR scan of order 1 or 2 over nseg = 2 n_folds segments
 int64_t launch_scan(int nseg, bool pair, const MdrScanArgs &args, const MdrSeg &seg, int sms, int64_t max_blocks,
                     cudaStream_t st) {
     switch (nseg) {
@@ -558,6 +644,87 @@ void check_common(fs_dataset *ds, int64_t n_kept, int order, const int32_t *fold
                (long long)n_kept, order);
     FS_REQUIRE(n_folds >= 2 && n_folds <= kMdrMaxFolds, FS_ERR_INVALID, "mdr: n_folds = %d outside [2, %d]", n_folds,
                kMdrMaxFolds);
+}
+
+// Scan of the prepared planes and the merges of the block lists (plus, for MDR, the fold-best reduction):
+// ksa selects the evaluation policy.  all (device, nullable): [2, n_combos] for MDR, [n_combos] for KSA.
+// Returns the merged list (device, n_top entries) and sets *blocks to the scan's grid.
+MdrCand *run_scan(fs_dataset *ds, int64_t n_kept, int order, int64_t n_top, bool ksa, double *all, PhaseTimer &tm,
+                  int *launches, int64_t *blocks) {
+    cudaStream_t st = ds->stream;
+    const int nseg = ds->mdr_nseg, n_folds = ksa ? 0 : nseg / 2;
+    tm.begin(&fs_stats::ms_dist_general);
+    int sms = 0;
+    FS_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, ds->device));
+    MdrScanArgs args{};
+    args.planes = ds->mdr_planes.ptr;
+    args.marg = ds->mdr_marg.ptr;
+    args.start = ds->disc.start.ptr;
+    args.W = ds->mdr_W;
+    args.n_kept = n_kept;
+    args.n_top = (int)n_top;
+    if (order == 2) {
+        args.tiles_side = ceil_div(n_kept, kMdrTile);
+        args.n_tiles = args.tiles_side * (args.tiles_side + 1) / 2;
+    } else {
+        args.tiles_side = 0;
+        args.n_tiles = ceil_div(n_kept, kMdrThreads);
+    }
+    if (all) {
+        args.all_train = ksa ? nullptr : all;
+        args.all_test = ksa ? all : all + mdr_combos(n_kept, order);
+    }
+    // at most as many blocks as the SMs hold at once (persistent), and never more than there are tiles
+    const int64_t max_blocks = 16LL * sms;
+    ds->mdr_top.reserve(2 * (size_t)max_blocks * n_top * sizeof(MdrCand));
+    ds->mdr_fold.reserve((size_t)max_blocks * std::max(n_folds, 1) * sizeof(MdrCand));
+    ds->mdr_best.reserve(kMdrMaxFolds);
+    args.top_out = reinterpret_cast<MdrCand *>(ds->mdr_top.ptr);
+    args.fold_out = reinterpret_cast<MdrCand *>(ds->mdr_fold.ptr);
+    static_assert(sizeof(MdrCand) == 24, "MdrCand layout");
+    const int64_t G = ksa ? launch_scan_t<2, true, KsaEval>(args, ds->mdr_seg, sms, max_blocks, st)
+                          : launch_scan(nseg, order == 2, args, ds->mdr_seg, sms, max_blocks, st);
+    ++*launches;
+    tm.end();
+    tm.begin(&fs_stats::ms_reduce);
+    MdrCand *cur = args.top_out, *nxt = cur + max_blocks * n_top;
+    for (int64_t L = G; L > 1; L = ceil_div(L, 2)) {
+        mdr_merge_kernel<<<(unsigned)ceil_div(L, 2), 256, 0, st>>>(cur, L, (int)n_top, nxt);
+        FS_CUDA(cudaGetLastError());
+        ++*launches;
+        std::swap(cur, nxt);
+    }
+    if (!ksa) {
+        mdr_fold_best_kernel<<<1, 32, 0, st>>>(args.fold_out, G, n_folds, ds->mdr_best.ptr);
+        FS_CUDA(cudaGetLastError());
+        ++*launches;
+    }
+    tm.end();
+    *blocks = G;
+    return cur;
+}
+
+void scan_stats(fs_stats *stats, PhaseTimer &tm, int launches, int64_t G, const fs_dataset *ds, int64_t n_combos) {
+    memset(stats, 0, sizeof(*stats));
+    tm.finish(stats);
+    stats->launches = launches;
+    stats->n_chunks = (int32_t)G;
+    stats->n_tensor_cols = ds->ws.pt;
+    stats->onehot_k = ds->ws.K_used;
+    stats->pairs_selected = n_combos;
+}
+
+// Positions (a, b) of the order-2 combination index idx over n positions: a from the quadratic, then exact
+// integer fix-ups (the inverse of the scan's a * n - a (a + 1) / 2 + (b - a - 1)).
+void decode_pair(int64_t idx, int64_t n, int64_t *a, int64_t *b) {
+    auto off = [n](int64_t v) { return v * n - v * (v + 1) / 2; };
+    const double q = 2.0 * (double)n - 1.0;
+    int64_t v = (int64_t)std::floor((q - std::sqrt(std::max(q * q - 8.0 * (double)idx, 0.0))) * 0.5);
+    v = std::min<int64_t>(std::max<int64_t>(v, 0), std::max<int64_t>(n - 2, 0));
+    while (v > 0 && off(v) > idx) --v;
+    while (v + 1 < n - 1 && off(v + 1) <= idx) ++v;
+    *a = v;
+    *b = idx - off(v) + v + 1;
 }
 
 }  // namespace
@@ -588,59 +755,20 @@ int fs_mdr_scan(fs_dataset *ds, const int64_t *feat_idx, int64_t n_kept, int32_t
         tm.begin(&fs_stats::ms_gather);
         mdr_prepare(ds, feat_idx, n_kept, fold, n_folds, &launches);
         tm.end();
-        tm.begin(&fs_stats::ms_dist_general);
-        const int nseg = ds->mdr_nseg;
-        int sms = 0;
-        FS_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, ds->device));
-        MdrScanArgs args{};
-        args.planes = ds->mdr_planes.ptr;
-        args.marg = ds->mdr_marg.ptr;
-        args.start = ds->disc.start.ptr;
-        args.W = ds->mdr_W;
-        args.n_kept = n_kept;
-        args.n_top = (int)n_top;
-        if (order == 2) {
-            args.tiles_side = ceil_div(n_kept, kMdrTile);
-            args.n_tiles = args.tiles_side * (args.tiles_side + 1) / 2;
-        } else {
-            args.tiles_side = 0;
-            args.n_tiles = ceil_div(n_kept, kMdrThreads);
-        }
+        double *all = nullptr;
         if (all_train) {
             ds->mdr_all.reserve(2 * (size_t)n_combos);
-            args.all_train = ds->mdr_all.ptr;
-            args.all_test = ds->mdr_all.ptr + n_combos;
+            all = ds->mdr_all.ptr;
         }
-        // at most as many blocks as the SMs hold at once (persistent), and never more than there are tiles
-        const int64_t max_blocks = 16LL * sms;
-        ds->mdr_top.reserve(2 * (size_t)max_blocks * n_top * sizeof(MdrCand));
-        ds->mdr_fold.reserve((size_t)max_blocks * n_folds * sizeof(MdrCand));
-        ds->mdr_best.reserve(kMdrMaxFolds);
-        args.top_out = reinterpret_cast<MdrCand *>(ds->mdr_top.ptr);
-        args.fold_out = reinterpret_cast<MdrCand *>(ds->mdr_fold.ptr);
-        static_assert(sizeof(MdrCand) == 24, "MdrCand layout");
-        const int64_t G = launch_scan(nseg, order == 2, args, ds->mdr_seg, sms, max_blocks, st);
-        ++launches;
-        tm.end();
-        tm.begin(&fs_stats::ms_reduce);
-        MdrCand *cur = args.top_out, *nxt = cur + max_blocks * n_top;
-        for (int64_t L = G; L > 1; L = ceil_div(L, 2)) {
-            mdr_merge_kernel<<<(unsigned)ceil_div(L, 2), 256, 0, st>>>(cur, L, (int)n_top, nxt);
-            FS_CUDA(cudaGetLastError());
-            ++launches;
-            std::swap(cur, nxt);
-        }
-        mdr_fold_best_kernel<<<1, 32, 0, st>>>(args.fold_out, G, n_folds, ds->mdr_best.ptr);
-        FS_CUDA(cudaGetLastError());
-        ++launches;
-        tm.end();
+        int64_t G = 0;
+        const MdrCand *cur = run_scan(ds, n_kept, order, n_top, false, all, tm, &launches, &G);
         tm.stop();          // ms_total ends before the results are copied back
         std::vector<MdrCand> top(n_top);
         FS_CUDA(cudaMemcpyAsync(top.data(), cur, n_top * sizeof(MdrCand), cudaMemcpyDeviceToHost, st));
         FS_CUDA(cudaMemcpyAsync(fold_best, ds->mdr_best.ptr, n_folds * sizeof(long long), cudaMemcpyDeviceToHost, st));
         if (all_train) {
-            FS_CUDA(cudaMemcpyAsync(all_train, args.all_train, n_combos * sizeof(double), cudaMemcpyDeviceToHost, st));
-            FS_CUDA(cudaMemcpyAsync(all_test, args.all_test, n_combos * sizeof(double), cudaMemcpyDeviceToHost, st));
+            FS_CUDA(cudaMemcpyAsync(all_train, all, n_combos * sizeof(double), cudaMemcpyDeviceToHost, st));
+            FS_CUDA(cudaMemcpyAsync(all_test, all + n_combos, n_combos * sizeof(double), cudaMemcpyDeviceToHost, st));
         }
         FS_CUDA(cudaStreamSynchronize(st));
         for (int64_t i = 0; i < n_top; ++i) {
@@ -648,15 +776,7 @@ int fs_mdr_scan(fs_dataset *ds, const int64_t *feat_idx, int64_t n_kept, int32_t
             top_test[i] = top[i].score;
             top_train[i] = top[i].train;
         }
-        if (stats) {
-            memset(stats, 0, sizeof(*stats));
-            tm.finish(stats);
-            stats->launches = launches;
-            stats->n_chunks = (int32_t)G;
-            stats->n_tensor_cols = ds->ws.pt;
-            stats->onehot_k = ds->ws.K_used;
-            stats->pairs_selected = n_combos;
-        }
+        if (stats) scan_stats(stats, tm, launches, G, ds, n_combos);
         return FS_OK;
     });
 }
@@ -689,6 +809,60 @@ int fs_mdr_tables(fs_dataset *ds, const int64_t *feat_idx, int64_t n_kept, int32
         FS_CUDA(cudaGetLastError());
         FS_CUDA(cudaMemcpyAsync(tables_out, ds->mdr_tables.ptr, cells * sizeof(int64_t), cudaMemcpyDeviceToHost, st));
         FS_CUDA(cudaStreamSynchronize(st));
+        return FS_OK;
+    });
+}
+
+int fs_interaction_scan(fs_dataset *ds, const int64_t *feat_idx, int64_t n_kept, int64_t n_top, int64_t *top_idx,
+                        double *top_ksa, int64_t *top_tables, double *all_ksa, fs_stats *stats) {
+    return api_call("fs_interaction_scan", [&] {
+        FS_REQUIRE(ds, FS_ERR_INVALID, "fs_interaction_scan: null data set");
+        if (!feat_idx) n_kept = ds->p;
+        FS_REQUIRE(top_idx && top_ksa && top_tables, FS_ERR_INVALID, "fs_interaction_scan: null output");
+        FS_REQUIRE(n_kept >= 2, FS_ERR_INVALID, "fs_interaction_scan: %lld columns form no pair", (long long)n_kept);
+        const int64_t n_pairs = mdr_combos(n_kept, 2);
+        FS_REQUIRE(n_top >= 1 && n_top <= std::min<int64_t>(FS_MDR_MAX_TOP, n_pairs), FS_ERR_INVALID,
+                   "fs_interaction_scan: n_top = %lld outside [1, min(%d, %lld pairs)]", (long long)n_top, FS_MDR_MAX_TOP,
+                   (long long)n_pairs);
+        FS_CUDA(cudaSetDevice(ds->device));
+        alloc_stream() = ds->stream;
+        cudaStream_t st = ds->stream;
+        int launches = 0;
+        PhaseTimer tm(stats != nullptr, st);
+        tm.begin(&fs_stats::ms_gather);
+        const std::vector<int32_t> fold(ds->n, 0);     // one fold: the segments are the two classes
+        mdr_prepare(ds, feat_idx, n_kept, fold.data(), 1, &launches, "interaction");
+        tm.end();
+        double *all = nullptr;
+        if (all_ksa) {
+            ds->mdr_all.reserve((size_t)n_pairs);
+            all = ds->mdr_all.ptr;
+        }
+        int64_t G = 0;
+        const MdrCand *cur = run_scan(ds, n_kept, 2, n_top, true, all, tm, &launches, &G);
+        tm.stop();          // ms_total ends before the results are copied back and the tables counted
+        std::vector<MdrCand> top(n_top);
+        FS_CUDA(cudaMemcpyAsync(top.data(), cur, n_top * sizeof(MdrCand), cudaMemcpyDeviceToHost, st));
+        if (all_ksa) FS_CUDA(cudaMemcpyAsync(all_ksa, all, n_pairs * sizeof(double), cudaMemcpyDeviceToHost, st));
+        FS_CUDA(cudaStreamSynchronize(st));
+        std::vector<int64_t> pairs(2 * n_top);
+        for (int64_t i = 0; i < n_top; ++i) {
+            top_idx[i] = top[i].idx;
+            top_ksa[i] = top[i].score;
+            decode_pair(top[i].idx, n_kept, &pairs[2 * i], &pairs[2 * i + 1]);
+        }
+        ds->mdr_combos.reserve((size_t)n_top * 2);
+        ds->mdr_tables.reserve((size_t)n_top * 2 * 9);
+        FS_CUDA(cudaMemcpyAsync(ds->mdr_combos.ptr, pairs.data(), pairs.size() * sizeof(int64_t), cudaMemcpyHostToDevice, st));
+        mdr_tables_kernel<<<(unsigned)ceil_div(n_top * 2, 128), 128, 0, st>>>(ds->mdr_planes.ptr, ds->mdr_W, ds->mdr_marg.ptr,
+                                                                              ds->disc.start.ptr, ds->mdr_seg, 2,
+                                                                              ds->mdr_combos.ptr, 2, n_top, ds->mdr_tables.ptr);
+        FS_CUDA(cudaGetLastError());
+        ++launches;
+        FS_CUDA(cudaMemcpyAsync(top_tables, ds->mdr_tables.ptr, (size_t)n_top * 2 * 9 * sizeof(int64_t),
+                                cudaMemcpyDeviceToHost, st));
+        FS_CUDA(cudaStreamSynchronize(st));
+        if (stats) scan_stats(stats, tm, launches, G, ds, n_pairs);
         return FS_OK;
     });
 }

@@ -32,7 +32,7 @@ extern "C" {
 #define FS_API
 #endif
 
-#define FS_ABI_VERSION 8
+#define FS_ABI_VERSION 9
 /* distinct values tracked per column by fs_dataset_create; a column with more
  * distinct values reports FS_DISTINCT_CAP + 1 */
 #define FS_DISTINCT_CAP 16
@@ -292,6 +292,31 @@ FS_API int fs_mdr_scan(fs_dataset *ds, const int64_t *feat_idx, int64_t n_kept, 
                        int64_t *fold_best, double *all_train, double *all_test, fs_stats *stats);
 FS_API int fs_mdr_tables(fs_dataset *ds, const int64_t *feat_idx, int64_t n_kept, int32_t order, const int32_t *fold,
                          int32_t n_folds, const int64_t *combos, int64_t m, int64_t *tables_out);
+
+/*
+ * Two-locus interaction screen (the KSA stage of BOOST; the semantics are this project's own, see DESIGN.md
+ * section 11): every pair (a, b), a < b, of the positions of feat_idx (NULL = all p) on the MDR planes of a
+ * single fold, so the two segments are the two classes.  The data set's y_enc is the class (n_classes must
+ * be 2); every scanned column must be discrete in fs_dataset_set_features and hold at most 3 distinct
+ * values (FS_ERR_INVALID otherwise); a column's state is the rank of its value among its sorted distinct
+ * values; n < 2^26.  Pair index: the order-2 index of fs_mdr_scan.
+ *
+ * Per pair, with n_ijk the samples of state i in a, state j in b and class k, and N = n:
+ *   q_ijk = (n_ij * n_ik * n_jk) / (n_i * n_j * n_k), 0 when a numerator margin is 0;   eta = sum q_ijk;
+ *   L_KSA = 2 * sum_{n_ijk > 0} n_ijk * log(n_ijk * eta / (N * q_ijk)),
+ * all in float64, the sums in cell order (i, j, k).  L_KSA bounds the likelihood-ratio statistic of the
+ * no-three-way-interaction model from above (G <= L_KSA).
+ *
+ * fs_interaction_scan: top_idx / top_ksa [n_top]: the n_top pairs with the highest L_KSA (lower index first
+ *   on ties); 1 <= n_top <= min(FS_MDR_MAX_TOP, n_pairs), n_pairs = n_kept * (n_kept - 1) / 2.
+ *   top_tables[(q * 2 + k) * 9 + i * 3 + j], int64 [n_top, 2, 9]: n_ijk of listed pair q, exact.  all_ksa
+ *   (nullable, [n_pairs] host array): L_KSA of every pair.  The bit-planes are those of fs_mdr_scan with the
+ *   fold vector of all zeros (built by the first call, reused by later ones).  In stats: ms_gather = encode +
+ *   pack (about 0 on a reuse), ms_dist_general = scan kernel, ms_reduce = merges, n_chunks = scan blocks,
+ *   pairs_selected = n_pairs; ms_total ends before the tables of the listed pairs are counted.
+ */
+FS_API int fs_interaction_scan(fs_dataset *ds, const int64_t *feat_idx, int64_t n_kept, int64_t n_top, int64_t *top_idx,
+                               double *top_ksa, int64_t *top_tables, double *all_ksa, fs_stats *stats);
 
 /*
  * Parity/debug view of the RESIDENT one-hot distance slab fs_score keeps between calls for TuRF's
