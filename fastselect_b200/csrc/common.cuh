@@ -211,8 +211,9 @@ enum : unsigned { kColContinuous = 0, kColTensor = 1, kColCompare = 2, kColConst
 
 // How the one-hot distance slab of a call is obtained: computed from scratch, updated by
 // subtracting the contribution of the columns removed since the cached slab (TuRF iterations:
-// d_ij -= sum over removed f of [x_if != x_jf], exact integers), or reused as it is.
-enum DistMode : int { kDistFull = 0, kDistIncremental = 1, kDistReuse = 2 };
+// d_ij -= sum over removed f of [x_if != x_jf], exact integers), or reused as it is.  kDistNone:
+// the call computes no distances (the joint-count and MDR paths read only At).
+enum DistMode : int { kDistNone = -1, kDistFull = 0, kDistIncremental = 1, kDistReuse = 2 };
 
 // Who owns which target rows (one process per GPU) and where their distance slabs live; passed
 // by value to the distance kernel.  A single rank is the trivial case {starts = {0, n}}.
@@ -281,10 +282,10 @@ struct WorkSet {
     std::vector<int64_t> h_gcol, h_gout;
     std::vector<uint8_t> h_ctype;
     std::vector<float> h_rg;
-    // cache of the column lists of an all-columns call (see build_workset)
-    bool lists_all = false, lists_uploaded = false;
-    uint64_t lists_typing = 0, lists_version = 0;
-    int64_t lists_flags = -1, lists_n = -1;
+    // the column lists are those of `key` under the typing lists_typing (see build_lists)
+    std::vector<int64_t> key;
+    bool lists_uploaded = false;
+    uint64_t lists_typing = ~0ull, lists_version = 0;
     int64_t n_cont = 0, n_cmp = 0;
     // one-hot tensor-core path (filled by onehot.cu).  A column with V distinct values owns
     // V - 1 "reduced" one-hot rows (values 0..V-2); the last value is implied (see onehot.cu)
@@ -320,9 +321,7 @@ struct WorkSet {
     DevBuf<int32_t> roff;
     DevBuf<int8_t> Ur, Wdr;         // [n, Kr]
     DevBuf<int32_t> srow_r;         // [n]
-    // cache key
-    std::vector<int64_t> key;
-    bool valid = false;
+    bool valid = false;             // the operands are those of the column lists
     uint64_t build_id = 0;          // bumped by every rebuild: state derived from At is stale when it changes
     // feature-sharded accumulation (multi-GPU group): At / codesT / krow hold only the tensor columns
     // [a0, a1) of the active list -- this rank's share -- with one-hot rows numbered from 0
@@ -331,7 +330,27 @@ struct WorkSet {
     DevBuf<int32_t> atoff;         // [a1 - a0 + 1] first reduced row of each slice column, from 0
     PinnedBuf<int32_t> p_atoff;
     bool acc_split = false;
-    bool group_call = false;       // built for a collective call of a multi-GPU group (restricted Wd rows)
+};
+
+// What the one-hot distance slab holds after the last call (kept for TuRF's incremental distance update):
+// the buffer, the tensor-path columns it sums over and the target rows it covers
+struct SlabCache {
+    bool valid = false;
+    const int32_t *buf = nullptr;
+    std::vector<int64_t> cols;
+    uint64_t version = ~0ull;       // WorkSet::lists_version cols were filled for
+    int64_t r0 = -1, R = -1;
+    void forget() { valid = false; }
+    void record(const int32_t *b, const WorkSet &ws, int64_t r0_, int64_t R_) {
+        buf = b;
+        if (version != ws.lists_version || (int64_t)cols.size() != ws.pt) {
+            cols.assign(ws.p_tcol.ptr, ws.p_tcol.ptr + ws.pt);
+            version = ws.lists_version;
+        }
+        r0 = r0_;
+        R = R_;
+        valid = true;
+    }
 };
 
 }  // namespace fs
@@ -409,7 +428,7 @@ struct fs_dataset {
     // typing
     bool have_features = false;
     uint64_t typing_epoch = 0;               // bumped whenever the typing (or the group's column shares) changes
-    uint64_t ct_version = ~0ull, dd_version = ~0ull;   // WorkSet::lists_version ct_pos / dd_cols were filled for
+    uint64_t ct_version = ~0ull;             // WorkSet::lists_version ct_pos was filled for
     int arith = FS_ARITH_F32;
     std::vector<uint8_t> is_discrete;
     std::vector<float> recip;
@@ -421,19 +440,11 @@ struct fs_dataset {
     fs::WorkSet ws;
     fs::DevBuf<double> Dc;        // [R, ldn] continuous/general distance part
     fs::DevBuf<int32_t> Dd;       // [R, ldn] one-hot mismatch counts
-    // what Dd holds after the last call (kept for TuRF's incremental distance update):
-    // the tensor-path columns it sums over and the target rows it covers
-    bool dd_valid = false;
-    std::vector<int64_t> dd_cols;
-    int64_t dd_r0 = -1, dd_R = -1;
-    const int32_t *dd_buf = nullptr;
-    // multi-GPU symmetric distances (fs_dataset_set_peers): this rank's IPC-exportable slab, the
-    // peers' mapped slabs, and the cross-rank barrier called between distances and selection
+    fs::SlabCache slab;           // what Dd or peer_slab holds after the last call
+    // multi-GPU symmetric distances (fs_dataset_attach_comm): this rank's slab in its arena and the
+    // peers' mapped slabs
     fs::DistPeers peers{};
-    bool peers_on = false;
     int32_t *peer_slab = nullptr;
-    size_t peer_slab_count = 0;
-    bool last_dist_exchanged = false;        // the last distance launch stored into peer slabs
     fs::DevBuf<int8_t> sel;       // [R, ldn] neighbour codes
     fs::DevBuf<fs::RowInfo> rinfo;
     fs::DevBuf<int64_t> row_ids;
@@ -454,7 +465,6 @@ struct fs_dataset {
     fs::GroupLayout glayout{};
     fs::DevBuf<int64_t> all_ids;             // 0 .. n-1 (the sharded accumulation runs over all target rows)
     std::vector<int64_t> all_ids_h;
-    std::vector<int64_t> tcol_all_sorted;    // tensor-path columns of the whole data set (ascending): static ownership
     std::vector<int64_t> owner_bound;        // [world + 1] original-column boundaries of the ranks' accumulation shares
     fs::DevBuf<int8_t> a_gather;  // gathered one-hot target rows (fs_debug_rows)
     // ReliefF reference tie order (select.cu): compacted list of tied rows, [R, n] (key, index) pairs
@@ -491,14 +501,16 @@ struct fs_dataset {
 
 namespace fs {
 
-// dataset.cu
-// r0 / R / slab_cacheable: the (contiguous) target rows of this call and whether their distance
-// slab fits one chunk -- decides between a full, an incremental and no distance computation
-// want_split: a multi-GPU group call that may shard the accumulation by one-hot columns (WorkSet::acc_split)
-// dist_ops: build the distance operands U / Wd / srow too (the joint-count and MDR paths read only At)
-void build_workset(fs_dataset *ds, const int64_t *feat_idx, int64_t n_kept, bool need_codes,
-                   int64_t r0, int64_t R, bool contiguous, bool slab_cacheable, bool want_split, bool group_call,
-                   bool dist_ops, int *launches);
+// dataset.cu: the working set of the columns feat_idx (all p columns when null), in two halves.
+// build_lists: the columns split by path, the accumulation slice of a multi-GPU group call that may shard the
+// accumulation by one-hot columns (want_split; WorkSet::acc_split), uploaded; kept while the call's columns,
+// flags and the typing stay.  Marks the operands stale when the lists change.
+void build_lists(fs_dataset *ds, const int64_t *feat_idx, int64_t n_kept, bool want_split, bool group_call);
+// build_operands: the general columns gathered and the one-hot operands (build_onehot) for the distance mode
+// `dist_mode` of target rows [u_lo, u_hi), unless the operands built last serve; those being the full distance
+// operands, an incremental update becomes a full computation.  Sets ws.dist_mode.
+void build_operands(fs_dataset *ds, bool need_codes, int dist_mode, int64_t u_lo, int64_t u_hi, bool group_call,
+                    int *launches);
 
 // joint.cu: the operand of the discrete columns feat_idx (all p columns when null) of a data set whose features
 // are set.  Every column must be constant or a tensor-path column with at most max_values distinct values
@@ -513,15 +525,16 @@ void comm_check(fs_comm *c);
 void comm_push(fs_comm *c, size_t off, size_t bytes, cudaStream_t st, int *launches);
 
 // onehot.cu: the reduced one-hot operands of the working set's tensor-path columns (U, Wd, srow when
-// ws.have_dist_ops; At, krow, codesT or tpos; codes when ws.have_codes) and, for an incremental distance
-// update, those of the removed columns
-void build_onehot(fs_dataset *ds, WorkSet &ws, int *launches);
+// ws.have_dist_ops -- Wd only of the rows this rank's distance kernel reads in a group call; At, krow, codesT
+// or tpos; codes when ws.have_codes) and, for an incremental distance update, those of the removed columns
+void build_onehot(fs_dataset *ds, WorkSet &ws, bool group_call, int *launches);
 
 // tc_dist.cu: the one-hot mismatch counts of R target rows (internal order; h_row_ids / d_row_ids, or the
 // contiguous range from r0_internal) against all samples, into the slab Dd [R, ldn] (or subtracted from it for
-// an incremental update); symmetric and mirrored into the peers' slabs when this rank scores its shard
+// an incremental update); with `exchange` (this rank computes its whole shard into its arena slab) symmetric
+// and mirrored into the peers' slabs
 void launch_dist_tensor(fs_dataset *ds, const WorkSet &ws, int64_t r0_internal, const int64_t *h_row_ids,
-                        const int64_t *d_row_ids, bool contiguous, int64_t R, int32_t *Dd, int64_t ldn,
+                        const int64_t *d_row_ids, bool contiguous, int64_t R, int32_t *Dd, int64_t ldn, bool exchange,
                         cudaStream_t st, int *launches, double *ops);
 // The distance GEMM itself: D[r, j] = srow[ids[r]] + srow[j] - sum_k a[r, k] b[j, k] (subtract: D[r, j] -= that)
 // over the FP4 operands a (R rows) and b (n rows), row_bytes wide at a pitch of `pitch` bytes, contracted over K

@@ -325,6 +325,19 @@ static void compute_owner_bounds(fs_dataset *ds) {
     }
 }
 
+// Drop what was derived from the typing or the group: the working set's operands and the cached distance slab
+// always, the resident codesT with `codes`, and with `retyped` the column lists (typing_epoch) and the ranks'
+// accumulation shares
+static void forget_derived(fs_dataset *ds, bool codes, bool retyped) {
+    ds->ws.valid = false;
+    ds->slab.forget();
+    if (codes) ds->ct_valid = false;
+    if (retyped) {
+        ++ds->typing_epoch;
+        compute_owner_bounds(ds);
+    }
+}
+
 static int usable_devices() {
     int count = 0;
     if (cudaGetDeviceCount(&count) != cudaSuccess) {
@@ -415,68 +428,24 @@ static void run_gather(fs_dataset *ds, WorkSet &ws, int *launches) {
     ++*launches;
 }
 
-// Can the cached distance slab serve this call?  tcol[0..pt) are the tensor-path columns now active.
-static int plan_dist(fs_dataset *ds, const int64_t *tcol, int64_t pt, int64_t r0, int64_t R, bool cacheable,
-                     std::vector<int64_t> &removed) {
-    removed.clear();
-    const char *env = getenv("FS_B200_INCREMENTAL");
-    if (env && env[0] == '0') return kDistFull;
-    if (!cacheable || !ds->dd_valid || ds->dd_r0 != r0 || ds->dd_R != R || pt == 0) return kDistFull;
-    const std::vector<int64_t> &old = ds->dd_cols;
-    if ((size_t)pt > old.size()) return kDistFull;
-    // the active columns must be a subsequence of the cached ones (TuRF only ever deletes)
-    size_t j = 0;
-    for (int64_t i = 0; i < pt; ++i) {
-        while (j < old.size() && old[j] != tcol[i]) removed.push_back(old[j++]);
-        if (j == old.size()) {
-            removed.clear();
-            return kDistFull;
-        }
-        ++j;
-    }
-    while (j < old.size()) removed.push_back(old[j++]);
-    if (removed.empty()) return kDistReuse;
-    if ((int64_t)removed.size() >= pt) {           // subtracting would cost more than recomputing
-        removed.clear();
-        return kDistFull;
-    }
-    return kDistIncremental;
-}
-
-void build_workset(fs_dataset *ds, const int64_t *feat_idx, int64_t n_kept, bool need_codes,
-                   int64_t r0, int64_t R, bool contiguous, bool slab_cacheable, bool want_split, bool group_call,
-                   bool dist_ops, int *launches) {
+void build_lists(fs_dataset *ds, const int64_t *feat_idx, int64_t n_kept, bool want_split, bool group_call) {
     WorkSet &ws = ds->ws;
-    // sample rows the target-side distance operand U has to hold
-    const int64_t want_lo = contiguous ? r0 : 0, want_hi = contiguous ? r0 + R : ds->n;
-    Trace tr_all("build_workset");
-    // cache key: flags + the explicit column list (none when every column is active)
+    Trace tr_all("build_lists");
+    // key: flags + the explicit column list (none when every column is active)
     const bool all = feat_idx == nullptr;
     std::vector<int64_t> key(3 + (all ? 0 : n_kept));
     key[0] = (want_split ? 1 : 0) | (group_call ? 2 : 0);
-    ws.group_call = group_call;
     key[1] = ds->arith;
     key[2] = all ? -1 : n_kept;
     if (!all) memcpy(key.data() + 3, feat_idx, n_kept * sizeof(int64_t));
-    if (ws.valid && ws.key == key && (ws.have_codes || !need_codes || ws.pt == 0)) {
-        // same columns as the last call: the slab is either still there or recomputed in full
-        const int mode = plan_dist(ds, ws.p_tcol.ptr, ws.pt, r0, R, slab_cacheable, ws.removed);
-        if (mode == kDistReuse || (ws.have_dist_ops && ws.u_lo <= want_lo && want_hi <= ws.u_hi) || ws.pt == 0 ||
-            !dist_ops) {                     // only At is needed, and it is always built
-            ws.dist_mode = mode == kDistReuse ? kDistReuse : kDistFull;
-            return;
-        }
-    }
+    // the lists depend only on the key and the typing (fs_dataset_set_features, and the group's column shares):
+    // they are kept (host vectors, pinned staging and their device copies) until one of those changes, so that
+    // re-scoring the same columns does not walk them on the host again
+    if (ws.key == key && ws.lists_typing == ds->typing_epoch) return;
     ws.valid = false;
+    ws.key.clear();                 // until the lists are complete (a bad column below throws)
     const int chunk = kChunkBytes / (ds->arith == FS_ARITH_F64 ? 8 : 4);
     ws.elem = ds->arith == FS_ARITH_F64 ? 8 : 4;
-
-    // The column lists of an all-columns call depend only on the typing (fs_dataset_set_features) and the
-    // call's flags: they are kept (host vectors, pinned staging and their device copies) until one of those
-    // changes, so that re-scoring the same data set does not walk all p columns on the host again.
-    const bool lists_ok = all && ws.lists_all && ws.lists_typing == ds->typing_epoch && ws.lists_flags == key[0] &&
-                          ws.lists_n == n_kept;
-    if (!lists_ok) {
     // split the active columns: one-hot tensor path (discrete, 2 <= V <= FS_DISTINCT_CAP),
     // continuous, and wide discrete ("compare") columns.  The tensor-path lists are written
     // straight into the pinned staging buffers the encode kernel's inputs are copied from;
@@ -591,13 +560,23 @@ void build_workset(fs_dataset *ds, const int64_t *feat_idx, int64_t n_kept, bool
         FS_CUDA(cudaMemcpyAsync(ws.gcol.ptr, ws.h_gcol.data(), ws.pg * sizeof(int64_t), cudaMemcpyHostToDevice, ds->stream));
         FS_CUDA(cudaMemcpyAsync(ws.gout.ptr, ws.h_gout.data(), ws.pg * sizeof(int64_t), cudaMemcpyHostToDevice, ds->stream));
     }
-    ws.lists_all = all;
+    ws.key = std::move(key);
     ws.lists_typing = ds->typing_epoch;
-    ws.lists_flags = key[0];
-    ws.lists_n = n_kept;
     ++ws.lists_version;
     ws.lists_uploaded = false;
-    }   // !lists_ok
+}
+
+void build_operands(fs_dataset *ds, bool need_codes, int dist_mode, int64_t u_lo, int64_t u_hi, bool group_call,
+                    int *launches) {
+    WorkSet &ws = ds->ws;
+    if (ws.valid && (ws.have_codes || !need_codes || ws.pt == 0) &&
+        (dist_mode == kDistNone || dist_mode == kDistReuse || ws.pt == 0 ||
+         (ws.have_dist_ops && ws.u_lo <= u_lo && u_hi <= ws.u_hi))) {
+        ws.dist_mode = dist_mode == kDistIncremental ? kDistFull : dist_mode;
+        return;
+    }
+    Trace tr_all("build_operands");
+    ws.valid = false;
     ws.have_xg32 = false;
     if (ws.pg > 0) {
         ws.xg.reserve((size_t)ds->n * ws.ldg * ws.elem);
@@ -619,18 +598,14 @@ void build_workset(fs_dataset *ds, const int64_t *feat_idx, int64_t n_kept, bool
     }
     ws.K = 0;
     ws.have_codes = need_codes;
-    {
-        Trace tr("  plan_dist");
-        ws.dist_mode = plan_dist(ds, ws.p_tcol.ptr, ws.pt, r0, R, slab_cacheable, ws.removed);
-    }
-    ws.have_dist_ops = ws.dist_mode == kDistFull && dist_ops;
-    ws.u_lo = want_lo;
-    ws.u_hi = want_hi;
+    ws.dist_mode = dist_mode;
+    ws.have_dist_ops = dist_mode == kDistFull;
+    ws.u_lo = u_lo;
+    ws.u_hi = u_hi;
     if (ws.pt > 0) {
         Trace tr("  build_onehot");
-        build_onehot(ds, ws, launches);
+        build_onehot(ds, ws, group_call, launches);
     }
-    ws.key = std::move(key);
     ws.valid = true;
     ++ws.build_id;
 }
@@ -801,16 +776,13 @@ int fs_dataset_set_features(fs_dataset *ds, const uint8_t *is_discrete, const fl
                       memcmp(ds->is_discrete.data(), is_discrete, ds->p) == 0 &&
                       memcmp(ds->recip.data(), recip, ds->p * sizeof(float)) == 0;
     if (same) {
-        ds->ws.valid = false;
-        ds->dd_valid = false;
-        ds->ct_valid = false;
+        forget_derived(ds, true, false);
         return FS_OK;
     }
-    ++ds->typing_epoch;
     ds->is_discrete.assign(is_discrete, is_discrete + ds->p);
     ds->recip.assign(recip, recip + ds->p);
     ds->arith = arith;
-    // per-column path of the scoring pipeline, decided once (build_workset reads one byte per column)
+    // per-column path of the scoring pipeline, decided once (build_lists reads one byte per column)
     ds->col_info.resize(ds->p);
     const bool byte_input = ds->dtype == FS_U8 || ds->dtype == FS_I8;
     for (int64_t f = 0; f < ds->p; ++f) {
@@ -830,10 +802,7 @@ int fs_dataset_set_features(fs_dataset *ds, const uint8_t *is_discrete, const fl
         ds->col_info[f] = (uint8_t)ci;
     }
     ds->have_features = true;
-    ds->ws.valid = false;
-    ds->dd_valid = false;
-    ds->ct_valid = false;
-    compute_owner_bounds(ds);
+    forget_derived(ds, true, true);
     return FS_OK;
 }
 
@@ -851,12 +820,8 @@ int fs_dataset_attach_comm(fs_dataset *ds, fs_comm *comm, const int64_t *row_sta
         FS_REQUIRE(ds, FS_ERR_INVALID, "fs_dataset_attach_comm: null data set");
         if (comm == nullptr || comm->world <= 1) {         // detach: plain single-rank behaviour
             ds->comm = nullptr;
-            ds->peers_on = false;
             ds->peer_slab = nullptr;
-            ds->dd_valid = false;
-            ds->ws.valid = false;
-            ++ds->typing_epoch;
-            ds->owner_bound.clear();
+            forget_derived(ds, false, true);
             return FS_OK;
         }
         FS_REQUIRE(row_starts, FS_ERR_INVALID, "fs_dataset_attach_comm: row_starts missing");
@@ -898,12 +863,7 @@ int fs_dataset_attach_comm(fs_dataset *ds, fs_comm *comm, const int64_t *row_sta
         ds->peers = pr;
         ds->comm = comm;
         ds->peer_slab = pr.slab[rank];
-        ds->peer_slab_count = (L.off_mask_h - L.off_slab) / sizeof(int32_t);
-        ds->peers_on = true;
-        ds->dd_valid = false;
-        ds->ws.valid = false;
-        ++ds->typing_epoch;          // the accumulation shares changed: cached column lists are stale
-        compute_owner_bounds(ds);
+        forget_derived(ds, false, true);          // the accumulation shares changed: cached column lists are stale
         return FS_OK;
     });
 }

@@ -78,7 +78,8 @@ const DiscreteOperand &discrete_operand(fs_dataset *ds, const int64_t *feat_idx,
             max_rows = std::max(max_rows, rows);
         }
         op.valid = false;
-        build_workset(ds, feat_idx, n_kept, false, 0, ds->n, true, false, false, false, false, launches);
+        build_lists(ds, feat_idx, n_kept, false, false);
+        build_operands(ds, false, kDistNone, 0, ds->n, false, launches);
         FS_REQUIRE(ws.K_used == start[n_kept], FS_ERR_STATE, "%s: working set holds %lld reduced rows, expected %lld",
                    what, (long long)ws.K_used, (long long)start[n_kept]);
         op.start_h = std::move(start);

@@ -597,9 +597,9 @@ static void build_removed(fs_dataset *ds, WorkSet &ws, int *launches) {
                   nullptr, nullptr, ws.srow_r.ptr, nullptr, 0, n, nullptr, 0, 0, WdRows{0, n, 0, 0}, st, launches);
 }
 
-void build_onehot(fs_dataset *ds, WorkSet &ws, int *launches) {
+void build_onehot(fs_dataset *ds, WorkSet &ws, bool group_call, int *launches) {
     const int64_t n = ds->n, pt = ws.pt;
-    // tcol / tout / toff, K_used, all_ident and the accumulation slice [a0, a1) were filled by build_workset
+    // tcol / tout / toff, K_used, all_ident and the accumulation slice [a0, a1) were filled by build_lists
     ws.K = round_up(ws.K_used, 256);          // elements (FP4 nibbles); U / Wd rows are K / 2 bytes
     ws.ldt = round_up(n, 128);
     ws.ldc = round_up(pt, 16);
@@ -678,7 +678,7 @@ void build_onehot(fs_dataset *ds, WorkSet &ws, int *launches) {
     // samples), then the accumulation operands of this rank's slice only.
     // Wd rows this rank's distance kernel reads (see WdRows)
     WdRows wr{0, n, 0, 0};
-    if (ws.group_call && ds->peers_on && ds->peers.world > 1) {
+    if (group_call) {
         const DistPeers &pr = ds->peers;
         const int G = pr.world, r = pr.rank, last = r + G / 2;          // ranks r .. r + floor(G / 2) on the ring
         if (last < G) {

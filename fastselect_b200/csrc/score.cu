@@ -45,6 +45,38 @@ static int64_t chunk_rows(bool have_general, bool have_tensor, int64_t ldn, int 
     return rows;
 }
 
+// Can the slab cached in `buf` serve this call's target rows [r0, r0 + R) and active tensor-path columns?  Fills
+// ws.removed with the columns an incremental update subtracts.
+static int plan_dist(fs_dataset *ds, const int32_t *buf, int64_t r0, int64_t R, bool cacheable) {
+    const SlabCache &c = ds->slab;
+    WorkSet &ws = ds->ws;
+    std::vector<int64_t> &removed = ws.removed;
+    const int64_t *tcol = ws.p_tcol.ptr, pt = ws.pt;
+    removed.clear();
+    const char *env = getenv("FS_B200_INCREMENTAL");
+    if (env && env[0] == '0') return kDistFull;
+    if (!cacheable || !c.valid || c.buf != buf || c.r0 != r0 || c.R != R || pt == 0) return kDistFull;
+    const std::vector<int64_t> &old = c.cols;
+    if ((size_t)pt > old.size()) return kDistFull;
+    // the active columns must be a subsequence of the cached ones (TuRF only ever deletes)
+    size_t j = 0;
+    for (int64_t i = 0; i < pt; ++i) {
+        while (j < old.size() && old[j] != tcol[i]) removed.push_back(old[j++]);
+        if (j == old.size()) {
+            removed.clear();
+            return kDistFull;
+        }
+        ++j;
+    }
+    while (j < old.size()) removed.push_back(old[j++]);
+    if (removed.empty()) return kDistReuse;
+    if ((int64_t)removed.size() >= pt) {           // subtracting would cost more than recomputing
+        removed.clear();
+        return kDistFull;
+    }
+    return kDistIncremental;
+}
+
 static void run_pipeline(fs_dataset *ds, int algo, int use_star, int32_t k, const float *class_probs,
                          const int64_t *feat_idx, int64_t n_kept, const std::vector<int64_t> &targets,
                          bool contiguous, double *d_wsum, DebugOut *dbg, fs_stats *stats) {
@@ -71,9 +103,9 @@ static void run_pipeline(fs_dataset *ds, int algo, int use_star, int32_t k, cons
     // columns, and wsum_out receives the COMPLETE sums on every rank.
     fs_comm *comm = ds->comm;
     int64_t max_shard = 0;
-    for (int q = 0; ds->peers_on && q < ds->peers.world; ++q)
+    for (int q = 0; comm != nullptr && q < ds->peers.world; ++q)
         max_shard = std::max<int64_t>(max_shard, ds->peers.starts[q + 1] - ds->peers.starts[q]);
-    const bool group_call = ds->peers_on && comm != nullptr && comm->world > 1 && contiguous && dbg == nullptr &&
+    const bool group_call = comm != nullptr && comm->world > 1 && contiguous && dbg == nullptr &&
                             targets[0] == ds->peers.starts[ds->peers.rank] &&
                             (int64_t)targets.size() == ds->peers.starts[ds->peers.rank + 1] - ds->peers.starts[ds->peers.rank] &&
                             round_up(max_shard, 128) <= chunk_rows(true, true, ldn, algo);
@@ -85,16 +117,11 @@ static void run_pipeline(fs_dataset *ds, int algo, int use_star, int32_t k, cons
     // (with peers configured the decision is taken for the largest shard, so that all ranks agree)
     const int64_t cache_rows = std::max<int64_t>((int64_t)targets.size(), max_shard);
     const bool slab_cacheable = contiguous && dbg == nullptr && round_up(cache_rows, 128) <= chunk_rows(true, true, ldn, algo);
-    if (!slab_cacheable) ds->dd_valid = false;
+    if (!slab_cacheable) ds->slab.forget();
     timer.begin(&fs_stats::ms_gather);
     const auto prep0 = std::chrono::steady_clock::now();
-    build_workset(ds, feat_idx, n_kept, algo == FS_RELIEFF, targets[0], (int64_t)targets.size(),
-                  contiguous, slab_cacheable, want_split, group_call, true, &launches);
-    const double ms_prep = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - prep0).count();
-    timer.end();
+    build_lists(ds, feat_idx, n_kept, want_split, group_call);
     const WorkSet &ws = ds->ws;
-    const bool fshard = group_call && ws.acc_split && ws.pt > 0;
-
     const int64_t Rmax = std::min<int64_t>(chunk_rows(ws.pg > 0, ws.pt > 0, ldn, algo), round_up((int64_t)targets.size(), 128));
     if (ws.pg > 0) ds->Dc.reserve((size_t)Rmax * ldn);
     // the one-hot distance slab: this rank's slab inside its exchange arena for a group call (the
@@ -107,18 +134,15 @@ static void run_pipeline(fs_dataset *ds, int algo, int use_star, int32_t k, cons
             ds->Dd.reserve((size_t)Rmax * ldn);
             Dd = ds->Dd.ptr;
         }
-        if (ds->dd_buf != Dd) {
-            // the cached slab lives in the other buffer: recompute in full (the working set may
-            // have been built for an incremental update)
-            if (ds->dd_valid && ws.dist_mode != kDistFull) {
-                ds->dd_valid = false;
-                ds->ws.valid = false;
-                build_workset(ds, feat_idx, n_kept, algo == FS_RELIEFF, targets[0], (int64_t)targets.size(),
-                              contiguous, slab_cacheable, want_split, group_call, true, &launches);
-            }
-            ds->dd_valid = false;
-        }
     }
+    const int64_t u_lo = contiguous ? targets[0] : 0, u_hi = contiguous ? targets[0] + (int64_t)targets.size() : n;
+    build_operands(ds, algo == FS_RELIEFF, plan_dist(ds, Dd, targets[0], (int64_t)targets.size(), slab_cacheable),
+                   u_lo, u_hi, group_call, &launches);
+    const double ms_prep = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - prep0).count();
+    timer.end();
+    const bool fshard = group_call && ws.acc_split && ws.pt > 0;
+    // a group call's full distance pass is symmetric across the ranks: each stores tiles into the others' slabs
+    const bool exchange = group_call && ws.dist_mode == kDistFull;
     ds->sel.reserve((size_t)Rmax * ldn);
     const bool use_masks = ws.pt > 0 && algo != FS_RELIEFF;
     // neighbour masks and row constants: inside a group call they live in the arena at the rows of this
@@ -186,28 +210,20 @@ static void run_pipeline(fs_dataset *ds, int algo, int use_star, int32_t k, cons
         }
         // ---- distances
         if (ws.pt > 0 && ws.dist_mode != kDistReuse) {
-            ds->dd_valid = false;
+            ds->slab.forget();
             timer.begin(&fs_stats::ms_dist_tensor);
-            launch_dist_tensor(ds, ws, h_ids[0], h_ids, ds->row_ids.ptr, contiguous, R, Dd, ldn, st, &launches, &ops_dist);
+            launch_dist_tensor(ds, ws, h_ids[0], h_ids, ds->row_ids.ptr, contiguous, R, Dd, ldn, exchange, st, &launches,
+                               &ops_dist);
             timer.end();
-            if (ds->last_dist_exchanged) {
+            if (exchange) {
                 // tiles computed here were also stored into the peers' slabs and theirs into this one:
                 // every rank must have finished its distance kernel before anyone selects (device-side
                 // barrier over flags in the arenas: no host synchronisation inside the step)
                 comm_barrier(comm, st, &launches);
             }
         }
-        if (ws.pt > 0 && slab_cacheable) {
-            ds->dd_buf = Dd;
-            // Dd now holds the mismatch counts of exactly these columns for these target rows
-            if (ds->dd_version != ws.lists_version || (int64_t)ds->dd_cols.size() != ws.pt) {
-                ds->dd_cols.assign(ws.p_tcol.ptr, ws.p_tcol.ptr + ws.pt);
-                ds->dd_version = ws.lists_version;
-            }
-            ds->dd_r0 = targets[0];
-            ds->dd_R = (int64_t)targets.size();
-            ds->dd_valid = true;
-        }
+        // Dd now holds the mismatch counts of exactly these columns for these target rows
+        if (ws.pt > 0 && slab_cacheable) ds->slab.record(Dd, ws, targets[0], (int64_t)targets.size());
         if (ws.pg > 0) {
             timer.begin(&fs_stats::ms_dist_general);
             launch_dist_general(ws, xa, R, ws.xg.ptr, n, ds->Dc.ptr, ldn, st, &launches);
@@ -403,19 +419,20 @@ int fs_debug_rows(fs_dataset *ds, int algo, int use_star, int32_t k, const float
 int fs_debug_slab(fs_dataset *ds, int64_t row_begin, int64_t nrows, int32_t *out, int64_t *info_out) {
     return api_call("fs_debug_slab", [&] {
         FS_REQUIRE(ds && out && nrows >= 1, FS_ERR_INVALID, "fs_debug_slab: invalid argument");
-        FS_REQUIRE(ds->dd_valid && ds->dd_buf != nullptr, FS_ERR_STATE, "fs_debug_slab: no distance slab is cached");
-        FS_REQUIRE(row_begin >= ds->dd_r0 && row_begin + nrows <= ds->dd_r0 + ds->dd_R, FS_ERR_STATE,
+        const SlabCache &c = ds->slab;
+        FS_REQUIRE(c.valid && c.buf != nullptr, FS_ERR_STATE, "fs_debug_slab: no distance slab is cached");
+        FS_REQUIRE(row_begin >= c.r0 && row_begin + nrows <= c.r0 + c.R, FS_ERR_STATE,
                    "fs_debug_slab: rows [%lld, %lld) outside the cached range [%lld, %lld)", (long long)row_begin,
-                   (long long)(row_begin + nrows), (long long)ds->dd_r0, (long long)(ds->dd_r0 + ds->dd_R));
+                   (long long)(row_begin + nrows), (long long)c.r0, (long long)(c.r0 + c.R));
         FS_CUDA(cudaSetDevice(ds->device));
         FS_CUDA(cudaStreamSynchronize(ds->stream));
         const int64_t ldn = round_up(ds->n, 128);
-        FS_CUDA(cudaMemcpy2D(out, ds->n * sizeof(int32_t), ds->dd_buf + (size_t)(row_begin - ds->dd_r0) * ldn,
+        FS_CUDA(cudaMemcpy2D(out, ds->n * sizeof(int32_t), c.buf + (size_t)(row_begin - c.r0) * ldn,
                              ldn * sizeof(int32_t), ds->n * sizeof(int32_t), nrows, cudaMemcpyDeviceToHost));
         if (info_out) {
-            info_out[0] = ds->dd_r0;
-            info_out[1] = ds->dd_R;
-            info_out[2] = (int64_t)ds->dd_cols.size();
+            info_out[0] = c.r0;
+            info_out[1] = c.R;
+            info_out[2] = (int64_t)c.cols.size();
         }
         return FS_OK;
     });

@@ -344,7 +344,7 @@ void launch_tc_dist(const int8_t *a, const int8_t *b, int64_t row_bytes, int64_t
 }
 
 void launch_dist_tensor(fs_dataset *ds, const WorkSet &ws, int64_t r0_internal, const int64_t *h_row_ids,
-                        const int64_t *d_row_ids, bool contiguous, int64_t R, int32_t *Dd, int64_t ldn,
+                        const int64_t *d_row_ids, bool contiguous, int64_t R, int32_t *Dd, int64_t ldn, bool exchange,
                         cudaStream_t st, int *launches, double *ops) {
     // incremental update: the operands are those of the removed columns and the result is subtracted
     const bool incr = ws.dist_mode == kDistIncremental;
@@ -367,15 +367,12 @@ void launch_dist_tensor(fs_dataset *ds, const WorkSet &ws, int64_t r0_internal, 
     }
     // Symmetric mode: the target rows of all ranks together cover every sample, so half of the
     // off-diagonal super-blocks are computed and mirrored (see the file head).  One rank scoring all rows
-    // is the trivial case; with peers configured (fs_dataset_set_peers) this rank's rows must be
-    // exactly its shard and Dd its exported slab.  An incremental update across ranks stays
-    // non-symmetric (it would need remote read-modify-writes).
-    const bool own_shard = contiguous && ds->peers_on && Dd == ds->peer_slab && r0_internal == ds->peers.starts[ds->peers.rank] &&
-                           R == ds->peers.starts[ds->peers.rank + 1] - ds->peers.starts[ds->peers.rank] && !incr;
-    const DistPeers peers = own_shard ? ds->peers : single_rank_peers(Dd, ds->n);
-    const bool symmetric = own_shard || (contiguous && r0_internal == 0 && R == ds->n);
+    // is the trivial case; in a multi-GPU group the caller says so (`exchange`: this rank's rows are
+    // exactly its shard and Dd its arena slab).  An incremental update across ranks stays
+    // non-symmetric (it would need remote read-modify-writes): the caller never asks for both.
+    const DistPeers peers = exchange ? ds->peers : single_rank_peers(Dd, ds->n);
+    const bool symmetric = exchange || (contiguous && r0_internal == 0 && R == ds->n);
     launch_tc_dist(a_rows, Wop, K, K, K, sop, d_row_ids, R, ds->n, ldn, symmetric, incr, peers, st, launches, ops);
-    ds->last_dist_exchanged = symmetric && peers.world > 1;
 }
 
 }  // namespace fs

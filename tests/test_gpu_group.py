@@ -198,3 +198,122 @@ def test_single_process_multi_gpu_entry(native, monkeypatch):
         monkeypatch.delenv("FASTSELECT_B200_GPUS")
         t0 = fsb.TuRF(fsb.MultiSURF(backend="gpu", n_features_to_select=5), n_features_to_select=20, pct_remove=0.2).fit(x, y)
         assert np.array_equal(t0.top_features_, t1.top_features_)
+
+
+# ---- a call's distance plan across buffers: the slab of a collective call lives in the rank's arena, that of any
+# other call in the data set's own buffer.  A slab cached in one of them must never seed an incremental update or
+# a reuse in the other.
+
+def _turf_columns(p):
+    rs = np.random.RandomState(5)
+    a1 = np.sort(rs.choice(p, int(p * 0.9), replace=False))
+    a2 = np.sort(rs.choice(a1, int(a1.size * 0.9), replace=False))
+    a3 = np.sort(rs.choice(a2, int(a2.size * 0.9), replace=False))
+    return a1, a2, a3
+
+
+def _fresh(native, x, y32, **call):
+    """Score and slab of one call on a data set that has never scored before."""
+    with native.Dataset(x, y32, 2) as ds:
+        ds.set_features(np.ones(x.shape[1], bool), np.ones(x.shape[1], np.float32), native.FS_ARITH_F32)
+        w = ds.score(native.FS_MULTISURF, **call)
+        lo = call.get("row_begin", 0)
+        hi = call.get("row_end", x.shape[0])
+        return w, ds.debug_slab(lo, hi - lo)
+
+
+def test_group_then_alone_recomputes_the_slab(native, monkeypatch):
+    n, p = 900, 700
+    x, y = epistatic_genotypes(47, n, p)
+    y32 = y.astype(np.int32)
+    a1, a2, a3 = _turf_columns(p)
+    g = EmulatedGroup(native, x, y32, 2, 2, False, monkeypatch)
+    try:
+        g.set_features(np.ones(p, bool), np.ones(p, np.float32), native.FS_ARITH_F32)
+        for cols in (None, a1):                   # a1: incremental update of the arena slab
+            want, _ = _fresh(native, x, y32, feat_idx=cols)
+            for got in g.score(native.FS_MULTISURF, feat_idx=cols):
+                assert np.array_equal(got, want)
+        ds = g.sets[0]
+        ds.attach_comm(None, None)
+        # alone, on the rows and a subset of the columns the arena slab was cached for, then on all rows
+        for call in (dict(feat_idx=a2, row_begin=g.starts[0], row_end=g.starts[1]), dict(feat_idx=a3)):
+            want, (want_slab, want_info) = _fresh(native, x, y32, **call)
+            assert np.array_equal(ds.score(native.FS_MULTISURF, **call), want)
+            lo, hi = call.get("row_begin", 0), call.get("row_end", n)
+            got_slab, got_info = ds.debug_slab(lo, hi - lo)
+            assert got_info == want_info and np.array_equal(got_slab, want_slab)
+    finally:
+        g.close()
+
+
+def test_alone_then_group_recomputes_the_slab(native, monkeypatch):
+    n, p = 900, 700
+    x, y = epistatic_genotypes(48, n, p)
+    y32 = y.astype(np.int32)
+    isd, recip = np.ones(p, bool), np.ones(p, np.float32)
+    a1, a2, _ = _turf_columns(p)
+    fresh = EmulatedGroup(native, x, y32, 2, 2, False, monkeypatch)
+    try:
+        fresh.set_features(isd, recip, native.FS_ARITH_F32)
+        want = fresh.score(native.FS_MULTISURF, feat_idx=a2)
+    finally:
+        fresh.close()
+    g = EmulatedGroup(native, x, y32, 2, 2, False, monkeypatch)
+    try:
+        # each rank alone caches the slab of all columns over its shard in its own buffer
+        for r, ds in enumerate(g.sets):
+            ds.set_features(isd, recip, native.FS_ARITH_F32)
+            w, _ = _fresh(native, x, y32, row_begin=g.starts[r], row_end=g.starts[r + 1])
+            assert np.array_equal(ds.score(native.FS_MULTISURF, row_begin=g.starts[r], row_end=g.starts[r + 1]), w)
+            ds.attach_comm(g.comms[r], g.starts)
+        got = g.score(native.FS_MULTISURF, feat_idx=a1)
+        assert np.array_equal(got[0], got[1])
+        got = g.score(native.FS_MULTISURF, feat_idx=a2)
+        for r in range(2):
+            assert np.array_equal(got[r], want[r])
+    finally:
+        g.close()
+
+
+def test_score_after_joint_columns_rebuilds_the_working_set(native):
+    n, p = 900, 700
+    x, y = epistatic_genotypes(49, n, p)
+    y32 = y.astype(np.int32)
+    a1, _, _ = _turf_columns(p)
+    want, (want_slab, want_info) = _fresh(native, x, y32, feat_idx=a1)
+    with native.Dataset(x, y32, 2) as ds:
+        ds.set_features(np.ones(p, bool), np.ones(p, np.float32), native.FS_ARITH_F32)
+        ds.score(native.FS_MULTISURF)
+        # the joint path builds the working set of a1 without distance operands
+        ds.joint_columns(native.FS_JOINT_MI, 2.0, [0, 3], feat_idx=a1)
+        assert np.array_equal(ds.score(native.FS_MULTISURF, feat_idx=a1), want)
+        got_slab, got_info = ds.debug_slab(0, n)
+        assert got_info == want_info and np.array_equal(got_slab, want_slab)
+
+
+# (launches, n_chunks) of every call of a TuRF-like sequence: all columns, then two shrinking subsets.  A
+# working set or operand built twice, or a slab recomputed where it could be updated, changes the counts.
+TURF_LAUNCHES_ALONE = [(8, 1), (9, 1), (9, 1)]
+TURF_LAUNCHES_GROUP = [[(18, 1)] * 2, [(17, 1)] * 2, [(17, 1)] * 2]     # per rank
+
+
+def test_turf_sequence_launch_counts(native, monkeypatch):
+    n, p = 900, 700
+    x, y = epistatic_genotypes(50, n, p)
+    y32 = y.astype(np.int32)
+    isd, recip = np.ones(p, bool), np.ones(p, np.float32)
+    a1, a2, _ = _turf_columns(p)
+    seq = (None, a1, a2)
+    with native.Dataset(x, y32, 2) as ds:
+        ds.set_features(isd, recip, native.FS_ARITH_F32)
+        alone = [ds.score(native.FS_MULTISURF, feat_idx=c, want_stats=True)[1] for c in seq]
+    g = EmulatedGroup(native, x, y32, 2, 2, False, monkeypatch)
+    try:
+        g.set_features(isd, recip, native.FS_ARITH_F32)
+        group = [[s for _, s in g.score(native.FS_MULTISURF, feat_idx=c, want_stats=True)] for c in seq]
+    finally:
+        g.close()
+    got_alone = [(s["launches"], s["n_chunks"]) for s in alone]
+    got_group = [[(s["launches"], s["n_chunks"]) for s in ranks] for ranks in group]
+    assert (got_alone, got_group) == (TURF_LAUNCHES_ALONE, TURF_LAUNCHES_GROUP), repr((got_alone, got_group))
