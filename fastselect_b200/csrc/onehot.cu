@@ -12,6 +12,7 @@
 // Samples are in the data set's class-sorted internal order.  HBM-bound streaming kernel:
 // reads n*pt elements once, writes 1.5*n*K + n*pt bytes.
 #include <algorithm>
+#include <type_traits>
 
 #include "common.cuh"
 
@@ -34,9 +35,12 @@ namespace fs {
 // Tile: 128 samples x 64 columns per CTA.  Step 1 reads x and keeps the value codes in
 // shared memory in both orientations; step 2 emits the U / Wd rows (one-hot index
 // contiguous) and the per-sample counts s; step 3 the At and codesT rows (sample index
-// contiguous).  On the 0/1/2 fast path all global stores are 8- or 16-byte vectors and every
-// byte of the tile's footprint is written exactly once (no memset of the operands); the general
-// path ORs the words at unaligned tile edges into operands the host cleared.
+// contiguous).  One kernel template, onehot_encode_kernel<Tin, kLean>, does all three steps: its
+// lean instantiation (one-byte 0/1/2 genotypes) writes every byte of the tile's footprint exactly
+// once, so the host clears only the K padding of U / Wd; the general instantiations (any input
+// type, up to FS_DISTINCT_CAP values) OR the words at unaligned tile edges into operands the host
+// cleared whole (clear_dist_ops).  Where every column of a tile holds three values, both take the
+// same 0/1/2 paths, whose global stores are 8- or 16-byte vectors.
 constexpr int ENC_ROWS = 128;
 constexpr int ENC_COLS = 64;
 constexpr int ENC_CR_LD = ENC_ROWS + 4;                       // conflict-free transposed stores
@@ -74,8 +78,14 @@ struct WdRows {
     __host__ __device__ bool touches(int64_t a, int64_t b) const { return (a < hi0 && b > lo0) || (a < hi1 && b > lo1); }
 };
 
-template <typename Tin>
-__global__ void __launch_bounds__(256) onehot_encode_kernel(
+// kLean: the instantiation for the case that matters most, one-byte input whose columns all hold exactly the
+// values 0/1/2 (the value is its own code, two reduced rows per column).  It has no code tables and no per-column
+// bookkeeping, so registers stay low enough for 6 CTAs per SM, which is what hides the perm -> x load chain of
+// this streaming kernel.  It alone stages short column spans in shared memory (step 1) and writes a ragged column
+// tile byte by byte (step 2); only the general instantiations translate values to codes and OR partial words in.
+// (A minimum of 0 CTAs per SM sets none: the general instantiations' register allocation changes under a minimum of 1.)
+template <typename Tin, bool kLean>
+__global__ void __launch_bounds__(256, kLean ? 6 : 0) onehot_encode_kernel(
     const Tin *__restrict__ x, int64_t ldx, const int64_t *__restrict__ perm, const int64_t *__restrict__ tcol,
     const int32_t *__restrict__ toff, const double *__restrict__ vals, int as_f32, int64_t n, int64_t pt, int64_t K,
     int64_t ldt, int64_t ldc, int8_t *__restrict__ U, int8_t *__restrict__ Wd, int8_t *__restrict__ At,
@@ -86,9 +96,9 @@ __global__ void __launch_bounds__(256) onehot_encode_kernel(
     // columns numbers At / krow rows from 0 but addresses the distance operands globally)
     __shared__ __align__(16) uint8_t code_rc[ENC_ROWS][ENC_COLS];       // [sample][column]
     __shared__ __align__(16) uint8_t code_cr[ENC_COLS][ENC_CR_LD];      // [column][sample]
-    __shared__ uint8_t kcol[ENC_KMAX];                                  // reduced row -> column in tile
-    __shared__ uint8_t kval[ENC_KMAX];                                  // reduced row -> value code
-    __shared__ uint8_t clast[ENC_COLS];                                 // last code of each column
+    __shared__ uint8_t kcol[ENC_KMAX];                                  // general: reduced row -> column in tile
+    __shared__ uint8_t kval[ENC_KMAX];                                  // general: reduced row -> value code
+    __shared__ uint8_t clast[ENC_COLS];                                 // general: last code of each column
     __shared__ int64_t sperm[ENC_ROWS];
     const int tid = threadIdx.x, lane = tid & 31;
     // row tiles vary fastest: the CTAs resident at one time cover every sample of a band of
@@ -116,25 +126,29 @@ __global__ void __launch_bounds__(256) onehot_encode_kernel(
         float vf[FS_DISTINCT_CAP];
         if (c < ncols) {
             f = tcol[c0 + c];
-            const int off = toff[c0 + c];
-            V = toff[c0 + c + 1] - off + 1;
-            if (!all_ident) {
+            const int off = kLean ? k0 + 2 * c : toff[c0 + c];
+            V = kLean ? 3 : toff[c0 + c + 1] - off + 1;
+            if constexpr (!kLean) {
+                if (!all_ident) {
 #pragma unroll
-                for (int q = 0; q < FS_DISTINCT_CAP; ++q) {
-                    const double d = q < V ? vals[f * FS_DISTINCT_CAP + q] : 0.0;
-                    v[q] = (Tin)d;
-                    vf[q] = (float)d;
-                    ident = ident && (q >= V || d == (double)q);
+                    for (int q = 0; q < FS_DISTINCT_CAP; ++q) {
+                        const double d = q < V ? vals[f * FS_DISTINCT_CAP + q] : 0.0;
+                        v[q] = (Tin)d;
+                        vf[q] = (float)d;
+                        ident = ident && (q >= V || d == (double)q);
+                    }
                 }
             }
             if (tid < ENC_COLS) {
-                clast[c] = (uint8_t)(V - 1);
-                for (int q = 0; q < V - 1; ++q) {
-                    kcol[off - k0 + q] = (uint8_t)c;
-                    kval[off - k0 + q] = (uint8_t)q;
-                    if (tile_y == 0 && krow)
-                        krow[off + q] = (uint32_t)(tpos ? tpos[c0 + c] : (int32_t)(c0 + c)) | ((uint32_t)q << 24) | ((uint32_t)(V - 1) << 28);
+                if constexpr (!kLean) {
+                    clast[c] = (uint8_t)(V - 1);
+                    for (int q = 0; q < V - 1; ++q) {
+                        kcol[off - k0 + q] = (uint8_t)c;
+                        kval[off - k0 + q] = (uint8_t)q;
+                    }
                 }
+                for (int q = 0; tile_y == 0 && krow && q < V - 1; ++q)
+                    krow[off + q] = (uint32_t)(tpos ? tpos[c0 + c] : (int32_t)(c0 + c)) | ((uint32_t)q << 24) | ((uint32_t)(V - 1) << 28);
             }
         }
         // whole-tile fast path: one-byte input, identity codes, and the tile's 64 columns are 64
@@ -142,23 +156,34 @@ __global__ void __launch_bounds__(256) onehot_encode_kernel(
         const int64_t f0 = tcol[c0];
         const bool fast1 = __syncthreads_and(sizeof(Tin) == 1 && ncols == ENC_COLS && ident && f == f0 + c &&
                                              (ldx & 15) == 0 && ((reinterpret_cast<uintptr_t>(x) + f0) & 15) == 0);
+        // lean second choice: the tile's columns lie within kSpan bytes of x (16-byte aligned base)
+        constexpr int kSpan = 256, kSpanRows = 32;
+        const int64_t fbase = f0 & ~(int64_t)15;
+        const int64_t flast = tcol[c0 + ncols - 1];
+        const bool span_ok = kLean && __syncthreads_and(!fast1 && (ldx & 15) == 0 && (reinterpret_cast<uintptr_t>(x) & 15) == 0 &&
+                                                        flast - fbase < kSpan && (c >= ncols || (f >= fbase && f <= flast)));
         if (fast1) {
+            // two 16-byte loads per thread, both in flight before either is used
+            uint4 q[2];
 #pragma unroll
             for (int i = 0; i < 2; ++i) {
-                const int item = tid + 256 * i, rr = item >> 2, ch = item & 3;
-                uint4 q = make_uint4(0u, 0u, 0u, 0u);
-                if (rr < nrows) {
-                    q = *reinterpret_cast<const uint4 *>(reinterpret_cast<const uint8_t *>(x) + sperm[rr] * ldx + f0 + 16 * ch);
-                    if (codes) *reinterpret_cast<uint4 *>(codes + (r0 + rr) * ldc + c0 + 16 * ch) = q;   // ldc, c0: multiples of 16
-                }
-                *reinterpret_cast<uint4 *>(&code_rc[rr][16 * ch]) = q;
-                const uint32_t qw[4] = {q.x, q.y, q.z, q.w};
+                const int rr = (tid + 256 * i) >> 2, ch = tid & 3;
+                q[i] = rr < nrows ? *reinterpret_cast<const uint4 *>(reinterpret_cast<const uint8_t *>(x) + sperm[rr] * ldx + f0 + 16 * ch)
+                                  : make_uint4(0u, 0u, 0u, 0u);
+            }
+#pragma unroll
+            for (int i = 0; i < 2; ++i) {
+                const int rr = (tid + 256 * i) >> 2, ch = tid & 3;
+                if (codes && rr < nrows) *reinterpret_cast<uint4 *>(codes + (r0 + rr) * ldc + c0 + 16 * ch) = q[i];   // ldc, c0: multiples of 16
+                *reinterpret_cast<uint4 *>(&code_rc[rr][16 * ch]) = q[i];
+                const uint32_t qw[4] = {q[i].x, q[i].y, q[i].z, q[i].w};
 #pragma unroll
                 for (int b = 0; b < 16; ++b) code_cr[16 * ch + b][rr] = (uint8_t)(qw[b >> 2] >> (8 * (b & 3)));
             }
-        } else {
-            // 32 samples per thread (rows tid/64 + 4i): the loads of a batch of 8 are issued before
-            // any of them is used, so 8 requests per thread are in flight
+        } else if (!span_ok) {
+            // gathered columns (TuRF iterations): one column per thread, 32 samples per thread (rows
+            // tid/64 + 4i); the loads of a batch of 8 are issued before any of them is used, so 8
+            // requests per thread are in flight
             constexpr int kBatch = 8;
             for (int i0 = 0; i0 < ENC_ROWS / 4; i0 += kBatch) {
                 Tin xv[kBatch];
@@ -175,18 +200,20 @@ __global__ void __launch_bounds__(256) onehot_encode_kernel(
                         int found = 0;
                         if (ident) {
                             found = (int)xv[u];
-                        } else if (V <= 4) {                 // genotype-like columns: 3 compares, no loop
+                        } else if constexpr (!kLean) {
+                            if (V <= 4) {                   // genotype-like columns: 3 compares, no loop
 #pragma unroll
-                            for (int q = 3; q >= 1; --q) {
-                                const bool eq = as_f32 ? ((float)xv[u] == vf[q]) : (xv[u] == v[q]);
-                                if (q < V && eq) found = q;
-                            }
-                            if (as_f32 ? ((float)xv[u] == vf[0]) : (xv[u] == v[0])) found = 0;   // lowest match wins
-                        } else {
+                                for (int q = 3; q >= 1; --q) {
+                                    const bool eq = as_f32 ? ((float)xv[u] == vf[q]) : (xv[u] == v[q]);
+                                    if (q < V && eq) found = q;
+                                }
+                                if (as_f32 ? ((float)xv[u] == vf[0]) : (xv[u] == v[0])) found = 0;   // lowest match wins
+                            } else {
 #pragma unroll
-                            for (int q = FS_DISTINCT_CAP - 1; q >= 0; --q) {
-                                const bool eq = as_f32 ? ((float)xv[u] == vf[q]) : (xv[u] == v[q]);
-                                if (q < V && eq) found = q;
+                                for (int q = FS_DISTINCT_CAP - 1; q >= 0; --q) {
+                                    const bool eq = as_f32 ? ((float)xv[u] == vf[q]) : (xv[u] == v[q]);
+                                    if (q < V && eq) found = q;
+                                }
                             }
                         }
                         code = (uint8_t)found;
@@ -196,23 +223,49 @@ __global__ void __launch_bounds__(256) onehot_encode_kernel(
                     code_cr[c][rr] = code;
                 }
             }
+        } else if constexpr (kLean) {
+            // gathered columns whose span in x is short (TuRF's early iterations: ascending columns with
+            // a few gaps): the span [fbase, fbase + kSpan) of 32 rows at a time is staged in shared memory
+            // with coalesced 16-byte loads, and every thread picks its column's bytes from there
+            __shared__ __align__(16) uint8_t raw[kSpanRows][kSpan];
+            const int span_chunks = (int)((flast - fbase) >> 4) + 1;          // 16-byte chunks that hold a wanted column
+            for (int rb = 0; rb < ENC_ROWS; rb += kSpanRows) {
+                // fixed 16-chunk indexing (no division by the run-time chunk count); chunks past the span idle
+                for (int item = tid; item < kSpanRows * (kSpan / 16); item += 256) {
+                    const int rr = rb + (item >> 4), ch = item & 15;
+                    if (ch >= span_chunks) continue;
+                    uint4 q = make_uint4(0u, 0u, 0u, 0u);
+                    if (rr < nrows && fbase + 16 * ch < ldx) q = *reinterpret_cast<const uint4 *>(x + sperm[rr] * ldx + fbase + 16 * ch);
+                    *reinterpret_cast<uint4 *>(&raw[rr - rb][16 * ch]) = q;
+                }
+                __syncthreads();
+#pragma unroll
+                for (int u = 0; u < kSpanRows / 4; ++u) {
+                    const int rl = (tid >> 6) + 4 * u, rr = rb + rl;
+                    const uint8_t xv = (c < ncols && rr < nrows) ? raw[rl][(int)(f - fbase)] : (uint8_t)0;
+                    if (codes && c < ncols && rr < nrows) codes[(r0 + rr) * ldc + c0 + c] = xv;
+                    code_rc[rr][c] = xv;
+                    code_cr[c][rr] = xv;
+                }
+                __syncthreads();
+            }
         }
     }
     __syncthreads();
 
     // ---- step 2: U[r, k0..k1), Wd[r, k0..k1), s[r]
-    // fast path (every column of the tile has 3 values and k0 is 16-byte aligned, i.e. 0/1/2
-    // genotypes): 8 codes -> 16 bytes of U and of Wd, built with shifts
     const int kg0 = k0 + uk0, kg1 = k1 + uk0;          // the same rows in U / Wd
-    const bool v3 = __syncthreads_and((tid >= ncols) || clast[tid < ncols ? tid : 0] == 2) && (kg0 & 31) == 0 &&
-                    (ncols & 15) == 0;
+    // every column of the tile has 3 values (0/1/2 genotypes): two reduced rows per column, codes are the rows' bits
+    bool all3 = true;
+    if constexpr (!kLean) all3 = __syncthreads_and((tid >= ncols) || clast[tid < ncols ? tid : 0] == 2);
     if (U == nullptr) {
         // distance operands not wanted (the slab is updated incrementally from other columns)
-    } else if (v3) {
+    } else if (all3 && (kg0 & 31) == 0 && (ncols & 15) == 0) {
         // 16 columns per item: 16 code bytes -> 16 bytes of U and of Wd (one byte per column)
         const int ngroups = ncols >> 4;
-        for (int item = tid; item < ENC_ROWS * 4; item += 256) {      // uniform trip count (shuffles below)
-            const int rr = item >> 2, g = item & 3;
+#pragma unroll
+        for (int it = 0; it < ENC_ROWS * 4 / 256; ++it) {                 // uniform trip count (shuffles below)
+            const int item = tid + 256 * it, rr = item >> 2, g = item & 3;
             int cnt = 0;
             if (rr < nrows && g < ngroups) {
                 const uint4 cw = *reinterpret_cast<const uint4 *>(&code_rc[rr][16 * g]);
@@ -229,6 +282,23 @@ __global__ void __launch_bounds__(256) onehot_encode_kernel(
             cnt += __shfl_xor_sync(0xffffffffu, cnt, 1);
             cnt += __shfl_xor_sync(0xffffffffu, cnt, 2);
             if (g == 0 && rr < nrows && cnt) atomicAdd(&srow[r0 + rr], cnt);
+        }
+    } else if constexpr (kLean) {
+        // ragged last column tile: one (sample, column) byte per step
+        for (int rr = tid >> 5; rr < ENC_ROWS; rr += 8) {
+            int cnt = 0;
+            if (rr < nrows)
+                for (int cc = lane; cc < ncols; cc += 32) {
+                    const uint32_t code = code_rc[rr][cc];
+                    const int64_t o = (r0 + rr) * K + (kg0 >> 1) + cc;
+                    if (r0 + rr >= u_lo && r0 + rr < u_hi)
+                        U[o - u_lo * K] = (int8_t)(code == 0u ? 0x02u : code == 1u ? 0x20u : 0u);
+                    if (wr.has(r0 + rr)) Wd[o] = (int8_t)(code == 0u ? 0x24u : code == 1u ? 0x42u : 0u);
+                    cnt += code != 2u ? 1 : 0;
+                }
+#pragma unroll
+            for (int o = 16; o >= 1; o >>= 1) cnt += __shfl_xor_sync(0xffffffffu, cnt, o);
+            if (lane == 0 && rr < nrows && cnt) atomicAdd(&srow[r0 + rr], cnt);
         }
     } else {
         // general path: nibbles k0..k1 of the row; 32-bit words (8 nibbles) that belong to this tile
@@ -275,8 +345,8 @@ __global__ void __launch_bounds__(256) onehot_encode_kernel(
     // ---- step 3: At[k, r0..r0+128) and codesT[c, r0..r0+128): 16 samples per store
     if (At == nullptr) {
         // accumulation operands not wanted (columns that only update the distance slab)
-    } else if (v3 && nrows == ENC_ROWS) {
-        // 0/1/2 fast path: one item = 16 samples of one column -> its two At rows and its codesT row
+    } else if (all3) {
+        // one item = 16 samples of one column -> its two At rows and its codesT row
         for (int item = tid; item < ncols * 8; item += 256) {
             const int c = item >> 3, seg = item & 7;
             const uint32_t *src = reinterpret_cast<const uint32_t *>(&code_cr[c][16 * seg]);
@@ -288,11 +358,28 @@ __global__ void __launch_bounds__(256) onehot_encode_kernel(
             e1.w = w.w & 0x01010101u; e0.w = ((w.w >> 1) & 0x01010101u) ^ 0x01010101u ^ e1.w;
             const int64_t o = r0 + 16 * seg;                                  // r0, ldt multiples of 128: aligned
             const int64_t lda = ldt >> 1;                                     // At: two samples per byte
-            *reinterpret_cast<uint2 *>(At + (int64_t)(k0 + 2 * c) * lda + (o >> 1)) = pack_fp4_flags16(e0.x, e0.y, e0.z, e0.w);
-            *reinterpret_cast<uint2 *>(At + (int64_t)(k0 + 2 * c + 1) * lda + (o >> 1)) = pack_fp4_flags16(e1.x, e1.y, e1.z, e1.w);
-            if (codesT) *reinterpret_cast<uint4 *>(codesT + (c0 + c) * ldt + o) = w;
+            int8_t *a0 = At + (int64_t)(k0 + 2 * c) * lda + (o >> 1), *a1 = a0 + lda;
+            uint8_t *ct = codesT ? codesT + (c0 + c) * ldt + o : nullptr;
+            if (16 * seg + 16 <= nrows) {
+                *reinterpret_cast<uint2 *>(a0) = pack_fp4_flags16(e0.x, e0.y, e0.z, e0.w);
+                *reinterpret_cast<uint2 *>(a1) = pack_fp4_flags16(e1.x, e1.y, e1.z, e1.w);
+                if (ct) *reinterpret_cast<uint4 *>(ct) = w;
+            } else {
+                // ragged last row tile: whole bytes only where a sample lives, zero nibbles past nrows
+                for (int b = 0; b < 16 && 16 * seg + b < nrows; b += 2) {
+                    const uint32_t ca = code_cr[c][16 * seg + b];
+                    const bool two = 16 * seg + b + 1 < nrows;
+                    const uint32_t cb = two ? code_cr[c][16 * seg + b + 1] : 3u;     // 3 matches no value
+                    a0[b >> 1] = (int8_t)((ca == 0u ? 0x02u : 0u) | (cb == 0u ? 0x20u : 0u));
+                    a1[b >> 1] = (int8_t)((ca == 1u ? 0x02u : 0u) | (cb == 1u ? 0x20u : 0u));
+                    if (ct) {
+                        ct[b] = (uint8_t)ca;
+                        if (two) ct[b + 1] = (uint8_t)cb;
+                    }
+                }
+            }
         }
-    } else {
+    } else if constexpr (!kLean) {
         const int nk = k1 - k0;
         for (int item = tid; item < nk * 8; item += 256) {
             const int kk = item >> 3, seg = item & 7;
@@ -337,214 +424,49 @@ __global__ void __launch_bounds__(256) onehot_encode_kernel(
     }
 }
 
-// Lean variant for the case that matters most: one-byte input whose active columns all hold
-// exactly the values 0/1/2 (the value is its own code, two reduced rows per column, k0 = 2 c0).
-// No code tables, no per-column bookkeeping: registers stay low enough for 6 CTAs per SM, which
-// is what hides the perm -> x load chain of this streaming kernel.
-__global__ void __launch_bounds__(256, 6) onehot_encode_v3_kernel(
-    const uint8_t *__restrict__ x, int64_t ldx, const int64_t *__restrict__ perm, const int64_t *__restrict__ tcol,
-    int64_t n, int64_t pt, int64_t K, int64_t ldt, int64_t ldc, int8_t *__restrict__ U, int8_t *__restrict__ Wd,
-    int8_t *__restrict__ At, uint8_t *__restrict__ codesT, uint8_t *__restrict__ codes, int32_t *__restrict__ srow,
-    uint32_t *__restrict__ krow, int64_t u_lo, int64_t u_hi, const int32_t *__restrict__ tpos, int64_t ucol0, WdRows wr) {
-    // ucol0: column of U / Wd that this launch's column 0 stands for (see onehot_encode_kernel's uk0)
-    __shared__ __align__(16) uint8_t code_rc[ENC_ROWS][ENC_COLS];       // [sample][column]
-    __shared__ __align__(16) uint8_t code_cr[ENC_COLS][ENC_CR_LD];      // [column][sample]
-    __shared__ int64_t sperm[ENC_ROWS];
-    const int tid = threadIdx.x;
-    // row tiles vary fastest: the CTAs resident at one time cover every sample of a band of
-    // columns, so the feature-major rows (At, codesT) are written as whole contiguous rows
-    const int tiles_y = (int)((n + ENC_ROWS - 1) / ENC_ROWS);
-    const int tile_x = (int)(blockIdx.x / tiles_y), tile_y = (int)(blockIdx.x % tiles_y);
-    const int64_t c0 = (int64_t)tile_x * ENC_COLS, r0 = (int64_t)tile_y * ENC_ROWS;
-    const int ncols = (int)(pt - c0 < ENC_COLS ? pt - c0 : ENC_COLS);
-    const int nrows = (int)(n - r0 < ENC_ROWS ? n - r0 : ENC_ROWS);
-    const int64_t k0 = 2 * c0;
-    // a distance-only launch has nothing to do for a row tile whose samples' Wd rows nobody reads
-    if (At == nullptr && codes == nullptr && !wr.touches(r0, r0 + nrows)) return;
-    if (tid < ENC_ROWS) sperm[tid] = tid < nrows ? perm[r0 + tid] : 0;
-    const int c = tid & (ENC_COLS - 1);
-    const int64_t f = c < ncols ? tcol[c0 + c] : 0, f0 = tcol[c0];
-    if (tile_y == 0 && krow && tid < ncols) {
-        const uint32_t crow = (uint32_t)(tpos ? tpos[c0 + tid] : (int32_t)(c0 + tid));   // codesT row of this column
-        krow[k0 + 2 * tid] = crow | (2u << 28);
-        krow[k0 + 2 * tid + 1] = crow | (1u << 24) | (2u << 28);
-    }
-    // ---- step 1: codes (= values) into shared memory, both orientations
-    const bool fast1 = __syncthreads_and(ncols == ENC_COLS && f == f0 + c && (ldx & 15) == 0 &&
-                                         ((reinterpret_cast<uintptr_t>(x) + f0) & 15) == 0);
-    // second choice: the tile's columns lie within kSpan bytes of x (16-byte aligned base)
-    constexpr int kSpan = 256, kSpanRows = 32;
-    __shared__ __align__(16) uint8_t raw[kSpanRows][kSpan];
-    const int64_t fbase = f0 & ~(int64_t)15;
-    const int64_t flast = tcol[c0 + ncols - 1];
-    const bool span_ok = __syncthreads_and(!fast1 && (ldx & 15) == 0 && (reinterpret_cast<uintptr_t>(x) & 15) == 0 &&
-                                           flast - fbase < kSpan && (c >= ncols || (f >= fbase && f <= flast)));
-    const int span_chunks = (int)((flast - fbase) >> 4) + 1;          // 16-byte chunks that hold a wanted column
-    if (fast1) {
-        // the tile's 64 columns are 64 consecutive, 16-byte aligned bytes of every row of x
-#pragma unroll
-        for (int i = 0; i < 2; ++i) {
-            const int item = tid + 256 * i, rr = item >> 2, ch = item & 3;
-            uint4 q = make_uint4(0u, 0u, 0u, 0u);
-            if (rr < nrows) {
-                q = *reinterpret_cast<const uint4 *>(x + sperm[rr] * ldx + f0 + 16 * ch);
-                if (codes) *reinterpret_cast<uint4 *>(codes + (r0 + rr) * ldc + c0 + 16 * ch) = q;
-            }
-            *reinterpret_cast<uint4 *>(&code_rc[rr][16 * ch]) = q;
-            const uint32_t qw[4] = {q.x, q.y, q.z, q.w};
-#pragma unroll
-            for (int b = 0; b < 16; ++b) code_cr[16 * ch + b][rr] = (uint8_t)(qw[b >> 2] >> (8 * (b & 3)));
-        }
-    } else if (span_ok) {
-        // gathered columns whose span in x is short (TuRF's early iterations: ascending columns with
-        // a few gaps): the span [fbase, fbase + kSpan) of 32 rows at a time is staged in shared memory
-        // with coalesced 16-byte loads, and every thread picks its column's bytes from there
-        for (int rb = 0; rb < ENC_ROWS; rb += kSpanRows) {
-            // fixed 16-chunk indexing (no division by the run-time chunk count); chunks past the span idle
-            for (int item = tid; item < kSpanRows * (kSpan / 16); item += 256) {
-                const int rr = rb + (item >> 4), ch = item & 15;
-                if (ch >= span_chunks) continue;
-                uint4 q = make_uint4(0u, 0u, 0u, 0u);
-                if (rr < nrows && fbase + 16 * ch < ldx) q = *reinterpret_cast<const uint4 *>(x + sperm[rr] * ldx + fbase + 16 * ch);
-                *reinterpret_cast<uint4 *>(&raw[rr - rb][16 * ch]) = q;
-            }
-            __syncthreads();
-#pragma unroll
-            for (int u = 0; u < kSpanRows / 4; ++u) {
-                const int rl = (tid >> 6) + 4 * u, rr = rb + rl;
-                const uint8_t xv = (c < ncols && rr < nrows) ? raw[rl][(int)(f - fbase)] : (uint8_t)0;
-                if (codes && c < ncols && rr < nrows) codes[(r0 + rr) * ldc + c0 + c] = xv;
-                code_rc[rr][c] = xv;
-                code_cr[c][rr] = xv;
-            }
-            __syncthreads();
-        }
-    } else {
-        // gathered columns (TuRF iterations): one column per thread, 8 loads in flight
-        constexpr int kBatch = 8;
-        for (int i0 = 0; i0 < ENC_ROWS / 4; i0 += kBatch) {
-            uint8_t xv[kBatch];
-#pragma unroll
-            for (int u = 0; u < kBatch; ++u) {
-                const int rr = (tid >> 6) + 4 * (i0 + u);
-                xv[u] = (c < ncols && rr < nrows) ? x[sperm[rr] * ldx + f] : (uint8_t)0;
-            }
-#pragma unroll
-            for (int u = 0; u < kBatch; ++u) {
-                const int rr = (tid >> 6) + 4 * (i0 + u);
-                if (codes && c < ncols && rr < nrows) codes[(r0 + rr) * ldc + c0 + c] = xv[u];
-                code_rc[rr][c] = xv[u];
-                code_cr[c][rr] = xv[u];
-            }
-        }
-    }
-    __syncthreads();
-    // ---- step 2: U, Wd (16 bytes per 8 codes) and the per-sample counts s
-    if (U != nullptr) {
-        if ((ncols & 15) == 0) {
-            // 16 columns per item: 16 code bytes -> 16 bytes of U and of Wd (one byte per column)
-            const int ngroups = ncols >> 4;
-#pragma unroll
-            for (int it = 0; it < ENC_ROWS * 4 / 256; ++it) {
-                const int item = tid + 256 * it, rr = item >> 2, g = item & 3;
-                int cnt = 0;
-                if (rr < nrows && g < ngroups) {
-                    const uint4 cw = *reinterpret_cast<const uint4 *>(&code_rc[rr][16 * g]);
-                    uint4 u, w;
-                    expand_v3_fp4(cw.x, u.x, w.x, cnt);
-                    expand_v3_fp4(cw.y, u.y, w.y, cnt);
-                    expand_v3_fp4(cw.z, u.z, w.z, cnt);
-                    expand_v3_fp4(cw.w, u.w, w.w, cnt);
-                    const int64_t o = (r0 + rr) * K + ucol0 + c0 + 16 * g;       // K = row pitch in bytes; one byte per column
-                    // U holds only the rows [u_lo, u_hi) (the target rows of this rank)
-                    if (r0 + rr >= u_lo && r0 + rr < u_hi) *reinterpret_cast<uint4 *>(U + o - u_lo * K) = u;
-                    if (wr.has(r0 + rr)) *reinterpret_cast<uint4 *>(Wd + o) = w;
-                }
-                cnt += __shfl_xor_sync(0xffffffffu, cnt, 1);
-                cnt += __shfl_xor_sync(0xffffffffu, cnt, 2);
-                if (g == 0 && rr < nrows && cnt) atomicAdd(&srow[r0 + rr], cnt);
-            }
-        } else {
-            // ragged last column tile: one (sample, column) byte per step
-            for (int rr = tid >> 5; rr < ENC_ROWS; rr += 8) {
-                int cnt = 0;
-                if (rr < nrows)
-                    for (int cc = tid & 31; cc < ncols; cc += 32) {
-                        const uint32_t code = code_rc[rr][cc];
-                        const int64_t o = (r0 + rr) * K + ucol0 + c0 + cc;
-                        if (r0 + rr >= u_lo && r0 + rr < u_hi)
-                            U[o - u_lo * K] = (int8_t)(code == 0u ? 0x02u : code == 1u ? 0x20u : 0u);
-                        if (wr.has(r0 + rr)) Wd[o] = (int8_t)(code == 0u ? 0x24u : code == 1u ? 0x42u : 0u);
-                        cnt += code != 2u ? 1 : 0;
-                    }
-#pragma unroll
-                for (int o = 16; o >= 1; o >>= 1) cnt += __shfl_xor_sync(0xffffffffu, cnt, o);
-                if ((tid & 31) == 0 && rr < nrows && cnt) atomicAdd(&srow[r0 + rr], cnt);
-            }
-        }
-    }
-    // ---- step 3: the two At rows and the codesT row of each column, 16 samples per store
-    if (At != nullptr) {
-        for (int item = tid; item < ncols * 8; item += 256) {
-            const int cc = item >> 3, seg = item & 7;
-            const uint32_t *src = reinterpret_cast<const uint32_t *>(&code_cr[cc][16 * seg]);
-            const uint4 w = make_uint4(src[0], src[1], src[2], src[3]);
-            uint4 e0, e1;
-            e1.x = w.x & 0x01010101u; e0.x = ((w.x >> 1) & 0x01010101u) ^ 0x01010101u ^ e1.x;
-            e1.y = w.y & 0x01010101u; e0.y = ((w.y >> 1) & 0x01010101u) ^ 0x01010101u ^ e1.y;
-            e1.z = w.z & 0x01010101u; e0.z = ((w.z >> 1) & 0x01010101u) ^ 0x01010101u ^ e1.z;
-            e1.w = w.w & 0x01010101u; e0.w = ((w.w >> 1) & 0x01010101u) ^ 0x01010101u ^ e1.w;
-            const int64_t o = r0 + 16 * seg;                                  // r0, ldt multiples of 128: aligned
-            const int64_t lda = ldt >> 1;                                     // At: two samples per byte (FP4 nibbles)
-            int8_t *a0 = At + (k0 + 2 * cc) * lda + (o >> 1), *a1 = a0 + lda;
-            uint8_t *ct = codesT ? codesT + (c0 + cc) * ldt + o : nullptr;
-            if (16 * seg + 16 <= nrows) {
-                *reinterpret_cast<uint2 *>(a0) = pack_fp4_flags16(e0.x, e0.y, e0.z, e0.w);
-                *reinterpret_cast<uint2 *>(a1) = pack_fp4_flags16(e1.x, e1.y, e1.z, e1.w);
-                if (ct) *reinterpret_cast<uint4 *>(ct) = w;
-            } else {
-                for (int b = 0; b < 16 && 16 * seg + b < nrows; b += 2) {
-                    const uint32_t ca = code_cr[cc][16 * seg + b];
-                    const bool two = 16 * seg + b + 1 < nrows;
-                    const uint32_t cb = two ? code_cr[cc][16 * seg + b + 1] : 3u;     // 3 matches no value
-                    a0[b >> 1] = (int8_t)((ca == 0u ? 0x02u : 0u) | (cb == 0u ? 0x20u : 0u));
-                    a1[b >> 1] = (int8_t)((ca == 1u ? 0x02u : 0u) | (cb == 1u ? 0x20u : 0u));
-                    if (ct) {
-                        ct[b] = (uint8_t)ca;
-                        if (two) ct[b + 1] = (uint8_t)cb;
-                    }
-                }
-            }
-        }
+// The lean instantiation hard-codes 0/1/2 genotypes: identity codes AND exactly three values in EVERY column of a
+// non-empty list (K_used == 2 * pt alone also holds for, say, one 2-valued plus one 4-valued column).
+static bool lean_encode(bool all_ident, bool all_v3, int64_t pc) { return all_ident && all_v3 && pc > 0; }
+
+// Clears what the encode launches that fill the distance operands U [u_rows, K/2 bytes] and Wd [n, K/2 bytes]
+// do not write.  The lean kernel writes every byte of its columns, so only the K padding (reduced rows
+// K_used..K); the general kernel ORs the words at unaligned tile edges in, so everything.
+static void clear_dist_ops(bool lean, int8_t *U, int64_t u_rows, int8_t *Wd, int64_t n, int64_t K_used, int64_t K,
+                           cudaStream_t st) {
+    const size_t Kb = (size_t)K / 2;
+    if (!lean) {
+        FS_CUDA(cudaMemsetAsync(U, 0, (size_t)u_rows * Kb, st));
+        FS_CUDA(cudaMemsetAsync(Wd, 0, (size_t)n * Kb, st));
+    } else if (K > K_used) {
+        FS_CUDA(cudaMemset2DAsync(U + K_used / 2, Kb, 0, (size_t)(K - K_used) / 2, (size_t)u_rows, st));
+        FS_CUDA(cudaMemset2DAsync(Wd + K_used / 2, Kb, 0, (size_t)(K - K_used) / 2, (size_t)n, st));
     }
 }
 
-// One launch of the encode over the columns tcol[0, pc): the lean kernel (every column holds exactly the values 0/1/2
-// of a one-byte input), else the general kernel in the input's type.  off: the columns' first reduced rows; uk0 /
-// ucol0: the reduced row / column of U and Wd that the launch's first one stands for.  Null outputs are not written.
+// One launch of the encode over the columns tcol[0, pc): the lean kernel (see lean_encode), else the general
+// kernel in the input's type.  off: the columns' first reduced rows; uk0: the reduced row of U and Wd that off's
+// row 0 stands for.  Null outputs are not written.
 static void launch_encode(const fs_dataset *ds, bool lean, int all_ident, const int64_t *tcol, const int32_t *off, int64_t pc,
                           int64_t K, int64_t ldt, int64_t ldc, int8_t *U, int8_t *Wd, int8_t *At, uint8_t *codesT,
                           uint8_t *codes, int32_t *srow, uint32_t *krow, int64_t u_lo, int64_t u_hi, const int32_t *tpos,
-                          int uk0, int64_t ucol0, WdRows wr, cudaStream_t st, int *launches) {
+                          int uk0, WdRows wr, cudaStream_t st, int *launches) {
     const int64_t n = ds->n;
     const unsigned grid = (unsigned)(ceil_div(pc, ENC_COLS) * ceil_div(n, ENC_ROWS));
     const int as_f32 = (ds->arith == FS_ARITH_F32 && ds->dtype == FS_F64) ? 1 : 0;
-    auto general = [&](auto type_tag) {
+    auto encode = [&](auto type_tag, auto lean_tag) {
         using T = decltype(type_tag);
-        onehot_encode_kernel<T><<<grid, 256, 0, st>>>(static_cast<const T *>(ds->x), ds->ldx, ds->d_perm.ptr, tcol, off,
-                                                      ds->d_vals.ptr, as_f32, n, pc, K, ldt, ldc, U, Wd, At, codesT, codes,
-                                                      srow, krow, all_ident, u_lo, u_hi, tpos, uk0, wr);
+        onehot_encode_kernel<T, decltype(lean_tag)::value><<<grid, 256, 0, st>>>(
+            static_cast<const T *>(ds->x), ds->ldx, ds->d_perm.ptr, tcol, off, ds->d_vals.ptr, as_f32, n, pc, K, ldt, ldc,
+            U, Wd, At, codesT, codes, srow, krow, all_ident, u_lo, u_hi, tpos, uk0, wr);
     };
     if (lean) {
-        onehot_encode_v3_kernel<<<grid, 256, 0, st>>>(static_cast<const uint8_t *>(ds->x), ds->ldx, ds->d_perm.ptr, tcol, n, pc,
-                                                      K, ldt, ldc, U, Wd, At, codesT, codes, srow, krow, u_lo, u_hi, tpos,
-                                                      ucol0, wr);
+        encode(uint8_t{}, std::true_type{});      // FS_U8 and FS_I8 alike: the bytes are the codes 0/1/2
     } else {
         switch (ds->dtype) {
-            case FS_U8: general(uint8_t{}); break;
-            case FS_I8: general(int8_t{}); break;
-            case FS_F32: general(float{}); break;
-            case FS_F64: general(double{}); break;
+            case FS_U8: encode(uint8_t{}, std::false_type{}); break;
+            case FS_I8: encode(int8_t{}, std::false_type{}); break;
+            case FS_F32: encode(float{}, std::false_type{}); break;
+            case FS_F64: encode(double{}, std::false_type{}); break;
         }
     }
     FS_CUDA(cudaGetLastError());
@@ -582,19 +504,10 @@ static void build_removed(fs_dataset *ds, WorkSet &ws, int *launches) {
     FS_CUDA(cudaMemcpyAsync(ws.roff.ptr, ws.p_roff.ptr, (pr + 1) * sizeof(int32_t), cudaMemcpyHostToDevice, st));
     FS_CUDA(cudaMemsetAsync(ws.srow_r.ptr, 0, ws.ldt * sizeof(int32_t), st));
     const int all_ident = (ident & kColIdent) ? 1 : 0;
-    // the lean kernel hard-codes 0/1/2: EVERY column must have exactly three values (a mix of 2- and
-    // 4-valued columns can also add up to two reduced rows per column on average)
-    const bool lean = all_ident && v3 && pr > 0;
-    if (!lean) {
-        // general encoder ORs partial words in: clear everything
-        FS_CUDA(cudaMemsetAsync(ws.Ur.ptr, 0, (size_t)n * Kb, st));
-        FS_CUDA(cudaMemsetAsync(ws.Wdr.ptr, 0, (size_t)n * Kb, st));
-    } else if (ws.Kr > ws.Kr_used) {
-        FS_CUDA(cudaMemset2DAsync(ws.Ur.ptr + ws.Kr_used / 2, Kb, 0, (size_t)(ws.Kr - ws.Kr_used) / 2, (size_t)n, st));
-        FS_CUDA(cudaMemset2DAsync(ws.Wdr.ptr + ws.Kr_used / 2, Kb, 0, (size_t)(ws.Kr - ws.Kr_used) / 2, (size_t)n, st));
-    }
+    const bool lean = lean_encode(all_ident, v3, pr);
+    clear_dist_ops(lean, ws.Ur.ptr, n, ws.Wdr.ptr, n, ws.Kr_used, ws.Kr, st);
     launch_encode(ds, lean, all_ident, ws.rcol.ptr, ws.roff.ptr, pr, (int64_t)Kb, ws.ldt, 0, ws.Ur.ptr, ws.Wdr.ptr, nullptr,
-                  nullptr, nullptr, ws.srow_r.ptr, nullptr, 0, n, nullptr, 0, 0, WdRows{0, n, 0, 0}, st, launches);
+                  nullptr, nullptr, ws.srow_r.ptr, nullptr, 0, n, nullptr, 0, WdRows{0, n, 0, 0}, st, launches);
 }
 
 void build_onehot(fs_dataset *ds, WorkSet &ws, bool group_call, int *launches) {
@@ -654,22 +567,15 @@ void build_onehot(fs_dataset *ds, WorkSet &ws, bool group_call, int *launches) {
         FS_CUDA(cudaMemcpyAsync(ws.atoff.ptr, ws.p_atoff.ptr, (pa + 1) * sizeof(int32_t), cudaMemcpyHostToDevice, st));
         ws.lists_uploaded = true;
     }
-    // the encode kernel writes every used byte of U, Wd, At and codesT exactly once; only the K
-    // padding (reduced rows K_used..K) has to be cleared.  Sample padding of the feature-major
-    // rows (columns n..ldt) is never read (the TMA maps are n bytes wide).
-    if (ops) FS_CUDA(cudaMemsetAsync(ws.srow.ptr, 0, ws.ldt * sizeof(int32_t), st));
     const size_t Kb = (size_t)ws.K / 2;
-    // the lean kernel hard-codes 0/1/2 genotypes: identity codes AND exactly three values in EVERY column
-    // (K_used == 2 * pt alone also holds for, say, one 2-valued plus one 4-valued column)
-    const bool lean = ws.all_ident && ws.all_v3;
-    if (ops && !lean) {
-        // the general encoder ORs the words at unaligned tile edges in: clear the operands first
-        FS_CUDA(cudaMemsetAsync(ws.U.ptr, 0, (size_t)(ws.u_hi - ws.u_lo) * Kb, st));
-        FS_CUDA(cudaMemsetAsync(ws.Wd.ptr, 0, (size_t)n * Kb, st));
-    } else if (ops && ws.K > ws.K_used) {
-        FS_CUDA(cudaMemset2DAsync(ws.U.ptr + ws.K_used / 2, Kb, 0, (size_t)(ws.K - ws.K_used) / 2, (size_t)(ws.u_hi - ws.u_lo), st));
-        FS_CUDA(cudaMemset2DAsync(ws.Wd.ptr + ws.K_used / 2, Kb, 0, (size_t)(ws.K - ws.K_used) / 2, (size_t)n, st));
+    const bool lean = lean_encode(ws.all_ident, ws.all_v3, pt);
+    if (ops) {
+        FS_CUDA(cudaMemsetAsync(ws.srow.ptr, 0, ws.ldt * sizeof(int32_t), st));
+        clear_dist_ops(lean, ws.U.ptr, ws.u_hi - ws.u_lo, ws.Wd.ptr, n, ws.K_used, ws.K, st);
     }
+    // the encode writes every used byte of At and codesT exactly once; only the K padding (reduced rows
+    // Ka_used..Ka) has to be cleared.  Sample padding of the feature-major rows (columns n..ldt) is never
+    // read (the TMA maps are n bytes wide).
     if (ws.Ka > ws.Ka_used)
         FS_CUDA(cudaMemsetAsync(ws.At.ptr + (size_t)ws.Ka_used * (ws.ldt / 2), 0, (size_t)(ws.Ka - ws.Ka_used) * (ws.ldt / 2), st));
     const int all_ident = ws.all_ident ? 1 : 0;
@@ -702,7 +608,7 @@ void build_onehot(fs_dataset *ds, WorkSet &ws, bool group_call, int *launches) {
         int32_t *So = want_dist ? ws.srow.ptr : nullptr;
         uint8_t *codes = want_codes ? ws.codes.ptr : nullptr;       // sample-major value codes (ReliefF)
         launch_encode(ds, lean, all_ident, ws.tcol.ptr + c_lo, off, pc, (int64_t)Kb, ws.ldt, ws.ldc, Uo, Wo, Ao, Co, codes, So,
-                      Ko, ws.u_lo, ws.u_hi, To, uk0, c_lo, wr, st, launches);
+                      Ko, ws.u_lo, ws.u_hi, To, uk0, wr, st, launches);
     };
     if (!split) {
         launch(0, pt, ops, true, ws.have_codes);
