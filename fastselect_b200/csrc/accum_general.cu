@@ -222,52 +222,52 @@ int64_t accum_general_partials(const WorkSet &ws, int64_t R) {
     return ceil_div(R, rows_per_cta_for(R, ws.ldg));
 }
 
-void launch_accum_general(const WorkSet &ws, int64_t n, const void *xa, const int8_t *sel, int64_t ldn,
+void launch_accum_general(const WorkSet &ws, int64_t n, int64_t row0, const int8_t *sel, int64_t ldn,
                           const RowInfo *rinfo, int64_t R, double *partial, int64_t n_part, cudaStream_t st,
                           int *launches) {
     if (ws.pg == 0 || R == 0) return;
     const int64_t rows = rows_per_cta_for(R, ws.ldg);
     dim3 grid((unsigned)n_part, (unsigned)ceil_div(ws.ldg, kAccThreads));
+    const size_t a_off = (size_t)row0 * ws.ldg;        // the target rows: a view of the matrix
     // float64 arithmetic (SURF) with only continuous columns: the reference STORES each term as float32
     // (diffs_from_i, SURF.py:143-158) and adds float32 sums, so the accumulation runs on the float32 image
     // of the offset-free columns (x - column minimum: |x'| <= range, so the image keeps 2^-24 of the RANGE,
     // not of |x|) with the float32 kernel -- FP32 pipe instead of three FP64 operations per (pair, feature).
-    // Target rows given as a view into xg (the production path); a gathered copy (fs_debug_rows) stays on
-    // the float64 kernel.
-    const char *xg_lo = ws.xg.ptr, *xg_hi = ws.xg.ptr + (size_t)n * ws.ldg * ws.elem;
-    const bool view = static_cast<const char *>(xa) >= xg_lo && static_cast<const char *>(xa) < xg_hi;
-    if (ws.elem == 8 && ws.have_xg32 && view) {
-        const int64_t row0 = (static_cast<const char *>(xa) - xg_lo) / ((int64_t)ws.ldg * ws.elem);
+    // float64 data with compare columns stays on the float64 kernel.
+    if (ws.elem == 8 && ws.have_xg32) {
         accum_general_kernel<float><<<grid, kAccThreads, 0, st>>>(
-            ws.xg32.ptr, n, ws.ldg, ws.rg.ptr, ws.ctype.ptr, ws.xg32.ptr + (size_t)row0 * ws.ldg, sel, ldn, rinfo, R, rows,
+            ws.xg32.ptr, n, ws.ldg, ws.rg.ptr, ws.ctype.ptr, ws.xg32.ptr + a_off, sel, ldn, rinfo, R, rows,
             partial, kChunkBytes / 8);
-    } else if (ws.elem == 4)
+    } else if (ws.elem == 4) {
+        const float *xg = reinterpret_cast<const float *>(ws.xg.ptr);
         accum_general_kernel<float><<<grid, kAccThreads, 0, st>>>(
-            reinterpret_cast<const float *>(ws.xg.ptr), n, ws.ldg, ws.rg.ptr, ws.ctype.ptr,
-            static_cast<const float *>(xa), sel, ldn, rinfo, R, rows, partial, kChunkBytes / 4);
-    else
+            xg, n, ws.ldg, ws.rg.ptr, ws.ctype.ptr, xg + a_off, sel, ldn, rinfo, R, rows, partial, kChunkBytes / 4);
+    } else {
+        const double *xg = reinterpret_cast<const double *>(ws.xg.ptr);
         accum_general_kernel<double><<<grid, kAccThreads, 0, st>>>(
-            reinterpret_cast<const double *>(ws.xg.ptr), n, ws.ldg, ws.rg.ptr, ws.ctype.ptr,
-            static_cast<const double *>(xa), sel, ldn, rinfo, R, rows, partial, kChunkBytes / 8);
+            xg, n, ws.ldg, ws.rg.ptr, ws.ctype.ptr, xg + a_off, sel, ldn, rinfo, R, rows, partial, kChunkBytes / 8);
+    }
     FS_CUDA(cudaGetLastError());
     ++*launches;
 }
 
-void launch_relieff_gather(const WorkSet &ws, int64_t n, const void *xa, const int32_t *nbr_idx,
+void launch_relieff_gather(const WorkSet &ws, int64_t n, int64_t row0, const int32_t *nbr_idx,
                            const double *nbr_w, const int32_t *nbr_cnt, int32_t nbr_cap, int64_t R,
                            double *partial, int64_t n_part, cudaStream_t st, int *launches) {
     (void)n;
     if (ws.pg == 0 || R == 0) return;
     const int64_t rows = rows_per_cta_for(R, ws.ldg);
     dim3 grid((unsigned)n_part, (unsigned)ceil_div(ws.ldg, kAccThreads));
-    if (ws.elem == 4)
-        relieff_gather_kernel<float><<<grid, kAccThreads, 0, st>>>(
-            reinterpret_cast<const float *>(ws.xg.ptr), ws.ldg, ws.rg.ptr, ws.ctype.ptr,
-            static_cast<const float *>(xa), nbr_idx, nbr_w, nbr_cnt, nbr_cap, R, rows, partial);
-    else
-        relieff_gather_kernel<double><<<grid, kAccThreads, 0, st>>>(
-            reinterpret_cast<const double *>(ws.xg.ptr), ws.ldg, ws.rg.ptr, ws.ctype.ptr,
-            static_cast<const double *>(xa), nbr_idx, nbr_w, nbr_cnt, nbr_cap, R, rows, partial);
+    const size_t a_off = (size_t)row0 * ws.ldg;        // the target rows: a view of the matrix
+    if (ws.elem == 4) {
+        const float *xg = reinterpret_cast<const float *>(ws.xg.ptr);
+        relieff_gather_kernel<float><<<grid, kAccThreads, 0, st>>>(xg, ws.ldg, ws.rg.ptr, ws.ctype.ptr, xg + a_off, nbr_idx,
+                                                                   nbr_w, nbr_cnt, nbr_cap, R, rows, partial);
+    } else {
+        const double *xg = reinterpret_cast<const double *>(ws.xg.ptr);
+        relieff_gather_kernel<double><<<grid, kAccThreads, 0, st>>>(xg, ws.ldg, ws.rg.ptr, ws.ctype.ptr, xg + a_off, nbr_idx,
+                                                                    nbr_w, nbr_cnt, nbr_cap, R, rows, partial);
+    }
     FS_CUDA(cudaGetLastError());
     ++*launches;
 }
@@ -275,7 +275,7 @@ void launch_relieff_gather(const WorkSet &ws, int64_t n, const void *xa, const i
 // ReliefF on the one-hot columns: sparse neighbour lists, value codes compared directly
 // (ReliefF.py:181-216; at most C*k neighbours per target) -- HBM/L2-bound gather.
 __global__ void __launch_bounds__(128) relieff_codes_gather_kernel(
-    const uint8_t *__restrict__ codes, int64_t ldc, int64_t pt, const int64_t *__restrict__ ids,
+    const uint8_t *__restrict__ codes, int64_t ldc, int64_t pt, int64_t row0,
     const int32_t *__restrict__ nbr_idx, const double *__restrict__ nbr_w, const int32_t *__restrict__ nbr_cnt,
     int nbr_cap, int64_t R, int64_t rows_per_cta, double *__restrict__ partial) {
     __shared__ int32_t sidx[256];
@@ -288,7 +288,7 @@ __global__ void __launch_bounds__(128) relieff_codes_gather_kernel(
     const int64_t r_end = r_begin + rows_per_cta < R ? r_begin + rows_per_cta : R;
     double total = 0.0;
     for (int64_t row = r_begin; row < r_end; ++row) {
-        const uint8_t ci = codes[ids[row] * ldc + cc];
+        const uint8_t ci = codes[(row0 + row) * ldc + cc];
         const int cnt = nbr_cnt[row];
         for (int s0 = 0; s0 < cnt; s0 += 256) {
             const int m = cnt - s0 < 256 ? cnt - s0 : 256;
@@ -319,7 +319,7 @@ __global__ void __launch_bounds__(256) reduce_code_partials_kernel(const double 
 }
 
 // Grid: 128-column strips x chunks of target rows, about 8 CTAs per SM of a B200 (148 SMs) in all.
-void launch_relieff_codes(const WorkSet &ws, const int64_t *ids, const int32_t *nbr_idx, const double *nbr_w,
+void launch_relieff_codes(const WorkSet &ws, int64_t row0, const int32_t *nbr_idx, const double *nbr_w,
                           const int32_t *nbr_cnt, int32_t nbr_cap, int64_t R, DevBuf<double> &partial, double *wsum,
                           cudaStream_t st, int *launches) {
     const int64_t ctiles = ceil_div(ws.pt, 128);
@@ -328,7 +328,7 @@ void launch_relieff_codes(const WorkSet &ws, const int64_t *ids, const int32_t *
     const int64_t n_part = ceil_div(R, rows);
     partial.reserve((size_t)n_part * ws.pt);
     dim3 grid((unsigned)n_part, (unsigned)ctiles);
-    relieff_codes_gather_kernel<<<grid, 128, 0, st>>>(ws.codes.ptr, ws.ldc, ws.pt, ids, nbr_idx, nbr_w, nbr_cnt, nbr_cap, R,
+    relieff_codes_gather_kernel<<<grid, 128, 0, st>>>(ws.codes.ptr, ws.ldc, ws.pt, row0, nbr_idx, nbr_w, nbr_cnt, nbr_cap, R,
                                                       rows, partial.ptr);
     FS_CUDA(cudaGetLastError());
     reduce_code_partials_kernel<<<(unsigned)ceil_div(ws.pt, 256), 256, 0, st>>>(partial.ptr, n_part, ws.pt, ws.tout.ptr, wsum);

@@ -447,14 +447,12 @@ struct fs_dataset {
     int32_t *peer_slab = nullptr;
     fs::DevBuf<int8_t> sel;       // [R, ldn] neighbour codes
     fs::DevBuf<fs::RowInfo> rinfo;
-    fs::DevBuf<int64_t> row_ids;
     fs::DevBuf<double> partial;   // accumulation partials
     fs::DevBuf<double> wsum;      // [n_kept]
     fs::DevBuf<int32_t> nbr_idx;  // ReliefF neighbour lists
     fs::DevBuf<double> nbr_w;
     fs::DevBuf<int32_t> nbr_cnt;
     fs::DevBuf<float> d_class_probs;
-    fs::DevBuf<char> xa_gather;   // gathered target rows (fs_debug_rows)
     fs::DevBuf<double> tpartial;  // tensor-path accumulation partials
     fs::DevBuf<int32_t> tile_desc; // target-tile descriptors of the accumulation kernel
     fs::DevBuf<int32_t> tile_consts; // per-(tile, phase, target) coefficient limbs and mask row sums
@@ -463,10 +461,7 @@ struct fs_dataset {
     fs_comm *comm = nullptr;
     bool x_in_arena = false;                 // fs_dataset_create_group: the raw matrix lives in the arena
     fs::GroupLayout glayout{};
-    fs::DevBuf<int64_t> all_ids;             // 0 .. n-1 (the sharded accumulation runs over all target rows)
-    std::vector<int64_t> all_ids_h;
     std::vector<int64_t> owner_bound;        // [world + 1] original-column boundaries of the ranks' accumulation shares
-    fs::DevBuf<int8_t> a_gather;  // gathered one-hot target rows (fs_debug_rows)
     // ReliefF reference tie order (select.cu): compacted list of tied rows, [R, n] (key, index) pairs
     fs::DevBuf<int32_t> tie_list;
     fs::DevBuf<uint2> tie_pairs;
@@ -475,7 +470,6 @@ struct fs_dataset {
     fs::DiscreteOperand disc;
     fs::DevBuf<double> joint_out;       // [n_kept, n_kept]
     fs::DevBuf<int32_t> joint_zero;     // zeros: the s_i / s_j vector of the reused distance kernel
-    fs::DevBuf<int64_t> joint_ids;      // zeros: its row-id vector
     fs::DevBuf<int32_t> joint_slab;     // [band rows, ldd] negated reduced joint counts of one band
     fs::DevBuf<int64_t> joint_pairs, joint_tables;
     // column path (fs_joint_columns)
@@ -529,50 +523,48 @@ void comm_push(fs_comm *c, size_t off, size_t bytes, cudaStream_t st, int *launc
 // or tpos; codes when ws.have_codes) and, for an incremental distance update, those of the removed columns
 void build_onehot(fs_dataset *ds, WorkSet &ws, bool group_call, int *launches);
 
-// tc_dist.cu: the one-hot mismatch counts of R target rows (internal order; h_row_ids / d_row_ids, or the
-// contiguous range from r0_internal) against all samples, into the slab Dd [R, ldn] (or subtracted from it for
-// an incremental update); with `exchange` (this rank computes its whole shard into its arena slab) symmetric
-// and mirrored into the peers' slabs
-void launch_dist_tensor(fs_dataset *ds, const WorkSet &ws, int64_t r0_internal, const int64_t *h_row_ids,
-                        const int64_t *d_row_ids, bool contiguous, int64_t R, int32_t *Dd, int64_t ldn, bool exchange,
+// tc_dist.cu: the one-hot mismatch counts of the target rows [r0, r0 + R) (internal order) against all samples,
+// into the slab Dd [R, ldn] (or subtracted from it for an incremental update); with `exchange` (this rank computes
+// its whole shard into its arena slab) symmetric and mirrored into the peers' slabs
+void launch_dist_tensor(fs_dataset *ds, const WorkSet &ws, int64_t r0, int64_t R, int32_t *Dd, int64_t ldn, bool exchange,
                         cudaStream_t st, int *launches, double *ops);
-// The distance GEMM itself: D[r, j] = srow[ids[r]] + srow[j] - sum_k a[r, k] b[j, k] (subtract: D[r, j] -= that)
+// The distance GEMM itself: D[r, j] = srow[r0 + r] + srow[j] - sum_k a[r, k] b[j, k] (subtract: D[r, j] -= that)
 // over the FP4 operands a (R rows) and b (n rows), row_bytes wide at a pitch of `pitch` bytes, contracted over K
 // bytes (a multiple of 128; bytes past row_bytes are the tensor maps' zero fill)
 void launch_tc_dist(const int8_t *a, const int8_t *b, int64_t row_bytes, int64_t pitch, int64_t K, const int32_t *srow,
-                    const int64_t *d_ids, int64_t R, int64_t n, int64_t ldd, bool symmetric, bool subtract,
+                    int64_t r0, int64_t R, int64_t n, int64_t ldd, bool symmetric, bool subtract,
                     const DistPeers &peers, cudaStream_t st, int *launches, double *ops);
 
 // tc_accum.cu: wsum[tout[c]] += the MultiSURF / SURF weight of every one-hot column c of the working set's
-// accumulation slice over R target rows, from the FP4 neighbour masks (rows of ldn / 2 bytes, kAccumMaskPadRows
-// rows of padding behind them) and the row constants rinfo
-void launch_accum_tensor(fs_dataset *ds, const WorkSet &ws, const int64_t *d_row_ids, const int64_t *h_row_ids,
-                         bool contiguous, int64_t R, const int8_t *mask_h, const int8_t *mask_m, int64_t ldn,
-                         const RowInfo *rinfo, double *wsum, cudaStream_t st, int *launches, double *ops);
+// accumulation slice over the target rows [row0, row0 + R), from the FP4 neighbour masks (rows of ldn / 2 bytes,
+// kAccumMaskPadRows rows of padding behind them) and the row constants rinfo
+void launch_accum_tensor(fs_dataset *ds, const WorkSet &ws, int64_t row0, int64_t R, const int8_t *mask_h,
+                         const int8_t *mask_m, int64_t ldn, const RowInfo *rinfo, double *wsum, cudaStream_t st,
+                         int *launches, double *ops);
 
 // dist_general.cu: D[r, j] = sum over general columns of the per-feature term
 // between target row r (rows of xa) and sample j (rows of xb).
 void launch_dist_general(const WorkSet &ws, const void *xa, int64_t na, const void *xb, int64_t nb,
                          double *D, int64_t ldd, cudaStream_t st, int *launches);
 
-// select.cu
-void launch_select(fs_dataset *ds, int algo, int use_star, int32_t k, const int64_t *row_ids, int64_t R,
+// select.cu: neighbours of the target rows [r0, r0 + R)
+void launch_select(fs_dataset *ds, int algo, int use_star, int32_t k, int64_t r0, int64_t R,
                    const double *Dc, const int32_t *Dd, int64_t ldn, int8_t *sel, int8_t *mask_h, int8_t *mask_m,
                    RowInfo *rinfo,
                    int32_t *nbr_idx, double *nbr_w, int32_t *nbr_cnt, int32_t nbr_cap,
                    const float *class_probs, cudaStream_t st, int *launches);
 
-// accum_general.cu
+// accum_general.cu: the target rows are the rows [row0, row0 + R) of the general matrix
 int64_t accum_general_partials(const WorkSet &ws, int64_t R);
-void launch_accum_general(const WorkSet &ws, int64_t n, const void *xa, const int8_t *sel, int64_t ldn,
+void launch_accum_general(const WorkSet &ws, int64_t n, int64_t row0, const int8_t *sel, int64_t ldn,
                           const RowInfo *rinfo, int64_t R, double *partial, int64_t n_part,
                           cudaStream_t st, int *launches);
-void launch_relieff_gather(const WorkSet &ws, int64_t n, const void *xa, const int32_t *nbr_idx,
+void launch_relieff_gather(const WorkSet &ws, int64_t n, int64_t row0, const int32_t *nbr_idx,
                            const double *nbr_w, const int32_t *nbr_cnt, int32_t nbr_cap, int64_t R,
                            double *partial, int64_t n_part, cudaStream_t st, int *launches);
 // ReliefF on the one-hot columns: wsum[tout[c]] += the weight of every tensor-path column c from the value codes
-// (ws.codes) of the R target rows ids and of their neighbours; partial is scratch
-void launch_relieff_codes(const WorkSet &ws, const int64_t *ids, const int32_t *nbr_idx, const double *nbr_w,
+// (ws.codes) of the target rows [row0, row0 + R) and of their neighbours; partial is scratch
+void launch_relieff_codes(const WorkSet &ws, int64_t row0, const int32_t *nbr_idx, const double *nbr_w,
                           const int32_t *nbr_cnt, int32_t nbr_cap, int64_t R, DevBuf<double> &partial, double *wsum,
                           cudaStream_t st, int *launches);
 // wsum[gout[c]] += sum_q partial[q, c]  (fixed order => bitwise reproducible)

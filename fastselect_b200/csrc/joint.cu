@@ -172,7 +172,7 @@ void run_joint(fs_dataset *ds, int kind, double log_base, const int64_t *feat_id
     const int64_t row_bytes = (n + 1) / 2, pitch = ws.ldt / 2;     // At: two samples per byte
     tm.end();
 
-    // the reused distance kernel adds s_i + s_j (zeros here) and looks its rows up through an id vector
+    // the reused distance kernel adds s_i + s_j: zeros here, for the band's rows (from 0) and columns
     const int64_t zero_len = round_up(std::max<int64_t>(K, 1), 256) + 256;
     ds->joint_zero.reserve(zero_len);
     FS_CUDA(cudaMemsetAsync(ds->joint_zero.ptr, 0, zero_len * sizeof(int32_t), st));
@@ -195,10 +195,8 @@ void run_joint(fs_dataset *ds, int kind, double log_base, const int64_t *feat_id
         if (R > 0) {
             tm.begin(&fs_stats::ms_dist_tensor);
             ds->joint_slab.reserve((size_t)round_up(R, 128) * ldd);
-            ds->joint_ids.reserve(round_up(R, 128));
-            FS_CUDA(cudaMemsetAsync(ds->joint_ids.ptr, 0, round_up(R, 128) * sizeof(int64_t), st));
             const int8_t *base = ws.At.ptr + (size_t)b0 * pitch;
-            launch_tc_dist(base, base, row_bytes, pitch, k_bytes, ds->joint_zero.ptr, ds->joint_ids.ptr, R, ncols, ldd, false,
+            launch_tc_dist(base, base, row_bytes, pitch, k_bytes, ds->joint_zero.ptr, 0, R, ncols, ldd, false,
                            false, single_rank_peers(ds->joint_slab.ptr, ncols), st, &launches, &ops);
             tm.end();
         }

@@ -7,15 +7,22 @@
 #include <algorithm>
 #include <chrono>
 #include <cstring>
+#include <utility>
 
 #include "common.cuh"
 
 namespace fs {
 
+// A run of consecutive internal (class-sorted) target rows [r0, r0 + R): every pipeline pass scores a contiguous range
+struct RowRun {
+    int64_t r0, R;
+};
+
 struct DebugOut {
     double *dist = nullptr;    // [nt, n] original sample order
     double *thresh = nullptr;  // [nt]
     int8_t *mask = nullptr;    // [nt, n]
+    const int64_t *pos = nullptr;  // [nt] position in the caller's target list of every row of the runs, in run order
 };
 
 __global__ void count_selected_kernel(const RowInfo *rinfo, int64_t R, unsigned long long *out) {
@@ -78,8 +85,8 @@ static int plan_dist(fs_dataset *ds, const int32_t *buf, int64_t r0, int64_t R, 
 }
 
 static void run_pipeline(fs_dataset *ds, int algo, int use_star, int32_t k, const float *class_probs,
-                         const int64_t *feat_idx, int64_t n_kept, const std::vector<int64_t> &targets,
-                         bool contiguous, double *d_wsum, DebugOut *dbg, fs_stats *stats) {
+                         const int64_t *feat_idx, int64_t n_kept, const std::vector<RowRun> &runs,
+                         double *d_wsum, DebugOut *dbg, fs_stats *stats) {
     FS_REQUIRE(ds->have_features, FS_ERR_STATE, "fs_score: call fs_dataset_set_features first");
     FS_REQUIRE(algo == FS_RELIEFF || algo == FS_SURF || algo == FS_MULTISURF, FS_ERR_INVALID, "unknown algo %d", algo);
     FS_REQUIRE(n_kept >= 1, FS_ERR_INVALID, "fs_score: n_kept must be >= 1");
@@ -96,6 +103,14 @@ static void run_pipeline(fs_dataset *ds, int algo, int use_star, int32_t k, cons
     PhaseTimer timer(stats != nullptr, st);
 
     const int64_t ldn = round_up(n, 128);
+    // target rows in all and the hull [u_lo, u_hi) of the runs.  fs_score passes one run, [u_lo, u_hi) itself, and
+    // only fs_score (dbg == nullptr) joins a group call or keeps its slab: those decisions read the hull as the range
+    int64_t nt = 0, u_lo = n, u_hi = 0;
+    for (const RowRun &u : runs) {
+        nt += u.R;
+        u_lo = std::min(u_lo, u.r0);
+        u_hi = std::max(u_hi, u.r0 + u.R);
+    }
     // Multi-GPU group call: this rank scores exactly its shard of the target rows, every rank does the
     // same with the same arguments, and the shard fits one chunk on every rank (the decision must be
     // identical everywhere: it is taken for the LARGEST shard with the most demanding slab set).  Then
@@ -105,9 +120,9 @@ static void run_pipeline(fs_dataset *ds, int algo, int use_star, int32_t k, cons
     int64_t max_shard = 0;
     for (int q = 0; comm != nullptr && q < ds->peers.world; ++q)
         max_shard = std::max<int64_t>(max_shard, ds->peers.starts[q + 1] - ds->peers.starts[q]);
-    const bool group_call = comm != nullptr && comm->world > 1 && contiguous && dbg == nullptr &&
-                            targets[0] == ds->peers.starts[ds->peers.rank] &&
-                            (int64_t)targets.size() == ds->peers.starts[ds->peers.rank + 1] - ds->peers.starts[ds->peers.rank] &&
+    const bool group_call = comm != nullptr && comm->world > 1 && dbg == nullptr &&
+                            u_lo == ds->peers.starts[ds->peers.rank] &&
+                            nt == ds->peers.starts[ds->peers.rank + 1] - ds->peers.starts[ds->peers.rank] &&
                             round_up(max_shard, 128) <= chunk_rows(true, true, ldn, algo);
     if (group_call) FS_REQUIRE(comm->connected, FS_ERR_STATE, "fs_score: the multi-GPU group is not connected");
     const char *env_fs = getenv("FS_B200_FEATURE_SHARD");
@@ -115,14 +130,14 @@ static void run_pipeline(fs_dataset *ds, int algo, int use_star, int32_t k, cons
     // the one-hot distance slab of a contiguous target range that fits one chunk is kept between
     // calls: TuRF's next iteration subtracts the removed columns instead of recomputing it
     // (with peers configured the decision is taken for the largest shard, so that all ranks agree)
-    const int64_t cache_rows = std::max<int64_t>((int64_t)targets.size(), max_shard);
-    const bool slab_cacheable = contiguous && dbg == nullptr && round_up(cache_rows, 128) <= chunk_rows(true, true, ldn, algo);
+    const int64_t cache_rows = std::max<int64_t>(nt, max_shard);
+    const bool slab_cacheable = dbg == nullptr && round_up(cache_rows, 128) <= chunk_rows(true, true, ldn, algo);
     if (!slab_cacheable) ds->slab.forget();
     timer.begin(&fs_stats::ms_gather);
     const auto prep0 = std::chrono::steady_clock::now();
     build_lists(ds, feat_idx, n_kept, want_split, group_call);
     const WorkSet &ws = ds->ws;
-    const int64_t Rmax = std::min<int64_t>(chunk_rows(ws.pg > 0, ws.pt > 0, ldn, algo), round_up((int64_t)targets.size(), 128));
+    const int64_t Rmax = std::min<int64_t>(chunk_rows(ws.pg > 0, ws.pt > 0, ldn, algo), round_up(nt, 128));
     if (ws.pg > 0) ds->Dc.reserve((size_t)Rmax * ldn);
     // the one-hot distance slab: this rank's slab inside its exchange arena for a group call (the
     // peers store their mirrored tiles into it), else the data set's own buffer
@@ -135,9 +150,7 @@ static void run_pipeline(fs_dataset *ds, int algo, int use_star, int32_t k, cons
             Dd = ds->Dd.ptr;
         }
     }
-    const int64_t u_lo = contiguous ? targets[0] : 0, u_hi = contiguous ? targets[0] + (int64_t)targets.size() : n;
-    build_operands(ds, algo == FS_RELIEFF, plan_dist(ds, Dd, targets[0], (int64_t)targets.size(), slab_cacheable),
-                   u_lo, u_hi, group_call, &launches);
+    build_operands(ds, algo == FS_RELIEFF, plan_dist(ds, Dd, u_lo, nt, slab_cacheable), u_lo, u_hi, group_call, &launches);
     const double ms_prep = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - prep0).count();
     timer.end();
     const bool fshard = group_call && ws.acc_split && ws.pt > 0;
@@ -150,7 +163,7 @@ static void run_pipeline(fs_dataset *ds, int algo, int use_star, int32_t k, cons
     int8_t *mask_h = nullptr, *mask_m = nullptr;
     RowInfo *rinfo_buf = nullptr;
     char *arena = group_call ? static_cast<char *>(comm->arena) : nullptr;
-    const int64_t shard0 = group_call ? targets[0] : 0;
+    const int64_t shard0 = group_call ? u_lo : 0;
     if (group_call) {
         mask_h = reinterpret_cast<int8_t *>(arena + ds->glayout.off_mask_h) + (size_t)shard0 * (ldn / 2);
         mask_m = reinterpret_cast<int8_t *>(arena + ds->glayout.off_mask_m) + (size_t)shard0 * (ldn / 2);
@@ -172,7 +185,6 @@ static void run_pipeline(fs_dataset *ds, int algo, int use_star, int32_t k, cons
         FS_REQUIRE(n_kept <= ds->p, FS_ERR_INVALID, "fs_score: more output columns than the data set has");
         acc_out = reinterpret_cast<double *>(arena + ds->glayout.off_w) + (size_t)comm->rank * ds->p;
     }
-    ds->row_ids.reserve(Rmax);
     int32_t nbr_cap = 0;
     if (algo == FS_RELIEFF) {
         nbr_cap = (int32_t)std::min<int64_t>((int64_t)ds->n_classes * k, n);
@@ -187,33 +199,18 @@ static void run_pipeline(fs_dataset *ds, int algo, int use_star, int32_t k, cons
     FS_CUDA(cudaMemsetAsync(ds->counters.ptr, 0, sizeof(unsigned long long), st));
     FS_CUDA(cudaMemsetAsync(acc_out, 0, n_kept * sizeof(double), st));
 
-    int n_chunks = 0;
-    for (int64_t t0 = 0; t0 < (int64_t)targets.size(); t0 += Rmax) {
-        const int64_t R = std::min<int64_t>(Rmax, (int64_t)targets.size() - t0);
-        const int64_t *h_ids = targets.data() + t0;
-        ++n_chunks;
-        FS_CUDA(cudaMemcpyAsync(ds->row_ids.ptr, h_ids, R * sizeof(int64_t), cudaMemcpyHostToDevice, st));
-        // target rows of the general matrix: a view for a contiguous range, a gathered copy otherwise
-        const char *xa = nullptr;
-        if (ws.pg > 0) {
-            const size_t row_bytes = (size_t)ws.ldg * ws.elem;
-            if (contiguous) {
-                xa = ws.xg.ptr + (size_t)h_ids[0] * row_bytes;
-            } else {
-                ds->xa_gather.reserve((size_t)R * row_bytes);
-                for (int64_t r = 0; r < R; ++r)
-                    FS_CUDA(cudaMemcpyAsync(ds->xa_gather.ptr + (size_t)r * row_bytes,
-                                            ws.xg.ptr + (size_t)h_ids[r] * row_bytes, row_bytes,
-                                            cudaMemcpyDeviceToDevice, st));
-                xa = ds->xa_gather.ptr;
-            }
-        }
+    // the chunks: the runs cut into ranges of at most Rmax rows
+    std::vector<RowRun> chunks;
+    for (const RowRun &u : runs)
+        for (int64_t r = u.r0; r < u.r0 + u.R; r += Rmax) chunks.push_back({r, std::min<int64_t>(Rmax, u.r0 + u.R - r)});
+    int64_t t0 = 0;     // rows of the chunks before this one
+    for (const RowRun &chunk : chunks) {
+        const int64_t r0 = chunk.r0, R = chunk.R;
         // ---- distances
         if (ws.pt > 0 && ws.dist_mode != kDistReuse) {
             ds->slab.forget();
             timer.begin(&fs_stats::ms_dist_tensor);
-            launch_dist_tensor(ds, ws, h_ids[0], h_ids, ds->row_ids.ptr, contiguous, R, Dd, ldn, exchange, st, &launches,
-                               &ops_dist);
+            launch_dist_tensor(ds, ws, r0, R, Dd, ldn, exchange, st, &launches, &ops_dist);
             timer.end();
             if (exchange) {
                 // tiles computed here were also stored into the peers' slabs and theirs into this one:
@@ -223,15 +220,16 @@ static void run_pipeline(fs_dataset *ds, int algo, int use_star, int32_t k, cons
             }
         }
         // Dd now holds the mismatch counts of exactly these columns for these target rows
-        if (ws.pt > 0 && slab_cacheable) ds->slab.record(Dd, ws, targets[0], (int64_t)targets.size());
+        if (ws.pt > 0 && slab_cacheable) ds->slab.record(Dd, ws, u_lo, nt);
         if (ws.pg > 0) {
             timer.begin(&fs_stats::ms_dist_general);
-            launch_dist_general(ws, xa, R, ws.xg.ptr, n, ds->Dc.ptr, ldn, st, &launches);
+            launch_dist_general(ws, ws.xg.ptr + (size_t)r0 * ws.ldg * ws.elem, R, ws.xg.ptr, n, ds->Dc.ptr, ldn, st,
+                                &launches);
             timer.end();
         }
         // ---- neighbour selection
         timer.begin(&fs_stats::ms_select);
-        launch_select(ds, algo, use_star, k, ds->row_ids.ptr, R, ws.pg > 0 ? ds->Dc.ptr : nullptr,
+        launch_select(ds, algo, use_star, k, r0, R, ws.pg > 0 ? ds->Dc.ptr : nullptr,
                       ws.pt > 0 ? Dd : nullptr, ldn, ds->sel.ptr, use_masks ? mask_h : nullptr,
                       use_masks ? mask_m : nullptr, rinfo_buf, ds->nbr_idx.ptr,
                       ds->nbr_w.ptr, ds->nbr_cnt.ptr, nbr_cap, ds->d_class_probs.ptr, st, &launches);
@@ -251,14 +249,7 @@ static void run_pipeline(fs_dataset *ds, int algo, int use_star, int32_t k, cons
             comm_push(comm, ds->glayout.off_mask_m + (size_t)shard0 * mrow, (size_t)R * mrow, st, &launches);
             comm_push(comm, ds->glayout.off_rinfo + (size_t)shard0 * sizeof(RowInfo), (size_t)R * sizeof(RowInfo), st, &launches);
             comm_barrier(comm, st, &launches);
-            if ((int64_t)ds->all_ids_h.size() != n) {
-                ds->all_ids_h.resize(n);
-                for (int64_t r = 0; r < n; ++r) ds->all_ids_h[r] = r;
-                ds->all_ids.alloc(n);
-                FS_CUDA(cudaMemcpyAsync(ds->all_ids.ptr, ds->all_ids_h.data(), n * sizeof(int64_t), cudaMemcpyHostToDevice, st));
-            }
-            launch_accum_tensor(ds, ws, ds->all_ids.ptr, ds->all_ids_h.data(), true, n,
-                                reinterpret_cast<const int8_t *>(arena + ds->glayout.off_mask_h),
+            launch_accum_tensor(ds, ws, 0, n, reinterpret_cast<const int8_t *>(arena + ds->glayout.off_mask_h),
                                 reinterpret_cast<const int8_t *>(arena + ds->glayout.off_mask_m), ldn,
                                 reinterpret_cast<const RowInfo *>(arena + ds->glayout.off_rinfo), acc_out, st, &launches,
                                 &ops_accum);
@@ -266,11 +257,10 @@ static void run_pipeline(fs_dataset *ds, int algo, int use_star, int32_t k, cons
         } else if (ws.pt > 0) {
             timer.begin(&fs_stats::ms_accum_tensor);
             if (algo == FS_RELIEFF)
-                launch_relieff_codes(ws, ds->row_ids.ptr, ds->nbr_idx.ptr, ds->nbr_w.ptr, ds->nbr_cnt.ptr, nbr_cap, R,
-                                     ds->tpartial, acc_out, st, &launches);
+                launch_relieff_codes(ws, r0, ds->nbr_idx.ptr, ds->nbr_w.ptr, ds->nbr_cnt.ptr, nbr_cap, R, ds->tpartial,
+                                     acc_out, st, &launches);
             else
-                launch_accum_tensor(ds, ws, ds->row_ids.ptr, h_ids, contiguous, R, mask_h, mask_m, ldn, rinfo_buf,
-                                    acc_out, st, &launches, &ops_accum);
+                launch_accum_tensor(ds, ws, r0, R, mask_h, mask_m, ldn, rinfo_buf, acc_out, st, &launches, &ops_accum);
             timer.end();
         }
         if (ws.pg > 0) {
@@ -278,10 +268,10 @@ static void run_pipeline(fs_dataset *ds, int algo, int use_star, int32_t k, cons
             ds->partial.reserve((size_t)n_part * ws.ldg);
             timer.begin(&fs_stats::ms_accum_general);
             if (algo == FS_RELIEFF)
-                launch_relieff_gather(ws, n, xa, ds->nbr_idx.ptr, ds->nbr_w.ptr, ds->nbr_cnt.ptr, nbr_cap, R,
+                launch_relieff_gather(ws, n, r0, ds->nbr_idx.ptr, ds->nbr_w.ptr, ds->nbr_cnt.ptr, nbr_cap, R,
                                       ds->partial.ptr, n_part, st, &launches);
             else
-                launch_accum_general(ws, n, xa, ds->sel.ptr, ldn, rinfo_buf, R, ds->partial.ptr, n_part, st,
+                launch_accum_general(ws, n, r0, ds->sel.ptr, ldn, rinfo_buf, R, ds->partial.ptr, n_part, st,
                                      &launches);
             timer.end();
             timer.begin(&fs_stats::ms_reduce);
@@ -306,7 +296,7 @@ static void run_pipeline(fs_dataset *ds, int algo, int use_star, int32_t k, cons
             FS_CUDA(cudaMemcpy(hs.data(), ds->sel.ptr, hs.size(), cudaMemcpyDeviceToHost));
             FS_CUDA(cudaMemcpy(hr.data(), rinfo_buf, R * sizeof(RowInfo), cudaMemcpyDeviceToHost));
             for (int64_t r = 0; r < R; ++r) {
-                const int64_t t = t0 + r;
+                const int64_t t = dbg->pos[t0 + r];
                 if (dbg->thresh) dbg->thresh[t] = hr[r].thresh;
                 for (int64_t j = 0; j < n; ++j) {
                     const int64_t orig = ds->perm[j];
@@ -315,12 +305,13 @@ static void run_pipeline(fs_dataset *ds, int algo, int use_star, int32_t k, cons
                         if (ws.pg > 0) d += hd[(size_t)r * ldn + j];
                         if (ws.pt > 0) d += (double)hdd[(size_t)r * ldn + j];
                         if (algo != FS_MULTISURF) d = (double)(float)d;   // SURF.py:160, ReliefF.py:155
-                        dbg->dist[(size_t)t * n + orig] = (j == h_ids[r]) ? 0.0 : d;
+                        dbg->dist[(size_t)t * n + orig] = (j == r0 + r) ? 0.0 : d;
                     }
                     if (dbg->mask) dbg->mask[(size_t)t * n + orig] = hs[(size_t)r * ldn + j];
                 }
             }
         }
+        t0 += R;
     }
     if (group_call) {
         // every rank's contribution (its share of the one-hot columns in full, or partial sums over its
@@ -345,7 +336,7 @@ static void run_pipeline(fs_dataset *ds, int algo, int use_star, int32_t k, cons
         unsigned long long sel_pairs = 0;
         FS_CUDA(cudaMemcpy(&sel_pairs, ds->counters.ptr, sizeof(sel_pairs), cudaMemcpyDeviceToHost));
         stats->launches = launches;
-        stats->n_chunks = n_chunks;
+        stats->n_chunks = (int)chunks.size();
         stats->n_tensor_cols = ws.pt;
         stats->n_general_cols = ws.n_cont + ws.n_cmp;
         stats->onehot_k = ws.K;
@@ -373,18 +364,17 @@ int fs_score(fs_dataset *ds, int algo, int use_star, int32_t k, const float *cla
                    (long long)ds->n);
         FS_CUDA(cudaSetDevice(ds->device));
         alloc_stream() = ds->stream;
-        std::vector<int64_t> targets(row_end - row_begin);
-        for (int64_t r = row_begin; r < row_end; ++r) targets[r - row_begin] = r;
         double *d_out = wsum_out;
         if (!out_on_device) {
             ds->wsum.reserve(n_kept);
             d_out = ds->wsum.ptr;
         }
-        if (targets.empty()) {
+        if (row_begin == row_end) {
             FS_CUDA(cudaMemsetAsync(d_out, 0, n_kept * sizeof(double), ds->stream));
             if (stats) memset(stats, 0, sizeof(*stats));
         } else {
-            run_pipeline(ds, algo, use_star, k, class_probs, feat_idx, n_kept, targets, true, d_out, nullptr, stats);
+            run_pipeline(ds, algo, use_star, k, class_probs, feat_idx, n_kept, {{row_begin, row_end - row_begin}}, d_out,
+                         nullptr, stats);
         }
         if (!out_on_device) {
             FS_CUDA(cudaMemcpyAsync(wsum_out, d_out, n_kept * sizeof(double), cudaMemcpyDeviceToHost, ds->stream));
@@ -402,15 +392,26 @@ int fs_debug_rows(fs_dataset *ds, int algo, int use_star, int32_t k, const float
         if (!feat_idx) n_kept = ds->p;
         FS_CUDA(cudaSetDevice(ds->device));
         alloc_stream() = ds->stream;
-        std::vector<int64_t> ids(nt);
+        // (internal row, position) of every target, in row order, cut into runs of consecutive internal rows (a
+        // repeated target starts a new run): each run is scored as a contiguous range, like fs_score's, and each row's
+        // outputs go to its position
+        std::vector<std::pair<int64_t, int64_t>> order(nt);
         for (int64_t t = 0; t < nt; ++t) {
             FS_REQUIRE(targets[t] >= 0 && targets[t] < ds->n, FS_ERR_INVALID, "fs_debug_rows: target %lld out of range",
                        (long long)targets[t]);
-            ids[t] = ds->inv_perm[targets[t]];
+            order[t] = {ds->inv_perm[targets[t]], t};
+        }
+        std::sort(order.begin(), order.end());
+        std::vector<RowRun> runs;
+        std::vector<int64_t> pos(nt);
+        for (int64_t t = 0; t < nt; ++t) {
+            if (t > 0 && order[t].first == order[t - 1].first + 1) ++runs.back().R;
+            else runs.push_back({order[t].first, 1});
+            pos[t] = order[t].second;
         }
         ds->wsum.reserve(n_kept);
-        DebugOut dbg{dist_out, thresh_out, mask_out};
-        run_pipeline(ds, algo, use_star, k, class_probs, feat_idx, n_kept, ids, false, ds->wsum.ptr, &dbg, nullptr);
+        DebugOut dbg{dist_out, thresh_out, mask_out, pos.data()};
+        run_pipeline(ds, algo, use_star, k, class_probs, feat_idx, n_kept, runs, ds->wsum.ptr, &dbg, nullptr);
         if (wsum_out) FS_CUDA(cudaMemcpy(wsum_out, ds->wsum.ptr, n_kept * sizeof(double), cudaMemcpyDeviceToHost));
         return FS_OK;
     });

@@ -36,7 +36,7 @@ __device__ __forceinline__ T block_sum(T v, T *scratch /*[8]*/) {
 template <int ALGO>
 __global__ void __launch_bounds__(256) select_threshold_kernel(const double *__restrict__ Dc,
                                                                const int32_t *__restrict__ Dd, int64_t ldn,
-                                                               int64_t n, const int64_t *__restrict__ row_ids,
+                                                               int64_t n, int64_t r0,
                                                                const int32_t *__restrict__ y,
                                                                const int64_t *__restrict__ inv_perm, int use_star,
                                                                int8_t *__restrict__ sel,
@@ -47,7 +47,7 @@ __global__ void __launch_bounds__(256) select_threshold_kernel(const double *__r
     __shared__ int si[8];
     __shared__ double s_thresh;
     const int64_t r = blockIdx.x;
-    const int64_t self = row_ids[r];
+    const int64_t self = r0 + r;
     const int64_t base = r * ldn;
     const int tid = threadIdx.x;
     const double inv = 1.0 / (double)(n - 1);
@@ -207,7 +207,7 @@ __device__ __forceinline__ int block_rank(bool flag, int *warp_tot /*[8]*/, int 
 
 __global__ void __launch_bounds__(256) relieff_select_kernel(
     const double *__restrict__ Dc, const int32_t *__restrict__ Dd, int64_t ldn, int64_t n,
-    const int64_t *__restrict__ row_ids, const int32_t *__restrict__ y, const int64_t *__restrict__ cls_start,
+    int64_t r0, const int32_t *__restrict__ y, const int64_t *__restrict__ cls_start,
     int n_classes, int k, const float *__restrict__ class_probs, int8_t *__restrict__ sel,
     RowInfo *__restrict__ rinfo, int32_t *__restrict__ nbr_idx, double *__restrict__ nbr_w,
     int32_t *__restrict__ nbr_cnt, int nbr_cap, int32_t *__restrict__ tie_list) {
@@ -216,7 +216,7 @@ __global__ void __launch_bounds__(256) relieff_select_kernel(
     __shared__ unsigned s_prefix;
     __shared__ int s_remaining;
     const int64_t r = blockIdx.x;
-    const int64_t self = row_ids[r];
+    const int64_t self = r0 + r;
     const int64_t base = r * ldn;
     const int tid = threadIdx.x;
     const int ci = y[self];
@@ -402,7 +402,7 @@ __device__ __forceinline__ void numba_argsort_pairs(uint2 *P, int64_t n) {
 template <bool kShared>
 __global__ void __launch_bounds__(kShared ? kTieThreadsSmem : kTieThreadsGlobal) relieff_ties_kernel(
     const double *__restrict__ Dc, const int32_t *__restrict__ Dd, int64_t ldn, int64_t n,
-    const int64_t *__restrict__ row_ids, const int32_t *__restrict__ y, const int64_t *__restrict__ inv_perm,
+    int64_t r0, const int32_t *__restrict__ y, const int64_t *__restrict__ inv_perm,
     int n_classes, int k, const float *__restrict__ class_probs, const int32_t *__restrict__ tie_list,
     uint2 *scratch, int8_t *__restrict__ sel, int32_t *__restrict__ nbr_idx, double *__restrict__ nbr_w,
     int32_t *__restrict__ nbr_cnt, int nbr_cap) {
@@ -411,7 +411,7 @@ __global__ void __launch_bounds__(kShared ? kTieThreadsSmem : kTieThreadsGlobal)
     uint2 *P = kShared ? reinterpret_cast<uint2 *>(ties_smem) : scratch + (int64_t)blockIdx.x * tie_row_pairs(n, n_classes);
     int32_t *found = reinterpret_cast<int32_t *>(P + n);      // neighbours taken per class
     const int64_t r = tie_list[1 + blockIdx.x];
-    const int64_t self = row_ids[r];
+    const int64_t self = r0 + r;
     const int64_t base = r * ldn;
     for (int64_t o = threadIdx.x; o < n; o += blockDim.x) {
         const int64_t j = inv_perm[o];
@@ -449,18 +449,18 @@ __global__ void __launch_bounds__(kShared ? kTieThreadsSmem : kTieThreadsGlobal)
     nbr_cnt[r] = m;
 }
 
-void launch_select(fs_dataset *ds, int algo, int use_star, int32_t k, const int64_t *row_ids, int64_t R,
+void launch_select(fs_dataset *ds, int algo, int use_star, int32_t k, int64_t r0, int64_t R,
                    const double *Dc, const int32_t *Dd, int64_t ldn, int8_t *sel, int8_t *mask_h, int8_t *mask_m,
                    RowInfo *rinfo, int32_t *nbr_idx, double *nbr_w, int32_t *nbr_cnt, int32_t nbr_cap, const float *class_probs,
                    cudaStream_t st, int *launches) {
     if (R == 0) return;
     dim3 grid((unsigned)R);
     if (algo == FS_MULTISURF)
-        select_threshold_kernel<FS_MULTISURF><<<grid, 256, 0, st>>>(Dc, Dd, ldn, ds->n, row_ids, ds->d_y.ptr,
+        select_threshold_kernel<FS_MULTISURF><<<grid, 256, 0, st>>>(Dc, Dd, ldn, ds->n, r0, ds->d_y.ptr,
                                                                     ds->d_inv_perm.ptr, use_star, sel, mask_h, mask_m,
                                                                     rinfo);
     else if (algo == FS_SURF)
-        select_threshold_kernel<FS_SURF><<<grid, 256, 0, st>>>(Dc, Dd, ldn, ds->n, row_ids, ds->d_y.ptr,
+        select_threshold_kernel<FS_SURF><<<grid, 256, 0, st>>>(Dc, Dd, ldn, ds->n, r0, ds->d_y.ptr,
                                                                ds->d_inv_perm.ptr, use_star, sel, mask_h, mask_m, rinfo);
     else {
         // reference tie order unless FS_B200_RELIEFF_TIES=index (ties then go by sample index)
@@ -470,7 +470,7 @@ void launch_select(fs_dataset *ds, int algo, int use_star, int32_t k, const int6
             ds->tie_list.reserve(R + 1);
             FS_CUDA(cudaMemsetAsync(ds->tie_list.ptr, 0, sizeof(int32_t), st));
         }
-        relieff_select_kernel<<<grid, 256, 0, st>>>(Dc, Dd, ldn, ds->n, row_ids, ds->d_y.ptr, ds->d_cls_start.ptr,
+        relieff_select_kernel<<<grid, 256, 0, st>>>(Dc, Dd, ldn, ds->n, r0, ds->d_y.ptr, ds->d_cls_start.ptr,
                                                     ds->n_classes, k, class_probs, sel, rinfo, nbr_idx, nbr_w,
                                                     nbr_cnt, nbr_cap, emulate ? ds->tie_list.ptr : nullptr);
         if (emulate) {
@@ -486,7 +486,7 @@ void launch_select(fs_dataset *ds, int algo, int use_star, int32_t k, const int6
             else
                 ds->tie_pairs.reserve((size_t)R * tie_row_pairs(ds->n, ds->n_classes));
             kernel<<<grid, smem ? kTieThreadsSmem : kTieThreadsGlobal, smem ? row_bytes : 0, st>>>(
-                Dc, Dd, ldn, ds->n, row_ids, ds->d_y.ptr, ds->d_inv_perm.ptr, ds->n_classes, k, class_probs,
+                Dc, Dd, ldn, ds->n, r0, ds->d_y.ptr, ds->d_inv_perm.ptr, ds->n_classes, k, class_probs,
                 ds->tie_list.ptr, smem ? nullptr : ds->tie_pairs.ptr, sel, nbr_idx, nbr_w, nbr_cnt, nbr_cap);
         }
     }

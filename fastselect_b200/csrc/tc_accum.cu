@@ -160,9 +160,9 @@ __global__ void __launch_bounds__(256) accum_consts_kernel(const TileDesc *__res
 template <bool kPair>
 __global__ void __launch_bounds__(THREADS, 1)
 tc_accum_kernel(const __grid_constant__ CUtensorMap tmap_at, const __grid_constant__ CUtensorMap tmap_mh,
-                const __grid_constant__ CUtensorMap tmap_mm, int num_k_blocks, int64_t R,
+                const __grid_constant__ CUtensorMap tmap_mm, int num_k_blocks,
                 const TileDesc *__restrict__ tiles, int num_tiles, int groups, int group_tiles, int m_blocks,
-                const int64_t *__restrict__ ids, int contiguous, const int2 *__restrict__ limbs,
+                int64_t row0, const int2 *__restrict__ limbs,
                 const int32_t *__restrict__ rsum, const uint8_t *__restrict__ codesT, int64_t ldt,
                 const uint32_t *__restrict__ krow, int64_t K_rows, double *__restrict__ tpartial) {
     extern __shared__ __align__(1024) unsigned char smem_raw[];
@@ -290,7 +290,6 @@ tc_accum_kernel(const __grid_constant__ CUtensorMap tmap_at, const __grid_consta
         const int half = (warp - 2) >> 2;
         const int et = q * 32 + lane;                         // 0..127: TMEM lane / local one-hot row
         const uint32_t parity = (uint32_t)lane & 1u;          // kPair: plane of this one-hot row (row 2c + parity)
-        const int64_t ids0 = contiguous ? ids[0] : 0;
         int item = 0;
         for (int u = blockIdx.x; u < units; u += gridDim.x) {
             const int g = u % groups;
@@ -314,72 +313,43 @@ tc_accum_kernel(const __grid_constant__ CUtensorMap tmap_at, const __grid_consta
                 uint32_t oh[kPair ? HALF / 8 : HALF / 4];
                 if constexpr (kPair) {
                     const int64_t rbase = (int64_t)d.row0 + half * HALF + 8 * (int)parity;
-                    if (contiguous) {
-                        const int64_t id0 = ids0 + rbase;
-                        if ((id0 & 7) == 0) {
+                    const int64_t id0 = row0 + rbase;
+                    if ((id0 & 7) == 0) {
 #pragma unroll
-                            for (int j = 0; j < HALF / 16; ++j) {
-                                const uint2 a = *reinterpret_cast<const uint2 *>(at_row + id0 + 16 * j);
-                                oh[2 * j] = a.x; oh[2 * j + 1] = a.y;
-                            }
-                        } else {
-                            // unaligned start (class-aligned tiles): aligned words + funnel shift
-                            const uint32_t *src = reinterpret_cast<const uint32_t *>(at_row + (id0 & ~(int64_t)3));
-                            const uint32_t sh = (uint32_t)(id0 & 3) * 8u;
-#pragma unroll
-                            for (int j = 0; j < HALF / 16; ++j) {
-                                const uint32_t w0 = src[4 * j], w1 = src[4 * j + 1], w2 = src[4 * j + 2];
-                                oh[2 * j] = __funnelshift_r(w0, w1, sh);
-                                oh[2 * j + 1] = __funnelshift_r(w1, w2, sh);
-                            }
+                        for (int j = 0; j < HALF / 16; ++j) {
+                            const uint2 a = *reinterpret_cast<const uint2 *>(at_row + id0 + 16 * j);
+                            oh[2 * j] = a.x; oh[2 * j + 1] = a.y;
                         }
                     } else {
+                        // unaligned start (class-aligned tiles): aligned words + funnel shift
+                        const uint32_t *src = reinterpret_cast<const uint32_t *>(at_row + (id0 & ~(int64_t)3));
+                        const uint32_t sh = (uint32_t)(id0 & 3) * 8u;
 #pragma unroll
-                        for (int w = 0; w < HALF / 8; ++w) {
-                            uint32_t x = 0;
-#pragma unroll
-                            for (int b = 0; b < 4; ++b) {
-                                const int64_t r = rbase + (w >> 1) * 16 + (w & 1) * 4 + b;
-                                const uint32_t byte = r < R ? (uint32_t)at_row[ids[r]] : 0xffu;
-                                x |= byte << (8 * b);
-                            }
-                            oh[w] = x;
+                        for (int j = 0; j < HALF / 16; ++j) {
+                            const uint32_t w0 = src[4 * j], w1 = src[4 * j + 1], w2 = src[4 * j + 2];
+                            oh[2 * j] = __funnelshift_r(w0, w1, sh);
+                            oh[2 * j + 1] = __funnelshift_r(w1, w2, sh);
                         }
                     }
                 } else {
-                    const int64_t rbase = (int64_t)d.row0 + half * HALF;
-                    if (contiguous) {
-                        const int64_t id0 = ids0 + rbase;
-                        if ((id0 & 15) == 0) {
-                            const uint4 *src = reinterpret_cast<const uint4 *>(at_row + id0);
+                    const int64_t id0 = row0 + d.row0 + half * HALF;
+                    if ((id0 & 15) == 0) {
+                        const uint4 *src = reinterpret_cast<const uint4 *>(at_row + id0);
 #pragma unroll
-                            for (int w = 0; w < HALF / 16; ++w) {
-                                const uint4 a = src[w];
-                                oh[4 * w] = a.x; oh[4 * w + 1] = a.y; oh[4 * w + 2] = a.z; oh[4 * w + 3] = a.w;
-                            }
-                        } else {
-                            // unaligned start (class-aligned tiles): aligned words + funnel shift
-                            const uint32_t *src = reinterpret_cast<const uint32_t *>(at_row + (id0 & ~(int64_t)3));
-                            const uint32_t sh = (uint32_t)(id0 & 3) * 8u;
-                            uint32_t prev = src[0];
-#pragma unroll
-                            for (int w = 0; w < HALF / 4; ++w) {
-                                const uint32_t next = src[w + 1];
-                                oh[w] = __funnelshift_r(prev, next, sh);
-                                prev = next;
-                            }
+                        for (int w = 0; w < HALF / 16; ++w) {
+                            const uint4 a = src[w];
+                            oh[4 * w] = a.x; oh[4 * w + 1] = a.y; oh[4 * w + 2] = a.z; oh[4 * w + 3] = a.w;
                         }
                     } else {
+                        // unaligned start (class-aligned tiles): aligned words + funnel shift
+                        const uint32_t *src = reinterpret_cast<const uint32_t *>(at_row + (id0 & ~(int64_t)3));
+                        const uint32_t sh = (uint32_t)(id0 & 3) * 8u;
+                        uint32_t prev = src[0];
 #pragma unroll
                         for (int w = 0; w < HALF / 4; ++w) {
-                            uint32_t x = 0;
-#pragma unroll
-                            for (int b = 0; b < 4; ++b) {
-                                const int64_t r = rbase + w * 4 + b;
-                                const uint32_t byte = r < R ? (uint32_t)at_row[ids[r]] : 0xffu;
-                                x |= byte << (8 * b);
-                            }
-                            oh[w] = x;
+                            const uint32_t next = src[w + 1];
+                            oh[w] = __funnelshift_r(prev, next, sh);
+                            prev = next;
                         }
                     }
                 }
@@ -522,9 +492,9 @@ struct ChunkConsts {
 // GPU: the same ceiling the distance GEMM hit before it became CTA pairs) -- the pair moves 30 KB.
 __global__ void __launch_bounds__(M_THREADS, 1)
 tc_accum_merged_kernel(const __grid_constant__ CUtensorMap tmap_at, const __grid_constant__ CUtensorMap tmap_mh,
-                       const __grid_constant__ CUtensorMap tmap_mm, int num_k_blocks, int64_t R,
+                       const __grid_constant__ CUtensorMap tmap_mm, int num_k_blocks,
                        const __grid_constant__ TileTable tt, int num_tiles, int groups, int group_tiles, int m_blocks, int group_span,
-                       const int64_t *__restrict__ ids, int contiguous, const int2 *__restrict__ limbs,
+                       int64_t row0, const int2 *__restrict__ limbs,
                        const int32_t *__restrict__ rsum, const uint8_t *__restrict__ codesT, int64_t ldt,
                        const uint32_t *__restrict__ krow, int64_t K_rows, double *__restrict__ tpartial) {
     extern __shared__ __align__(1024) unsigned char smem_raw[];
@@ -678,7 +648,6 @@ tc_accum_merged_kernel(const __grid_constant__ CUtensorMap tmap_at, const __grid
         const int q = warp & 3;
         const int part = warp >> 2;
         const int j = lane & 3, r8 = lane >> 2;
-        const int64_t ids0 = contiguous ? ids[0] : 0;
         const uint32_t tquarter = tmem_base + ((uint32_t)(q * 32) << 16);
         // hand an accumulator buffer back to the MMA issuer (this thread's TMEM loads have completed)
         auto release_acc = [&](uint64_t *bar) {
@@ -705,42 +674,25 @@ tc_accum_merged_kernel(const __grid_constant__ CUtensorMap tmap_at, const __grid
                 // (issued before the accumulator wait; shared by both phases).  Targets beyond the tile's
                 // rows get whatever follows: their coefficient is 0.
                 uint32_t oh0[M_CHUNKS], oh1[M_CHUNKS];
-                if (contiguous) {
-                    const int64_t a0 = ids0 + d.row0 + 16 * part + 4 * j;   // chunk i: + 16 M_PARTS i
-                    if ((a0 & 3) == 0) {
-#pragma unroll
-                        for (int i = 0; i < M_CHUNKS; ++i)
-                            if (i < n_my) {
-                                oh0[i] = *reinterpret_cast<const uint32_t *>(at0 + a0 + 16 * M_PARTS * i);
-                                oh1[i] = *reinterpret_cast<const uint32_t *>(at1 + a0 + 16 * M_PARTS * i);
-                            }
-                    } else {
-                        // unaligned start (class-aligned tiles): two aligned words + funnel shift
-                        const uint32_t sh = (uint32_t)(a0 & 3) * 8u;
-                        const int64_t ab = a0 & ~(int64_t)3;
-#pragma unroll
-                        for (int i = 0; i < M_CHUNKS; ++i)
-                            if (i < n_my) {
-                                const uint32_t *s0 = reinterpret_cast<const uint32_t *>(at0 + ab + 16 * M_PARTS * i);
-                                const uint32_t *s1 = reinterpret_cast<const uint32_t *>(at1 + ab + 16 * M_PARTS * i);
-                                oh0[i] = __funnelshift_r(s0[0], s0[1], sh);
-                                oh1[i] = __funnelshift_r(s1[0], s1[1], sh);
-                            }
-                    }
-                } else {
+                const int64_t a0 = row0 + d.row0 + 16 * part + 4 * j;   // chunk i: + 16 M_PARTS i
+                if ((a0 & 3) == 0) {
 #pragma unroll
                     for (int i = 0; i < M_CHUNKS; ++i)
                         if (i < n_my) {
-                            uint32_t x0 = 0, x1 = 0;
+                            oh0[i] = *reinterpret_cast<const uint32_t *>(at0 + a0 + 16 * M_PARTS * i);
+                            oh1[i] = *reinterpret_cast<const uint32_t *>(at1 + a0 + 16 * M_PARTS * i);
+                        }
+                } else {
+                    // unaligned start (class-aligned tiles): two aligned words + funnel shift
+                    const uint32_t sh = (uint32_t)(a0 & 3) * 8u;
+                    const int64_t ab = a0 & ~(int64_t)3;
 #pragma unroll
-                            for (int b = 0; b < 4; ++b) {
-                                const int64_t r = (int64_t)d.row0 + 16 * (part + M_PARTS * i) + 4 * j + b;
-                                const int64_t id = r < R ? ids[r] : -1;
-                                x0 |= (id >= 0 ? (uint32_t)at0[id] : 0xffu) << (8 * b);
-                                x1 |= (id >= 0 ? (uint32_t)at1[id] : 0xffu) << (8 * b);
-                            }
-                            oh0[i] = x0;
-                            oh1[i] = x1;
+                    for (int i = 0; i < M_CHUNKS; ++i)
+                        if (i < n_my) {
+                            const uint32_t *s0 = reinterpret_cast<const uint32_t *>(at0 + ab + 16 * M_PARTS * i);
+                            const uint32_t *s1 = reinterpret_cast<const uint32_t *>(at1 + ab + 16 * M_PARTS * i);
+                            oh0[i] = __funnelshift_r(s0[0], s0[1], sh);
+                            oh1[i] = __funnelshift_r(s1[0], s1[1], sh);
                         }
                 }
                 for (int phase = 0; phase < 2; ++phase) {
@@ -872,38 +824,29 @@ struct AccumPlan {
     double blocks = 0;       // K blocks contracted per one-hot row block (both phases, all tiles), in units of full 256-column tiles
 };
 
-static AccumPlan make_plan(int64_t n, int64_t R, bool contiguous, const int64_t *h_ids, const int32_t *h_y,
-                           const int64_t *h_cls_start, int bn, int n_round) {
+static AccumPlan make_plan(int64_t n, int64_t row0, int64_t R, const int32_t *h_y, const int64_t *h_cls_start, int bn,
+                           int n_round) {
     AccumPlan plan;
     const int nkb = (int)ceil_div(n, KS);
-    auto add = [&](int64_t row0, int64_t rows, int64_t hs, int64_t he, bool mixed) {
+    auto add = [&](int64_t r, int64_t rows, int64_t hs, int64_t he) {
         TileDesc d{};
-        d.row0 = (int32_t)row0;
+        d.row0 = (int32_t)r;
         d.rows = (int32_t)rows;
-        if (mixed) {
-            d.hb0 = 0; d.hb1 = nkb; d.ib0 = nkb; d.ib1 = nkb;      // both masks over every block
-        } else {
-            d.hb0 = (int32_t)(hs / KS);
-            d.hb1 = (int32_t)ceil_div(he, KS);
-            // blocks entirely inside [hs, he) hold no misses of this class
-            d.ib0 = (int32_t)ceil_div(hs, KS);
-            d.ib1 = he == n ? nkb : (int32_t)(he / KS);
-            if (d.ib1 < d.ib0) d.ib1 = d.ib0;
-        }
+        d.hb0 = (int32_t)(hs / KS);
+        d.hb1 = (int32_t)ceil_div(he, KS);
+        // blocks entirely inside [hs, he) hold no misses of this class
+        d.ib0 = (int32_t)ceil_div(hs, KS);
+        d.ib1 = he == n ? nkb : (int32_t)(he / KS);
+        if (d.ib1 < d.ib0) d.ib1 = d.ib0;
         // MMA N: the tile's rows rounded up to n_round (16; CTA pairs 32), in units of full 240-column tiles
         plan.blocks += (double)((d.hb1 - d.hb0) + d.ib0 + (nkb - d.ib1)) * (double)(ceil_div(rows, n_round) * n_round) / BN;
         plan.tiles.push_back(d);
     };
-    if (!contiguous) {
-        for (int64_t r = 0; r < R; r += bn) add(r, std::min<int64_t>(bn, R - r), 0, n, true);
-        return plan;
-    }
-    const int64_t id0 = h_ids[0];
     int64_t r = 0;
     while (r < R) {
-        const int c = h_y[id0 + r];
-        const int64_t cls_end = std::min<int64_t>(h_cls_start[c + 1] - id0, R);   // first row past this class
-        for (; r < cls_end; r += bn) add(r, std::min<int64_t>(bn, cls_end - r), h_cls_start[c], h_cls_start[c + 1], false);
+        const int c = h_y[row0 + r];
+        const int64_t cls_end = std::min<int64_t>(h_cls_start[c + 1] - row0, R);   // first row past this class
+        for (; r < cls_end; r += bn) add(r, std::min<int64_t>(bn, cls_end - r), h_cls_start[c], h_cls_start[c + 1]);
         r = cls_end;
     }
     return plan;
@@ -922,9 +865,9 @@ __global__ void __launch_bounds__(256) reduce_tensor_partials_kernel(const doubl
     wsum[tout[c]] += s;
 }
 
-void launch_accum_tensor(fs_dataset *ds, const WorkSet &ws, const int64_t *d_row_ids, const int64_t *h_row_ids,
-                         bool contiguous, int64_t R, const int8_t *mask_h, const int8_t *mask_m, int64_t ldn,
-                         const RowInfo *rinfo, double *wsum, cudaStream_t st, int *launches, double *ops) {
+void launch_accum_tensor(fs_dataset *ds, const WorkSet &ws, int64_t row0, int64_t R, const int8_t *mask_h,
+                         const int8_t *mask_m, int64_t ldn, const RowInfo *rinfo, double *wsum, cudaStream_t st,
+                         int *launches, double *ops) {
     const int64_t n = ds->n;
     // the accumulation operands hold the columns [a0, a1) of the active list (everything outside a
     // multi-GPU group; this rank's share inside one), one-hot rows numbered from 0
@@ -970,8 +913,8 @@ void launch_accum_tensor(fs_dataset *ds, const WorkSet &ws, const int64_t *d_row
     FS_CUDA(cudaGetDevice(&dev));
     FS_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
     FS_REQUIRE(n < (1LL << 22), FS_ERR_INVALID, "one-hot accumulation supports up to 2^22 samples (got %lld)", (long long)n);
-    const AccumPlan plan = make_plan(n, R, contiguous, h_row_ids, ds->y_sorted.data(), ds->cls_start.data(),
-                                     merged ? CG2_BN : BN, merged ? 32 : 16);
+    const AccumPlan plan = make_plan(n, row0, R, ds->y_sorted.data(), ds->cls_start.data(), merged ? CG2_BN : BN,
+                                     merged ? 32 : 16);
     const int m_blocks = (int)ceil_div(K_rows, BM);
     // Tile groups.  Work units (128 one-hot rows x one group) are dealt round-robin, so the ~sms
     // units resident at one time span sms / groups one-hot row blocks, each streaming its own
@@ -1031,15 +974,15 @@ void launch_accum_tensor(fs_dataset *ds, const WorkSet &ws, const int64_t *d_row
             attr.val.clusterDim.z = 1;
             cfg.attrs = &attr;
             cfg.numAttrs = 1;
-            FS_CUDA(cudaLaunchKernelEx(&cfg, tc_accum_merged_kernel, tmap_at, tmap_mh, tmap_mm, (int)ceil_div(n, KS), R, table,
-                                       nt, groups, group_tiles, m_blocks, group_span, d_row_ids, contiguous ? 1 : 0,
+            FS_CUDA(cudaLaunchKernelEx(&cfg, tc_accum_merged_kernel, tmap_at, tmap_mh, tmap_mm, (int)ceil_div(n, KS), table,
+                                       nt, groups, group_tiles, m_blocks, group_span, row0,
                                        (const int2 *)limbs, (const int32_t *)rsum, ws.codesT.ptr, ws.ldt, ws.krow.ptr, K_rows, tpartial.ptr));
         } else {
             const int units = m_blocks * groups;
             const int grid = units < sms ? units : sms;
             kernel<<<grid, THREADS, smem_bytes, st>>>(
-                tmap_at, tmap_mh, tmap_mm, (int)ceil_div(n, KS), R, d_tiles, nt,
-                groups, group_tiles, m_blocks, d_row_ids, contiguous ? 1 : 0, limbs, rsum, ws.codesT.ptr, ws.ldt, ws.krow.ptr, K_rows,
+                tmap_at, tmap_mh, tmap_mm, (int)ceil_div(n, KS), d_tiles, nt,
+                groups, group_tiles, m_blocks, row0, limbs, rsum, ws.codesT.ptr, ws.ldt, ws.krow.ptr, K_rows,
                 tpartial.ptr + (size_t)groups_done * PARTS * K_rows);
         }
         FS_CUDA(cudaGetLastError());

@@ -203,7 +203,7 @@ __device__ __forceinline__ void dist_store_tile(uint32_t tmem_base, int q, int64
 // symmetric scheme.
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(THREADS, 1)
 tc_dist_pair_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b,
-                    int num_k_blocks, const int32_t *__restrict__ srow, const int64_t *__restrict__ ids, int64_t R,
+                    int num_k_blocks, const int32_t *__restrict__ srow, int64_t r0, int64_t R,
                     int64_t n, int64_t ldd, int symmetric, int subtract, int pair_rows, int tiles_x,
                     const __grid_constant__ DistPeers peers) {
     const uint32_t crank = tc::cluster_ctarank();
@@ -303,7 +303,7 @@ tc_dist_pair_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
         // ===== epilogue: this CTA's 128 TMEM lanes =====
         const int q = warp & 3;
         const int64_t row = (int64_t)m0 + q * 32 + lane;
-        const int32_t s_i = row < R ? srow[ids[row]] : 0;
+        const int32_t s_i = row < R ? srow[r0 + row] : 0;
         tc::mbar_wait(accum_bar, 0);
         tc::tc_fence_after();
         dist_store_tile(tmem_base, q, row, s_i, R, n0, cend, srow, ldd, subtract, mirror, Dd, Dm, peers.starts[owner], row_global0);
@@ -318,7 +318,7 @@ tc_dist_pair_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
 }
 
 void launch_tc_dist(const int8_t *a, const int8_t *b, int64_t row_bytes, int64_t pitch, int64_t K, const int32_t *srow,
-                    const int64_t *d_ids, int64_t R, int64_t n, int64_t ldd, bool symmetric, bool subtract,
+                    int64_t r0, int64_t R, int64_t n, int64_t ldd, bool symmetric, bool subtract,
                     const DistPeers &peers, cudaStream_t st, int *launches, double *ops) {
     const CUtensorMap tmap_a = make_tmap_u8_sw128(a, row_bytes, R, pitch, BM);
     const CUtensorMap tmap_b = make_tmap_u8_sw128(b, row_bytes, n, pitch, BN / 2);   // each CTA of a pair stages half of the sample rows
@@ -326,7 +326,7 @@ void launch_tc_dist(const int8_t *a, const int8_t *b, int64_t row_bytes, int64_t
     // per launch: the attribute belongs to the CURRENT device (several devices per process: fs_multi_*)
     FS_CUDA(cudaFuncSetAttribute(tc_dist_pair_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
     tc_dist_pair_kernel<<<(unsigned)(2 * tiles_x * pair_rows), THREADS, SMEM_BYTES, st>>>(
-        tmap_a, tmap_b, (int)(K / BK), srow, d_ids, R, n, ldd, symmetric ? 1 : 0, subtract ? 1 : 0, pair_rows, tiles_x, peers);
+        tmap_a, tmap_b, (int)(K / BK), srow, r0, R, n, ldd, symmetric ? 1 : 0, subtract ? 1 : 0, pair_rows, tiles_x, peers);
     FS_CUDA(cudaGetLastError());
     ++*launches;
     if (ops) {
@@ -343,8 +343,7 @@ void launch_tc_dist(const int8_t *a, const int8_t *b, int64_t row_bytes, int64_t
     }
 }
 
-void launch_dist_tensor(fs_dataset *ds, const WorkSet &ws, int64_t r0_internal, const int64_t *h_row_ids,
-                        const int64_t *d_row_ids, bool contiguous, int64_t R, int32_t *Dd, int64_t ldn, bool exchange,
+void launch_dist_tensor(fs_dataset *ds, const WorkSet &ws, int64_t r0, int64_t R, int32_t *Dd, int64_t ldn, bool exchange,
                         cudaStream_t st, int *launches, double *ops) {
     // incremental update: the operands are those of the removed columns and the result is subtracted
     const bool incr = ws.dist_mode == kDistIncremental;
@@ -353,26 +352,16 @@ void launch_dist_tensor(fs_dataset *ds, const WorkSet &ws, int64_t r0_internal, 
     const int64_t K = (incr ? ws.Kr : ws.K) / 2;        // operand row bytes (FP4 nibbles)
     // every column adds at most 2 to an FP32 accumulator: exact while the sums stay below 2^24
     FS_REQUIRE(2 * ws.pt < (1LL << 24), FS_ERR_INVALID, "too many one-hot columns for exact FP32 accumulation (%lld)", (long long)ws.pt);
-    const int8_t *a_rows;
     const int64_t u_lo = incr ? 0 : ws.u_lo;           // first sample row held by the target-side operand
-    if (contiguous) {
-        a_rows = Uop + (size_t)(r0_internal - u_lo) * K;
-    } else {
-        DevBuf<int8_t> &g = ds->a_gather;
-        g.reserve((size_t)R * K);
-        for (int64_t r = 0; r < R; ++r)
-            FS_CUDA(cudaMemcpyAsync(g.ptr + (size_t)r * K, Uop + (size_t)(h_row_ids[r] - u_lo) * K, K,
-                                    cudaMemcpyDeviceToDevice, st));
-        a_rows = g.ptr;
-    }
+    const int8_t *a_rows = Uop + (size_t)(r0 - u_lo) * K;
     // Symmetric mode: the target rows of all ranks together cover every sample, so half of the
     // off-diagonal super-blocks are computed and mirrored (see the file head).  One rank scoring all rows
     // is the trivial case; in a multi-GPU group the caller says so (`exchange`: this rank's rows are
     // exactly its shard and Dd its arena slab).  An incremental update across ranks stays
     // non-symmetric (it would need remote read-modify-writes): the caller never asks for both.
     const DistPeers peers = exchange ? ds->peers : single_rank_peers(Dd, ds->n);
-    const bool symmetric = exchange || (contiguous && r0_internal == 0 && R == ds->n);
-    launch_tc_dist(a_rows, Wop, K, K, K, sop, d_row_ids, R, ds->n, ldn, symmetric, incr, peers, st, launches, ops);
+    const bool symmetric = exchange || (r0 == 0 && R == ds->n);
+    launch_tc_dist(a_rows, Wop, K, K, K, sop, r0, R, ds->n, ldn, symmetric, incr, peers, st, launches, ops);
 }
 
 }  // namespace fs

@@ -8,7 +8,7 @@ per-feature term is exact in float32 and float64, every distance is exact in any
 of d and d^2 and SURF's float32 row sum are exact (while n * p * 32 < 2^24), so distances, thresholds and neighbour
 masks must equal the CPU oracle's bit for bit:
 
-* Selection: ``fs_debug_rows`` on gathered targets -- distances, thresholds and masks of MultiSURF(*) and SURF(*).
+* Selection: ``fs_debug_rows`` on scattered targets -- distances, thresholds and masks of MultiSURF(*) and SURF(*).
 * SURF and SURF*: coefficients +-1, so the general accumulation is exact on both instantiations (float32 tiles of at
   most 128 multiples of 1/8, the float32 image ``x - min`` at any row offset, the float64 kernel); weights bitwise.
   ``FS_ARITH_F32`` runs SURF on the kernels MultiSURF and ReliefF use, which makes it the exact probe of those.
@@ -299,7 +299,7 @@ def _check_rows(native, ds, d, algo, star, tg, arith):
 @pytest.mark.gpu
 @pytest.mark.parametrize("n,arith,p,mixed", _dist_params())
 def test_distances_thresholds_masks_are_exact(native, n, arith, p, mixed):
-    """fs_debug_rows on gathered targets (the duplicated pair included, several 64-row tiles where n allows):
+    """fs_debug_rows on scattered targets (the duplicated pair included, several 64-row tiles where n allows):
     distances, thresholds and masks of MultiSURF(*) and SURF(*) bitwise, SURF weights bitwise, MultiSURF weights
     within the float32-coefficient bound."""
     d = dist_data(n, p, mixed)

@@ -4,7 +4,8 @@ promises on genotype data, at the tile, K-block, class and launch edges where th
 * Accumulation: ``fs_score`` over contiguous internal row ranges (class-aligned tiles, skipped K blocks) with each
   kernel -- ``FS_B200_ACCUM_PAIR`` = 3 (merged-plane CTA pairs, the default for 0/1/2 columns), 1 (paired epilogue),
   0 (one thread per one-hot row, the default for every other value count) -- and ``fs_debug_rows`` on scattered
-  targets (mixed tiles), against the CPU oracle's weights at a tolerance derived from the number formats
+  targets (runs of consecutive internal rows on the same plan), against the CPU oracle's weights at a tolerance
+  derived from the number formats
   (``exact_tolerance``) instead of rtol 1e-5: a single miscounted (target, sample, feature) triple fails.
 * Distances: the resident slab of ``tc_dist_pair_kernel`` (symmetric mirrored tiles for the full range, plain tiles
   for a range off the 128-row grid, the incremental subtract update) bitwise against exact integer distances.

@@ -7,7 +7,7 @@ production-path gap):
   distance slab bit-exact against oracle distances;
 * the PRODUCTION entry point (fs_score over a contiguous internal row range: class-aligned tiles,
   skipped K blocks, paired epilogue) against the oracle's weights for exactly those rows on C3 and C4
-  -- fs_debug_rows takes the non-contiguous plan, so it does not cover those code paths.
+  -- fs_debug_rows runs the same plan on runs of consecutive internal rows of its targets.
 
 Each test body also runs at a reduced shape so that a failure localises quickly."""
 import numpy as np
